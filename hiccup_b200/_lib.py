@@ -154,6 +154,9 @@ SIGNATURES = {
     "hic_decode_sync": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.POINTER(ctypes.c_uint64), c_void_p]),
     "hic_decode_export_restarts": (c_int, [c_void_p, c_void_p, c_void_p, ctypes.c_uint64, c_void_p]),
     "hic_decode_run_restarts": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_uint64, c_void_p, c_void_p]),
+    "hic_decode_run_dc": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_uint64, c_void_p, c_void_p]),
+    "hic_dct_thumbnail_shape": (c_int, [c_int32, c_int32, ctypes.POINTER(c_int32), ctypes.POINTER(c_int32)]),
+    "hic_dct_thumbnail": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
 }
 
 _lock = threading.Lock()
@@ -204,6 +207,13 @@ def geometry(h, w):
     g = Geometry()
     check(load().hic_dct_geometry_of(int(h), int(w), ctypes.byref(g)))
     return g
+
+
+def thumbnail_shape(h, w):
+    """(th, tw) of the 1/8-scale thumbnail of a DCT-mode image of h x w (host only)."""
+    th, tw = c_int32(), c_int32()
+    check(load().hic_dct_thumbnail_shape(int(h), int(w), ctypes.byref(th), ctypes.byref(tw)))
+    return int(th.value), int(tw.value)
 
 
 def tie_capacity(n, h, w):

@@ -281,6 +281,60 @@ class DctBatchCodec(_BatchCodec):
     def _after_decode(self):
         self.inverse_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
 
+    # ---- 1/8-scale thumbnails from the DC streams alone (codec.jpeg_thumbnail for the whole batch) ---------------
+    @property
+    def thumbnail_shape(self):
+        th, tw = _lib.thumbnail_shape(self.h, self.w)
+        return (self.n, th, tw, 3)
+
+    def _thumb_buffers(self):
+        if getattr(self, "d_dc", None) is None:          # made on first use: a codec that never previews pays nothing
+            self.d_dc = _lib.DeviceBuffer(2 * self.blocks)
+            self.d_thumb = _lib.DeviceBuffer(int(np.prod(self.thumbnail_shape)))
+            self._h_thumb = None
+            self._buffers += [self.d_dc, self.d_thumb]
+        return self.d_dc, self.d_thumb
+
+    def thumbnails_device(self):
+        """DC-only D1 + D3 and the thumbnail kernel from the encoder's own device-resident output (decode_device's
+        hand-over); the thumbnails stay on the device (fetch_thumbnails)."""
+        d_dc, d_thumb = self._thumb_buffers()
+        st = self.stream
+        enc = self.encoder
+        d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
+        self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
+        self.decoder.run_dc(enc._out.ptr, enc.byte_off, enc.nbits, d_dc.ptr, st)
+        _lib.check(self.lib.hic_dct_thumbnail(d_dc.ptr, self.n, self.h, self.w, d_thumb.ptr, st))
+
+    def thumbnails(self, enc, out=None):
+        """Thumbnails of an EncodedStreams (encode() or read_files() / streams_from_files()), host to host: only the
+        DC streams' tables and bytes go up, n x th x tw x 3 comes down.  out: optional preallocated uint8 array of
+        thumbnail_shape."""
+        d_dc, d_thumb = self._thumb_buffers()
+        index, symbols, packed, data, byte_off, nbits = entropy.dc_streams_only(enc)
+        self.decoder.decode_dc(index, symbols, packed, data, byte_off, nbits, d_dc.ptr, self.stream)
+        _lib.check(self.lib.hic_dct_thumbnail(d_dc.ptr, self.n, self.h, self.w, d_thumb.ptr, self.stream))
+        return self.fetch_thumbnails(out)
+
+    def fetch_thumbnails(self, out=None):
+        """Download the thumbnails of the last thumbnails() / thumbnails_device()."""
+        _, d_thumb = self._thumb_buffers()
+        count = int(np.prod(self.thumbnail_shape))
+        if out is None:
+            if self._h_thumb is None:
+                self._h_thumb = _lib.PinnedBuffer(count)
+            out = self._h_thumb.array(np.uint8, count)
+        else:
+            assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
+            out = out.reshape(-1)
+        return d_thumb.download(np.uint8, count, self.stream, out=out).reshape(self.thumbnail_shape)
+
+    def close(self):
+        if getattr(self, "_h_thumb", None) is not None:
+            self._h_thumb.free()
+            self._h_thumb = None
+        super().close()
+
     def coefficients(self):
         """Download the quantised zigzag blocks of the last encode: (n, blocks_per_image, 64) int16."""
         c = self.d_coef.download(np.int16, self.blocks * 64, self.stream)

@@ -137,9 +137,10 @@ def _stream_order(hic):
     return tabs, bits, 6
 
 
-def _records_in_stream_order(hic, nbits):
+def _records_in_stream_order(hic, nbits, kinds=(0, 1, 2)):
     """The file's restart records re-ordered to stream order and concatenated, or None when the file has none
-    (or they do not fit its bit strings: the extension is advisory, the decoder then synchronises by itself)."""
+    (or they do not fit its bit strings: the extension is advisory, the decoder then synchronises by itself).
+    kinds: the symbol kinds whose records are wanted (the DC-only decode takes kind 0 alone)."""
     ext = getattr(hic, "restarts", None)
     if ext is None:
         return None
@@ -150,7 +151,7 @@ def _records_in_stream_order(hic, nbits):
     want = entropy.EntropyDecoder.subsequences(nbits)
     offs, cnts = [], []
     for s, i in enumerate(bits):
-        if i is None:
+        if i is None or s % 3 not in kinds:
             continue
         off, cnt = ext.records[i - first]
         if off.size != want[s] or cnt.size != want[s]:
@@ -247,6 +248,45 @@ def jpeg_decode(hic: hicimage.HicImage) -> model.CompressedImage:
     finally:
         coef.free()
     return out
+
+
+def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
+    """The 1/8-scale preview of a DCT-mode file: (th, tw, 3) uint8, one pixel per 8x8 tile of what jpeg_decode +
+    compression.jpeg_decompression return (th = ceil(out_h / 8)), from the three DC streams alone (hic_dct_thumbnail).
+    Only the DC tables and DC bit strings go to the device; the file's restart records of the DC streams are used
+    when it has them."""
+    if not (hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"):
+        raise NotImplementedError("thumbnails come from the DC streams of a DCT-mode (JPEG) file; a wavelet (HIC) file has "
+                                  "none -- its coarse band would need a prefix decode of the value and length streams")
+    settings.check_supported()
+    _lib.require_device()
+    p = hic.payloads
+    lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
+    h, w = int(lum_shape[0]), int(lum_shape[1])
+    g = _lib.geometry(h, w)
+    if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
+        raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
+    # stream order s = channel * 3 + kind; the DC table / bit string of channel c is payload c / 9 + c
+    rows, syms, lens, codes = _tables_to_arrays([p[c] for c in range(3)])
+    index = np.zeros((9, 2), np.uint32)
+    index[0::3, 1] = rows
+    index[0::3, 0] = np.concatenate(([0], np.cumsum(rows)[:-1]))
+    packed = (lens.astype(np.uint64) << np.uint64(58)) | (codes & entropy.CODE_MASK)
+    data, offs3, nbits3 = _gather_payload_bytes([p[9 + c] for c in range(3)])
+    offs, nbits = np.zeros(9, np.uint64), np.zeros(9, np.uint64)
+    offs[0::3], nbits[0::3] = offs3, nbits3
+    records = _records_in_stream_order(hic, nbits, kinds=(entropy.KIND_DC,))
+    th, tw = _lib.thumbnail_shape(h, w)
+    dec = entropy.cached_decoder(_lib.layout_dct(1, h, w))
+    d_dc = _lib.scratch(2 * g.blocks_per_image)
+    out = _lib.scratch(3 * th * tw)
+    try:
+        dec.decode_dc(index, syms, packed, data, offs, nbits, d_dc.ptr, restarts=records)
+        _lib.check(_lib.load().hic_dct_thumbnail(d_dc.ptr, 1, h, w, out.ptr, None))
+        return out.download(np.uint8, 3 * th * tw).reshape(th, tw, 3)
+    finally:
+        d_dc.free()
+        out.free()
 
 
 def wavelet_encode(compressed: model.CompressedImage, restarts: bool = False) -> hicimage.HicImage:

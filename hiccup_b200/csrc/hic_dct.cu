@@ -1077,6 +1077,47 @@ upsample_colour_vec_kernel(const uint8_t* __restrict__ yp, const uint8_t* __rest
             o[k] = (uint32_t)px[4 * k] | ((uint32_t)px[4 * k + 1] << 8) | ((uint32_t)px[4 * k + 2] << 16) | ((uint32_t)px[4 * k + 3] << 24);
     }
 }
+
+// A block whose AC terms are all zero decodes (K7: q T00 through the IDCT, /256, +128, astype(uint8)) to one
+// constant sample: trunc(q T00 / 256 + 128) mod 256 = ((q T00 + 32768) / 256, truncated toward zero) & 255.
+__device__ __forceinline__ int dc_block_sample(int q, int t00) { return ((q * t00 + 32768) / 256) & 255; }
+
+// Thumbnail: one pixel per 8x8 tile of the full decode's output (th = ceil(out_h / 8), tw = ceil(out_w / 8)),
+// from the DC values alone (one int16 per block, global block order).  The luminance block (ty, tx) gives Y; the
+// chroma planes of block samples (nby_c x nbx_c) go through K8's pyrUp taps on the fly, s[-1] = s[1] and s[n] =
+// s[n-1] per axis, and are cropped to th x tw with Y; then K8's ycrcb_to_rgb.  One thread per thumbnail pixel.
+__global__ void __launch_bounds__(256)
+thumbnail_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int n, int th, int tw, uint8_t* __restrict__ rgb) {
+    const int64_t per = (int64_t)th * tw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * n) return;
+    const int64_t img = gid / per;
+    const int64_t rem = gid - img * per;
+    const int ty = (int)(rem / tw), tx = (int)(rem % tw);
+    const int16_t* blocks = dc + img * g.blocks_per_image;
+    const int t_l = c_tab.qi[0][0], t_c = c_tab.qi[1][0];
+    const int y = dc_block_sample(__ldg(blocks + (int64_t)ty * g.nbx_l + tx), t_l);
+    const int cy = ty >> 1, cx = tx >> 1;
+    const bool odd_y = ty & 1, odd_x = tx & 1;
+    const int ym = cy > 0 ? cy - 1 : (g.nby_c > 1 ? 1 : 0), yn = cy + 1 < g.nby_c ? cy + 1 : g.nby_c - 1;
+    const int xm = cx > 0 ? cx - 1 : (g.nbx_c > 1 ? 1 : 0), xn = cx + 1 < g.nbx_c ? cx + 1 : g.nbx_c - 1;
+    int up[2];
+#pragma unroll
+    for (int ch = 0; ch < 2; ++ch) {
+        const int16_t* p = blocks + g.nb_l + ch * g.nb_c;
+        auto s = [&](int r, int c) { return dc_block_sample(__ldg(p + (int64_t)r * g.nbx_c + c), t_c); };
+        // horizontal pass on the rows the vertical tap needs, then the vertical tap
+        auto hor = [&](int r) { return odd_x ? 4 * (s(r, cx) + s(r, xn)) : s(r, xm) + 6 * s(r, cx) + s(r, xn); };
+        const int v = odd_y ? 4 * (hor(cy) + hor(yn)) : hor(ym) + 6 * hor(cy) + hor(yn);
+        up[ch] = (v + 32) >> 6;
+    }
+    int r, gg, b;
+    ycrcb_to_rgb(y, up[0], up[1], r, gg, b);
+    uint8_t* o = rgb + gid * 3;
+    o[0] = (uint8_t)r;
+    o[1] = (uint8_t)gg;
+    o[2] = (uint8_t)b;
+}
 }  // namespace k7
 
 // ------------------------------------------------------------------------------------------------
@@ -1330,6 +1371,34 @@ int hic_dct_inverse(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, uint
         HIC_LAUNCH("upsample_colour_kernel", st, k7::upsample_colour_vec_kernel<<<grid_for(quads / 4, 256), 256, 0, st>>>(d_y, d_cr, d_cb, g, n, d_rgb_out));
     else
         HIC_LAUNCH("upsample_colour_kernel", st, k7::upsample_colour_kernel<<<grid_for(quads, 256), 256, 0, st>>>(d_y, d_cr, d_cb, g, n, d_rgb_out));
+    return HIC_OK;
+}
+
+int hic_dct_thumbnail_shape(int32_t h, int32_t w, int32_t* th, int32_t* tw) {
+    using namespace hic;
+    HIC_REQUIRE(th && tw, "NULL argument");
+    hic_dct_geometry g;
+    const int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    *th = ceil_div(g.out_h, 8);
+    *tw = ceil_div(g.out_w, 8);
+    return HIC_OK;
+}
+
+int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint8_t* d_rgb_out, void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_dc && d_rgb_out, "NULL device pointer");
+    HIC_REQUIRE(n >= 1, "batch size must be positive");
+    hic_dct_geometry g;
+    int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    int32_t th = 0, tw = 0;
+    rc = hic_dct_thumbnail_shape(h, w, &th, &tw);
+    if (rc) return rc;
+    rc = ensure_tables();
+    if (rc) return rc;
+    cudaStream_t st = as_stream(stream);
+    HIC_LAUNCH("thumbnail_kernel", st, k7::thumbnail_kernel<<<grid_for((int64_t)n * th * tw, 256), 256, 0, st>>>(d_dc, g, n, th, tw, d_rgb_out));
     return HIC_OK;
 }
 

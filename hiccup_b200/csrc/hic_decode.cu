@@ -1103,6 +1103,13 @@ __global__ void validate_kernel(Geom g, const int16_t* __restrict__ values, cons
     if (trailing ? (total > g.L.len[c]) : (total != g.L.len[c])) atomicOr(err, 16u);
 }
 
+// the DC-only decode's check: every DC stream held exactly one symbol per block of its channel
+__global__ void validate_dc_kernel(Geom g, const uint32_t* __restrict__ nsym_arr, uint32_t* __restrict__ err) {
+    const int cs = blockIdx.x * blockDim.x + threadIdx.x;
+    if (cs >= g.L.n_images * 3) return;
+    if (nsym_arr[cs * 3 + HIC_KIND_DC] != (uint32_t)g.L.nb[cs % 3]) atomicOr(err, 8u);
+}
+
 // ------------------------------------------------------------------------------------------------
 // D3: DC prefix sum (utils.invert_differences) written to element 0 of every block
 // ------------------------------------------------------------------------------------------------
@@ -1363,7 +1370,9 @@ int hic_decode_set_tables(hic_decode_plan* p, const uint32_t* h_rows, const int3
 }  // extern "C"
 
 // mode 0: the whole decode; mode 1: D1's synchronisation only (what the restart records are exported from);
-// h_roff / h_rcnt: restart records of every subsequence in stream order, or NULL
+// mode 2: the DC streams alone -- D1 on the kind-0 streams and D3 into d_coef, which is then one int16 DC value
+// per block (the other streams' offsets and bit counts are ignored, their bytes never read);
+// h_roff / h_rcnt: restart records of every subsequence in stream order (of the decoded streams), or NULL
 static int decode_run_impl(hic_decode_plan* p, const uint8_t* d_bytes, const uint64_t* h_byte_off, const uint64_t* h_nbits,
                            int16_t* d_coef, void* stream, int mode, const uint8_t* h_roff, const uint8_t* h_rcnt,
                            uint64_t n_restart) {
@@ -1383,8 +1392,12 @@ static int decode_run_impl(hic_decode_plan* p, const uint8_t* d_bytes, const uin
     const dec::Geom& g = p->g;
     cudaStream_t st = as_stream(stream);
     const int nss = p->n_ss;
-    std::vector<uint64_t> nbits(h_nbits, h_nbits + nss), off(h_byte_off, h_byte_off + nss);
+    if (mode == 2) HIC_REQUIRE(g.L.skip_first, "a flat (wavelet) layout has no DC streams");
+    std::vector<uint64_t> nbits(nss), off(nss);
     for (int s = 0; s < nss; ++s) {
+        const bool used = mode != 2 || s % 3 == HIC_KIND_DC;
+        nbits[s] = used ? h_nbits[s] : 0;
+        off[s] = used ? h_byte_off[s] : 0;
         HIC_REQUIRE((off[s] & 3) == 0, "stream %d is not 4-byte aligned", s);
         // a framed payload is its pad-count byte + ceil(nbits / 8) bytes; the decoders read whole 32-bit words of it
         if (p->data_bytes && nbits[s])
@@ -1446,6 +1459,7 @@ static int decode_run_impl(hic_decode_plan* p, const uint8_t* d_bytes, const uin
         if (rc) return rc;
     }
     HIC_CUDA(cudaMemsetAsync(p->d_nsym, 0, sizeof(uint32_t) * nss, st));
+    int16_t* const dc = mode == 2 ? d_coef : p->d_dc;      // the DC-only mode decodes straight into the caller's buffer
     if (n_tiles) {
         {
             int rc = hic::small_h2d(p->xfer, p->d_tiles, tiles.data(), sizeof(SyncTile) * n_tiles, st);
@@ -1502,7 +1516,7 @@ static int decode_run_impl(hic_decode_plan* p, const uint8_t* d_bytes, const uin
                 HIC_CUDA(cudaFuncSetAttribute(huffman_write_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WRITE_SMEM));
                 if (dev < 64) attr_set[dev] = true;
             }
-            HIC_LAUNCH("huffman_write_kernel", st, huffman_write_kernel<<<(unsigned)n_tiles, SUB_PER_CTA, WRITE_SMEM, st>>>(a, g, p->d_tile_symoff, p->d_dc, p->d_values, p->d_lengths, p->d_err));
+            HIC_LAUNCH("huffman_write_kernel", st, huffman_write_kernel<<<(unsigned)n_tiles, SUB_PER_CTA, WRITE_SMEM, st>>>(a, g, p->d_tile_symoff, dc, p->d_values, p->d_lengths, p->d_err));
         }
     }
     if (mode == 1) {
@@ -1511,19 +1525,23 @@ static int decode_run_impl(hic_decode_plan* p, const uint8_t* d_bytes, const uin
         return HIC_OK;
     }
     if (g.L.skip_first) {           // D3 first: the expansion below writes the DC values with the blocks they belong to
-        HIC_LAUNCH("dc_tile_sum_kernel", st, dc_tile_sum_kernel<<<(unsigned)p->total_dtiles, XTHREADS, 0, st>>>(g, p->d_dc, p->d_tile_sum));
+        HIC_LAUNCH("dc_tile_sum_kernel", st, dc_tile_sum_kernel<<<(unsigned)p->total_dtiles, XTHREADS, 0, st>>>(g, dc, p->d_tile_sum));
         HIC_LAUNCH("stream_scan64_kernel", st, stream_scan64_kernel<<<p->n_cs, SCAN_THREADS, 0, st>>>(p->n_cs, g.dtiles[0], g.dtiles[1], g.dtiles[2],
                                                                    g.dtiles_per_image, p->d_tile_sum, p->d_tile_off,
                                                                    p->d_stream_total));
-        HIC_LAUNCH("dc_prefix_kernel", st, dc_prefix_kernel<<<(unsigned)p->total_dtiles, XTHREADS, 0, st>>>(g, p->d_dc, p->d_tile_off));
+        HIC_LAUNCH("dc_prefix_kernel", st, dc_prefix_kernel<<<(unsigned)p->total_dtiles, XTHREADS, 0, st>>>(g, dc, p->d_tile_off));
     }
-    HIC_LAUNCH("expand_tile_sum_kernel", st, expand_tile_sum_kernel<<<(unsigned)((p->total_xtiles + XTHREADS / 32 - 1) / (XTHREADS / 32)), XTHREADS, 0, st>>>(g, p->d_lengths, p->d_nsym, p->d_tile_sum, p->total_xtiles));
-    HIC_LAUNCH("stream_scan64_kernel", st, stream_scan64_kernel<<<p->n_cs, SCAN_THREADS, 0, st>>>(p->n_cs, g.xtiles[0], g.xtiles[1], g.xtiles[2],
-                                                               g.xtiles_per_image, p->d_tile_sum, p->d_tile_off,
-                                                               p->d_stream_total));
-    HIC_LAUNCH("expand_scatter_kernel", st, expand_scatter_kernel<<<(unsigned)p->total_xtiles, XTHREADS, 0, st>>>(g, p->d_values, p->d_lengths, p->d_dc, p->d_nsym,
-                                                                         p->d_tile_off, p->d_stream_total, d_coef, p->d_err));
-    HIC_LAUNCH("validate_kernel", st, validate_kernel<<<(p->n_cs + 127) / 128, 128, 0, st>>>(g, p->d_values, p->d_lengths, p->d_nsym, p->d_stream_total, p->d_err));
+    if (mode == 2) {
+        HIC_LAUNCH("validate_dc_kernel", st, validate_dc_kernel<<<(p->n_cs + 127) / 128, 128, 0, st>>>(g, p->d_nsym, p->d_err));
+    } else {
+        HIC_LAUNCH("expand_tile_sum_kernel", st, expand_tile_sum_kernel<<<(unsigned)((p->total_xtiles + XTHREADS / 32 - 1) / (XTHREADS / 32)), XTHREADS, 0, st>>>(g, p->d_lengths, p->d_nsym, p->d_tile_sum, p->total_xtiles));
+        HIC_LAUNCH("stream_scan64_kernel", st, stream_scan64_kernel<<<p->n_cs, SCAN_THREADS, 0, st>>>(p->n_cs, g.xtiles[0], g.xtiles[1], g.xtiles[2],
+                                                                   g.xtiles_per_image, p->d_tile_sum, p->d_tile_off,
+                                                                   p->d_stream_total));
+        HIC_LAUNCH("expand_scatter_kernel", st, expand_scatter_kernel<<<(unsigned)p->total_xtiles, XTHREADS, 0, st>>>(g, p->d_values, p->d_lengths, p->d_dc, p->d_nsym,
+                                                                             p->d_tile_off, p->d_stream_total, d_coef, p->d_err));
+        HIC_LAUNCH("validate_kernel", st, validate_kernel<<<(p->n_cs + 127) / 128, 128, 0, st>>>(g, p->d_values, p->d_lengths, p->d_nsym, p->d_stream_total, p->d_err));
+    }
     const void* h_flags = nullptr;
     {
         int rc = hic::small_d2h(p->xfer, p->d_err, 4 * sizeof(uint32_t), st, &h_flags);
@@ -1554,6 +1572,12 @@ int hic_decode_run_restarts(hic_decode_plan* p, const uint8_t* d_bytes, const ui
                             const uint8_t* h_off, const uint8_t* h_cnt, uint64_t n_sub, int16_t* d_coef, void* stream) {
     HIC_REQUIRE(h_off && h_cnt, "NULL restart records");
     return decode_run_impl(p, d_bytes, h_byte_off, h_nbits, d_coef, stream, 0, h_off, h_cnt, n_sub);
+}
+
+int hic_decode_run_dc(hic_decode_plan* p, const uint8_t* d_bytes, const uint64_t* h_byte_off, const uint64_t* h_nbits,
+                      const uint8_t* h_off, const uint8_t* h_cnt, uint64_t n_sub, int16_t* d_dc, void* stream) {
+    HIC_REQUIRE((h_off == nullptr) == (h_cnt == nullptr), "restart records need both `off` and `cnt`");
+    return decode_run_impl(p, d_bytes, h_byte_off, h_nbits, d_dc, stream, 2, h_off, h_cnt, n_sub);
 }
 
 int hic_decode_sync(hic_decode_plan* p, const uint8_t* d_bytes, const uint64_t* h_byte_off, const uint64_t* h_nbits,

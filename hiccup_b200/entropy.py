@@ -335,6 +335,75 @@ class EntropyDecoder:
         _lib.check(self.lib.hic_decode_run(self.plan, d_data, byte_off.ctypes.data, nbits.ctypes.data, d_coef, stream))
         return None
 
+    def run_dc(self, d_data, byte_off, nbits, d_dc, stream=None, restarts=None):
+        """DC-only decode (hic_decode_run_dc) with the tables already installed: d_dc receives one int16 DC value per
+        block.  Only the DC streams' entries of byte_off / nbits and their bytes are read.  restarts = (off, cnt): the
+        DC streams' records in stream order; records that do not fit mean decoding the long way (and failing there
+        if the streams are bad), never a silent mis-decode."""
+        byte_off = np.ascontiguousarray(byte_off, np.uint64)
+        nbits = np.ascontiguousarray(nbits, np.uint64)
+        if restarts is not None:
+            off = np.ascontiguousarray(restarts[0], np.uint8)
+            cnt = np.ascontiguousarray(restarts[1], np.uint8)
+            assert off.size == cnt.size
+            try:
+                _lib.check(self.lib.hic_decode_run_dc(self.plan, d_data, byte_off.ctypes.data, nbits.ctypes.data,
+                                                      off.ctypes.data, cnt.ctypes.data, int(off.size), d_dc, stream))
+                return True
+            except _lib.HicError:
+                pass
+        _lib.check(self.lib.hic_decode_run_dc(self.plan, d_data, byte_off.ctypes.data, nbits.ctypes.data, None, None, 0, d_dc, stream))
+        return False
+
+    def decode_dc(self, index, symbols, packed, data, byte_off, nbits, d_dc, stream=None, restarts=None):
+        """Packed host tables (the AC streams may have no rows) + framed payloads in a host array (the DC streams'
+        bytes at least) -> run_dc.  The data bound is checked against `data`.  Returns whether the records were used."""
+        index = np.ascontiguousarray(index, np.uint32)
+        symbols = np.ascontiguousarray(symbols, np.int32)
+        packed = np.ascontiguousarray(packed, np.uint64)
+        _lib.check(self.lib.hic_decode_set_tables_packed(self.plan, index.ctypes.data, symbols.ctypes.data,
+                                                         packed.ctypes.data, int(symbols.size), stream))
+        data = np.ascontiguousarray(data, np.uint8)
+        need = data.nbytes + 16
+        if self._in is None or self._in.nbytes < need:
+            if self._in is not None:
+                self._in.free()
+            self._in = _lib.DeviceBuffer(need + need // 4)
+        self._in.upload(data, stream)
+        _lib.check(self.lib.hic_decode_set_data_bytes(self.plan, int(data.nbytes)))
+        try:
+            return self.run_dc(self._in.ptr, byte_off, nbits, d_dc, stream, restarts)
+        finally:
+            _lib.check(self.lib.hic_decode_set_data_bytes(self.plan, 0))
+
+
+def dc_streams_only(enc):
+    """The DC streams of an EncodedStreams alone, for decode_dc: (index, symbols, packed, data, byte_off, nbits) with
+    the AC streams at zero rows and zero bits, and the DC streams' tables and framed bytes packed together."""
+    n_s = enc.index.shape[0]
+    dc = np.arange(0, n_s, 3)
+    start = enc.index[dc, 0].astype(np.int64)
+    rows = enc.index[dc, 1].astype(np.int64)
+    index = np.zeros((n_s, 2), np.uint32)
+    index[dc, 1] = rows
+    index[dc, 0] = np.concatenate(([0], np.cumsum(rows)[:-1])).astype(np.uint32)
+    b_off = np.asarray(enc.byte_off, np.int64)[dc]
+    b_len = np.asarray(enc.byte_len, np.int64)[dc]
+    b_pad = (b_len + 3) & ~3                                             # whole words: every stream starts 4-byte aligned
+    byte_off = np.zeros(n_s, np.uint64)
+    byte_off[dc] = np.concatenate(([0], np.cumsum(b_pad)[:-1])).astype(np.uint64)
+    data = np.zeros(int(b_pad.sum()) + 16, np.uint8)
+    src = np.asarray(enc.data, np.uint8)
+    # slices, one per stream: a few thousand of them cost less than an element-wise gather of megabytes
+    for a, o, n in zip(byte_off[dc].tolist(), b_off.tolist(), b_len.tolist()):
+        data[a:a + n] = src[o:o + n]
+    symbols, packed = np.asarray(enc.symbols), np.asarray(enc.packed)
+    pick = [slice(a, a + n) for a, n in zip(start.tolist(), rows.tolist())]
+    cat = lambda arr: np.concatenate([arr[s] for s in pick]) if pick else arr[:0]
+    nbits = np.zeros(n_s, np.uint64)
+    nbits[dc] = np.asarray(enc.nbits, np.uint64)[dc]
+    return index, cat(symbols), cat(packed), data, byte_off, nbits
+
 
 # ------------------------------------------------------------------------------------------------
 # plan cache of the single-image entry points (codec.jpeg_encode / jpeg_decode / wavelet_*): an entropy plan

@@ -3,14 +3,15 @@ rank 1) plus a directory mode that feeds the batched GPU path.
 
     compress(path, output, style)      run.py:18-29   image file -> <output>/<name>.<STYLE>-hic
     decompress(path)                   run.py:32-43   .hic file -> pixels (the reference shows them in a window;
-                                                       here they are returned, and written with `save=`)
+                                                       here they are returned, and written with `save=`);
+                                                       thumbnail=True: the 1/8-scale preview of a DCT-mode file instead
     compress_many(paths, output, ...)  additive: same-shaped images are encoded as one GPU batch and their files
                                        written by the library's host threads (batch.write_files)
     decompress_many(paths, ...)        additive: same-shaped `.hic` files are read and decoded as one GPU batch
 
 Like the reference, `cv2.imread` delivers BGR and the codec treats channel 0 as R (run.py:19), so files
 are interchangeable with the reference's in both directions.  Command line: python -m hiccup_b200.run
--c IMG... | -d HIC... [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
+-c IMG... | -d HIC... [-t] [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
 """
 import argparse
 import os
@@ -45,9 +46,20 @@ def compress(path, output, c=model.Compression.JPEG, restarts=False):
     return out
 
 
-def decompress(path, save=None):
+def _no_wavelet_thumbnails(path):
+    raise NotImplementedError("%s is a wavelet (HIC) file: thumbnails come from the DC streams of DCT-mode (JPEG) files, "
+                              "and wavelet files have none" % (path,))
+
+
+def decompress(path, save=None, thumbnail=False):
+    """thumbnail=True: the 1/8-scale preview (one pixel per 8x8 tile of the decoded image) of a DCT-mode file from its DC streams alone
+    (codec.jpeg_thumbnail); a wavelet file raises NotImplementedError."""
     hi = hicimage.HicImage.from_file(path)
-    if hi.hic_type == model.Compression.JPEG:
+    if thumbnail:
+        if hi.hic_type != model.Compression.JPEG:
+            _no_wavelet_thumbnails(path)
+        rgb = codec.jpeg_thumbnail(hi)
+    elif hi.hic_type == model.Compression.JPEG:
         rgb = compression.jpeg_decompression(codec.jpeg_decode(hi))
     elif hi.hic_type == model.Compression.HIC:
         rgb = compression.wavelet_decompression(codec.wavelet_decode(hi))
@@ -101,22 +113,28 @@ def _peek(raw):
     return mode, shape
 
 
-def decompress_many(paths, save_dir=None, max_batch=256):
+def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False):
     """Decode many `.hic` files; files of one mode and image shape go through the batched codec together.  Returns the
-    pixel arrays in the order of `paths` (equal to what decompress() returns for each); save_dir: also write them as PNG."""
+    pixel arrays in the order of `paths` (equal to what decompress() returns for each); save_dir: also write them as PNG
+    (<name>.png, or <name>.thumb.png for thumbnails).  thumbnail=True: the previews of DCT-mode files
+    (DctBatchCodec.thumbnails); a wavelet file among them raises NotImplementedError before anything is decoded."""
     from hiccup_b200.batch import DctBatchCodec, WaveletBatchCodec
     groups, out = {}, [None] * len(paths)
     for i, p in enumerate(paths):
         with open(p, "rb") as f:
             raw = f.read()
-        groups.setdefault(_peek(raw), []).append((i, raw))
+        key = _peek(raw)
+        if thumbnail and key[0] != model.Compression.JPEG:
+            _no_wavelet_thumbnails(p)
+        groups.setdefault(key, []).append((i, raw))
     for (mode, (h, w)), items in groups.items():
         cls = DctBatchCodec if mode == model.Compression.JPEG else WaveletBatchCodec
         for a in range(0, len(items), max_batch):
             part = items[a:a + max_batch]
             bc = cls(len(part), h, w)
             try:
-                pixels = bc.decode(bc.streams_from_files([raw for _, raw in part]))
+                enc = bc.streams_from_files([raw for _, raw in part])
+                pixels = bc.thumbnails(enc) if thumbnail else bc.decode(enc)
                 for (i, _), rgb in zip(part, pixels):
                     out[i] = rgb.copy()
             finally:
@@ -124,8 +142,12 @@ def decompress_many(paths, save_dir=None, max_batch=256):
     if save_dir is not None:
         import cv2
         for p, rgb in zip(paths, out):
-            cv2.imwrite(os.path.join(save_dir, os.path.split(p)[-1] + ".png"), rgb)
+            cv2.imwrite(os.path.join(save_dir, _png_name(p, thumbnail)), rgb)
     return out
+
+
+def _png_name(path, thumbnail):
+    return os.path.split(path)[-1] + (".thumb.png" if thumbnail else ".png")
 
 
 def main(argv=None):
@@ -137,7 +159,11 @@ def main(argv=None):
     ap.add_argument("--output", "-o", metavar="OUT", default=".")
     ap.add_argument("--restarts", "-r", action="store_true",
                     help="append restart records to the .hic files (ignored by the reference's reader; faster decode here)")
+    ap.add_argument("--thumbnail", "-t", action="store_true",
+                    help="with -d: write the 1/8-scale preview of each DCT-mode file (<name>.thumb.png) from its DC streams alone")
     args = ap.parse_args(argv)
+    if args.thumbnail and not args.decompress:
+        ap.error("-t/--thumbnail goes with -d/--decompress")
     style = model.Compression(args.compression)
     if args.compress:
         for out in (compress_many(args.compress, args.output, style, restarts=args.restarts) if len(args.compress) > 1
@@ -145,11 +171,12 @@ def main(argv=None):
             print(out)
     elif args.decompress:
         if len(args.decompress) > 1:
-            decompress_many(args.decompress, save_dir=args.output)
+            decompress_many(args.decompress, save_dir=args.output, thumbnail=args.thumbnail)
         else:
-            decompress(args.decompress[0], save=os.path.join(args.output, os.path.split(args.decompress[0])[-1] + ".png"))
+            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], args.thumbnail)),
+                       thumbnail=args.thumbnail)
         for p in args.decompress:
-            print(os.path.join(args.output, os.path.split(p)[-1] + ".png"))
+            print(os.path.join(args.output, _png_name(p, args.thumbnail)))
     else:
         raise RuntimeError("Illegal state")
 

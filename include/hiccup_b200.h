@@ -139,6 +139,18 @@ int hic_dct_inverse(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, uint
                     uint8_t* d_cr, uint8_t* d_cb, uint8_t* d_rgb_out, hic_tie_record* d_ties,
                     uint32_t tie_capacity, uint32_t* d_stats, void* stream);
 
+/* Thumbnail -- a 1/8-scale preview from the DC terms alone: one pixel per 8x8 tile of the image
+ * compression.jpeg_decompression (compression.py:42-56) returns, th = ceil(out_h / 8) rows of tw =
+ * ceil(out_w / 8).  Each block counts as its DC-only decode through transform.inv_dct_channel
+ * (transform.py:169-179), the constant ((q T00 + 32768) / 256 truncated toward zero) & 255 (T00 = 16
+ * luminance, 17 chroma); the chroma planes of those values go through cv2.pyrUp (transform.py:151-157),
+ * all three are cropped to th x tw and converted by cv2.cvtColor YCrCb->RGB (compression.py:56), the
+ * integer arithmetic of K8.  d_dc: one int16 DC value per block in global block order (image *
+ * blocks_per_image + block), as hic_decode_run_dc leaves them; d_rgb_out: n * th * tw * 3.
+ * hic_dct_thumbnail_shape is host only (no device needed). */
+int hic_dct_thumbnail_shape(int32_t h, int32_t w, int32_t* th, int32_t* tw);
+int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint8_t* d_rgb_out, void* stream);
+
 /* ---- wavelet ("HIC") mode --------------------------------------------------------------------- */
 /* Sub-band geometry of pywt.wavedec2(channel, "db1", level=3) (transform.py:196-209): level sizes
  * ceil(n / 2) per level; ten sub-bands per channel in the order [cA3, cH3, cV3, cD3, cH2, cV2, cD2,
@@ -373,6 +385,17 @@ int hic_decode_export_restarts(hic_decode_plan* plan, uint8_t* h_off, uint8_t* h
 int hic_decode_run_restarts(hic_decode_plan* plan, const uint8_t* d_bytes, const uint64_t* h_byte_off,
                             const uint64_t* h_nbits, const uint8_t* h_off, const uint8_t* h_cnt, uint64_t n_sub,
                             int16_t* d_coef, void* stream);
+
+/* DC-only decode (DCT layouts; a flat layout gives HIC_ERR_INVALID) -- the DC half of codec.jpeg_decode
+ * (codec.py:337-426): HuffmanTree.decode_data (huffman.py:149-174) of the three DC bit strings of every image
+ * and utils.invert_differences (utils.py:66-74).  Only the kind-0 streams are read: the offsets, bit counts
+ * and bytes of kinds 1 and 2 are ignored (their tables may have no rows), and hic_decode_set_data_bytes
+ * bounds apply to the DC streams.  d_dc receives one int16 DC value per block, index image *
+ * blocks_per_image + block.  h_off / h_cnt / n_sub: the restart records of the DC streams alone, in stream
+ * order, or NULL / NULL / 0 to synchronise.  Synchronises `stream`; HIC_ERR_CORRUPT if a DC stream does
+ * not decode to exactly one symbol per block of its channel (or the records do not belong to it). */
+int hic_decode_run_dc(hic_decode_plan* plan, const uint8_t* d_bytes, const uint64_t* h_byte_off, const uint64_t* h_nbits,
+                      const uint8_t* h_off, const uint8_t* h_cnt, uint64_t n_sub, int16_t* d_dc, void* stream);
 
 /* ---- host-side helpers of the `.hic` container (no device involved) -------------------------------------
  * The rows of one Huffman table to / from the byte strings the reference pickles them as, one pickle per row

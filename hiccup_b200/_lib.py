@@ -157,6 +157,10 @@ SIGNATURES = {
     "hic_decode_run_dc": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_uint64, c_void_p, c_void_p]),
     "hic_dct_thumbnail_shape": (c_int, [c_int32, c_int32, ctypes.POINTER(c_int32), ctypes.POINTER(c_int32)]),
     "hic_dct_thumbnail": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    "hic_dct_region_blocks": (c_int, [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_int32)]),
+    "hic_dct_region_sizes": (c_int, [c_int32, c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_size_t), ctypes.POINTER(c_uint32)]),
+    "hic_dct_region": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_size_t, c_void_p,
+                               c_uint32, c_void_p, c_void_p, c_void_p]),
 }
 
 _lock = threading.Lock()
@@ -214,6 +218,40 @@ def thumbnail_shape(h, w):
     th, tw = c_int32(), c_int32()
     check(load().hic_dct_thumbnail_shape(int(h), int(w), ctypes.byref(th), ctypes.byref(tw)))
     return int(th.value), int(tw.value)
+
+
+def region_blocks(h, w, top, left, rh, rw):
+    """The block rectangles a window of rh x rw at (top, left) of the decoded image selects (host only):
+    ((by, bx, nby, nbx) of the luminance plane, the same of each chroma plane).  HicError for an invalid window."""
+    rect = (c_int32 * 8)()
+    check(load().hic_dct_region_blocks(int(h), int(w), int(top), int(left), int(rh), int(rw), rect))
+    return tuple(rect[0:4]), tuple(rect[4:8])
+
+
+def region_sizes(n, h, w, rh, rw):
+    """(work bytes, tie capacity) hic_dct_region needs for n windows of rh x rw (host only)."""
+    work, cap = c_size_t(), c_uint32()
+    check(load().hic_dct_region_sizes(int(n), int(h), int(w), int(rh), int(rw), ctypes.byref(work), ctypes.byref(cap)))
+    return int(work.value), int(cap.value)
+
+
+def region_origins(h, w, origins, size):
+    """Check windows of size = (rh, rw) at origins ((n, 2) (top, left)) against the h x w image's decoded output
+    (out_h x out_w) on the host: the origins as a contiguous (n, 2) int32 array, or ValueError."""
+    g = geometry(h, w)
+    rh, rw = (int(v) for v in size)
+    o = np.asarray(origins)
+    if o.ndim != 2 or o.shape[1] != 2 or o.shape[0] < 1 or not np.issubdtype(o.dtype, np.integer):
+        raise ValueError("origins must be a non-empty (n, 2) integer array of (top, left), got shape %r" % (o.shape,))
+    o = o.astype(np.int64)
+    if rh < 1 or rw < 1:
+        raise ValueError("empty region %dx%d" % (rh, rw))
+    bad = (o[:, 0] < 0) | (o[:, 1] < 0) | (o[:, 0] + rh > g.out_h) | (o[:, 1] + rw > g.out_w)
+    if bad.any():
+        i = int(np.argmax(bad))
+        raise ValueError("region %dx%d at (%d, %d) is not inside the %dx%d decoded image"
+                         % (rh, rw, o[i, 0], o[i, 1], g.out_h, g.out_w))
+    return np.ascontiguousarray(o, np.int32)
 
 
 def tie_capacity(n, h, w):

@@ -329,10 +329,75 @@ class DctBatchCodec(_BatchCodec):
             out = out.reshape(-1)
         return d_thumb.download(np.uint8, count, self.stream, out=out).reshape(self.thumbnail_shape)
 
+    # ---- regions: one height x width window per image at full resolution (codec.jpeg_region for the whole batch) ----
+    def _region_buffers(self, origins, size):
+        """Check the windows (ValueError before any device work) and make the work and output buffers for their size
+        on first use; returns the origins as (n, 2) int32."""
+        origins = _lib.region_origins(self.h, self.w, origins, size)
+        if origins.shape[0] != self.n:
+            raise ValueError("%d origins for a batch of %d images" % (origins.shape[0], self.n))
+        size = (int(size[0]), int(size[1]))
+        if getattr(self, "_region_size", None) != size:
+            for b in (getattr(self, "d_region_work", None), getattr(self, "d_region", None), getattr(self, "_h_region", None)):
+                if b is not None:
+                    b.free()
+                    if b in self._buffers:
+                        self._buffers.remove(b)
+            self.region_work_bytes, self.region_tie_capacity = _lib.region_sizes(self.n, self.h, self.w, *size)
+            self.d_region_work = _lib.DeviceBuffer(self.region_work_bytes)
+            self.d_region = _lib.DeviceBuffer(self.n * size[0] * size[1] * 3)
+            self._h_region = None
+            self._buffers += [self.d_region_work, self.d_region]
+            self._region_size = size
+        return origins
+
+    def _region(self, origins):
+        rh, rw = self._region_size
+        _lib.check(self.lib.hic_dct_region(self.d_coef_dec.ptr, self.n, self.h, self.w, origins.ctypes.data, rh, rw,
+                                           self.d_region_work.ptr, self.region_work_bytes, self.d_ties.ptr,
+                                           self.region_tie_capacity, self.d_stats.ptr, self.d_region.ptr, self.stream))
+
+    def decode_regions_device(self, origins, size):
+        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the windows of
+        size = (height, width) at origins ((n, 2) of (top, left)); they stay on the device (fetch_regions)."""
+        origins = self._region_buffers(origins, size)
+        st = self.stream
+        enc = self.encoder
+        d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
+        self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
+        self.decoder.run(enc._out.ptr, enc.byte_off, enc.nbits, self.d_coef_dec.ptr, st)
+        self._region(origins)
+
+    def decode_regions(self, enc, origins, size, out=None):
+        """Windows of an EncodedStreams, host to host: image i's window is decode(enc)[i, top:top+height,
+        left:left+width] with (top, left) = origins[i] and (height, width) = size, bit for bit.  out: optional
+        preallocated uint8 array of (n, height, width, 3)."""
+        origins = self._region_buffers(origins, size)
+        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
+        self._region(origins)
+        return self.fetch_regions(out)
+
+    def fetch_regions(self, out=None):
+        """Download the windows of the last decode_regions() / decode_regions_device() (and their tie statistics
+        into region_stats)."""
+        rh, rw = self._region_size
+        count = self.n * rh * rw * 3
+        if out is None:
+            if self._h_region is None:
+                self._h_region = _lib.PinnedBuffer(count)
+            out = self._h_region.array(np.uint8, count)
+        else:
+            assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
+            out = out.reshape(-1)
+        out = self.d_region.download(np.uint8, count, self.stream, out=out)
+        self.region_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
+        return out.reshape(self.n, rh, rw, 3)
+
     def close(self):
-        if getattr(self, "_h_thumb", None) is not None:
-            self._h_thumb.free()
-            self._h_thumb = None
+        for name in ("_h_thumb", "_h_region"):
+            if getattr(self, name, None) is not None:
+                getattr(self, name).free()
+                setattr(self, name, None)
         super().close()
 
     def coefficients(self):

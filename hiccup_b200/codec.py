@@ -289,6 +289,42 @@ def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
         out.free()
 
 
+def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int) -> np.ndarray:
+    """One window of a DCT-mode file at full resolution: (height, width, 3) uint8, equal to
+    compression.jpeg_decompression(jpeg_decode(hic))[top:top+height, left:left+width] bit for bit.  The entropy
+    decode is jpeg_decode's (restart records used when the file has them); then only the blocks the window reads are
+    inverse-transformed and only its pixels upsampled and converted (hic_dct_region).  ValueError for a window
+    outside the decoded image, NotImplementedError for a wavelet file, both before any device work."""
+    if not (hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"):
+        raise NotImplementedError("region decode works on DCT-mode (JPEG) files; this is a wavelet (HIC) file")
+    p = hic.payloads
+    lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
+    h, w = int(lum_shape[0]), int(lum_shape[1])
+    g = _lib.geometry(h, w)
+    if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
+        raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
+    origin = _lib.region_origins(h, w, [(top, left)], (height, width))
+    settings.check_supported()
+    _lib.require_device()
+    work_bytes, tie_cap = _lib.region_sizes(1, h, w, height, width)
+    order = [kind * 3 + c for c in range(3) for kind in range(3)]
+    rows, syms, lens, codes = _tables_to_arrays([p[i] for i in order])
+    data, offs, nbits = _gather_payload_bytes([p[9 + i] for i in order])
+    dec = entropy.cached_decoder(_lib.layout_dct(1, h, w))
+    lib = _lib.load()
+    bufs = [_lib.scratch(g.blocks_per_image * 128), _lib.scratch(work_bytes), _lib.scratch(tie_cap * _lib.TIE_RECORD_BYTES),
+            _lib.scratch(4 * _lib.TIE_STATS), _lib.scratch(3 * int(height) * int(width))]
+    coef, work, ties, stats, out = bufs
+    try:
+        _entropy_decode(dec, hic, rows, syms, lens, codes, data, offs, nbits, coef.ptr)
+        _lib.check(lib.hic_dct_region(coef.ptr, 1, h, w, origin.ctypes.data, int(height), int(width), work.ptr, work_bytes,
+                                      ties.ptr, tie_cap, stats.ptr, out.ptr, None))
+        return out.download(np.uint8, 3 * int(height) * int(width)).reshape(int(height), int(width), 3)
+    finally:
+        for b in bufs:
+            b.free()
+
+
 def wavelet_encode(compressed: model.CompressedImage, restarts: bool = False) -> hicimage.HicImage:
     from hiccup_b200 import wavelet
     hic = wavelet.wavelet_encode(compressed)

@@ -93,6 +93,54 @@ static int geometry_of(int h, int w, hic_dct_geometry* g) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// region decode: the blocks a window of the output reads
+// ------------------------------------------------------------------------------------------------
+// Output pixel (oy, ox) reads luminance sample (oy, ox) and K8's chroma taps: rows cy - 1 .. cy + 1 of cy = oy / 2
+// (row 1 for cy = 0, clamped to hc - 1 at the bottom), the same for columns.  So a window of rh output rows at top
+// reads luminance rows [top, top + rh - 1] and chroma rows [max(0, top/2 - 1), min(hc - 1, (top + rh - 1)/2 + 1)]
+// -- at most rh / 2 + 3 of them.  Every window of one size gets a block rectangle of one size per plane kind: the
+// most blocks those rows (columns) can touch, at most the plane's block count.  It starts at the block of the first
+// row the window reads, moved back where it would run past the plane's last block.
+struct RegionSpan {
+    int ny_l, nx_l;   // luminance rectangle, blocks
+    int ny_c, nx_c;   // chroma rectangle (Cr and Cb alike)
+};
+
+__host__ __device__ inline int region_span_l(int r, int nb) { return min(nb, (r + 6) / 8 + 1); }   // r samples
+__host__ __device__ inline int region_span_c(int r, int nb) { return min(nb, (r / 2 + 3 + 6) / 8 + 1); }
+__host__ __device__ inline RegionSpan region_span(const hic_dct_geometry& g, int rh, int rw) {
+    return {region_span_l(rh, g.nby_l), region_span_l(rw, g.nbx_l), region_span_c(rh, g.nby_c), region_span_c(rw, g.nbx_c)};
+}
+// first block row (column) of the luminance / chroma rectangle of a window whose first output row (column) is t
+__host__ __device__ inline int region_first_l(int t, int span, int nb) { return min(t >> 3, nb - span); }
+__host__ __device__ inline int region_first_c(int t, int span, int nb) { return min(max(0, (t >> 1) - 1) >> 3, nb - span); }
+
+static int region_check(const hic_dct_geometry& g, int64_t top, int64_t left, int64_t rh, int64_t rw) {
+    HIC_REQUIRE(rh >= 1 && rw >= 1, "empty region %lldx%lld", (long long)rh, (long long)rw);
+    HIC_REQUIRE(top >= 0 && left >= 0 && top + rh <= g.out_h && left + rw <= g.out_w,
+                "region %lldx%lld at (%lld, %lld) is not inside the %dx%d decoded image", (long long)rh, (long long)rw,
+                (long long)top, (long long)left, g.out_h, g.out_w);
+    return HIC_OK;
+}
+
+// window-local planes of one image (bytes) and the work buffer: n origins, then the n Y planes, Cr planes, Cb planes
+struct RegionLayout {
+    RegionSpan s;
+    size_t head, ly, lc, total;
+    uint64_t blocks;      // selected blocks of the batch
+};
+static RegionLayout region_layout(int n, const hic_dct_geometry& g, int rh, int rw) {
+    RegionLayout L;
+    L.s = region_span(g, rh, rw);
+    L.head = ((size_t)n * 2 * sizeof(int32_t) + 255) / 256 * 256;
+    L.ly = (size_t)64 * L.s.ny_l * L.s.nx_l;
+    L.lc = (size_t)64 * L.s.ny_c * L.s.nx_c;
+    L.total = L.head + (size_t)n * (L.ly + 2 * L.lc);
+    L.blocks = (uint64_t)n * (L.ly + 2 * L.lc) / 64;
+    return L;
+}
+
+// ------------------------------------------------------------------------------------------------
 // K1: fused encode transform
 // ------------------------------------------------------------------------------------------------
 namespace k1 {
@@ -892,11 +940,18 @@ inverse_kernel(const __grid_constant__ CUtensorMap tmap_blocks, hic_dct_geometry
     }
 }
 
-// Float64 re-evaluation of every flagged sample with scipy's exact operation order.
-__global__ void __launch_bounds__(128)
-inverse_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_t* __restrict__ yp,
-                     uint8_t* __restrict__ crp, uint8_t* __restrict__ cbp, const hic_tie_record* __restrict__ ties,
-                     uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+// Where a flagged block's samples go: the plane (row stride pw, ph rows) and the block's position in it.
+struct BlockDst {
+    uint8_t* plane;
+    int ph, pw, BY, BX;
+};
+
+// Float64 re-evaluation of every flagged sample with scipy's exact operation order.  locate(img, p, BY, BX) maps
+// block (BY, BX) of plane p (0 = Y, 1 = Cr, 2 = Cb) of image img to its BlockDst.
+template <class Locate>
+__device__ __forceinline__ void inverse_fixup_body(const int16_t* __restrict__ coef, const hic_dct_geometry& g,
+                                                   const hic_tie_record* __restrict__ ties, uint32_t tie_capacity,
+                                                   uint32_t* __restrict__ stats, Locate locate) {
     // eight lanes per flagged block (four blocks per warp): lane r runs the block's row r, then its column
     // r, in exact_decoded_block's order (rows first, then columns, /256, +128); the row results cross the
     // lanes through shared memory
@@ -909,24 +964,22 @@ inverse_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8
         const uint32_t i = base + grp;
         const bool mine = i < n_rec;
         double* a = s_a[warp][grp];
-        int kind = 0, ph = g.h, pw = g.w, nbx = g.nbx_l;
-        uint8_t* plane = nullptr;
-        int BY = 0, BX = 0;
+        int kind = 0, nbx = g.nbx_l;
+        BlockDst d = {nullptr, 0, 0, 0, 0};
         if (mine) {
             const hic_tie_record rec = ties[i];
             const int64_t img = rec.block / g.blocks_per_image;
             int64_t local = rec.block - img * g.blocks_per_image;
-            plane = yp + (size_t)img * g.h * g.w;
+            int p = 0;
             if (local >= g.nb_l) {
                 kind = 1;
                 local -= g.nb_l;
-                const int p = (int)(local / g.nb_c);
+                p = (int)(local / g.nb_c);
                 local -= (int64_t)p * g.nb_c;
-                ph = g.hc; pw = g.wc; nbx = g.nbx_c;
-                plane = (p == 0 ? crp : cbp) + (size_t)img * g.hc * g.wc;
+                nbx = g.nbx_c;
+                ++p;
             }
-            BY = (int)(local / nbx);
-            BX = (int)(local % nbx);
+            d = locate(img, p, (int)(local / nbx), (int)(local % nbx));
             const int16_t* blk = coef + (size_t)rec.block * 64;
             double row[8];
 #pragma unroll
@@ -947,9 +1000,9 @@ inverse_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8
             uint32_t changed = 0;
 #pragma unroll
             for (int y = 0; y < 8; ++y) {
-                if (8 * BY + y >= ph || 8 * BX + l8 >= pw) continue;
+                if (8 * d.BY + y >= d.ph || 8 * d.BX + l8 >= d.pw) continue;
                 const uint8_t v = wrap_u8(dadd(ddiv(col[y], 256.0), 128.0));
-                uint8_t* dst = plane + (size_t)(8 * BY + y) * pw + 8 * BX + l8;
+                uint8_t* dst = d.plane + (size_t)(8 * d.BY + y) * d.pw + 8 * d.BX + l8;
                 if (*dst != v) {
                     *dst = v;
                     ++changed;
@@ -969,6 +1022,16 @@ inverse_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8
         if (done) atomicAdd(&stats[1], 64u * done);
         if (changed_total) atomicAdd(&stats[2], changed_total);
     }
+}
+
+__global__ void __launch_bounds__(128)
+inverse_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_t* __restrict__ yp,
+                     uint8_t* __restrict__ crp, uint8_t* __restrict__ cbp, const hic_tie_record* __restrict__ ties,
+                     uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    inverse_fixup_body(coef, g, ties, tie_capacity, stats, [&](int64_t img, int p, int BY, int BX) {
+        if (p == 0) return BlockDst{yp + (size_t)img * g.h * g.w, g.h, g.w, BY, BX};
+        return BlockDst{(p == 1 ? crp : cbp) + (size_t)img * g.hc * g.wc, g.hc, g.wc, BY, BX};
+    });
 }
 
 // K8: cv2.pyrUp of both chroma planes + crop + YCrCb -> RGB.  One thread per chroma sample,
@@ -1117,6 +1180,146 @@ thumbnail_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int n, int 
     o[0] = (uint8_t)r;
     o[1] = (uint8_t)gg;
     o[2] = (uint8_t)b;
+}
+
+// ---- region decode: K7R, its fix-up, K8R (one rh x rw window per image, its origin per image) -----------------
+// Image i's window-local planes: Y at y + i * ly, 8 ny_l rows of 8 nx_l samples holding the luminance block
+// rectangle (region_first_l, region_span); Cr and Cb at cr / cb + i * lc, the chroma rectangle likewise.
+struct RegionArgs {
+    const int32_t* origin;      // n x (top, left), output coordinates
+    uint8_t *y, *cr, *cb;
+    size_t ly, lc;
+    RegionSpan s;
+    int rh, rw;
+};
+struct RegionFirst {
+    int by_l, bx_l, by_c, bx_c;
+};
+__device__ __forceinline__ RegionFirst region_first(const hic_dct_geometry& g, const RegionArgs& a, int64_t img) {
+    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
+    return {region_first_l(top, a.s.ny_l, g.nby_l), region_first_l(left, a.s.nx_l, g.nbx_l),
+            region_first_c(top, a.s.ny_c, g.nby_c), region_first_c(left, a.s.nx_c, g.nbx_c)};
+}
+
+// K7R: one selected block per thread through K7's inverse_block, into the window-local planes; ties are recorded
+// with the global block index, so exactly the blocks K7 flags are flagged.  The selected blocks are one run per
+// block row of each rectangle, so there is no box of consecutive blocks for one TMA load: the CTA's 128 blocks
+// come in by plain 16-byte loads, a warp reading four whole 128-byte blocks per instruction, into shared memory
+// with K7's 128-byte swizzle (piece j of block t at j ^ (t & 7)).
+constexpr int K7R_THREADS = 128;
+__global__ void __launch_bounds__(K7R_THREADS)
+region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, int n, RegionArgs a,
+                      hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    __shared__ int4 s_blk[K7R_THREADS * 8];
+    __shared__ uint32_t s_src[K7R_THREADS];
+    const int64_t nl = (int64_t)a.s.ny_l * a.s.nx_l, nc = (int64_t)a.s.ny_c * a.s.nx_c, per = nl + 2 * nc;
+    const int64_t first = (int64_t)blockIdx.x * K7R_THREADS, gid = first + threadIdx.x;
+    const bool live = gid < per * n;
+    int64_t img = 0;
+    int p = 0, ly = 0, lx = 0;
+    if (live) {
+        img = gid / per;
+        int64_t local = gid - img * per;
+        const RegionFirst f = region_first(g, a, img);
+        int64_t block = img * g.blocks_per_image;
+        if (local < nl) {
+            ly = (int)(local / a.s.nx_l);
+            lx = (int)(local % a.s.nx_l);
+            block += (int64_t)(f.by_l + ly) * g.nbx_l + f.bx_l + lx;
+        } else {
+            local -= nl;
+            p = 1 + (int)(local / nc);
+            local -= (int64_t)(p - 1) * nc;
+            ly = (int)(local / a.s.nx_c);
+            lx = (int)(local % a.s.nx_c);
+            block += g.nb_l + (int64_t)(p - 1) * g.nb_c + (int64_t)(f.by_c + ly) * g.nbx_c + f.bx_c + lx;
+        }
+        s_src[threadIdx.x] = (uint32_t)block;
+    }
+    __syncthreads();
+    const int count = (int)min((int64_t)K7R_THREADS, per * n - first);
+    const int4* c4 = reinterpret_cast<const int4*>(coef);
+    for (int q = threadIdx.x; q < 8 * count; q += K7R_THREADS) {
+        const int t = q >> 3, j = q & 7;
+        s_blk[8 * t + (j ^ (t & 7))] = __ldg(c4 + (size_t)s_src[t] * 8 + j);
+    }
+    __syncthreads();
+    if (!live) return;
+    const int4* src = &s_blk[threadIdx.x * 8];
+    const int sw = threadIdx.x & 7;
+    if (p == 0)
+        inverse_block<0>(src, sw, a.y + img * a.ly, 8 * a.s.ny_l, 8 * a.s.nx_l, ly, lx, s_src[threadIdx.x], ties,
+                         tie_capacity, stats);
+    else
+        inverse_block<1>(src, sw, (p == 1 ? a.cr : a.cb) + img * a.lc, 8 * a.s.ny_c, 8 * a.s.nx_c, ly, lx,
+                         s_src[threadIdx.x], ties, tie_capacity, stats);
+}
+
+// The fix-up of K7R's flagged blocks: inverse_fixup_kernel's arithmetic, each block landing in its window.
+__global__ void __launch_bounds__(128)
+region_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, RegionArgs a,
+                    const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    inverse_fixup_body(coef, g, ties, tie_capacity, stats, [&](int64_t img, int p, int BY, int BX) {
+        const RegionFirst f = region_first(g, a, img);
+        if (p == 0) return BlockDst{a.y + img * a.ly, 8 * a.s.ny_l, 8 * a.s.nx_l, BY - f.by_l, BX - f.bx_l};
+        return BlockDst{(p == 1 ? a.cr : a.cb) + img * a.lc, 8 * a.s.ny_c, 8 * a.s.nx_c, BY - f.by_c, BX - f.bx_c};
+    });
+}
+
+// K8R: K8's pyrUp taps and ycrcb_to_rgb over one window per image: a thread per chroma sample the window covers,
+// producing the pixels of its 2x2 output quad that lie inside the window (cw = rw / 2 + 1 samples per row cover any
+// origin's columns, ch = rh / 2 + 1 its rows).  The neighbours are chosen in image coordinates (hc, wc of the whole
+// image: reflect at row / column 0, replicate at the last) and then read from the window-local planes; the
+// n x rh x rw x 3 result is written directly.
+__global__ void __launch_bounds__(256)
+region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restrict__ rgb) {
+    const int ch = a.rh / 2 + 1, cw = a.rw / 2 + 1;
+    const int64_t per = (int64_t)ch * cw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * n) return;
+    const int64_t img = gid / per;
+    const int64_t rem = gid - img * per;
+    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
+    const int cy = (top >> 1) + (int)(rem / cw), cx = (left >> 1) + (int)(rem % cw);
+    if (2 * cy > top + a.rh - 1 || 2 * cx > left + a.rw - 1) return;
+    const RegionFirst f = region_first(g, a, img);
+    const int ym = cy > 0 ? cy - 1 : (g.hc > 1 ? 1 : 0), yn = cy + 1 < g.hc ? cy + 1 : g.hc - 1;
+    const int xm = cx > 0 ? cx - 1 : (g.wc > 1 ? 1 : 0), xn = cx + 1 < g.wc ? cx + 1 : g.wc - 1;
+    const int r0 = 8 * f.by_c, c0 = 8 * f.bx_c, pw = 8 * a.s.nx_c;
+    int up[2][4];      // [channel][2*dy + dx], as K8
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+        const uint8_t* p = (c == 0 ? a.cr : a.cb) + img * a.lc;
+        auto row = [&](int r, int* v) {
+            const uint8_t* q = p + (size_t)(r - r0) * pw - c0;
+            v[0] = q[xm]; v[1] = q[cx]; v[2] = q[xn];
+        };
+        int s0[3], s1[3], s2[3];
+        row(ym, s0); row(cy, s1); row(yn, s2);
+        const int e0 = s0[0] + 6 * s0[1] + s0[2], o0 = 4 * (s0[1] + s0[2]);
+        const int e1 = s1[0] + 6 * s1[1] + s1[2], o1 = 4 * (s1[1] + s1[2]);
+        const int e2 = s2[0] + 6 * s2[1] + s2[2], o2 = 4 * (s2[1] + s2[2]);
+        up[c][0] = (e0 + 6 * e1 + e2 + 32) >> 6;
+        up[c][1] = (o0 + 6 * o1 + o2 + 32) >> 6;
+        up[c][2] = (4 * (e1 + e2) + 32) >> 6;
+        up[c][3] = (4 * (o1 + o2) + 32) >> 6;
+    }
+    const uint8_t* ysrc = a.y + img * a.ly;
+    uint8_t* dst = rgb + (size_t)img * a.rh * a.rw * 3;
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < 2; ++dx) {
+            const int oy = 2 * cy + dy, ox = 2 * cx + dx;
+            if (oy < top || oy >= top + a.rh || ox < left || ox >= left + a.rw) continue;
+            int r, gg, b;
+            ycrcb_to_rgb(ysrc[(size_t)(oy - 8 * f.by_l) * (8 * a.s.nx_l) + (ox - 8 * f.bx_l)], up[0][2 * dy + dx],
+                         up[1][2 * dy + dx], r, gg, b);
+            uint8_t* o = dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3;
+            o[0] = (uint8_t)r;
+            o[1] = (uint8_t)gg;
+            o[2] = (uint8_t)b;
+        }
 }
 }  // namespace k7
 
@@ -1399,6 +1602,76 @@ int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint
     if (rc) return rc;
     cudaStream_t st = as_stream(stream);
     HIC_LAUNCH("thumbnail_kernel", st, k7::thumbnail_kernel<<<grid_for((int64_t)n * th * tw, 256), 256, 0, st>>>(d_dc, g, n, th, tw, d_rgb_out));
+    return HIC_OK;
+}
+
+int hic_dct_region_blocks(int32_t h, int32_t w, int32_t top, int32_t left, int32_t rh, int32_t rw, int32_t* rect) {
+    using namespace hic;
+    HIC_REQUIRE(rect != nullptr, "NULL argument");
+    hic_dct_geometry g;
+    int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    rc = region_check(g, top, left, rh, rw);
+    if (rc) return rc;
+    const RegionSpan s = region_span(g, rh, rw);
+    const int32_t out[8] = {region_first_l(top, s.ny_l, g.nby_l), region_first_l(left, s.nx_l, g.nbx_l), s.ny_l, s.nx_l,
+                            region_first_c(top, s.ny_c, g.nby_c), region_first_c(left, s.nx_c, g.nbx_c), s.ny_c, s.nx_c};
+    memcpy(rect, out, sizeof(out));
+    return HIC_OK;
+}
+
+int hic_dct_region_sizes(int32_t n, int32_t h, int32_t w, int32_t rh, int32_t rw, size_t* work_bytes, uint32_t* tie_capacity) {
+    using namespace hic;
+    HIC_REQUIRE(work_bytes && tie_capacity, "NULL argument");
+    HIC_REQUIRE(n >= 1, "batch size must be positive");
+    hic_dct_geometry g;
+    int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    rc = region_check(g, 0, 0, rh, rw);
+    if (rc) return rc;
+    const RegionLayout L = region_layout(n, g, rh, rw);
+    HIC_REQUIRE(L.blocks < (1ull << 32), "batch too large: %llu selected blocks", (unsigned long long)L.blocks);
+    *work_bytes = L.total;
+    *tie_capacity = (uint32_t)L.blocks;
+    return HIC_OK;
+}
+
+int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const int32_t* h_origin, int32_t rh,
+                   int32_t rw, uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity,
+                   uint32_t* d_stats, uint8_t* d_rgb_out, void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_coef && h_origin && d_work && d_ties && d_stats && d_rgb_out, "NULL pointer");
+    HIC_REQUIRE(n >= 1, "batch size must be positive");
+    hic_dct_geometry g;
+    int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    HIC_REQUIRE((int64_t)n * g.blocks_per_image < (1ll << 32), "batch too large: %lld blocks", (long long)n * g.blocks_per_image);
+    for (int i = 0; i < n; ++i) {
+        rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw);
+        if (rc) return rc;
+    }
+    const RegionLayout L = region_layout(n, g, rh, rw);
+    HIC_REQUIRE(work_bytes >= L.total, "work buffer of %zu bytes is too small: %zu needed (hic_dct_region_sizes)", work_bytes, L.total);
+    HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
+                "d_coef and d_work must be 16-byte aligned");
+    rc = ensure_tables();
+    if (rc) return rc;
+    cudaStream_t st = as_stream(stream);
+    HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
+    HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    k7::RegionArgs a;
+    a.origin = reinterpret_cast<const int32_t*>(d_work);
+    a.y = d_work + L.head;
+    a.cr = a.y + (size_t)n * L.ly;
+    a.cb = a.cr + (size_t)n * L.lc;
+    a.ly = L.ly;
+    a.lc = L.lc;
+    a.s = L.s;
+    a.rh = rh;
+    a.rw = rw;
+    HIC_LAUNCH("region_inverse_kernel", st, k7::region_inverse_kernel<<<grid_for((int64_t)L.blocks, k7::K7R_THREADS), k7::K7R_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH("region_fixup_kernel", st, k7::region_fixup_kernel<<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH("region_colour_kernel", st, k7::region_colour_kernel<<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
     return HIC_OK;
 }
 

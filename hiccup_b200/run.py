@@ -4,17 +4,20 @@ rank 1) plus a directory mode that feeds the batched GPU path.
     compress(path, output, style)      run.py:18-29   image file -> <output>/<name>.<STYLE>-hic
     decompress(path)                   run.py:32-43   .hic file -> pixels (the reference shows them in a window;
                                                        here they are returned, and written with `save=`);
-                                                       thumbnail=True: the 1/8-scale preview of a DCT-mode file instead
+                                                       thumbnail=True: the 1/8-scale preview of a DCT-mode file instead;
+                                                       region=(top, left, height, width): that window of it instead
     compress_many(paths, output, ...)  additive: same-shaped images are encoded as one GPU batch and their files
                                        written by the library's host threads (batch.write_files)
     decompress_many(paths, ...)        additive: same-shaped `.hic` files are read and decoded as one GPU batch
 
 Like the reference, `cv2.imread` delivers BGR and the codec treats channel 0 as R (run.py:19), so files
 are interchangeable with the reference's in both directions.  Command line: python -m hiccup_b200.run
--c IMG... | -d HIC... [-t] [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
+-c IMG... | -d HIC... [-t | --region T,L,H,W] [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
 """
 import argparse
 import os
+
+import numpy as np
 
 from hiccup_b200 import codec, compression, hicimage, model
 
@@ -51,11 +54,34 @@ def _no_wavelet_thumbnails(path):
                               "and wavelet files have none" % (path,))
 
 
-def decompress(path, save=None, thumbnail=False):
-    """thumbnail=True: the 1/8-scale preview (one pixel per 8x8 tile of the decoded image) of a DCT-mode file from its DC streams alone
-    (codec.jpeg_thumbnail); a wavelet file raises NotImplementedError."""
-    hi = hicimage.HicImage.from_file(path)
+def _no_wavelet_regions(path):
+    raise NotImplementedError("%s is a wavelet (HIC) file: region decode works on DCT-mode (JPEG) files" % (path,))
+
+
+def _region_args(region, thumbnail):
+    """region as ((top, left), (height, width)), or None; ValueError for a malformed one or one combined with thumbnail."""
+    if region is None:
+        return None
     if thumbnail:
+        raise ValueError("region and thumbnail do not go together")
+    r = tuple(region)
+    if len(r) != 4 or not all(isinstance(v, (int, np.integer)) for v in r):
+        raise ValueError("region must be four integers (top, left, height, width), got %r" % (region,))
+    return (int(r[0]), int(r[1])), (int(r[2]), int(r[3]))
+
+
+def decompress(path, save=None, thumbnail=False, region=None):
+    """thumbnail=True: the 1/8-scale preview (one pixel per 8x8 tile of the decoded image) of a DCT-mode file from its DC streams alone
+    (codec.jpeg_thumbnail); a wavelet file raises NotImplementedError.  region=(top, left, height, width): that window
+    of the decoded image at full resolution (codec.jpeg_region); a wavelet file raises NotImplementedError and a window
+    the image does not hold ValueError, before anything is decoded or written."""
+    win = _region_args(region, thumbnail)
+    hi = hicimage.HicImage.from_file(path)
+    if win is not None:
+        if hi.hic_type != model.Compression.JPEG:
+            _no_wavelet_regions(path)
+        rgb = codec.jpeg_region(hi, *win[0], *win[1])
+    elif thumbnail:
         if hi.hic_type != model.Compression.JPEG:
             _no_wavelet_thumbnails(path)
         rgb = codec.jpeg_thumbnail(hi)
@@ -113,12 +139,16 @@ def _peek(raw):
     return mode, shape
 
 
-def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False):
+def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region=None):
     """Decode many `.hic` files; files of one mode and image shape go through the batched codec together.  Returns the
     pixel arrays in the order of `paths` (equal to what decompress() returns for each); save_dir: also write them as PNG
     (<name>.png, or <name>.thumb.png for thumbnails).  thumbnail=True: the previews of DCT-mode files
-    (DctBatchCodec.thumbnails); a wavelet file among them raises NotImplementedError before anything is decoded."""
+    (DctBatchCodec.thumbnails); a wavelet file among them raises NotImplementedError before anything is decoded.
+    region=(top, left, height, width): that window of every file (DctBatchCodec.decode_regions, <name>.region.png); a
+    wavelet file, or a file whose image does not hold the window, raises before anything is decoded or written."""
+    from hiccup_b200 import _lib
     from hiccup_b200.batch import DctBatchCodec, WaveletBatchCodec
+    win = _region_args(region, thumbnail)
     groups, out = {}, [None] * len(paths)
     for i, p in enumerate(paths):
         with open(p, "rb") as f:
@@ -126,6 +156,10 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False):
         key = _peek(raw)
         if thumbnail and key[0] != model.Compression.JPEG:
             _no_wavelet_thumbnails(p)
+        if win is not None:
+            if key[0] != model.Compression.JPEG:
+                _no_wavelet_regions(p)
+            _lib.region_origins(*key[1], [win[0]], win[1])
         groups.setdefault(key, []).append((i, raw))
     for (mode, (h, w)), items in groups.items():
         cls = DctBatchCodec if mode == model.Compression.JPEG else WaveletBatchCodec
@@ -134,7 +168,12 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False):
             bc = cls(len(part), h, w)
             try:
                 enc = bc.streams_from_files([raw for _, raw in part])
-                pixels = bc.thumbnails(enc) if thumbnail else bc.decode(enc)
+                if win is not None:
+                    pixels = bc.decode_regions(enc, np.tile(np.asarray(win[0], np.int32), (len(part), 1)), win[1])
+                elif thumbnail:
+                    pixels = bc.thumbnails(enc)
+                else:
+                    pixels = bc.decode(enc)
                 for (i, _), rgb in zip(part, pixels):
                     out[i] = rgb.copy()
             finally:
@@ -142,12 +181,23 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False):
     if save_dir is not None:
         import cv2
         for p, rgb in zip(paths, out):
-            cv2.imwrite(os.path.join(save_dir, _png_name(p, thumbnail)), rgb)
+            cv2.imwrite(os.path.join(save_dir, _png_name(p, thumbnail, region)), rgb)
     return out
 
 
-def _png_name(path, thumbnail):
-    return os.path.split(path)[-1] + (".thumb.png" if thumbnail else ".png")
+def _png_name(path, thumbnail, region=None):
+    return os.path.split(path)[-1] + (".region.png" if region is not None else ".thumb.png" if thumbnail else ".png")
+
+
+def _parse_region(text):
+    parts = text.split(",")
+    try:
+        vals = tuple(int(v) for v in parts)
+    except ValueError:
+        vals = ()
+    if len(vals) != 4:
+        raise argparse.ArgumentTypeError("expected TOP,LEFT,HEIGHT,WIDTH (four integers), got %r" % (text,))
+    return vals
 
 
 def main(argv=None):
@@ -161,22 +211,29 @@ def main(argv=None):
                     help="append restart records to the .hic files (ignored by the reference's reader; faster decode here)")
     ap.add_argument("--thumbnail", "-t", action="store_true",
                     help="with -d: write the 1/8-scale preview of each DCT-mode file (<name>.thumb.png) from its DC streams alone")
+    ap.add_argument("--region", metavar="TOP,LEFT,HEIGHT,WIDTH", type=_parse_region,
+                    help="with -d: write that window of each DCT-mode file's decoded image (<name>.region.png) at full resolution")
     args = ap.parse_args(argv)
     if args.thumbnail and not args.decompress:
         ap.error("-t/--thumbnail goes with -d/--decompress")
+    if args.region is not None and not args.decompress:
+        ap.error("--region goes with -d/--decompress")
+    if args.region is not None and args.thumbnail:
+        ap.error("--region does not go with -t/--thumbnail")
     style = model.Compression(args.compression)
     if args.compress:
         for out in (compress_many(args.compress, args.output, style, restarts=args.restarts) if len(args.compress) > 1
                     else [compress(args.compress[0], args.output, style, restarts=args.restarts)]):
             print(out)
     elif args.decompress:
+        extra = {} if args.region is None else {"region": args.region}
         if len(args.decompress) > 1:
-            decompress_many(args.decompress, save_dir=args.output, thumbnail=args.thumbnail)
+            decompress_many(args.decompress, save_dir=args.output, thumbnail=args.thumbnail, **extra)
         else:
-            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], args.thumbnail)),
-                       thumbnail=args.thumbnail)
+            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], args.thumbnail, args.region)),
+                       thumbnail=args.thumbnail, **extra)
         for p in args.decompress:
-            print(os.path.join(args.output, _png_name(p, args.thumbnail)))
+            print(os.path.join(args.output, _png_name(p, args.thumbnail, args.region)))
     else:
         raise RuntimeError("Illegal state")
 

@@ -151,6 +151,31 @@ int hic_dct_inverse(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, uint
 int hic_dct_thumbnail_shape(int32_t h, int32_t w, int32_t* th, int32_t* tw);
 int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint8_t* d_rgb_out, void* stream);
 
+/* Region -- one rh x rw window of the decoded image per image of the batch, at full resolution:
+ * window i equals compression.jpeg_decompression(...)[top:top+rh, left:left+rw] (compression.py:42-56)
+ * bit for bit, (top, left) = h_origin[2i], h_origin[2i+1] in output coordinates; valid when top, left >= 0,
+ * rh, rw >= 1, top + rh <= out_h and left + rw <= out_w.  Output pixel (oy, ox) reads luminance sample
+ * (oy, ox) and the chroma samples of rows {ym, cy, yn} and columns {xm, cx, xn}, cy = oy >> 1, cx = ox >> 1,
+ * ym = cy > 0 ? cy - 1 : (hc > 1 ? 1 : 0), yn = min(cy + 1, hc - 1) (the same for columns): cv2.pyrUp's
+ * borders at the image's edges (reflect at the top and left, replicate at the bottom and right), the real
+ * neighbouring samples everywhere else.  Only the blocks covering those samples are inverse-transformed
+ * (K7's float32 path, its error band and float64 fix-up; tie records carry the global block index) into
+ * window-local planes in d_work, and only the window's pixels are upsampled and converted (K8's integer
+ * arithmetic) straight into d_rgb_out (n * rh * rw * 3).
+ * hic_dct_region_blocks (host only) gives the block rectangles a window at (top, left) selects:
+ * rect = {by, bx, nby, nbx} of the luminance plane, then the same of each chroma plane; every window of one
+ * size selects rectangles of one size.  hic_dct_region_sizes (host only) gives the d_work bytes and the tie
+ * capacity (one record per selected block) for n windows of rh x rw.  hic_dct_region checks every origin on
+ * the host (HIC_ERR_INVALID for a window outside out_h x out_w or an empty size) before anything is launched,
+ * and copies the origins to d_work with cudaMemcpyAsync on `stream`.  d_coef as hic_dct_inverse reads it
+ * (16-byte aligned); d_work 16-byte aligned; d_stats as for hic_dct_inverse, zeroed by this call. */
+int hic_dct_region_blocks(int32_t h, int32_t w, int32_t top, int32_t left, int32_t rh, int32_t rw, int32_t* rect);
+int hic_dct_region_sizes(int32_t n, int32_t h, int32_t w, int32_t rh, int32_t rw, size_t* work_bytes,
+                         uint32_t* tie_capacity);
+int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const int32_t* h_origin,
+                   int32_t rh, int32_t rw, uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties,
+                   uint32_t tie_capacity, uint32_t* d_stats, uint8_t* d_rgb_out, void* stream);
+
 /* ---- wavelet ("HIC") mode --------------------------------------------------------------------- */
 /* Sub-band geometry of pywt.wavedec2(channel, "db1", level=3) (transform.py:196-209): level sizes
  * ceil(n / 2) per level; ten sub-bands per channel in the order [cA3, cH3, cV3, cD3, cH2, cV2, cD2,

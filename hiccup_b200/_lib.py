@@ -161,6 +161,10 @@ SIGNATURES = {
     "hic_dct_region_sizes": (c_int, [c_int32, c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_size_t), ctypes.POINTER(c_uint32)]),
     "hic_dct_region": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_size_t, c_void_p,
                                c_uint32, c_void_p, c_void_p, c_void_p]),
+    "hic_dct_scaled_shape": (c_int, [c_int32, c_int32, c_int32, ctypes.POINTER(c_int32), ctypes.POINTER(c_int32)]),
+    "hic_dct_scaled_sizes": (c_int, [c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_size_t), ctypes.POINTER(c_uint32)]),
+    "hic_dct_scaled": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_size_t, c_void_p, c_uint32, c_void_p,
+                               c_void_p, c_void_p]),
 }
 
 _lock = threading.Lock()
@@ -252,6 +256,27 @@ def region_origins(h, w, origins, size):
         raise ValueError("region %dx%d at (%d, %d) is not inside the %dx%d decoded image"
                          % (rh, rw, o[i, 0], o[i, 1], g.out_h, g.out_w))
     return np.ascontiguousarray(o, np.int32)
+
+
+def scale_arg(scale):
+    """scale as an int if it is 2 or 4 (the scaled decode's factors; 8 is the thumbnail), else ValueError."""
+    if isinstance(scale, bool) or not isinstance(scale, (int, np.integer)) or int(scale) not in (2, 4):
+        raise ValueError("scale must be 2 or 4 (got %r; 1/8 scale is the thumbnail)" % (scale,))
+    return int(scale)
+
+
+def scaled_shape(h, w, scale):
+    """(sh, sw) = (ceil(out_h / scale), ceil(out_w / scale)) of the scaled decode (host only)."""
+    sh, sw = c_int32(), c_int32()
+    check(load().hic_dct_scaled_shape(int(h), int(w), int(scale), ctypes.byref(sh), ctypes.byref(sw)))
+    return int(sh.value), int(sw.value)
+
+
+def scaled_sizes(n, h, w, scale):
+    """(work bytes, tie capacity) hic_dct_scaled needs for n images (host only)."""
+    work, cap = c_size_t(), c_uint32()
+    check(load().hic_dct_scaled_sizes(int(n), int(h), int(w), int(scale), ctypes.byref(work), ctypes.byref(cap)))
+    return int(work.value), int(cap.value)
 
 
 def tie_capacity(n, h, w):

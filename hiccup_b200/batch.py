@@ -393,8 +393,71 @@ class DctBatchCodec(_BatchCodec):
         self.region_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
         return out.reshape(self.n, rh, rw, 3)
 
+    # ---- 1/2- and 1/4-scale images (codec.jpeg_scaled for the whole batch) ----------------------------------------
+    def scaled_shape(self, scale):
+        sh, sw = _lib.scaled_shape(self.h, self.w, _lib.scale_arg(scale))
+        return (self.n, sh, sw, 3)
+
+    def _scaled_buffers(self, scale):
+        """Check the scale (ValueError before any device work) and make the work and output buffers for it on first
+        use; returns it as an int."""
+        scale = _lib.scale_arg(scale)
+        if getattr(self, "_scale", None) != scale:
+            for b in (getattr(self, "d_scaled_work", None), getattr(self, "d_scaled", None), getattr(self, "_h_scaled", None)):
+                if b is not None:
+                    b.free()
+                    if b in self._buffers:
+                        self._buffers.remove(b)
+            self.scaled_work_bytes, self.scaled_tie_capacity = _lib.scaled_sizes(self.n, self.h, self.w, scale)
+            self.d_scaled_work = _lib.DeviceBuffer(self.scaled_work_bytes)
+            self.d_scaled = _lib.DeviceBuffer(int(np.prod(self.scaled_shape(scale))))
+            self._h_scaled = None
+            self._buffers += [self.d_scaled_work, self.d_scaled]
+            self._scale = scale
+        return scale
+
+    def _scaled(self):
+        _lib.check(self.lib.hic_dct_scaled(self.d_coef_dec.ptr, self.n, self.h, self.w, self._scale, self.d_scaled_work.ptr,
+                                           self.scaled_work_bytes, self.d_ties.ptr, self.scaled_tie_capacity,
+                                           self.d_stats.ptr, self.d_scaled.ptr, self.stream))
+
+    def decode_scaled_device(self, scale):
+        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the 1/scale images;
+        they stay on the device (fetch_scaled)."""
+        self._scaled_buffers(scale)
+        st = self.stream
+        enc = self.encoder
+        d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
+        self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
+        self.decoder.run(enc._out.ptr, enc.byte_off, enc.nbits, self.d_coef_dec.ptr, st)
+        self._scaled()
+
+    def decode_scaled(self, enc, scale, out=None):
+        """The 1/scale images (scale 2 or 4) of an EncodedStreams, host to host: image i equals
+        codec.jpeg_scaled of its file.  out: optional preallocated uint8 array of scaled_shape(scale)."""
+        self._scaled_buffers(scale)
+        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
+        self._scaled()
+        return self.fetch_scaled(out)
+
+    def fetch_scaled(self, out=None):
+        """Download the images of the last decode_scaled() / decode_scaled_device() (and their tie statistics into
+        scaled_stats)."""
+        shape = self.scaled_shape(self._scale)
+        count = int(np.prod(shape))
+        if out is None:
+            if self._h_scaled is None:
+                self._h_scaled = _lib.PinnedBuffer(count)
+            out = self._h_scaled.array(np.uint8, count)
+        else:
+            assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
+            out = out.reshape(-1)
+        out = self.d_scaled.download(np.uint8, count, self.stream, out=out)
+        self.scaled_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
+        return out.reshape(shape)
+
     def close(self):
-        for name in ("_h_thumb", "_h_region"):
+        for name in ("_h_thumb", "_h_region", "_h_scaled"):
             if getattr(self, name, None) is not None:
                 getattr(self, name).free()
                 setattr(self, name, None)

@@ -325,6 +325,44 @@ def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width:
             b.free()
 
 
+def jpeg_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
+    """The 1/2- or 1/4-scale image of a DCT-mode file: (ceil(out_h / scale), ceil(out_w / scale), 3) uint8.  Each
+    8x8 block gives an m x m tile (m = 8 / scale) by a reduced inverse transform of its low-frequency m x m
+    coefficients, the mean of each scale x scale tile of its IDCT, with the exact float64 definition of
+    hic_dct_scaled; the chroma planes are upsampled and converted with the full decode's integer rules.  The
+    entropy decode is jpeg_decode's (restart records used when the file has them).  ValueError for a scale other
+    than 2 or 4 (1/8 is jpeg_thumbnail), NotImplementedError for a wavelet file, both before any device work."""
+    if not (hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"):
+        raise NotImplementedError("scaled decode works on DCT-mode (JPEG) files; this is a wavelet (HIC) file")
+    scale = _lib.scale_arg(scale)
+    p = hic.payloads
+    lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
+    h, w = int(lum_shape[0]), int(lum_shape[1])
+    g = _lib.geometry(h, w)
+    if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
+        raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
+    settings.check_supported()
+    _lib.require_device()
+    sh, sw = _lib.scaled_shape(h, w, scale)
+    work_bytes, tie_cap = _lib.scaled_sizes(1, h, w, scale)
+    order = [kind * 3 + c for c in range(3) for kind in range(3)]
+    rows, syms, lens, codes = _tables_to_arrays([p[i] for i in order])
+    data, offs, nbits = _gather_payload_bytes([p[9 + i] for i in order])
+    dec = entropy.cached_decoder(_lib.layout_dct(1, h, w))
+    lib = _lib.load()
+    bufs = [_lib.scratch(g.blocks_per_image * 128), _lib.scratch(work_bytes), _lib.scratch(tie_cap * _lib.TIE_RECORD_BYTES),
+            _lib.scratch(4 * _lib.TIE_STATS), _lib.scratch(3 * sh * sw)]
+    coef, work, ties, stats, out = bufs
+    try:
+        _entropy_decode(dec, hic, rows, syms, lens, codes, data, offs, nbits, coef.ptr)
+        _lib.check(lib.hic_dct_scaled(coef.ptr, 1, h, w, scale, work.ptr, work_bytes, ties.ptr, tie_cap, stats.ptr, out.ptr,
+                                      None))
+        return out.download(np.uint8, 3 * sh * sw).reshape(sh, sw, 3)
+    finally:
+        for b in bufs:
+            b.free()
+
+
 def wavelet_encode(compressed: model.CompressedImage, restarts: bool = False) -> hicimage.HicImage:
     from hiccup_b200 import wavelet
     hic = wavelet.wavelet_encode(compressed)

@@ -419,6 +419,82 @@ inline double eo_inverse_prescale(int k) {
     return want / x[0];
 }
 
+// ------------------------------------------------------------------------------------------------
+// scaled decode: the m x m reduced inverse transform (m = 8 / s samples per block side, s = 2 or 4)
+//
+// B_s[k][0] = 1, B_s[k][n] = 2 D_s(n) cos(pi n (2k + 1) / (2m)), D_s(n) = sin(pi n s / 16) / (s sin(pi n / 16)):
+// for a block whose coefficients are non-zero only at u, v < m, B_s X B_s^T is the mean of each s x s tile of
+// the unrounded 8 x 8 IDCT.  Correctly rounded float64 values, row major [k][n]; tests/scaled_oracle.py holds
+// the same bits and tests/test_scaled_host.py checks both against the closed form.
+// ------------------------------------------------------------------------------------------------
+#define HIC_SCALED_B4 { \
+     0x1.0p+0,  0x1.cfefefc82ff2ap+0,  0x1.4e7ae9144f0fcp+0,  0x1.45d3819f43820p-1, \
+     0x1.0p+0,  0x1.8056948c8d24bp-1, -0x1.4e7ae9144f0fcp+0, -0x1.894e984d2e2bcp+0, \
+     0x1.0p+0, -0x1.8056948c8d24bp-1, -0x1.4e7ae9144f0fcp+0,  0x1.894e984d2e2bcp+0, \
+     0x1.0p+0, -0x1.cfefefc82ff2ap+0,  0x1.4e7ae9144f0fcp+0, -0x1.45d3819f43820p-1 }
+#define HIC_SCALED_B2 { \
+     0x1.0p+0,  0x1.480d9d073b428p+0, \
+     0x1.0p+0, -0x1.480d9d073b428p+0 }
+
+// The definition of a scaled block, in float64: cq = the dequantised coefficients q[u][v] T[u][v], u, v < M, row
+// major; rows first (A[u][k] = sum_v B[k][v] cq[u][v]), then columns (Y[j][k] = sum_u B[j][u] A[u][k]), every sum
+// left to right from its first product, every product and sum rounded; out[j][k] = Y / 256 + 128, the value
+// before the uint8 cast (wrap_u8).  The fix-up kernel and the CPU harness both run this.
+template <int M>
+HIC_HD void scaled_decoded_block(const int32_t* cq, double* out) {
+    static_assert(M == 4 || M == 2, "scale 2 or 4");
+    const double B4[16] = HIC_SCALED_B4, B2[4] = HIC_SCALED_B2;
+    const double* B = M == 4 ? B4 : B2;
+    double a[M * M];
+#pragma unroll
+    for (int u = 0; u < M; ++u)
+#pragma unroll
+        for (int k = 0; k < M; ++k) {
+            double acc = dmul(B[M * k], (double)cq[M * u]);
+#pragma unroll
+            for (int v = 1; v < M; ++v) acc = dadd(acc, dmul(B[M * k + v], (double)cq[M * u + v]));
+            a[M * u + k] = acc;
+        }
+#pragma unroll
+    for (int j = 0; j < M; ++j)
+#pragma unroll
+        for (int k = 0; k < M; ++k) {
+            double acc = dmul(B[M * j], a[k]);
+#pragma unroll
+            for (int u = 1; u < M; ++u) acc = dadd(acc, dmul(B[M * j + u], a[M * u + k]));
+            out[M * j + k] = dadd(ddiv(acc, 256.0), 128.0);
+        }
+}
+
+// The float32 fast path of the same transform, in place on v (M x M, row major): rows, then columns, each output a
+// dense M-point sum acc = x_0 (B[k][0] = 1), then eo_fma(B[k][n], x_n, acc).  T is float, or the bound-carrying
+// value of hic_dct_bound.h, which derives the error band of this code.
+template <int M, typename T>
+HIC_HD void scaled_transform(T* v) {
+    static_assert(M == 4 || M == 2, "scale 2 or 4");
+    const double B4[16] = HIC_SCALED_B4, B2[4] = HIC_SCALED_B2;
+    const double* B = M == 4 ? B4 : B2;
+#pragma unroll
+    for (int pass = 0; pass < 2; ++pass) {
+        const int step = pass == 0 ? 1 : M, stride = pass == 0 ? M : 1;    // rows: v[M r + n]; columns: v[r + M n]
+#pragma unroll
+        for (int r = 0; r < M; ++r) {
+            T x[M], y[M];
+#pragma unroll
+            for (int n = 0; n < M; ++n) x[n] = v[stride * r + step * n];
+#pragma unroll
+            for (int k = 0; k < M; ++k) {
+                T acc = x[0];
+#pragma unroll
+                for (int n = 1; n < M; ++n) acc = eo_fma(T(B[M * k + n]), x[n], acc);
+                y[k] = acc;
+            }
+#pragma unroll
+            for (int k = 0; k < M; ++k) v[stride * r + step * k] = y[k];
+        }
+    }
+}
+
 // The near-tie bands.  A float32 quantised value C/q is trusted when its distance to the nearest
 // half-integer exceeds kappa(u, v) * 4 u E / q (u = 2^-24, E = sum |x - 128| over the block); a float32
 // decoded sample when its distance to the nearest integer (where the reference's uint8 truncation steps)

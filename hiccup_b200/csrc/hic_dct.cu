@@ -1,5 +1,6 @@
 // hic_dct.cu -- DCT-mode transform stage: K1 (fused colour + pyrDown + DCT + quantise + zigzag),
-// the float64 tie fix-up, K7 (dequantise + IDCT) and K8 (pyrUp + colour), plus layout converters.
+// the float64 tie fix-up, K7 (dequantise + IDCT) and K8 (pyrUp + colour), their thumbnail, region and scaled
+// variants, plus layout converters.
 //
 // Data layout in HBM (see include/hiccup_b200.h): RGB u8 interleaved in; coefficients as int16
 // "zigzag blocks" (one 128-byte line per 8x8 block) out.  HBM-bound by design: 3 B/pixel read,
@@ -26,6 +27,7 @@ struct DctTables {
     float qw[2][64];     // inverse band weight: q * w(u, v) * margin
     int qi[2][64];       // q
     int izz[64];         // natural index -> scan position
+    float sqw[2][2][16]; // scaled decode band weight [0: M = 4, 1: M = 2][kind][M u + v]: T(u, v) * w_s(u, v) * margin
 };
 __constant__ DctTables c_tab;
 __constant__ uint8_t c_zigzag[64] = HIC_ZIGZAG8;
@@ -60,6 +62,16 @@ static int ensure_tables() {
                     t.qi[kind][nat] = q;
                 }
         for (int k = 0; k < 64; ++k) t.izz[h_zigzag[k]] = k;
+        double w4[16], w2[4];
+        scaled_bounds<4>(w4);
+        scaled_bounds<2>(w2);
+        for (int kind = 0; kind < 2; ++kind)
+            for (int u = 0; u < 4; ++u)
+                for (int v = 0; v < 4; ++v) {
+                    const int q = (kind == 0 ? h_lum : h_chroma)[8 * u + v];
+                    t.sqw[0][kind][4 * u + v] = (float)(q * w4[4 * u + v] * HIC_BAND_MARGIN);
+                    if (u < 2 && v < 2) t.sqw[1][kind][2 * u + v] = (float)(q * w2[2 * u + v] * HIC_BAND_MARGIN);
+                }
         built = true;
     }
     HIC_CUDA(cudaMemcpyToSymbol(c_tab, &t, sizeof(t)));
@@ -1145,6 +1157,19 @@ upsample_colour_vec_kernel(const uint8_t* __restrict__ yp, const uint8_t* __rest
 // constant sample: trunc(q T00 / 256 + 128) mod 256 = ((q T00 + 32768) / 256, truncated toward zero) & 255.
 __device__ __forceinline__ int dc_block_sample(int q, int t00) { return ((q * t00 + 32768) / 256) & 255; }
 
+// K8's pyrUp of one chroma sample's 2x2 output quad [2 dy + dx] from its 3x3 neighbourhood: r0, r1, r2 the rows
+// ym, cy, yn, each at columns xm, cx, xn (s[-1] = s[1], s[n] = s[n-1] already applied by the caller).  Per axis even =
+// s[i-1] + 6 s[i] + s[i+1], odd = 4 (s[i] + s[i+1]); (v + 32) >> 6 after both axes.
+__device__ __forceinline__ void pyr_up_quad(const int* r0, const int* r1, const int* r2, int* up) {
+    const int e0 = r0[0] + 6 * r0[1] + r0[2], o0 = 4 * (r0[1] + r0[2]);
+    const int e1 = r1[0] + 6 * r1[1] + r1[2], o1 = 4 * (r1[1] + r1[2]);
+    const int e2 = r2[0] + 6 * r2[1] + r2[2], o2 = 4 * (r2[1] + r2[2]);
+    up[0] = (e0 + 6 * e1 + e2 + 32) >> 6;
+    up[1] = (o0 + 6 * o1 + o2 + 32) >> 6;
+    up[2] = (4 * (e1 + e2) + 32) >> 6;
+    up[3] = (4 * (o1 + o2) + 32) >> 6;
+}
+
 // Thumbnail: one pixel per 8x8 tile of the full decode's output (th = ceil(out_h / 8), tw = ceil(out_w / 8)),
 // from the DC values alone (one int16 per block, global block order).  The luminance block (ty, tx) gives Y; the
 // chroma planes of block samples (nby_c x nbx_c) go through K8's pyrUp taps on the fly, s[-1] = s[1] and s[n] =
@@ -1296,13 +1321,7 @@ region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restric
         };
         int s0[3], s1[3], s2[3];
         row(ym, s0); row(cy, s1); row(yn, s2);
-        const int e0 = s0[0] + 6 * s0[1] + s0[2], o0 = 4 * (s0[1] + s0[2]);
-        const int e1 = s1[0] + 6 * s1[1] + s1[2], o1 = 4 * (s1[1] + s1[2]);
-        const int e2 = s2[0] + 6 * s2[1] + s2[2], o2 = 4 * (s2[1] + s2[2]);
-        up[c][0] = (e0 + 6 * e1 + e2 + 32) >> 6;
-        up[c][1] = (o0 + 6 * o1 + o2 + 32) >> 6;
-        up[c][2] = (4 * (e1 + e2) + 32) >> 6;
-        up[c][3] = (4 * (o1 + o2) + 32) >> 6;
+        pyr_up_quad(s0, s1, s2, up[c]);
     }
     const uint8_t* ysrc = a.y + img * a.ly;
     uint8_t* dst = rgb + (size_t)img * a.rh * a.rw * 3;
@@ -1316,6 +1335,196 @@ region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restric
             ycrcb_to_rgb(ysrc[(size_t)(oy - 8 * f.by_l) * (8 * a.s.nx_l) + (ox - 8 * f.bx_l)], up[0][2 * dy + dx],
                          up[1][2 * dy + dx], r, gg, b);
             uint8_t* o = dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3;
+            o[0] = (uint8_t)r;
+            o[1] = (uint8_t)gg;
+            o[2] = (uint8_t)b;
+        }
+}
+
+// ---- scaled decode: K7S, its fix-up, K8S (1/s scale, M = 8 / s samples per block side) ----------------------
+// The work buffer holds one M x M tile of samples per block of the batch, in global block order: block b's samples
+// at work + b M^2, row major.  K8S reads the reduced planes through that layout.
+__device__ __forceinline__ int tile_sample(const uint8_t* plane, int nbx, int M, int r, int c) {
+    return plane[(((r / M) * nbx + c / M) * M + r % M) * M + c % M];
+}
+
+// K7S: one block per thread.  The CTA's 128 blocks arrive by one TMA tensor load over K7's [block][64 int16] map of
+// the coefficient buffer, only the scan entries the block needs: M = 4 reads entries 0..31 (its 4 x 4 corner ends at
+// entry 24) as a box of {32, 128} in the 64-byte swizzle (piece j of block t at j ^ ((t >> 1) & 3): the eight blocks
+// of a quarter warp hit eight different 16-byte bank groups); M = 2 reads entries 0..7 (the 2 x 2 corner ends at 4)
+// as a box of {8, 128}.  The float32 path is scaled_transform<M> on q T / 256 (exact); a block with AC terms and a
+// sample within its band of an integer (where the uint8 truncation steps) is recorded for the float64 fix-up.
+constexpr int K7S_THREADS = 128;
+template <int M>
+struct K7SSmem {
+    static constexpr int PIECES = M == 4 ? 4 : 1;      // 16-byte pieces (8 scan entries each) read per block
+    alignas(1024) int4 blk[K7S_THREADS * PIECES];
+    alignas(8) unsigned long long bar;
+};
+
+template <int M>
+__global__ void __launch_bounds__(K7S_THREADS)
+scaled_inverse_kernel(const __grid_constant__ CUtensorMap tmap_blocks, hic_dct_geometry g, int n, uint8_t* __restrict__ tiles,
+                      hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    constexpr int PIECES = K7SSmem<M>::PIECES;
+    constexpr uint8_t zz[64] = HIC_ZIGZAG8;
+    __shared__ K7SSmem<M> s;
+    const uint32_t bar = (uint32_t)__cvta_generic_to_shared(&s.bar);
+    if (threadIdx.x == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)sizeof(s.blk)) : "memory");
+        asm volatile(
+            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+            ::"r"((uint32_t)__cvta_generic_to_shared(s.blk)), "l"(reinterpret_cast<uint64_t>(&tmap_blocks)), "r"(0),
+            "r"((int)(blockIdx.x * K7S_THREADS)), "r"(bar)
+            : "memory");
+    }
+    __syncthreads();
+    asm volatile(
+        "{\n"
+        ".reg .pred P1;\n"
+        "LAB_WAIT:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], 0;\n"
+        "@P1 bra DONE;\n"
+        "bra LAB_WAIT;\n"
+        "DONE:\n"
+        "}\n" ::"r"(bar)
+        : "memory");
+    const int64_t total = (int64_t)n * g.blocks_per_image;
+    const int64_t gid = (int64_t)blockIdx.x * K7S_THREADS + threadIdx.x;
+    if (gid >= total) return;
+    const int kind = gid % g.blocks_per_image < g.nb_l ? 0 : 1;
+    const int t = threadIdx.x;
+    int words[4 * PIECES];                              // the block's first 8 PIECES scan entries, two per word
+#pragma unroll
+    for (int j = 0; j < PIECES; ++j) {
+        const int4 wv = s.blk[PIECES * t + (M == 4 ? j ^ ((t >> 1) & 3) : j)];
+        words[4 * j] = wv.x; words[4 * j + 1] = wv.y; words[4 * j + 2] = wv.z; words[4 * j + 3] = wv.w;
+    }
+    float v[M * M];
+    float energy = 0.f;          // sum |q| T w_s margin: the error band of the samples
+    int ac_bits = 0;
+#pragma unroll
+    for (int k = 0; k < 8 * PIECES; ++k) {
+        const int nat = zz[k], u = nat >> 3, x = nat & 7;
+        if (u >= M || x >= M) continue;
+        const int q = (k & 1) ? words[k >> 1] >> 16 : (int)(short)(words[k >> 1] & 0xFFFF);
+        v[M * u + x] = (float)(q * c_tab.qi[kind][nat]) * (1.f / 256.f);
+        energy = fmaf(fabsf((float)q), c_tab.sqw[M == 4 ? 0 : 1][kind][M * u + x], energy);
+        if (k) ac_bits |= q;
+    }
+    scaled_transform<M>(v);
+    float margin = 1e30f;
+    uint32_t packed[M * M / 4];
+#pragma unroll
+    for (int i = 0; i < M * M; ++i) {
+        const float p = v[i] + 128.f;
+        const float r = (p + MAGIC) - MAGIC;
+        margin = fminf(margin, fabsf(p - r));
+        const uint32_t b = (uint32_t)__float2int_rz(p) & 0xFFu;               // truncate, wrap
+        if (i % 4 == 0) packed[i / 4] = b; else packed[i / 4] |= b << (8 * (i % 4));
+    }
+    if constexpr (M == 4)
+        reinterpret_cast<uint4*>(tiles)[gid] = make_uint4(packed[0], packed[1], packed[2], packed[3]);
+    else
+        reinterpret_cast<uint32_t*>(tiles)[gid] = packed[0];
+    // as K7: 2^-15 covers the rounding of the final + 128 below 1024 and of this comparison
+    const float band = (float)(4.0 / 16777216.0 / 256.0) * energy + 3.0517578125e-5f;
+    if (ac_bits != 0 && margin <= band) {
+        const uint32_t slot = atomicAdd(&stats[0], 1u);
+        if (slot < tie_capacity) {
+            hic_tie_record rec;
+            rec.block = (uint32_t)gid;
+            rec.reserved = 0;
+            rec.mask = ~0ull;
+            ties[slot] = rec;
+        } else {
+            atomicAdd(&stats[3], 1u);
+        }
+    }
+}
+
+// The fix-up of K7S's flagged blocks: one thread per record, scaled_decoded_block<M> (the float64 definition) into
+// the block's tile.  stats[1] counts the samples re-evaluated, stats[2] those that changed.
+template <int M>
+__global__ void __launch_bounds__(128)
+scaled_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_t* __restrict__ tiles,
+                    const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    const uint32_t n_rec = min(stats[0], tie_capacity);
+    uint32_t changed = 0, done = 0;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_rec; i += gridDim.x * blockDim.x) {
+        const uint32_t b = ties[i].block;
+        const int kind = b % g.blocks_per_image < g.nb_l ? 0 : 1;
+        const int16_t* blk = coef + (size_t)b * 64;
+        int32_t cq[M * M];
+#pragma unroll
+        for (int u = 0; u < M; ++u)
+#pragma unroll
+            for (int x = 0; x < M; ++x) cq[M * u + x] = (int32_t)blk[c_tab.izz[8 * u + x]] * c_tab.qi[kind][8 * u + x];
+        double y[M * M];
+        scaled_decoded_block<M>(cq, y);
+        uint8_t* dst = tiles + (size_t)b * M * M;
+#pragma unroll
+        for (int k = 0; k < M * M; ++k) {
+            const uint8_t val = wrap_u8(y[k]);
+            if (dst[k] != val) {
+                dst[k] = val;
+                ++changed;
+            }
+        }
+        ++done;
+    }
+#pragma unroll
+    for (int off = 16; off; off >>= 1) {
+        changed += __shfl_down_sync(0xffffffffu, changed, off);
+        done += __shfl_down_sync(0xffffffffu, done, off);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (done) atomicAdd(&stats[1], (uint32_t)(M * M) * done);
+        if (changed) atomicAdd(&stats[2], changed);
+    }
+}
+
+// K8S: one sample of the reduced chroma planes (M nby_c x M nbx_c, their whole block grids: the thumbnail's
+// convention) per thread, as K8: its 3x3 neighbourhood through pyr_up_quad, Y from the reduced luminance plane
+// (M nby_l x M nbx_l), K8's ycrcb_to_rgb, and the pixels of its 2x2 output quad inside sh x sw = ceil(out_h / s) x
+// ceil(out_w / s) written to n x sh x sw x 3 directly.
+template <int M>
+__global__ void __launch_bounds__(256)
+scaled_colour_kernel(const uint8_t* __restrict__ tiles, hic_dct_geometry g, int n, int sh, int sw, uint8_t* __restrict__ rgb) {
+    const int qh = (sh + 1) / 2, qw = (sw + 1) / 2;
+    const int64_t per = (int64_t)qh * qw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * n) return;
+    const int64_t img = gid / per;
+    const int64_t rem = gid - img * per;
+    const int cy = (int)(rem / qw), cx = (int)(rem % qw);
+    const int ny = M * g.nby_c, nx = M * g.nbx_c;
+    const int ym = cy > 0 ? cy - 1 : (ny > 1 ? 1 : 0), yn = cy + 1 < ny ? cy + 1 : ny - 1;
+    const int xm = cx > 0 ? cx - 1 : (nx > 1 ? 1 : 0), xn = cx + 1 < nx ? cx + 1 : nx - 1;
+    const uint8_t* base = tiles + (size_t)img * g.blocks_per_image * M * M;
+    int up[2][4];
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+        const uint8_t* p = base + (size_t)(g.nb_l + c * g.nb_c) * M * M;
+        auto row = [&](int r, int* v) {
+            v[0] = tile_sample(p, g.nbx_c, M, r, xm); v[1] = tile_sample(p, g.nbx_c, M, r, cx); v[2] = tile_sample(p, g.nbx_c, M, r, xn);
+        };
+        int s0[3], s1[3], s2[3];
+        row(ym, s0); row(cy, s1); row(yn, s2);
+        pyr_up_quad(s0, s1, s2, up[c]);
+    }
+    uint8_t* dst = rgb + (size_t)img * sh * sw * 3;
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < 2; ++dx) {
+            const int oy = 2 * cy + dy, ox = 2 * cx + dx;
+            if (oy >= sh || ox >= sw) continue;
+            int r, gg, b;
+            ycrcb_to_rgb(tile_sample(base, g.nbx_l, M, oy, ox), up[0][2 * dy + dx], up[1][2 * dy + dx], r, gg, b);
+            uint8_t* o = dst + ((size_t)oy * sw + ox) * 3;
             o[0] = (uint8_t)r;
             o[1] = (uint8_t)gg;
             o[2] = (uint8_t)b;
@@ -1672,6 +1881,82 @@ int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const
     HIC_LAUNCH("region_inverse_kernel", st, k7::region_inverse_kernel<<<grid_for((int64_t)L.blocks, k7::K7R_THREADS), k7::K7R_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("region_fixup_kernel", st, k7::region_fixup_kernel<<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("region_colour_kernel", st, k7::region_colour_kernel<<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
+    return HIC_OK;
+}
+
+int hic_dct_scaled_shape(int32_t h, int32_t w, int32_t scale, int32_t* sh, int32_t* sw) {
+    using namespace hic;
+    HIC_REQUIRE(sh && sw, "NULL argument");
+    HIC_REQUIRE(scale == 2 || scale == 4, "scale must be 2 or 4 (got %d; scale 8 is hic_dct_thumbnail)", scale);
+    hic_dct_geometry g;
+    const int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    *sh = ceil_div(g.out_h, scale);
+    *sw = ceil_div(g.out_w, scale);
+    return HIC_OK;
+}
+
+int hic_dct_scaled_sizes(int32_t n, int32_t h, int32_t w, int32_t scale, size_t* work_bytes, uint32_t* tie_capacity) {
+    using namespace hic;
+    HIC_REQUIRE(work_bytes && tie_capacity, "NULL argument");
+    HIC_REQUIRE(n >= 1, "batch size must be positive");
+    HIC_REQUIRE(scale == 2 || scale == 4, "scale must be 2 or 4 (got %d; scale 8 is hic_dct_thumbnail)", scale);
+    hic_dct_geometry g;
+    const int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    const int64_t blocks = (int64_t)n * g.blocks_per_image;
+    HIC_REQUIRE(blocks < (1ll << 32), "batch too large: %lld blocks", (long long)blocks);
+    const int m = 8 / scale;
+    *work_bytes = (size_t)blocks * m * m;
+    *tie_capacity = (uint32_t)blocks;
+    return HIC_OK;
+}
+
+int hic_dct_scaled(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32_t scale, uint8_t* d_work, size_t work_bytes,
+                   hic_tie_record* d_ties, uint32_t tie_capacity, uint32_t* d_stats, uint8_t* d_rgb_out, void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_coef && d_work && d_ties && d_stats && d_rgb_out, "NULL device pointer");
+    size_t need = 0;
+    uint32_t cap = 0;
+    int rc = hic_dct_scaled_sizes(n, h, w, scale, &need, &cap);
+    if (rc) return rc;
+    HIC_REQUIRE(work_bytes >= need, "work buffer of %zu bytes is too small: %zu needed (hic_dct_scaled_sizes)", work_bytes, need);
+    HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
+                "d_coef and d_work must be 16-byte aligned");
+    hic_dct_geometry g;
+    geometry_of(h, w, &g);
+    int32_t sh = 0, sw = 0;
+    hic_dct_scaled_shape(h, w, scale, &sh, &sw);
+    rc = ensure_tables();
+    if (rc) return rc;
+    cudaStream_t st = as_stream(stream);
+    HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
+    const int64_t blocks = (int64_t)n * g.blocks_per_image;
+    // K7's [block][64 int16] view of the coefficient buffer; the box takes the first 32 (M = 4) or 8 (M = 2) entries
+    CUtensorMap tmap_blocks;
+    {
+        EncodeTiledFn encode = nullptr;
+        rc = tensor_map_encoder(&encode);
+        if (rc) return rc;
+        const cuuint64_t dims[2] = {64, (cuuint64_t)blocks};
+        const cuuint64_t strides[1] = {128};
+        const cuuint32_t box[2] = {scale == 2 ? 32u : 8u, (cuuint32_t)k7::K7S_THREADS};
+        const cuuint32_t estr[2] = {1, 1};
+        const CUresult r = encode(&tmap_blocks, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, const_cast<int16_t*>(d_coef), dims, strides, box, estr,
+                                  CU_TENSOR_MAP_INTERLEAVE_NONE, scale == 2 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE,
+                                  CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return hic::fail(HIC_ERR_CUDA, "cuTensorMapEncodeTiled (coefficient blocks) failed: %d", (int)r);
+    }
+    const unsigned grid_inv = grid_for(blocks, k7::K7S_THREADS), grid_rgb = grid_for((int64_t)n * ((sh + 1) / 2) * ((sw + 1) / 2), 256);
+    if (scale == 2) {
+        HIC_LAUNCH("scaled_inverse_kernel", st, k7::scaled_inverse_kernel<4><<<grid_inv, k7::K7S_THREADS, 0, st>>>(tmap_blocks, g, n, d_work, d_ties, tie_capacity, d_stats));
+        HIC_LAUNCH("scaled_fixup_kernel", st, k7::scaled_fixup_kernel<4><<<148 * 4, 128, 0, st>>>(d_coef, g, d_work, d_ties, tie_capacity, d_stats));
+        HIC_LAUNCH("scaled_colour_kernel", st, k7::scaled_colour_kernel<4><<<grid_rgb, 256, 0, st>>>(d_work, g, n, sh, sw, d_rgb_out));
+    } else {
+        HIC_LAUNCH("scaled_inverse_kernel", st, k7::scaled_inverse_kernel<2><<<grid_inv, k7::K7S_THREADS, 0, st>>>(tmap_blocks, g, n, d_work, d_ties, tie_capacity, d_stats));
+        HIC_LAUNCH("scaled_fixup_kernel", st, k7::scaled_fixup_kernel<2><<<148 * 4, 128, 0, st>>>(d_coef, g, d_work, d_ties, tie_capacity, d_stats));
+        HIC_LAUNCH("scaled_colour_kernel", st, k7::scaled_colour_kernel<2><<<grid_rgb, 256, 0, st>>>(d_work, g, n, sh, sw, d_rgb_out));
+    }
     return HIC_OK;
 }
 

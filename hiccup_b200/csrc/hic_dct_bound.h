@@ -116,4 +116,23 @@ inline DctBounds dct_bounds() {
     return out;
 }
 
+// scaled decode (scaled_transform<M>): |p32 - p| <= (4 u / 256) sum_k w[k] |cq_k| + 2^-17 for every sample p = Y / 256
+// + 128 of an M x M block, cq_k = q T of input k = M u + v (the maximum over the M x M samples per input).  The
+// inputs cq / 256 are exact in float32 (|q T| < 2^22, a power-of-two scale); the final + 128 rounds once more, by at
+// most u |Y / 256| + 2^-17, hence the |c| added to each output's sum.
+template <int M>
+inline void scaled_bounds(double* w) {
+    static BoundV g[M * M];
+    for (int i = 0; i < M * M; ++i) {
+        g[i] = BoundV();
+        g[i].c[i] = 1.0 / 256.0;
+    }
+    scaled_transform<M>(g);
+    for (int k = 0; k < M * M; ++k) {
+        double worst = 0.0;
+        for (int s = 0; s < M * M; ++s) worst = fmax(worst, g[s].e[k] + fabs(g[s].c[k]));
+        w[k] = worst * 256.0 / 4.0;
+    }
+}
+
 }  // namespace hic

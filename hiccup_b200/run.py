@@ -5,14 +5,15 @@ rank 1) plus a directory mode that feeds the batched GPU path.
     decompress(path)                   run.py:32-43   .hic file -> pixels (the reference shows them in a window;
                                                        here they are returned, and written with `save=`);
                                                        thumbnail=True: the 1/8-scale preview of a DCT-mode file instead;
-                                                       region=(top, left, height, width): that window of it instead
+                                                       region=(top, left, height, width): that window of it instead;
+                                                       scale=2 or 4: its 1/2- or 1/4-scale image instead
     compress_many(paths, output, ...)  additive: same-shaped images are encoded as one GPU batch and their files
                                        written by the library's host threads (batch.write_files)
     decompress_many(paths, ...)        additive: same-shaped `.hic` files are read and decoded as one GPU batch
 
 Like the reference, `cv2.imread` delivers BGR and the codec treats channel 0 as R (run.py:19), so files
 are interchangeable with the reference's in both directions.  Command line: python -m hiccup_b200.run
--c IMG... | -d HIC... [-t | --region T,L,H,W] [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
+-c IMG... | -d HIC... [-t | --region T,L,H,W | --scale 2|4] [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
 """
 import argparse
 import os
@@ -70,14 +71,35 @@ def _region_args(region, thumbnail):
     return (int(r[0]), int(r[1])), (int(r[2]), int(r[3]))
 
 
-def decompress(path, save=None, thumbnail=False, region=None):
+def _no_wavelet_scaled(path):
+    raise NotImplementedError("%s is a wavelet (HIC) file: scaled decode works on DCT-mode (JPEG) files" % (path,))
+
+
+def _scale_args(scale, thumbnail, region):
+    """scale as an int (2 or 4), or None; ValueError for another value or one combined with thumbnail or region."""
+    if scale is None:
+        return None
+    if thumbnail or region is not None:
+        raise ValueError("scale does not go with thumbnail or region")
+    from hiccup_b200 import _lib
+    return _lib.scale_arg(scale)
+
+
+def decompress(path, save=None, thumbnail=False, region=None, scale=None):
     """thumbnail=True: the 1/8-scale preview (one pixel per 8x8 tile of the decoded image) of a DCT-mode file from its DC streams alone
     (codec.jpeg_thumbnail); a wavelet file raises NotImplementedError.  region=(top, left, height, width): that window
     of the decoded image at full resolution (codec.jpeg_region); a wavelet file raises NotImplementedError and a window
-    the image does not hold ValueError, before anything is decoded or written."""
+    the image does not hold ValueError, before anything is decoded or written.  scale=2 or 4: the 1/2- or 1/4-scale
+    image of a DCT-mode file (codec.jpeg_scaled); a wavelet file raises NotImplementedError and another scale
+    ValueError, before anything is decoded or written."""
     win = _region_args(region, thumbnail)
+    scale = _scale_args(scale, thumbnail, region)
     hi = hicimage.HicImage.from_file(path)
-    if win is not None:
+    if scale is not None:
+        if hi.hic_type != model.Compression.JPEG:
+            _no_wavelet_scaled(path)
+        rgb = codec.jpeg_scaled(hi, scale)
+    elif win is not None:
         if hi.hic_type != model.Compression.JPEG:
             _no_wavelet_regions(path)
         rgb = codec.jpeg_region(hi, *win[0], *win[1])
@@ -139,16 +161,19 @@ def _peek(raw):
     return mode, shape
 
 
-def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region=None):
+def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region=None, scale=None):
     """Decode many `.hic` files; files of one mode and image shape go through the batched codec together.  Returns the
     pixel arrays in the order of `paths` (equal to what decompress() returns for each); save_dir: also write them as PNG
     (<name>.png, or <name>.thumb.png for thumbnails).  thumbnail=True: the previews of DCT-mode files
     (DctBatchCodec.thumbnails); a wavelet file among them raises NotImplementedError before anything is decoded.
     region=(top, left, height, width): that window of every file (DctBatchCodec.decode_regions, <name>.region.png); a
-    wavelet file, or a file whose image does not hold the window, raises before anything is decoded or written."""
+    wavelet file, or a file whose image does not hold the window, raises before anything is decoded or written.
+    scale=2 or 4: the 1/2- or 1/4-scale image of every file (DctBatchCodec.decode_scaled, <name>.s2.png / <name>.s4.png);
+    a wavelet file or another scale raises before anything is decoded or written."""
     from hiccup_b200 import _lib
     from hiccup_b200.batch import DctBatchCodec, WaveletBatchCodec
     win = _region_args(region, thumbnail)
+    scale = _scale_args(scale, thumbnail, region)
     groups, out = {}, [None] * len(paths)
     for i, p in enumerate(paths):
         with open(p, "rb") as f:
@@ -160,6 +185,8 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region
             if key[0] != model.Compression.JPEG:
                 _no_wavelet_regions(p)
             _lib.region_origins(*key[1], [win[0]], win[1])
+        if scale is not None and key[0] != model.Compression.JPEG:
+            _no_wavelet_scaled(p)
         groups.setdefault(key, []).append((i, raw))
     for (mode, (h, w)), items in groups.items():
         cls = DctBatchCodec if mode == model.Compression.JPEG else WaveletBatchCodec
@@ -168,7 +195,9 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region
             bc = cls(len(part), h, w)
             try:
                 enc = bc.streams_from_files([raw for _, raw in part])
-                if win is not None:
+                if scale is not None:
+                    pixels = bc.decode_scaled(enc, scale)
+                elif win is not None:
                     pixels = bc.decode_regions(enc, np.tile(np.asarray(win[0], np.int32), (len(part), 1)), win[1])
                 elif thumbnail:
                     pixels = bc.thumbnails(enc)
@@ -181,11 +210,13 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region
     if save_dir is not None:
         import cv2
         for p, rgb in zip(paths, out):
-            cv2.imwrite(os.path.join(save_dir, _png_name(p, thumbnail, region)), rgb)
+            cv2.imwrite(os.path.join(save_dir, _png_name(p, thumbnail, region, scale)), rgb)
     return out
 
 
-def _png_name(path, thumbnail, region=None):
+def _png_name(path, thumbnail, region=None, scale=None):
+    if scale is not None:
+        return os.path.split(path)[-1] + ".s%d.png" % scale
     return os.path.split(path)[-1] + (".region.png" if region is not None else ".thumb.png" if thumbnail else ".png")
 
 
@@ -213,6 +244,8 @@ def main(argv=None):
                     help="with -d: write the 1/8-scale preview of each DCT-mode file (<name>.thumb.png) from its DC streams alone")
     ap.add_argument("--region", metavar="TOP,LEFT,HEIGHT,WIDTH", type=_parse_region,
                     help="with -d: write that window of each DCT-mode file's decoded image (<name>.region.png) at full resolution")
+    ap.add_argument("--scale", type=int, choices=(2, 4),
+                    help="with -d: write the 1/2- or 1/4-scale image of each DCT-mode file (<name>.s2.png / <name>.s4.png)")
     args = ap.parse_args(argv)
     if args.thumbnail and not args.decompress:
         ap.error("-t/--thumbnail goes with -d/--decompress")
@@ -220,6 +253,10 @@ def main(argv=None):
         ap.error("--region goes with -d/--decompress")
     if args.region is not None and args.thumbnail:
         ap.error("--region does not go with -t/--thumbnail")
+    if args.scale is not None and not args.decompress:
+        ap.error("--scale goes with -d/--decompress")
+    if args.scale is not None and (args.thumbnail or args.region is not None):
+        ap.error("--scale does not go with -t/--thumbnail or --region")
     style = model.Compression(args.compression)
     if args.compress:
         for out in (compress_many(args.compress, args.output, style, restarts=args.restarts) if len(args.compress) > 1
@@ -227,13 +264,15 @@ def main(argv=None):
             print(out)
     elif args.decompress:
         extra = {} if args.region is None else {"region": args.region}
+        if args.scale is not None:
+            extra["scale"] = args.scale
         if len(args.decompress) > 1:
             decompress_many(args.decompress, save_dir=args.output, thumbnail=args.thumbnail, **extra)
         else:
-            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], args.thumbnail, args.region)),
+            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], args.thumbnail, args.region, args.scale)),
                        thumbnail=args.thumbnail, **extra)
         for p in args.decompress:
-            print(os.path.join(args.output, _png_name(p, args.thumbnail, args.region)))
+            print(os.path.join(args.output, _png_name(p, args.thumbnail, args.region, args.scale)))
     else:
         raise RuntimeError("Illegal state")
 

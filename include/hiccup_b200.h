@@ -176,6 +176,29 @@ int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const
                    int32_t rh, int32_t rw, uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties,
                    uint32_t tie_capacity, uint32_t* d_stats, uint8_t* d_rgb_out, void* stream);
 
+/* Scaled decode -- the 1/s-scale image of each image of the batch, s = scale = 2 or 4 (scale 8 is
+ * hic_dct_thumbnail), m = 8 / s samples per block side.  Every block of the zero-padded planes gives an
+ * m x m tile: X = q T (u, v < m; the block's other coefficients are ignored), A = X B^T (rows first), Y = B A,
+ * each sum left to right in float64 with every product and sum rounded, sample = (uint8)(Y / 256 + 128)
+ * (truncation toward zero, wrap).  B_s[k][0] = 1, B_s[k][n] = 2 D(n) cos(pi n (2k+1) / (2m)),
+ * D(n) = sin(pi n s / 16) / (s sin(pi n / 16)) (hex literals in csrc/hic_core.cuh): B X B^T is the mean of each
+ * s x s tile of the unrounded 8 x 8 IDCT of a block with no coefficients beyond u, v < m.  The tiles form
+ * Y_s (m nby_l x m nbx_l) and Cr_s, Cb_s (m nby_c x m nbx_c); Cr_s and Cb_s go through cv2.pyrUp's integer
+ * rules, and all three are cropped to sh x sw = ceil(out_h / s) x ceil(out_w / s) and converted by
+ * ycrcb_to_rgb into d_rgb_out (n * sh * sw * 3) -- the thumbnail's convention, which is this definition at
+ * m = 1.  The coefficients come from K7's buffer (d_coef, 16-byte aligned), only the first 64 (s = 2) or 16
+ * (s = 4) bytes of each block; a float32 transform with a rigorous error band, whose flagged blocks are
+ * re-evaluated in float64 (tie records carry the global block index), writes the tiles to d_work
+ * (16-byte aligned).  hic_dct_scaled_shape and hic_dct_scaled_sizes (host only) give sh x sw and the d_work
+ * bytes and tie capacity (one record per block).  Every entry point returns HIC_ERR_INVALID for a scale other
+ * than 2 or 4 before anything is launched.  d_stats as for hic_dct_inverse, zeroed by this call; [1] counts
+ * samples re-evaluated. */
+int hic_dct_scaled_shape(int32_t h, int32_t w, int32_t scale, int32_t* sh, int32_t* sw);
+int hic_dct_scaled_sizes(int32_t n, int32_t h, int32_t w, int32_t scale, size_t* work_bytes, uint32_t* tie_capacity);
+int hic_dct_scaled(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32_t scale, uint8_t* d_work,
+                   size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity, uint32_t* d_stats,
+                   uint8_t* d_rgb_out, void* stream);
+
 /* ---- wavelet ("HIC") mode --------------------------------------------------------------------- */
 /* Sub-band geometry of pywt.wavedec2(channel, "db1", level=3) (transform.py:196-209): level sizes
  * ceil(n / 2) per level; ten sub-bands per channel in the order [cA3, cH3, cV3, cD3, cH2, cV2, cD2,

@@ -161,12 +161,18 @@ class _BatchCodec:
     def decode_device(self):
         """D1-D3 and the inverse transform from the encoder's own device-resident output (tables
         and bits are handed over device-to-device)."""
+        self._decode_from_encoder(self.d_coef_dec)
+        self._inverse()
+
+    def _decode_from_encoder(self, d_dst, dc_only=False):
+        """D1-D3 of the encoder's own device-resident output (tables and bits are handed over device-to-device) into
+        d_dst: the coefficient blocks, or with dc_only the DC streams alone, one value per block (EntropyDecoder.run_dc)."""
         st = self.stream
         enc = self.encoder
         d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
         self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
-        self.decoder.run(enc._out.ptr, enc.byte_off, enc.nbits, self.d_coef_dec.ptr, st)
-        self._inverse()
+        run = self.decoder.run_dc if dc_only else self.decoder.run
+        run(enc._out.ptr, enc.byte_off, enc.nbits, d_dst.ptr, st)
 
     # ---- host-to-host entry points -----------------------------------------------------------
     def encode(self, rgb):
@@ -218,17 +224,23 @@ class _BatchCodec:
 
     def fetch(self, out=None):
         """Download the pixels of the last decode_resident()."""
-        count = self.n * self.out_h * self.out_w * 3
+        pixels, self._h_out = self._download(self.d_out, self.out_shape, out, self._h_out)
+        self._after_decode()
+        return pixels
+
+    def _download(self, d_buf, shape, out, staging):
+        """The uint8 array of `shape` at the start of d_buf, downloaded into `out` (a C-contiguous uint8 array of its
+        size) or, without one, into `staging`, page-locked memory the caller keeps (made here when None).  Returns
+        (the array, staging)."""
+        count = int(np.prod(shape))
         if out is None:
-            if self._h_out is None:
-                self._h_out = _lib.PinnedBuffer(count)
-            out = self._h_out.array(np.uint8, count)
+            if staging is None:
+                staging = _lib.PinnedBuffer(count)
+            out = staging.array(np.uint8, count)
         else:
             assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
             out = out.reshape(-1)
-        out = self.d_out.download(np.uint8, count, self.stream, out=out)
-        self._after_decode()
-        return out.reshape(self.out_shape)
+        return d_buf.download(np.uint8, count, self.stream, out=out).reshape(shape), staging
 
     def _after_encode(self):
         pass
@@ -243,6 +255,22 @@ class _BatchCodec:
             if b is not None:
                 b.free()
         self._buffers, self._h_data, self._h_out, self._h_tab, self._h_tab_mem = [], None, None, None, []
+
+
+class _ReducedOutput:
+    """The device buffers of one reduced output of DctBatchCodec (thumbnails, regions or scaled images) for one key,
+    its parameters: the kernels' work area and the output, plus the page-locked staging a fetch without `out` makes."""
+
+    def __init__(self, key, shape, work_bytes, tie_capacity):
+        self.key, self.shape, self.work_bytes, self.tie_capacity = key, shape, work_bytes, tie_capacity
+        self.d_work = _lib.DeviceBuffer(work_bytes)
+        self.d_out = _lib.DeviceBuffer(int(np.prod(shape)))
+        self.h_out = None
+
+    def free(self):
+        for b in (self.d_work, self.d_out, self.h_out):
+            if b is not None:
+                b.free()
 
 
 class DctBatchCodec(_BatchCodec):
@@ -265,6 +293,7 @@ class DctBatchCodec(_BatchCodec):
         self._buffers += [self.d_ties, self.d_stats, self.d_y, self.d_cr, self.d_cb]
         self.forward_stats = np.zeros(4, np.uint32)
         self.inverse_stats = np.zeros(4, np.uint32)
+        self._reduced = {}
 
     def _forward(self):
         _lib.check(self.lib.hic_dct_forward(self.d_rgb.ptr, self.n, self.h, self.w, self.d_coef.ptr, self.d_ties.ptr,
@@ -281,117 +310,95 @@ class DctBatchCodec(_BatchCodec):
     def _after_decode(self):
         self.inverse_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
 
+    # ---- reduced outputs: thumbnails, regions and scaled images -----------------------------------------------------
+    def _reduced_buffers(self, kind, key, sizes):
+        """The buffers of reduced output `kind` for its parameters `key`.  Each kind keeps its own, made on first use (a
+        codec that never asks for one pays nothing) and remade only when its key changes; sizes() gives (output shape,
+        work bytes, tie capacity) for a new key."""
+        r = self._reduced.get(kind)
+        if r is not None and r.key == key:
+            return r
+        if r is not None:
+            self._reduced.pop(kind).free()
+        r = self._reduced[kind] = _ReducedOutput(key, *sizes())
+        return r
+
     # ---- 1/8-scale thumbnails from the DC streams alone (codec.jpeg_thumbnail for the whole batch) ---------------
     @property
     def thumbnail_shape(self):
         th, tw = _lib.thumbnail_shape(self.h, self.w)
         return (self.n, th, tw, 3)
 
-    def _thumb_buffers(self):
-        if getattr(self, "d_dc", None) is None:          # made on first use: a codec that never previews pays nothing
-            self.d_dc = _lib.DeviceBuffer(2 * self.blocks)
-            self.d_thumb = _lib.DeviceBuffer(int(np.prod(self.thumbnail_shape)))
-            self._h_thumb = None
-            self._buffers += [self.d_dc, self.d_thumb]
-        return self.d_dc, self.d_thumb
+    def _thumbnail_buffers(self):
+        """The work area holds the DC values, one int16 per block."""
+        return self._reduced_buffers("thumbnail", None, lambda: (self.thumbnail_shape, 2 * self.blocks, 0))
+
+    def _thumbnail(self, r):
+        _lib.check(self.lib.hic_dct_thumbnail(r.d_work.ptr, self.n, self.h, self.w, r.d_out.ptr, self.stream))
 
     def thumbnails_device(self):
         """DC-only D1 + D3 and the thumbnail kernel from the encoder's own device-resident output (decode_device's
         hand-over); the thumbnails stay on the device (fetch_thumbnails)."""
-        d_dc, d_thumb = self._thumb_buffers()
-        st = self.stream
-        enc = self.encoder
-        d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
-        self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
-        self.decoder.run_dc(enc._out.ptr, enc.byte_off, enc.nbits, d_dc.ptr, st)
-        _lib.check(self.lib.hic_dct_thumbnail(d_dc.ptr, self.n, self.h, self.w, d_thumb.ptr, st))
+        r = self._thumbnail_buffers()
+        self._decode_from_encoder(r.d_work, dc_only=True)
+        self._thumbnail(r)
 
     def thumbnails(self, enc, out=None):
         """Thumbnails of an EncodedStreams (encode() or read_files() / streams_from_files()), host to host: only the
         DC streams' tables and bytes go up, n x th x tw x 3 comes down.  out: optional preallocated uint8 array of
         thumbnail_shape."""
-        d_dc, d_thumb = self._thumb_buffers()
+        r = self._thumbnail_buffers()
         index, symbols, packed, data, byte_off, nbits = entropy.dc_streams_only(enc)
-        self.decoder.decode_dc(index, symbols, packed, data, byte_off, nbits, d_dc.ptr, self.stream)
-        _lib.check(self.lib.hic_dct_thumbnail(d_dc.ptr, self.n, self.h, self.w, d_thumb.ptr, self.stream))
+        self.decoder.decode_dc(index, symbols, packed, data, byte_off, nbits, r.d_work.ptr, self.stream)
+        self._thumbnail(r)
         return self.fetch_thumbnails(out)
 
     def fetch_thumbnails(self, out=None):
         """Download the thumbnails of the last thumbnails() / thumbnails_device()."""
-        _, d_thumb = self._thumb_buffers()
-        count = int(np.prod(self.thumbnail_shape))
-        if out is None:
-            if self._h_thumb is None:
-                self._h_thumb = _lib.PinnedBuffer(count)
-            out = self._h_thumb.array(np.uint8, count)
-        else:
-            assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
-            out = out.reshape(-1)
-        return d_thumb.download(np.uint8, count, self.stream, out=out).reshape(self.thumbnail_shape)
+        r = self._thumbnail_buffers()
+        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
+        return pixels
 
     # ---- regions: one height x width window per image at full resolution (codec.jpeg_region for the whole batch) ----
     def _region_buffers(self, origins, size):
-        """Check the windows (ValueError before any device work) and make the work and output buffers for their size
-        on first use; returns the origins as (n, 2) int32."""
+        """Check the windows (ValueError before any device work); returns the origins as (n, 2) int32 and the buffers
+        for their size."""
         origins = _lib.region_origins(self.h, self.w, origins, size)
         if origins.shape[0] != self.n:
             raise ValueError("%d origins for a batch of %d images" % (origins.shape[0], self.n))
-        size = (int(size[0]), int(size[1]))
-        if getattr(self, "_region_size", None) != size:
-            for b in (getattr(self, "d_region_work", None), getattr(self, "d_region", None), getattr(self, "_h_region", None)):
-                if b is not None:
-                    b.free()
-                    if b in self._buffers:
-                        self._buffers.remove(b)
-            self.region_work_bytes, self.region_tie_capacity = _lib.region_sizes(self.n, self.h, self.w, *size)
-            self.d_region_work = _lib.DeviceBuffer(self.region_work_bytes)
-            self.d_region = _lib.DeviceBuffer(self.n * size[0] * size[1] * 3)
-            self._h_region = None
-            self._buffers += [self.d_region_work, self.d_region]
-            self._region_size = size
-        return origins
+        rh, rw = int(size[0]), int(size[1])
+        return origins, self._reduced_buffers(
+            "region", (rh, rw), lambda: ((self.n, rh, rw, 3),) + _lib.region_sizes(self.n, self.h, self.w, rh, rw))
 
-    def _region(self, origins):
-        rh, rw = self._region_size
+    def _region(self, origins, r):
+        rh, rw = r.key
         _lib.check(self.lib.hic_dct_region(self.d_coef_dec.ptr, self.n, self.h, self.w, origins.ctypes.data, rh, rw,
-                                           self.d_region_work.ptr, self.region_work_bytes, self.d_ties.ptr,
-                                           self.region_tie_capacity, self.d_stats.ptr, self.d_region.ptr, self.stream))
+                                           r.d_work.ptr, r.work_bytes, self.d_ties.ptr, r.tie_capacity, self.d_stats.ptr,
+                                           r.d_out.ptr, self.stream))
 
     def decode_regions_device(self, origins, size):
         """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the windows of
         size = (height, width) at origins ((n, 2) of (top, left)); they stay on the device (fetch_regions)."""
-        origins = self._region_buffers(origins, size)
-        st = self.stream
-        enc = self.encoder
-        d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
-        self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
-        self.decoder.run(enc._out.ptr, enc.byte_off, enc.nbits, self.d_coef_dec.ptr, st)
-        self._region(origins)
+        origins, r = self._region_buffers(origins, size)
+        self._decode_from_encoder(self.d_coef_dec)
+        self._region(origins, r)
 
     def decode_regions(self, enc, origins, size, out=None):
         """Windows of an EncodedStreams, host to host: image i's window is decode(enc)[i, top:top+height,
         left:left+width] with (top, left) = origins[i] and (height, width) = size, bit for bit.  out: optional
         preallocated uint8 array of (n, height, width, 3)."""
-        origins = self._region_buffers(origins, size)
+        origins, r = self._region_buffers(origins, size)
         self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
-        self._region(origins)
+        self._region(origins, r)
         return self.fetch_regions(out)
 
     def fetch_regions(self, out=None):
         """Download the windows of the last decode_regions() / decode_regions_device() (and their tie statistics
         into region_stats)."""
-        rh, rw = self._region_size
-        count = self.n * rh * rw * 3
-        if out is None:
-            if self._h_region is None:
-                self._h_region = _lib.PinnedBuffer(count)
-            out = self._h_region.array(np.uint8, count)
-        else:
-            assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
-            out = out.reshape(-1)
-        out = self.d_region.download(np.uint8, count, self.stream, out=out)
+        r = self._reduced["region"]
+        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
         self.region_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
-        return out.reshape(self.n, rh, rw, 3)
+        return pixels
 
     # ---- 1/2- and 1/4-scale images (codec.jpeg_scaled for the whole batch) ----------------------------------------
     def scaled_shape(self, scale):
@@ -399,68 +406,42 @@ class DctBatchCodec(_BatchCodec):
         return (self.n, sh, sw, 3)
 
     def _scaled_buffers(self, scale):
-        """Check the scale (ValueError before any device work) and make the work and output buffers for it on first
-        use; returns it as an int."""
+        """Check the scale (ValueError before any device work); returns the buffers for it."""
         scale = _lib.scale_arg(scale)
-        if getattr(self, "_scale", None) != scale:
-            for b in (getattr(self, "d_scaled_work", None), getattr(self, "d_scaled", None), getattr(self, "_h_scaled", None)):
-                if b is not None:
-                    b.free()
-                    if b in self._buffers:
-                        self._buffers.remove(b)
-            self.scaled_work_bytes, self.scaled_tie_capacity = _lib.scaled_sizes(self.n, self.h, self.w, scale)
-            self.d_scaled_work = _lib.DeviceBuffer(self.scaled_work_bytes)
-            self.d_scaled = _lib.DeviceBuffer(int(np.prod(self.scaled_shape(scale))))
-            self._h_scaled = None
-            self._buffers += [self.d_scaled_work, self.d_scaled]
-            self._scale = scale
-        return scale
+        return self._reduced_buffers(
+            "scaled", scale, lambda: (self.scaled_shape(scale),) + _lib.scaled_sizes(self.n, self.h, self.w, scale))
 
-    def _scaled(self):
-        _lib.check(self.lib.hic_dct_scaled(self.d_coef_dec.ptr, self.n, self.h, self.w, self._scale, self.d_scaled_work.ptr,
-                                           self.scaled_work_bytes, self.d_ties.ptr, self.scaled_tie_capacity,
-                                           self.d_stats.ptr, self.d_scaled.ptr, self.stream))
+    def _scaled(self, r):
+        _lib.check(self.lib.hic_dct_scaled(self.d_coef_dec.ptr, self.n, self.h, self.w, r.key, r.d_work.ptr, r.work_bytes,
+                                           self.d_ties.ptr, r.tie_capacity, self.d_stats.ptr, r.d_out.ptr, self.stream))
 
     def decode_scaled_device(self, scale):
         """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the 1/scale images;
         they stay on the device (fetch_scaled)."""
-        self._scaled_buffers(scale)
-        st = self.stream
-        enc = self.encoder
-        d_index, d_row_sym, d_row_packed, _, _ = enc.device_tables()
-        self.decoder.set_tables_device(d_index, d_row_sym, d_row_packed, enc.total_rows, st)
-        self.decoder.run(enc._out.ptr, enc.byte_off, enc.nbits, self.d_coef_dec.ptr, st)
-        self._scaled()
+        r = self._scaled_buffers(scale)
+        self._decode_from_encoder(self.d_coef_dec)
+        self._scaled(r)
 
     def decode_scaled(self, enc, scale, out=None):
         """The 1/scale images (scale 2 or 4) of an EncodedStreams, host to host: image i equals
         codec.jpeg_scaled of its file.  out: optional preallocated uint8 array of scaled_shape(scale)."""
-        self._scaled_buffers(scale)
+        r = self._scaled_buffers(scale)
         self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
-        self._scaled()
+        self._scaled(r)
         return self.fetch_scaled(out)
 
     def fetch_scaled(self, out=None):
         """Download the images of the last decode_scaled() / decode_scaled_device() (and their tie statistics into
         scaled_stats)."""
-        shape = self.scaled_shape(self._scale)
-        count = int(np.prod(shape))
-        if out is None:
-            if self._h_scaled is None:
-                self._h_scaled = _lib.PinnedBuffer(count)
-            out = self._h_scaled.array(np.uint8, count)
-        else:
-            assert out.dtype == np.uint8 and out.size == count and out.flags.c_contiguous
-            out = out.reshape(-1)
-        out = self.d_scaled.download(np.uint8, count, self.stream, out=out)
+        r = self._reduced["scaled"]
+        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
         self.scaled_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
-        return out.reshape(shape)
+        return pixels
 
     def close(self):
-        for name in ("_h_thumb", "_h_region", "_h_scaled"):
-            if getattr(self, name, None) is not None:
-                getattr(self, name).free()
-                setattr(self, name, None)
+        for r in self._reduced.values():
+            r.free()
+        self._reduced = {}
         super().close()
 
     def coefficients(self):

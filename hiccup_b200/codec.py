@@ -126,8 +126,7 @@ def _gather_payload_bytes(bit_payloads):
 def _stream_order(hic):
     """File payload index of the table / bit string of every stream s of the entropy stage, (tables, bits);
     None where the stream does not exist (the DC streams of a wavelet file)."""
-    kind_is_jpeg = hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"
-    if kind_is_jpeg:       # reference order is (kind, channel); stream order is s = channel * 3 + kind
+    if _is_dct(hic):       # reference order is (kind, channel); stream order is s = channel * 3 + kind
         order = [kind * 3 + c for c in range(3) for kind in range(3)]
         return order, [9 + i for i in order], 9
     tabs, bits = [], []
@@ -215,26 +214,46 @@ def add_restart_records(hic: hicimage.HicImage) -> hicimage.HicImage:
     return hicimage.HicImage(hic.hic_type, hic.settings, list(p), others + [ext])
 
 
-def jpeg_decode(hic: hicimage.HicImage) -> model.CompressedImage:
-    settings.check_supported()
-    _lib.require_device()
-    assert hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"
+def _is_dct(hic):
+    return hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"
+
+
+def _require_dct(hic, what):
+    if not _is_dct(hic):
+        raise NotImplementedError("%s works on DCT-mode (JPEG) files; this is a wavelet (HIC) file" % what)
+
+
+def _dct_header(hic):
+    """(payloads, h, w, geometry) of a DCT-mode file; ValueError when its chroma shape does not belong to its luminance
+    shape."""
     p = hic.payloads
     lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
     h, w = int(lum_shape[0]), int(lum_shape[1])
     g = _lib.geometry(h, w)
     if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
         raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
-    # reorder the reference's (kind, channel) payload order into stream order s = channel * 3 + kind
-    order = [kind * 3 + c for c in range(3) for kind in range(3)]
-    rows, syms, lens, codes = _tables_to_arrays([p[i] for i in order])
-    data, offs, nbits = _gather_payload_bytes([p[9 + i] for i in order])
-    layout = _lib.layout_dct(1, h, w)
+    return p, h, w, g
+
+
+def _decode_coefficients(hic, h, w, d_coef):
+    """D1-D3 of all nine streams of a DCT-mode file into d_coef ([blocks][64] int16), with the file's restart records
+    when they fit."""
+    p = hic.payloads
+    tabs, bits, _ = _stream_order(hic)
+    rows, syms, lens, codes = _tables_to_arrays([p[i] for i in tabs])
+    data, offs, nbits = _gather_payload_bytes([p[i] for i in bits])
+    _entropy_decode(entropy.cached_decoder(_lib.layout_dct(1, h, w)), hic, rows, syms, lens, codes, data, offs, nbits, d_coef)
+
+
+def jpeg_decode(hic: hicimage.HicImage) -> model.CompressedImage:
+    settings.check_supported()
+    _lib.require_device()
+    assert _is_dct(hic)
+    _, h, w, g = _dct_header(hic)
     coef = _lib.scratch(g.blocks_per_image * 128)
-    dec = entropy.cached_decoder(layout)
     lib = _lib.load()
     try:
-        _entropy_decode(dec, hic, rows, syms, lens, codes, data, offs, nbits, coef.ptr)
+        _decode_coefficients(hic, h, w, coef.ptr)
         lum = _lib.scratch(4 * h * w)
         cr = _lib.scratch(4 * g.hc * g.wc)
         cb = _lib.scratch(4 * g.hc * g.wc)
@@ -255,17 +274,11 @@ def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
     compression.jpeg_decompression return (th = ceil(out_h / 8)), from the three DC streams alone (hic_dct_thumbnail).
     Only the DC tables and DC bit strings go to the device; the file's restart records of the DC streams are used
     when it has them."""
-    if not (hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"):
-        raise NotImplementedError("thumbnails come from the DC streams of a DCT-mode (JPEG) file; a wavelet (HIC) file has "
-                                  "none -- its coarse band would need a prefix decode of the value and length streams")
+    # a wavelet file has no DC streams: its coarse band would need a prefix decode of the value and length streams
+    _require_dct(hic, "thumbnail decode")
     settings.check_supported()
     _lib.require_device()
-    p = hic.payloads
-    lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
-    h, w = int(lum_shape[0]), int(lum_shape[1])
-    g = _lib.geometry(h, w)
-    if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
-        raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
+    p, h, w, g = _dct_header(hic)
     # stream order s = channel * 3 + kind; the DC table / bit string of channel c is payload c / 9 + c
     rows, syms, lens, codes = _tables_to_arrays([p[c] for c in range(3)])
     index = np.zeros((9, 2), np.uint32)
@@ -289,40 +302,37 @@ def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
         out.free()
 
 
+def _reduced_decode(hic, h, w, g, launch, params, sizes, shape):
+    """jpeg_decode's entropy stage into a coefficient buffer, then `launch` -- hic_dct_region or hic_dct_scaled, called as
+    (coef, 1, h, w, *params, work, work bytes, ties, tie capacity, stats, out, stream) with the (work bytes, tie capacity)
+    of `sizes` -- into a uint8 image of `shape`, which is returned."""
+    work_bytes, tie_cap = sizes
+    bufs = [_lib.scratch(g.blocks_per_image * 128), _lib.scratch(work_bytes), _lib.scratch(tie_cap * _lib.TIE_RECORD_BYTES),
+            _lib.scratch(4 * _lib.TIE_STATS), _lib.scratch(int(np.prod(shape)))]
+    coef, work, ties, stats, out = bufs
+    try:
+        _decode_coefficients(hic, h, w, coef.ptr)
+        _lib.check(launch(coef.ptr, 1, h, w, *params, work.ptr, work_bytes, ties.ptr, tie_cap, stats.ptr, out.ptr, None))
+        return out.download(np.uint8, int(np.prod(shape))).reshape(shape)
+    finally:
+        for b in bufs:
+            b.free()
+
+
 def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int) -> np.ndarray:
     """One window of a DCT-mode file at full resolution: (height, width, 3) uint8, equal to
     compression.jpeg_decompression(jpeg_decode(hic))[top:top+height, left:left+width] bit for bit.  The entropy
     decode is jpeg_decode's (restart records used when the file has them); then only the blocks the window reads are
     inverse-transformed and only its pixels upsampled and converted (hic_dct_region).  ValueError for a window
     outside the decoded image, NotImplementedError for a wavelet file, both before any device work."""
-    if not (hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"):
-        raise NotImplementedError("region decode works on DCT-mode (JPEG) files; this is a wavelet (HIC) file")
-    p = hic.payloads
-    lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
-    h, w = int(lum_shape[0]), int(lum_shape[1])
-    g = _lib.geometry(h, w)
-    if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
-        raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
+    _require_dct(hic, "region decode")
+    _, h, w, g = _dct_header(hic)
     origin = _lib.region_origins(h, w, [(top, left)], (height, width))
     settings.check_supported()
     _lib.require_device()
-    work_bytes, tie_cap = _lib.region_sizes(1, h, w, height, width)
-    order = [kind * 3 + c for c in range(3) for kind in range(3)]
-    rows, syms, lens, codes = _tables_to_arrays([p[i] for i in order])
-    data, offs, nbits = _gather_payload_bytes([p[9 + i] for i in order])
-    dec = entropy.cached_decoder(_lib.layout_dct(1, h, w))
-    lib = _lib.load()
-    bufs = [_lib.scratch(g.blocks_per_image * 128), _lib.scratch(work_bytes), _lib.scratch(tie_cap * _lib.TIE_RECORD_BYTES),
-            _lib.scratch(4 * _lib.TIE_STATS), _lib.scratch(3 * int(height) * int(width))]
-    coef, work, ties, stats, out = bufs
-    try:
-        _entropy_decode(dec, hic, rows, syms, lens, codes, data, offs, nbits, coef.ptr)
-        _lib.check(lib.hic_dct_region(coef.ptr, 1, h, w, origin.ctypes.data, int(height), int(width), work.ptr, work_bytes,
-                                      ties.ptr, tie_cap, stats.ptr, out.ptr, None))
-        return out.download(np.uint8, 3 * int(height) * int(width)).reshape(int(height), int(width), 3)
-    finally:
-        for b in bufs:
-            b.free()
+    height, width = int(height), int(width)
+    return _reduced_decode(hic, h, w, g, _lib.load().hic_dct_region, (origin.ctypes.data, height, width),
+                           _lib.region_sizes(1, h, w, height, width), (height, width, 3))
 
 
 def jpeg_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
@@ -332,35 +342,13 @@ def jpeg_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
     hic_dct_scaled; the chroma planes are upsampled and converted with the full decode's integer rules.  The
     entropy decode is jpeg_decode's (restart records used when the file has them).  ValueError for a scale other
     than 2 or 4 (1/8 is jpeg_thumbnail), NotImplementedError for a wavelet file, both before any device work."""
-    if not (hic.hic_type == model.Compression.JPEG or getattr(hic.hic_type, "value", None) == "JPEG"):
-        raise NotImplementedError("scaled decode works on DCT-mode (JPEG) files; this is a wavelet (HIC) file")
+    _require_dct(hic, "scaled decode")
     scale = _lib.scale_arg(scale)
-    p = hic.payloads
-    lum_shape, cr_shape = tuple(p[18].numbers), tuple(p[19].numbers)
-    h, w = int(lum_shape[0]), int(lum_shape[1])
-    g = _lib.geometry(h, w)
-    if (g.hc, g.wc) != (int(cr_shape[0]), int(cr_shape[1])):
-        raise ValueError("chroma shape %r does not belong to luminance shape %r" % (cr_shape, lum_shape))
+    _, h, w, g = _dct_header(hic)
     settings.check_supported()
     _lib.require_device()
-    sh, sw = _lib.scaled_shape(h, w, scale)
-    work_bytes, tie_cap = _lib.scaled_sizes(1, h, w, scale)
-    order = [kind * 3 + c for c in range(3) for kind in range(3)]
-    rows, syms, lens, codes = _tables_to_arrays([p[i] for i in order])
-    data, offs, nbits = _gather_payload_bytes([p[9 + i] for i in order])
-    dec = entropy.cached_decoder(_lib.layout_dct(1, h, w))
-    lib = _lib.load()
-    bufs = [_lib.scratch(g.blocks_per_image * 128), _lib.scratch(work_bytes), _lib.scratch(tie_cap * _lib.TIE_RECORD_BYTES),
-            _lib.scratch(4 * _lib.TIE_STATS), _lib.scratch(3 * sh * sw)]
-    coef, work, ties, stats, out = bufs
-    try:
-        _entropy_decode(dec, hic, rows, syms, lens, codes, data, offs, nbits, coef.ptr)
-        _lib.check(lib.hic_dct_scaled(coef.ptr, 1, h, w, scale, work.ptr, work_bytes, ties.ptr, tie_cap, stats.ptr, out.ptr,
-                                      None))
-        return out.download(np.uint8, 3 * sh * sw).reshape(sh, sw, 3)
-    finally:
-        for b in bufs:
-            b.free()
+    return _reduced_decode(hic, h, w, g, _lib.load().hic_dct_scaled, (scale,), _lib.scaled_sizes(1, h, w, scale),
+                           _lib.scaled_shape(h, w, scale) + (3,))
 
 
 def wavelet_encode(compressed: model.CompressedImage, restarts: bool = False) -> hicimage.HicImage:

@@ -1607,6 +1607,47 @@ static int tensor_map_encoder(EncodeTiledFn* out) {
     return HIC_OK;
 }
 
+// The decode entries' shared checks: n >= 1 images of h x w and (block_limit) a block count that fits 32-bit indices
+static int batch_geometry(int32_t n, int32_t h, int32_t w, bool block_limit, hic_dct_geometry* g) {
+    HIC_REQUIRE(n >= 1, "batch size must be positive");
+    const int rc = geometry_of(h, w, g);
+    if (rc) return rc;
+    if (block_limit) HIC_REQUIRE((int64_t)n * g->blocks_per_image < (1ll << 32), "batch too large: %lld blocks", (long long)n * g->blocks_per_image);
+    return HIC_OK;
+}
+
+// K7's [block][64 int16] view of the coefficient buffer; a box is the first box_cols entries of box_rows blocks
+static int coef_block_map(CUtensorMap* map, const int16_t* d_coef, int64_t blocks, cuuint32_t box_cols, cuuint32_t box_rows,
+                          CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2) {
+    EncodeTiledFn encode = nullptr;
+    const int rc = tensor_map_encoder(&encode);
+    if (rc) return rc;
+    const cuuint64_t dims[2] = {64, (cuuint64_t)blocks};
+    const cuuint64_t strides[1] = {128};
+    const cuuint32_t box[2] = {box_cols, box_rows};
+    const cuuint32_t estr[2] = {1, 1};
+    const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, const_cast<int16_t*>(d_coef), dims, strides, box, estr,
+                              CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return hic::fail(HIC_ERR_CUDA, "cuTensorMapEncodeTiled (coefficient blocks) failed: %d", (int)r);
+    return HIC_OK;
+}
+
+// K7S, its fix-up and K8S of hic_dct_scaled for M x M samples per block (scale 8 / M)
+template <int M>
+static int scaled_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, int sh, int sw, uint8_t* d_work,
+                         hic_tie_record* d_ties, uint32_t tie_capacity, uint32_t* d_stats, uint8_t* d_rgb_out, cudaStream_t st) {
+    const int64_t blocks = (int64_t)n * g.blocks_per_image;
+    CUtensorMap tmap_blocks;
+    const int rc = coef_block_map(&tmap_blocks, d_coef, blocks, M == 4 ? 32u : 8u, k7::K7S_THREADS,
+                                  M == 4 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+    if (rc) return rc;
+    const unsigned grid_inv = grid_for(blocks, k7::K7S_THREADS), grid_rgb = grid_for((int64_t)n * ((sh + 1) / 2) * ((sw + 1) / 2), 256);
+    HIC_LAUNCH("scaled_inverse_kernel", st, k7::scaled_inverse_kernel<M><<<grid_inv, k7::K7S_THREADS, 0, st>>>(tmap_blocks, g, n, d_work, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH("scaled_fixup_kernel", st, k7::scaled_fixup_kernel<M><<<148 * 4, 128, 0, st>>>(d_coef, g, d_work, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH("scaled_colour_kernel", st, k7::scaled_colour_kernel<M><<<grid_rgb, 256, 0, st>>>(d_work, g, n, sh, sw, d_rgb_out));
+    return HIC_OK;
+}
+
 }  // namespace hic
 
 // ------------------------------------------------------------------------------------------------
@@ -1719,9 +1760,8 @@ int hic_blocks_to_planes(const int16_t* d_coef, int32_t n, int32_t h, int32_t w,
                          int32_t* d_cb, void* stream) {
     using namespace hic;
     HIC_REQUIRE(d_coef && d_lum && d_cr && d_cb, "NULL device pointer");
-    HIC_REQUIRE(n >= 1, "batch size must be positive");
     hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
+    const int rc = batch_geometry(n, h, w, false, &g);
     if (rc) return rc;
     const int64_t items = (int64_t)n * g.blocks_per_image * 64;
     cudaStream_t st = as_stream(stream);
@@ -1733,9 +1773,8 @@ int hic_planes_to_blocks(const int32_t* d_lum, const int32_t* d_cr, const int32_
                          int32_t w, int16_t* d_coef, void* stream) {
     using namespace hic;
     HIC_REQUIRE(d_coef && d_lum && d_cr && d_cb, "NULL device pointer");
-    HIC_REQUIRE(n >= 1, "batch size must be positive");
     hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
+    const int rc = batch_geometry(n, h, w, false, &g);
     if (rc) return rc;
     const int64_t items = (int64_t)n * g.blocks_per_image * 64;
     cudaStream_t st = as_stream(stream);
@@ -1748,11 +1787,9 @@ int hic_dct_inverse(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, uint
                     uint32_t* d_stats, void* stream) {
     using namespace hic;
     HIC_REQUIRE(d_coef && d_y && d_cr && d_cb && d_rgb_out && d_ties && d_stats, "NULL device pointer");
-    HIC_REQUIRE(n >= 1, "batch size must be positive");
     hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
+    int rc = batch_geometry(n, h, w, true, &g);
     if (rc) return rc;
-    HIC_REQUIRE((int64_t)n * g.blocks_per_image < (1ll << 32), "batch too large: %lld blocks", (long long)n * g.blocks_per_image);
     rc = ensure_tables();
     if (rc) return rc;
     cudaStream_t st = as_stream(stream);
@@ -1760,19 +1797,8 @@ int hic_dct_inverse(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, uint
     const int64_t blocks = (int64_t)n * g.blocks_per_image;
     HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 127) == 0, "d_coef must be 128-byte aligned");
     CUtensorMap tmap_blocks;
-    {
-        EncodeTiledFn encode = nullptr;
-        rc = tensor_map_encoder(&encode);
-        if (rc) return rc;
-        const cuuint64_t dims[2] = {64, (cuuint64_t)blocks};
-        const cuuint64_t strides[1] = {128};
-        const cuuint32_t box[2] = {64, (cuuint32_t)k7::K7_THREADS};
-        const cuuint32_t estr[2] = {1, 1};
-        const CUresult r = encode(&tmap_blocks, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, const_cast<int16_t*>(d_coef), dims, strides, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return hic::fail(HIC_ERR_CUDA, "cuTensorMapEncodeTiled (coefficient blocks) failed: %d", (int)r);
-    }
+    rc = coef_block_map(&tmap_blocks, d_coef, blocks, 64, k7::K7_THREADS, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    if (rc) return rc;
     HIC_LAUNCH("inverse_kernel", st, k7::inverse_kernel<<<grid_for(blocks, k7::K7_THREADS), k7::K7_THREADS, 0, st>>>(tmap_blocks, g, n, d_y, d_cr, d_cb, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("inverse_fixup_kernel", st, k7::inverse_fixup_kernel<<<148 * 4, 128, 0, st>>>(d_coef, g, d_y, d_cr, d_cb, d_ties, tie_capacity, d_stats));
     const int64_t quads = (int64_t)n * g.hc * g.wc;
@@ -1800,9 +1826,8 @@ int hic_dct_thumbnail_shape(int32_t h, int32_t w, int32_t* th, int32_t* tw) {
 int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint8_t* d_rgb_out, void* stream) {
     using namespace hic;
     HIC_REQUIRE(d_dc && d_rgb_out, "NULL device pointer");
-    HIC_REQUIRE(n >= 1, "batch size must be positive");
     hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
+    int rc = batch_geometry(n, h, w, false, &g);
     if (rc) return rc;
     int32_t th = 0, tw = 0;
     rc = hic_dct_thumbnail_shape(h, w, &th, &tw);
@@ -1832,9 +1857,8 @@ int hic_dct_region_blocks(int32_t h, int32_t w, int32_t top, int32_t left, int32
 int hic_dct_region_sizes(int32_t n, int32_t h, int32_t w, int32_t rh, int32_t rw, size_t* work_bytes, uint32_t* tie_capacity) {
     using namespace hic;
     HIC_REQUIRE(work_bytes && tie_capacity, "NULL argument");
-    HIC_REQUIRE(n >= 1, "batch size must be positive");
     hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
+    int rc = batch_geometry(n, h, w, false, &g);
     if (rc) return rc;
     rc = region_check(g, 0, 0, rh, rw);
     if (rc) return rc;
@@ -1850,11 +1874,9 @@ int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const
                    uint32_t* d_stats, uint8_t* d_rgb_out, void* stream) {
     using namespace hic;
     HIC_REQUIRE(d_coef && h_origin && d_work && d_ties && d_stats && d_rgb_out, "NULL pointer");
-    HIC_REQUIRE(n >= 1, "batch size must be positive");
     hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
+    int rc = batch_geometry(n, h, w, true, &g);
     if (rc) return rc;
-    HIC_REQUIRE((int64_t)n * g.blocks_per_image < (1ll << 32), "batch too large: %lld blocks", (long long)n * g.blocks_per_image);
     for (int i = 0; i < n; ++i) {
         rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw);
         if (rc) return rc;
@@ -1924,40 +1946,17 @@ int hic_dct_scaled(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32
     HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
                 "d_coef and d_work must be 16-byte aligned");
     hic_dct_geometry g;
-    geometry_of(h, w, &g);
+    rc = batch_geometry(n, h, w, false, &g);
+    if (rc) return rc;
     int32_t sh = 0, sw = 0;
-    hic_dct_scaled_shape(h, w, scale, &sh, &sw);
+    rc = hic_dct_scaled_shape(h, w, scale, &sh, &sw);
+    if (rc) return rc;
     rc = ensure_tables();
     if (rc) return rc;
     cudaStream_t st = as_stream(stream);
     HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
-    const int64_t blocks = (int64_t)n * g.blocks_per_image;
-    // K7's [block][64 int16] view of the coefficient buffer; the box takes the first 32 (M = 4) or 8 (M = 2) entries
-    CUtensorMap tmap_blocks;
-    {
-        EncodeTiledFn encode = nullptr;
-        rc = tensor_map_encoder(&encode);
-        if (rc) return rc;
-        const cuuint64_t dims[2] = {64, (cuuint64_t)blocks};
-        const cuuint64_t strides[1] = {128};
-        const cuuint32_t box[2] = {scale == 2 ? 32u : 8u, (cuuint32_t)k7::K7S_THREADS};
-        const cuuint32_t estr[2] = {1, 1};
-        const CUresult r = encode(&tmap_blocks, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, const_cast<int16_t*>(d_coef), dims, strides, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, scale == 2 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE,
-                                  CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return hic::fail(HIC_ERR_CUDA, "cuTensorMapEncodeTiled (coefficient blocks) failed: %d", (int)r);
-    }
-    const unsigned grid_inv = grid_for(blocks, k7::K7S_THREADS), grid_rgb = grid_for((int64_t)n * ((sh + 1) / 2) * ((sw + 1) / 2), 256);
-    if (scale == 2) {
-        HIC_LAUNCH("scaled_inverse_kernel", st, k7::scaled_inverse_kernel<4><<<grid_inv, k7::K7S_THREADS, 0, st>>>(tmap_blocks, g, n, d_work, d_ties, tie_capacity, d_stats));
-        HIC_LAUNCH("scaled_fixup_kernel", st, k7::scaled_fixup_kernel<4><<<148 * 4, 128, 0, st>>>(d_coef, g, d_work, d_ties, tie_capacity, d_stats));
-        HIC_LAUNCH("scaled_colour_kernel", st, k7::scaled_colour_kernel<4><<<grid_rgb, 256, 0, st>>>(d_work, g, n, sh, sw, d_rgb_out));
-    } else {
-        HIC_LAUNCH("scaled_inverse_kernel", st, k7::scaled_inverse_kernel<2><<<grid_inv, k7::K7S_THREADS, 0, st>>>(tmap_blocks, g, n, d_work, d_ties, tie_capacity, d_stats));
-        HIC_LAUNCH("scaled_fixup_kernel", st, k7::scaled_fixup_kernel<2><<<148 * 4, 128, 0, st>>>(d_coef, g, d_work, d_ties, tie_capacity, d_stats));
-        HIC_LAUNCH("scaled_colour_kernel", st, k7::scaled_colour_kernel<2><<<grid_rgb, 256, 0, st>>>(d_work, g, n, sh, sw, d_rgb_out));
-    }
-    return HIC_OK;
+    return scale == 2 ? scaled_launch<4>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st)
+                      : scaled_launch<2>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st);
 }
 
 }  // extern "C"

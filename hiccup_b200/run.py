@@ -16,11 +16,12 @@ are interchangeable with the reference's in both directions.  Command line: pyth
 -c IMG... | -d HIC... [-t | --region T,L,H,W | --scale 2|4] [-s JPEG|HIC] [-o OUT] [-r], the subset of bin/belch.py:26-49 that does not need a display.
 """
 import argparse
+import collections
 import os
 
 import numpy as np
 
-from hiccup_b200 import codec, compression, hicimage, model
+from hiccup_b200 import _lib, codec, compression, hicimage, model
 
 
 def img_name(path, c):
@@ -50,39 +51,49 @@ def compress(path, output, c=model.Compression.JPEG, restarts=False):
     return out
 
 
-def _no_wavelet_thumbnails(path):
-    raise NotImplementedError("%s is a wavelet (HIC) file: thumbnails come from the DC streams of DCT-mode (JPEG) files, "
-                              "and wavelet files have none" % (path,))
+class _Output(collections.namedtuple("_Output", "suffix reduced decode decode_batch window")):
+    """What decompress() and decompress_many() make of each file: the PNG name suffix, the name of the reduced decode
+    (None for the full one), the single-file decode (HicImage -> pixels), the batch decode ((codec, EncodedStreams) ->
+    pixels) and the region's ((top, left), (height, width)) or None."""
+
+    def check(self, path, mode, shape=None):
+        """NotImplementedError for a wavelet file asked for a reduced decode; ValueError for an image of `shape` that
+        does not hold the window."""
+        if self.reduced and mode != model.Compression.JPEG:
+            raise NotImplementedError("%s is a wavelet (HIC) file: %s works on DCT-mode (JPEG) files" % (path, self.reduced))
+        if self.window is not None and shape is not None:
+            _lib.region_origins(*shape, [self.window[0]], self.window[1])
 
 
-def _no_wavelet_regions(path):
-    raise NotImplementedError("%s is a wavelet (HIC) file: region decode works on DCT-mode (JPEG) files" % (path,))
+def _decode(hi):
+    if hi.hic_type == model.Compression.JPEG:
+        return compression.jpeg_decompression(codec.jpeg_decode(hi))
+    if hi.hic_type == model.Compression.HIC:
+        return compression.wavelet_decompression(codec.wavelet_decode(hi))
+    raise RuntimeError("Unknown compression type")
 
 
-def _region_args(region, thumbnail):
-    """region as ((top, left), (height, width)), or None; ValueError for a malformed one or one combined with thumbnail."""
-    if region is None:
-        return None
+def _output(thumbnail=False, region=None, scale=None):
+    """The _Output for these options; ValueError for a malformed region, a scale other than 2 or 4, or more than one
+    of thumbnail, region and scale."""
+    if bool(thumbnail) + (region is not None) + (scale is not None) > 1:
+        raise ValueError("thumbnail, region and scale do not go together: choose one")
+    if region is not None:
+        r = tuple(region)
+        if len(r) != 4 or not all(isinstance(v, (int, np.integer)) for v in r):
+            raise ValueError("region must be four integers (top, left, height, width), got %r" % (region,))
+        top, left, height, width = (int(v) for v in r)
+        origin = np.array([[top, left]], np.int32)
+        return _Output(".region.png", "region decode", lambda hi: codec.jpeg_region(hi, top, left, height, width),
+                       lambda bc, enc: bc.decode_regions(enc, np.tile(origin, (bc.n, 1)), (height, width)),
+                       ((top, left), (height, width)))
+    if scale is not None:
+        scale = _lib.scale_arg(scale)
+        return _Output(".s%d.png" % scale, "scaled decode", lambda hi: codec.jpeg_scaled(hi, scale),
+                       lambda bc, enc: bc.decode_scaled(enc, scale), None)
     if thumbnail:
-        raise ValueError("region and thumbnail do not go together")
-    r = tuple(region)
-    if len(r) != 4 or not all(isinstance(v, (int, np.integer)) for v in r):
-        raise ValueError("region must be four integers (top, left, height, width), got %r" % (region,))
-    return (int(r[0]), int(r[1])), (int(r[2]), int(r[3]))
-
-
-def _no_wavelet_scaled(path):
-    raise NotImplementedError("%s is a wavelet (HIC) file: scaled decode works on DCT-mode (JPEG) files" % (path,))
-
-
-def _scale_args(scale, thumbnail, region):
-    """scale as an int (2 or 4), or None; ValueError for another value or one combined with thumbnail or region."""
-    if scale is None:
-        return None
-    if thumbnail or region is not None:
-        raise ValueError("scale does not go with thumbnail or region")
-    from hiccup_b200 import _lib
-    return _lib.scale_arg(scale)
+        return _Output(".thumb.png", "thumbnail decode", codec.jpeg_thumbnail, lambda bc, enc: bc.thumbnails(enc), None)
+    return _Output(".png", None, _decode, lambda bc, enc: bc.decode(enc), None)
 
 
 def decompress(path, save=None, thumbnail=False, region=None, scale=None):
@@ -92,27 +103,10 @@ def decompress(path, save=None, thumbnail=False, region=None, scale=None):
     the image does not hold ValueError, before anything is decoded or written.  scale=2 or 4: the 1/2- or 1/4-scale
     image of a DCT-mode file (codec.jpeg_scaled); a wavelet file raises NotImplementedError and another scale
     ValueError, before anything is decoded or written."""
-    win = _region_args(region, thumbnail)
-    scale = _scale_args(scale, thumbnail, region)
+    what = _output(thumbnail, region, scale)
     hi = hicimage.HicImage.from_file(path)
-    if scale is not None:
-        if hi.hic_type != model.Compression.JPEG:
-            _no_wavelet_scaled(path)
-        rgb = codec.jpeg_scaled(hi, scale)
-    elif win is not None:
-        if hi.hic_type != model.Compression.JPEG:
-            _no_wavelet_regions(path)
-        rgb = codec.jpeg_region(hi, *win[0], *win[1])
-    elif thumbnail:
-        if hi.hic_type != model.Compression.JPEG:
-            _no_wavelet_thumbnails(path)
-        rgb = codec.jpeg_thumbnail(hi)
-    elif hi.hic_type == model.Compression.JPEG:
-        rgb = compression.jpeg_decompression(codec.jpeg_decode(hi))
-    elif hi.hic_type == model.Compression.HIC:
-        rgb = compression.wavelet_decompression(codec.wavelet_decode(hi))
-    else:
-        raise RuntimeError("Unknown compression type")
+    what.check(path, hi.hic_type)
+    rgb = what.decode(hi)
     if save is not None:
         import cv2
         cv2.imwrite(save, rgb)
@@ -170,23 +164,14 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region
     wavelet file, or a file whose image does not hold the window, raises before anything is decoded or written.
     scale=2 or 4: the 1/2- or 1/4-scale image of every file (DctBatchCodec.decode_scaled, <name>.s2.png / <name>.s4.png);
     a wavelet file or another scale raises before anything is decoded or written."""
-    from hiccup_b200 import _lib
     from hiccup_b200.batch import DctBatchCodec, WaveletBatchCodec
-    win = _region_args(region, thumbnail)
-    scale = _scale_args(scale, thumbnail, region)
+    what = _output(thumbnail, region, scale)
     groups, out = {}, [None] * len(paths)
     for i, p in enumerate(paths):
         with open(p, "rb") as f:
             raw = f.read()
         key = _peek(raw)
-        if thumbnail and key[0] != model.Compression.JPEG:
-            _no_wavelet_thumbnails(p)
-        if win is not None:
-            if key[0] != model.Compression.JPEG:
-                _no_wavelet_regions(p)
-            _lib.region_origins(*key[1], [win[0]], win[1])
-        if scale is not None and key[0] != model.Compression.JPEG:
-            _no_wavelet_scaled(p)
+        what.check(p, *key)
         groups.setdefault(key, []).append((i, raw))
     for (mode, (h, w)), items in groups.items():
         cls = DctBatchCodec if mode == model.Compression.JPEG else WaveletBatchCodec
@@ -194,15 +179,7 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region
             part = items[a:a + max_batch]
             bc = cls(len(part), h, w)
             try:
-                enc = bc.streams_from_files([raw for _, raw in part])
-                if scale is not None:
-                    pixels = bc.decode_scaled(enc, scale)
-                elif win is not None:
-                    pixels = bc.decode_regions(enc, np.tile(np.asarray(win[0], np.int32), (len(part), 1)), win[1])
-                elif thumbnail:
-                    pixels = bc.thumbnails(enc)
-                else:
-                    pixels = bc.decode(enc)
+                pixels = what.decode_batch(bc, bc.streams_from_files([raw for _, raw in part]))
                 for (i, _), rgb in zip(part, pixels):
                     out[i] = rgb.copy()
             finally:
@@ -210,14 +187,12 @@ def decompress_many(paths, save_dir=None, max_batch=256, thumbnail=False, region
     if save_dir is not None:
         import cv2
         for p, rgb in zip(paths, out):
-            cv2.imwrite(os.path.join(save_dir, _png_name(p, thumbnail, region, scale)), rgb)
+            cv2.imwrite(os.path.join(save_dir, _png_name(p, what)), rgb)
     return out
 
 
-def _png_name(path, thumbnail, region=None, scale=None):
-    if scale is not None:
-        return os.path.split(path)[-1] + ".s%d.png" % scale
-    return os.path.split(path)[-1] + (".region.png" if region is not None else ".thumb.png" if thumbnail else ".png")
+def _png_name(path, what):
+    return os.path.split(path)[-1] + what.suffix
 
 
 def _parse_region(text):
@@ -247,32 +222,26 @@ def main(argv=None):
     ap.add_argument("--scale", type=int, choices=(2, 4),
                     help="with -d: write the 1/2- or 1/4-scale image of each DCT-mode file (<name>.s2.png / <name>.s4.png)")
     args = ap.parse_args(argv)
-    if args.thumbnail and not args.decompress:
-        ap.error("-t/--thumbnail goes with -d/--decompress")
-    if args.region is not None and not args.decompress:
-        ap.error("--region goes with -d/--decompress")
-    if args.region is not None and args.thumbnail:
-        ap.error("--region does not go with -t/--thumbnail")
-    if args.scale is not None and not args.decompress:
-        ap.error("--scale goes with -d/--decompress")
-    if args.scale is not None and (args.thumbnail or args.region is not None):
-        ap.error("--scale does not go with -t/--thumbnail or --region")
+    if (args.thumbnail or args.region is not None or args.scale is not None) and not args.decompress:
+        ap.error("-t/--thumbnail, --region and --scale go with -d/--decompress")
+    try:
+        what = _output(args.thumbnail, args.region, args.scale)
+    except ValueError as e:
+        ap.error(str(e))
     style = model.Compression(args.compression)
     if args.compress:
         for out in (compress_many(args.compress, args.output, style, restarts=args.restarts) if len(args.compress) > 1
                     else [compress(args.compress[0], args.output, style, restarts=args.restarts)]):
             print(out)
     elif args.decompress:
-        extra = {} if args.region is None else {"region": args.region}
-        if args.scale is not None:
-            extra["scale"] = args.scale
+        extra = {k: v for k, v in (("region", args.region), ("scale", args.scale)) if v is not None}
         if len(args.decompress) > 1:
             decompress_many(args.decompress, save_dir=args.output, thumbnail=args.thumbnail, **extra)
         else:
-            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], args.thumbnail, args.region, args.scale)),
+            decompress(args.decompress[0], save=os.path.join(args.output, _png_name(args.decompress[0], what)),
                        thumbnail=args.thumbnail, **extra)
         for p in args.decompress:
-            print(os.path.join(args.output, _png_name(p, args.thumbnail, args.region, args.scale)))
+            print(os.path.join(args.output, _png_name(p, what)))
     else:
         raise RuntimeError("Illegal state")
 

@@ -165,6 +165,13 @@ SIGNATURES = {
     "hic_dct_scaled_sizes": (c_int, [c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_size_t), ctypes.POINTER(c_uint32)]),
     "hic_dct_scaled": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_size_t, c_void_p, c_uint32, c_void_p,
                                c_void_p, c_void_p]),
+    "hic_dct_scaled_region_blocks": (c_int, [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_int32)]),
+    "hic_dct_scaled_region_sizes": (c_int, [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, ctypes.POINTER(c_size_t),
+                                            ctypes.POINTER(c_uint32)]),
+    "hic_dct_scaled_region": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_size_t,
+                                      c_void_p, c_uint32, c_void_p, c_void_p, c_void_p]),
+    "hic_dct_thumbnail_region": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_size_t,
+                                         c_void_p, c_void_p]),
 }
 
 _lock = threading.Lock()
@@ -239,10 +246,14 @@ def region_sizes(n, h, w, rh, rw):
     return int(work.value), int(cap.value)
 
 
-def region_origins(h, w, origins, size):
+def region_origins(h, w, origins, size, scale=1):
     """Check windows of size = (rh, rw) at origins ((n, 2) (top, left)) against the h x w image's decoded output
-    (out_h x out_w) on the host: the origins as a contiguous (n, 2) int32 array, or ValueError."""
+    (out_h x out_w), or with scale 2, 4 or 8 against its 1/scale image (ceil(out_h / scale) x ceil(out_w / scale)), on
+    the host: the origins as a contiguous (n, 2) int32 array, or ValueError."""
     g = geometry(h, w)
+    scale = region_scale_arg(scale)
+    ih, iw = (g.out_h, g.out_w) if scale == 1 else (-(-g.out_h // scale), -(-g.out_w // scale))
+    what = "decoded image" if scale == 1 else "1/%d-scale image" % scale
     rh, rw = (int(v) for v in size)
     o = np.asarray(origins)
     if o.ndim != 2 or o.shape[1] != 2 or o.shape[0] < 1 or not np.issubdtype(o.dtype, np.integer):
@@ -250,12 +261,34 @@ def region_origins(h, w, origins, size):
     o = o.astype(np.int64)
     if rh < 1 or rw < 1:
         raise ValueError("empty region %dx%d" % (rh, rw))
-    bad = (o[:, 0] < 0) | (o[:, 1] < 0) | (o[:, 0] + rh > g.out_h) | (o[:, 1] + rw > g.out_w)
+    bad = (o[:, 0] < 0) | (o[:, 1] < 0) | (o[:, 0] + rh > ih) | (o[:, 1] + rw > iw)
     if bad.any():
         i = int(np.argmax(bad))
-        raise ValueError("region %dx%d at (%d, %d) is not inside the %dx%d decoded image"
-                         % (rh, rw, o[i, 0], o[i, 1], g.out_h, g.out_w))
+        raise ValueError("region %dx%d at (%d, %d) is not inside the %dx%d %s" % (rh, rw, o[i, 0], o[i, 1], ih, iw, what))
     return np.ascontiguousarray(o, np.int32)
+
+
+def region_scale_arg(scale):
+    """scale as an int if it is a region decode's scale -- 1 (full resolution), 2, 4 or 8 -- else ValueError."""
+    if isinstance(scale, bool) or not isinstance(scale, (int, np.integer)) or int(scale) not in (1, 2, 4, 8):
+        raise ValueError("a region's scale must be 1, 2, 4 or 8 (got %r)" % (scale,))
+    return int(scale)
+
+
+def scaled_region_blocks(h, w, scale, top, left, rh, rw):
+    """region_blocks() for a window of the 1/scale image, scale 2 or 4 (host only)."""
+    rect = (c_int32 * 8)()
+    check(load().hic_dct_scaled_region_blocks(int(h), int(w), int(scale), int(top), int(left), int(rh), int(rw), rect))
+    return tuple(rect[0:4]), tuple(rect[4:8])
+
+
+def scaled_region_sizes(n, h, w, scale, rh, rw):
+    """(work bytes, tie capacity) hic_dct_scaled_region (scale 2, 4) or hic_dct_thumbnail_region (scale 8) needs for n
+    windows of rh x rw of the 1/scale image (host only)."""
+    work, cap = c_size_t(), c_uint32()
+    check(load().hic_dct_scaled_region_sizes(int(n), int(h), int(w), int(scale), int(rh), int(rw), ctypes.byref(work),
+                                             ctypes.byref(cap)))
+    return int(work.value), int(cap.value)
 
 
 def scale_arg(scale):

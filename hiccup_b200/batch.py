@@ -359,45 +359,69 @@ class DctBatchCodec(_BatchCodec):
         pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
         return pixels
 
-    # ---- regions: one height x width window per image at full resolution (codec.jpeg_region for the whole batch) ----
-    def _region_buffers(self, origins, size):
-        """Check the windows (ValueError before any device work); returns the origins as (n, 2) int32 and the buffers
-        for their size."""
-        origins = _lib.region_origins(self.h, self.w, origins, size)
+    # ---- regions: one height x width window per image, of the full-resolution image (codec.jpeg_region for the whole
+    # batch) or of the 1/2-, 1/4- or 1/8-scale image (jpeg_region(..., scale)) ----------------------------------------
+    def _region_buffers(self, origins, size, scale):
+        """Check the scale and the windows (ValueError before any device work); returns the origins as (n, 2) int32 and
+        the buffers for their size and scale."""
+        scale = _lib.region_scale_arg(scale)
+        origins = _lib.region_origins(self.h, self.w, origins, size, scale)
         if origins.shape[0] != self.n:
             raise ValueError("%d origins for a batch of %d images" % (origins.shape[0], self.n))
         rh, rw = int(size[0]), int(size[1])
-        return origins, self._reduced_buffers(
-            "region", (rh, rw), lambda: ((self.n, rh, rw, 3),) + _lib.region_sizes(self.n, self.h, self.w, rh, rw))
+        if scale == 1:
+            sizes = lambda: _lib.region_sizes(self.n, self.h, self.w, rh, rw)
+        else:
+            sizes = lambda: _lib.scaled_region_sizes(self.n, self.h, self.w, scale, rh, rw)
+        return origins, self._reduced_buffers("region", (rh, rw, scale), lambda: ((self.n, rh, rw, 3),) + sizes())
 
     def _region(self, origins, r):
-        rh, rw = r.key
-        _lib.check(self.lib.hic_dct_region(self.d_coef_dec.ptr, self.n, self.h, self.w, origins.ctypes.data, rh, rw,
-                                           r.d_work.ptr, r.work_bytes, self.d_ties.ptr, r.tie_capacity, self.d_stats.ptr,
-                                           r.d_out.ptr, self.stream))
+        """The region kernels of r's scale on the decoded coefficients -- at scale 8 on the DC values, which the DC-only
+        decode leaves in the coefficient buffer."""
+        rh, rw, scale = r.key
+        if scale == 1:
+            _lib.check(self.lib.hic_dct_region(self.d_coef_dec.ptr, self.n, self.h, self.w, origins.ctypes.data, rh, rw,
+                                               r.d_work.ptr, r.work_bytes, self.d_ties.ptr, r.tie_capacity, self.d_stats.ptr,
+                                               r.d_out.ptr, self.stream))
+        elif scale == 8:
+            _lib.check(self.lib.hic_dct_thumbnail_region(self.d_coef_dec.ptr, self.n, self.h, self.w, origins.ctypes.data, rh,
+                                                         rw, r.d_work.ptr, r.work_bytes, r.d_out.ptr, self.stream))
+        else:
+            _lib.check(self.lib.hic_dct_scaled_region(self.d_coef_dec.ptr, self.n, self.h, self.w, scale, origins.ctypes.data,
+                                                      rh, rw, r.d_work.ptr, r.work_bytes, self.d_ties.ptr, r.tie_capacity,
+                                                      self.d_stats.ptr, r.d_out.ptr, self.stream))
 
-    def decode_regions_device(self, origins, size):
-        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the windows of
-        size = (height, width) at origins ((n, 2) of (top, left)); they stay on the device (fetch_regions)."""
-        origins, r = self._region_buffers(origins, size)
-        self._decode_from_encoder(self.d_coef_dec)
+    def decode_regions_device(self, origins, size, scale=1):
+        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over; DC-only at scale 8, as
+        thumbnails_device), then the windows of size = (height, width) at origins ((n, 2) of (top, left), in the
+        coordinates of the 1/scale image); they stay on the device (fetch_regions)."""
+        origins, r = self._region_buffers(origins, size, scale)
+        self._decode_from_encoder(self.d_coef_dec, dc_only=r.key[2] == 8)
         self._region(origins, r)
 
-    def decode_regions(self, enc, origins, size, out=None):
+    def decode_regions(self, enc, origins, size, out=None, scale=1):
         """Windows of an EncodedStreams, host to host: image i's window is decode(enc)[i, top:top+height,
-        left:left+width] with (top, left) = origins[i] and (height, width) = size, bit for bit.  out: optional
-        preallocated uint8 array of (n, height, width, 3)."""
-        origins, r = self._region_buffers(origins, size)
-        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
+        left:left+width] with (top, left) = origins[i] and (height, width) = size, bit for bit -- or at scale 2 or 4 the
+        same window of decode_scaled(enc, scale)[i], at scale 8 of thumbnails(enc)[i] (only the DC streams go up).
+        out: optional preallocated uint8 array of (n, height, width, 3)."""
+        origins, r = self._region_buffers(origins, size, scale)
+        if r.key[2] == 8:
+            index, symbols, packed, data, byte_off, nbits = entropy.dc_streams_only(enc)
+            self.decoder.decode_dc(index, symbols, packed, data, byte_off, nbits, self.d_coef_dec.ptr, self.stream)
+        else:
+            self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
         self._region(origins, r)
         return self.fetch_regions(out)
 
     def fetch_regions(self, out=None):
         """Download the windows of the last decode_regions() / decode_regions_device() (and their tie statistics
-        into region_stats)."""
+        into region_stats; all zero at scale 8, which has no tie stage)."""
         r = self._reduced["region"]
         pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
-        self.region_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
+        if r.key[2] == 8:
+            self.region_stats = np.zeros(_lib.TIE_STATS, np.uint32)
+        else:
+            self.region_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
         return pixels
 
     # ---- 1/2- and 1/4-scale images (codec.jpeg_scaled for the whole batch) ----------------------------------------

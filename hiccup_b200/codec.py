@@ -278,7 +278,23 @@ def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
     _require_dct(hic, "thumbnail decode")
     settings.check_supported()
     _lib.require_device()
-    p, h, w, g = _dct_header(hic)
+    _, h, w, g = _dct_header(hic)
+    th, tw = _lib.thumbnail_shape(h, w)
+    d_dc = _lib.scratch(2 * g.blocks_per_image)
+    out = _lib.scratch(3 * th * tw)
+    try:
+        _decode_dc(hic, h, w, d_dc.ptr)
+        _lib.check(_lib.load().hic_dct_thumbnail(d_dc.ptr, 1, h, w, out.ptr, None))
+        return out.download(np.uint8, 3 * th * tw).reshape(th, tw, 3)
+    finally:
+        d_dc.free()
+        out.free()
+
+
+def _decode_dc(hic, h, w, d_dc):
+    """The DC-only entropy decode of a DCT-mode file into d_dc, one int16 per block: only the DC tables and DC bit
+    strings go to the device, with the file's restart records of the DC streams when it has them."""
+    p = hic.payloads
     # stream order s = channel * 3 + kind; the DC table / bit string of channel c is payload c / 9 + c
     rows, syms, lens, codes = _tables_to_arrays([p[c] for c in range(3)])
     index = np.zeros((9, 2), np.uint32)
@@ -289,17 +305,8 @@ def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
     offs, nbits = np.zeros(9, np.uint64), np.zeros(9, np.uint64)
     offs[0::3], nbits[0::3] = offs3, nbits3
     records = _records_in_stream_order(hic, nbits, kinds=(entropy.KIND_DC,))
-    th, tw = _lib.thumbnail_shape(h, w)
     dec = entropy.cached_decoder(_lib.layout_dct(1, h, w))
-    d_dc = _lib.scratch(2 * g.blocks_per_image)
-    out = _lib.scratch(3 * th * tw)
-    try:
-        dec.decode_dc(index, syms, packed, data, offs, nbits, d_dc.ptr, restarts=records)
-        _lib.check(_lib.load().hic_dct_thumbnail(d_dc.ptr, 1, h, w, out.ptr, None))
-        return out.download(np.uint8, 3 * th * tw).reshape(th, tw, 3)
-    finally:
-        d_dc.free()
-        out.free()
+    dec.decode_dc(index, syms, packed, data, offs, nbits, d_dc, restarts=records)
 
 
 def _reduced_decode(hic, h, w, g, launch, params, sizes, shape):
@@ -319,20 +326,41 @@ def _reduced_decode(hic, h, w, g, launch, params, sizes, shape):
             b.free()
 
 
-def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int) -> np.ndarray:
-    """One window of a DCT-mode file at full resolution: (height, width, 3) uint8, equal to
-    compression.jpeg_decompression(jpeg_decode(hic))[top:top+height, left:left+width] bit for bit.  The entropy
-    decode is jpeg_decode's (restart records used when the file has them); then only the blocks the window reads are
-    inverse-transformed and only its pixels upsampled and converted (hic_dct_region).  ValueError for a window
-    outside the decoded image, NotImplementedError for a wavelet file, both before any device work."""
+def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int, scale: int = 1) -> np.ndarray:
+    """One window of a DCT-mode file: (height, width, 3) uint8.  At scale 1 it is the window of the full-resolution
+    image, equal to compression.jpeg_decompression(jpeg_decode(hic))[top:top+height, left:left+width] bit for bit: the
+    entropy decode is jpeg_decode's (restart records used when the file has them); then only the blocks the window
+    reads are inverse-transformed and only its pixels upsampled and converted (hic_dct_region).  At scale 2 or 4 the
+    window is one of jpeg_scaled(hic, scale), equal to its crop, with only the window's blocks reduced-transformed
+    (hic_dct_scaled_region); at scale 8 one of jpeg_thumbnail(hic), from the DC streams alone
+    (hic_dct_thumbnail_region).  (top, left) is in the coordinates of the 1/scale image.  ValueError for a scale other
+    than 1, 2, 4 or 8 or a window outside the 1/scale image, NotImplementedError for a wavelet file, all before any
+    device work."""
     _require_dct(hic, "region decode")
+    scale = _lib.region_scale_arg(scale)
     _, h, w, g = _dct_header(hic)
-    origin = _lib.region_origins(h, w, [(top, left)], (height, width))
+    origin = _lib.region_origins(h, w, [(top, left)], (height, width), scale)
     settings.check_supported()
     _lib.require_device()
     height, width = int(height), int(width)
-    return _reduced_decode(hic, h, w, g, _lib.load().hic_dct_region, (origin.ctypes.data, height, width),
-                           _lib.region_sizes(1, h, w, height, width), (height, width, 3))
+    lib = _lib.load()
+    if scale == 1:
+        return _reduced_decode(hic, h, w, g, lib.hic_dct_region, (origin.ctypes.data, height, width),
+                               _lib.region_sizes(1, h, w, height, width), (height, width, 3))
+    sizes = _lib.scaled_region_sizes(1, h, w, scale, height, width)
+    if scale != 8:
+        return _reduced_decode(hic, h, w, g, lib.hic_dct_scaled_region, (scale, origin.ctypes.data, height, width), sizes,
+                               (height, width, 3))
+    bufs = [_lib.scratch(2 * g.blocks_per_image), _lib.scratch(sizes[0]), _lib.scratch(3 * height * width)]
+    d_dc, work, out = bufs
+    try:
+        _decode_dc(hic, h, w, d_dc.ptr)
+        _lib.check(lib.hic_dct_thumbnail_region(d_dc.ptr, 1, h, w, origin.ctypes.data, height, width, work.ptr, sizes[0],
+                                                out.ptr, None))
+        return out.download(np.uint8, 3 * height * width).reshape(height, width, 3)
+    finally:
+        for b in bufs:
+            b.free()
 
 
 def jpeg_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:

@@ -113,42 +113,71 @@ static int geometry_of(int h, int w, hic_dct_geometry* g) {
 // -- at most rh / 2 + 3 of them.  Every window of one size gets a block rectangle of one size per plane kind: the
 // most blocks those rows (columns) can touch, at most the plane's block count.  It starts at the block of the first
 // row the window reads, moved back where it would run past the plane's last block.
+// The scaled region decode uses the same rules at M = 8 / scale samples per block side: a window of the 1/scale image
+// reads rows of the reduced planes (M nby_l x M nbx_l luminance, M nby_c x M nbx_c chroma) exactly as a window of the
+// full decode reads rows of the full-size planes, so only the block size changes.  M is a template argument so that
+// the full-resolution callers (M = 8) compile to what they always did.
 struct RegionSpan {
     int ny_l, nx_l;   // luminance rectangle, blocks
     int ny_c, nx_c;   // chroma rectangle (Cr and Cb alike)
 };
 
-__host__ __device__ inline int region_span_l(int r, int nb) { return min(nb, (r + 6) / 8 + 1); }   // r samples
-__host__ __device__ inline int region_span_c(int r, int nb) { return min(nb, (r / 2 + 3 + 6) / 8 + 1); }
+template <int M>
+constexpr int log2_side() { return M == 8 ? 3 : (M == 4 ? 2 : 1); }
+template <int M = 8>
+__host__ __device__ inline int region_span_l(int r, int nb) { return min(nb, (r + M - 2) / M + 1); }   // r samples
+template <int M = 8>
+__host__ __device__ inline int region_span_c(int r, int nb) { return min(nb, (r / 2 + 3 + M - 2) / M + 1); }
+template <int M = 8>
 __host__ __device__ inline RegionSpan region_span(const hic_dct_geometry& g, int rh, int rw) {
-    return {region_span_l(rh, g.nby_l), region_span_l(rw, g.nbx_l), region_span_c(rh, g.nby_c), region_span_c(rw, g.nbx_c)};
+    return {region_span_l<M>(rh, g.nby_l), region_span_l<M>(rw, g.nbx_l), region_span_c<M>(rh, g.nby_c), region_span_c<M>(rw, g.nbx_c)};
 }
 // first block row (column) of the luminance / chroma rectangle of a window whose first output row (column) is t
-__host__ __device__ inline int region_first_l(int t, int span, int nb) { return min(t >> 3, nb - span); }
-__host__ __device__ inline int region_first_c(int t, int span, int nb) { return min(max(0, (t >> 1) - 1) >> 3, nb - span); }
+template <int M = 8>
+__host__ __device__ inline int region_first_l(int t, int span, int nb) { return min(t >> log2_side<M>(), nb - span); }
+template <int M = 8>
+__host__ __device__ inline int region_first_c(int t, int span, int nb) {
+    return min(max(0, (t >> 1) - 1) >> log2_side<M>(), nb - span);
+}
 
-static int region_check(const hic_dct_geometry& g, int64_t top, int64_t left, int64_t rh, int64_t rw) {
+// a window of the decoded image (scale 1) or of its 1/scale image, ceil(out_h / scale) x ceil(out_w / scale)
+static int region_check(const hic_dct_geometry& g, int64_t top, int64_t left, int64_t rh, int64_t rw, int scale = 1) {
     HIC_REQUIRE(rh >= 1 && rw >= 1, "empty region %lldx%lld", (long long)rh, (long long)rw);
-    HIC_REQUIRE(top >= 0 && left >= 0 && top + rh <= g.out_h && left + rw <= g.out_w,
-                "region %lldx%lld at (%lld, %lld) is not inside the %dx%d decoded image", (long long)rh, (long long)rw,
-                (long long)top, (long long)left, g.out_h, g.out_w);
+    const int ih = (g.out_h + scale - 1) / scale, iw = (g.out_w + scale - 1) / scale;
+    const bool inside = top >= 0 && left >= 0 && top + rh <= ih && left + rw <= iw;
+    if (scale == 1)
+        HIC_REQUIRE(inside, "region %lldx%lld at (%lld, %lld) is not inside the %dx%d decoded image", (long long)rh,
+                    (long long)rw, (long long)top, (long long)left, ih, iw);
+    HIC_REQUIRE(inside, "region %lldx%lld at (%lld, %lld) is not inside the %dx%d 1/%d-scale image", (long long)rh,
+                (long long)rw, (long long)top, (long long)left, ih, iw, scale);
     return HIC_OK;
 }
 
-// window-local planes of one image (bytes) and the work buffer: n origins, then the n Y planes, Cr planes, Cb planes
+// {by, bx, nby, nbx} of the luminance rectangle, then of each chroma rectangle, of a window at (top, left)
+template <int M>
+static void region_rect(const hic_dct_geometry& g, int top, int left, int rh, int rw, int32_t* rect) {
+    const RegionSpan s = region_span<M>(g, rh, rw);
+    const int32_t out[8] = {region_first_l<M>(top, s.ny_l, g.nby_l), region_first_l<M>(left, s.nx_l, g.nbx_l), s.ny_l, s.nx_l,
+                            region_first_c<M>(top, s.ny_c, g.nby_c), region_first_c<M>(left, s.nx_c, g.nbx_c), s.ny_c, s.nx_c};
+    memcpy(rect, out, sizeof(out));
+}
+
+// window-local planes of one image (bytes, M x M samples per block) and the work buffer: n origins, then the n Y
+// planes, Cr planes, Cb planes
 struct RegionLayout {
     RegionSpan s;
     size_t head, ly, lc, total;
     uint64_t blocks;      // selected blocks of the batch
 };
+template <int M = 8>
 static RegionLayout region_layout(int n, const hic_dct_geometry& g, int rh, int rw) {
     RegionLayout L;
-    L.s = region_span(g, rh, rw);
+    L.s = region_span<M>(g, rh, rw);
     L.head = ((size_t)n * 2 * sizeof(int32_t) + 255) / 256 * 256;
-    L.ly = (size_t)64 * L.s.ny_l * L.s.nx_l;
-    L.lc = (size_t)64 * L.s.ny_c * L.s.nx_c;
+    L.ly = (size_t)M * M * L.s.ny_l * L.s.nx_l;
+    L.lc = (size_t)M * M * L.s.ny_c * L.s.nx_c;
     L.total = L.head + (size_t)n * (L.ly + 2 * L.lc);
-    L.blocks = (uint64_t)n * (L.ly + 2 * L.lc) / 64;
+    L.blocks = (uint64_t)n * (L.ly + 2 * L.lc) / (M * M);
     return L;
 }
 
@@ -1174,15 +1203,9 @@ __device__ __forceinline__ void pyr_up_quad(const int* r0, const int* r1, const 
 // from the DC values alone (one int16 per block, global block order).  The luminance block (ty, tx) gives Y; the
 // chroma planes of block samples (nby_c x nbx_c) go through K8's pyrUp taps on the fly, s[-1] = s[1] and s[n] =
 // s[n-1] per axis, and are cropped to th x tw with Y; then K8's ycrcb_to_rgb.  One thread per thumbnail pixel.
-__global__ void __launch_bounds__(256)
-thumbnail_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int n, int th, int tw, uint8_t* __restrict__ rgb) {
-    const int64_t per = (int64_t)th * tw;
-    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= per * n) return;
-    const int64_t img = gid / per;
-    const int64_t rem = gid - img * per;
-    const int ty = (int)(rem / tw), tx = (int)(rem % tw);
-    const int16_t* blocks = dc + img * g.blocks_per_image;
+// thumbnail_pixel: pixel (ty, tx) of one image (blocks: its DC values) to o[0..2].
+__device__ __forceinline__ void thumbnail_pixel(const int16_t* __restrict__ blocks, const hic_dct_geometry& g, int ty, int tx,
+                                                uint8_t* __restrict__ o) {
     const int t_l = c_tab.qi[0][0], t_c = c_tab.qi[1][0];
     const int y = dc_block_sample(__ldg(blocks + (int64_t)ty * g.nbx_l + tx), t_l);
     const int cy = ty >> 1, cx = tx >> 1;
@@ -1201,17 +1224,41 @@ thumbnail_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int n, int 
     }
     int r, gg, b;
     ycrcb_to_rgb(y, up[0], up[1], r, gg, b);
-    uint8_t* o = rgb + gid * 3;
     o[0] = (uint8_t)r;
     o[1] = (uint8_t)gg;
     o[2] = (uint8_t)b;
 }
 
+__global__ void __launch_bounds__(256)
+thumbnail_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int n, int th, int tw, uint8_t* __restrict__ rgb) {
+    const int64_t per = (int64_t)th * tw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * n) return;
+    const int64_t img = gid / per;
+    const int64_t rem = gid - img * per;
+    thumbnail_pixel(dc + img * g.blocks_per_image, g, (int)(rem / tw), (int)(rem % tw), rgb + gid * 3);
+}
+
+// The 1/8-scale window: one rh x rw window of the thumbnail per image, its origin (top, left) per image in thumbnail
+// coordinates; one thread per window pixel, thumbnail_pixel straight from the DC values, n x rh x rw x 3 out.
+__global__ void __launch_bounds__(256)
+thumbnail_region_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int n, const int32_t* __restrict__ origin, int rh,
+                        int rw, uint8_t* __restrict__ rgb) {
+    const int64_t per = (int64_t)rh * rw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * n) return;
+    const int64_t img = gid / per;
+    const int64_t rem = gid - img * per;
+    const int top = __ldg(origin + 2 * img), left = __ldg(origin + 2 * img + 1);
+    thumbnail_pixel(dc + img * g.blocks_per_image, g, top + (int)(rem / rw), left + (int)(rem % rw), rgb + gid * 3);
+}
+
 // ---- region decode: K7R, its fix-up, K8R (one rh x rw window per image, its origin per image) -----------------
 // Image i's window-local planes: Y at y + i * ly, 8 ny_l rows of 8 nx_l samples holding the luminance block
-// rectangle (region_first_l, region_span); Cr and Cb at cr / cb + i * lc, the chroma rectangle likewise.
+// rectangle (region_first_l, region_span); Cr and Cb at cr / cb + i * lc, the chroma rectangle likewise.  (The scaled
+// region decode keeps M x M tiles of the rectangles' blocks there instead, block row by block row.)
 struct RegionArgs {
-    const int32_t* origin;      // n x (top, left), output coordinates
+    const int32_t* origin;      // n x (top, left), output coordinates (of the 1/scale image for the scaled decode)
     uint8_t *y, *cr, *cb;
     size_t ly, lc;
     RegionSpan s;
@@ -1220,10 +1267,33 @@ struct RegionArgs {
 struct RegionFirst {
     int by_l, bx_l, by_c, bx_c;
 };
+template <int M = 8>
 __device__ __forceinline__ RegionFirst region_first(const hic_dct_geometry& g, const RegionArgs& a, int64_t img) {
     const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
-    return {region_first_l(top, a.s.ny_l, g.nby_l), region_first_l(left, a.s.nx_l, g.nbx_l),
-            region_first_c(top, a.s.ny_c, g.nby_c), region_first_c(left, a.s.nx_c, g.nbx_c)};
+    return {region_first_l<M>(top, a.s.ny_l, g.nby_l), region_first_l<M>(left, a.s.nx_l, g.nbx_l),
+            region_first_c<M>(top, a.s.ny_c, g.nby_c), region_first_c<M>(left, a.s.nx_c, g.nbx_c)};
+}
+
+// Selected block `local` of image img (the nl luminance blocks of its rectangle row by row, then the nc of Cr, then
+// Cb): its plane p (0 = Y, 1 = Cr, 2 = Cb), its place (ly, lx) in the rectangle, and its global block index.
+template <int M = 8>
+__device__ __forceinline__ int64_t region_block(const hic_dct_geometry& g, const RegionArgs& a, int64_t img, int64_t local,
+                                                int64_t nl, int64_t nc, int& p, int& ly, int& lx) {
+    const RegionFirst f = region_first<M>(g, a, img);
+    int64_t block = img * g.blocks_per_image;
+    if (local < nl) {
+        ly = (int)(local / a.s.nx_l);
+        lx = (int)(local % a.s.nx_l);
+        block += (int64_t)(f.by_l + ly) * g.nbx_l + f.bx_l + lx;
+    } else {
+        local -= nl;
+        p = 1 + (int)(local / nc);
+        local -= (int64_t)(p - 1) * nc;
+        ly = (int)(local / a.s.nx_c);
+        lx = (int)(local % a.s.nx_c);
+        block += g.nb_l + (int64_t)(p - 1) * g.nb_c + (int64_t)(f.by_c + ly) * g.nbx_c + f.bx_c + lx;
+    }
+    return block;
 }
 
 // K7R: one selected block per thread through K7's inverse_block, into the window-local planes; ties are recorded
@@ -1244,22 +1314,7 @@ region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, int 
     int p = 0, ly = 0, lx = 0;
     if (live) {
         img = gid / per;
-        int64_t local = gid - img * per;
-        const RegionFirst f = region_first(g, a, img);
-        int64_t block = img * g.blocks_per_image;
-        if (local < nl) {
-            ly = (int)(local / a.s.nx_l);
-            lx = (int)(local % a.s.nx_l);
-            block += (int64_t)(f.by_l + ly) * g.nbx_l + f.bx_l + lx;
-        } else {
-            local -= nl;
-            p = 1 + (int)(local / nc);
-            local -= (int64_t)(p - 1) * nc;
-            ly = (int)(local / a.s.nx_c);
-            lx = (int)(local % a.s.nx_c);
-            block += g.nb_l + (int64_t)(p - 1) * g.nb_c + (int64_t)(f.by_c + ly) * g.nbx_c + f.bx_c + lx;
-        }
-        s_src[threadIdx.x] = (uint32_t)block;
+        s_src[threadIdx.x] = (uint32_t)region_block(g, a, img, gid - img * per, nl, nc, p, ly, lx);
     }
     __syncthreads();
     const int count = (int)min((int64_t)K7R_THREADS, per * n - first);
@@ -1362,12 +1417,77 @@ struct K7SSmem {
     alignas(8) unsigned long long bar;
 };
 
+// piece j of staged block t (16-byte units of the CTA's staging area)
+template <int M>
+__device__ __forceinline__ int scaled_piece(int t, int j) {
+    return K7SSmem<M>::PIECES * t + (M == 4 ? j ^ ((t >> 1) & 3) : j);
+}
+
+__device__ __forceinline__ void record_tie(uint32_t block, hic_tie_record* __restrict__ ties, uint32_t tie_capacity,
+                                           uint32_t* __restrict__ stats) {
+    const uint32_t slot = atomicAdd(&stats[0], 1u);
+    if (slot < tie_capacity) {
+        hic_tie_record rec;
+        rec.block = block;
+        rec.reserved = 0;
+        rec.mask = ~0ull;
+        ties[slot] = rec;
+    } else {
+        atomicAdd(&stats[3], 1u);
+    }
+}
+
+// K7S's arithmetic on staged block t of kind 0 (luminance) / 1 (chroma): its M x M tile, four samples per word, into
+// packed; true when the block has AC terms and a sample within its error band of an integer.
+template <int M>
+__device__ __forceinline__ bool scaled_block(const int4* __restrict__ blk, int t, int kind, uint32_t (&packed)[M * M / 4]) {
+    constexpr int PIECES = K7SSmem<M>::PIECES;
+    constexpr uint8_t zz[64] = HIC_ZIGZAG8;
+    int words[4 * PIECES];                              // the block's first 8 PIECES scan entries, two per word
+#pragma unroll
+    for (int j = 0; j < PIECES; ++j) {
+        const int4 wv = blk[scaled_piece<M>(t, j)];
+        words[4 * j] = wv.x; words[4 * j + 1] = wv.y; words[4 * j + 2] = wv.z; words[4 * j + 3] = wv.w;
+    }
+    float v[M * M];
+    float energy = 0.f;          // sum |q| T w_s margin: the error band of the samples
+    int ac_bits = 0;
+#pragma unroll
+    for (int k = 0; k < 8 * PIECES; ++k) {
+        const int nat = zz[k], u = nat >> 3, x = nat & 7;
+        if (u >= M || x >= M) continue;
+        const int q = (k & 1) ? words[k >> 1] >> 16 : (int)(short)(words[k >> 1] & 0xFFFF);
+        v[M * u + x] = (float)(q * c_tab.qi[kind][nat]) * (1.f / 256.f);
+        energy = fmaf(fabsf((float)q), c_tab.sqw[M == 4 ? 0 : 1][kind][M * u + x], energy);
+        if (k) ac_bits |= q;
+    }
+    scaled_transform<M>(v);
+    float margin = 1e30f;
+#pragma unroll
+    for (int i = 0; i < M * M; ++i) {
+        const float p = v[i] + 128.f;
+        const float r = (p + MAGIC) - MAGIC;
+        margin = fminf(margin, fabsf(p - r));
+        const uint32_t b = (uint32_t)__float2int_rz(p) & 0xFFu;               // truncate, wrap
+        if (i % 4 == 0) packed[i / 4] = b; else packed[i / 4] |= b << (8 * (i % 4));
+    }
+    // as K7: 2^-15 covers the rounding of the final + 128 below 1024 and of this comparison
+    const float band = (float)(4.0 / 16777216.0 / 256.0) * energy + 3.0517578125e-5f;
+    return ac_bits != 0 && margin <= band;
+}
+
+template <int M>
+__device__ __forceinline__ void store_tile(uint8_t* __restrict__ dst, const uint32_t (&packed)[M * M / 4]) {
+    if constexpr (M == 4)
+        *reinterpret_cast<uint4*>(dst) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
+    else
+        *reinterpret_cast<uint32_t*>(dst) = packed[0];
+}
+
 template <int M>
 __global__ void __launch_bounds__(K7S_THREADS)
 scaled_inverse_kernel(const __grid_constant__ CUtensorMap tmap_blocks, hic_dct_geometry g, int n, uint8_t* __restrict__ tiles,
                       hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
-    constexpr int PIECES = K7SSmem<M>::PIECES;
-    constexpr uint8_t zz[64] = HIC_ZIGZAG8;
     __shared__ K7SSmem<M> s;
     const uint32_t bar = (uint32_t)__cvta_generic_to_shared(&s.bar);
     if (threadIdx.x == 0) {
@@ -1395,62 +1515,19 @@ scaled_inverse_kernel(const __grid_constant__ CUtensorMap tmap_blocks, hic_dct_g
     const int64_t gid = (int64_t)blockIdx.x * K7S_THREADS + threadIdx.x;
     if (gid >= total) return;
     const int kind = gid % g.blocks_per_image < g.nb_l ? 0 : 1;
-    const int t = threadIdx.x;
-    int words[4 * PIECES];                              // the block's first 8 PIECES scan entries, two per word
-#pragma unroll
-    for (int j = 0; j < PIECES; ++j) {
-        const int4 wv = s.blk[PIECES * t + (M == 4 ? j ^ ((t >> 1) & 3) : j)];
-        words[4 * j] = wv.x; words[4 * j + 1] = wv.y; words[4 * j + 2] = wv.z; words[4 * j + 3] = wv.w;
-    }
-    float v[M * M];
-    float energy = 0.f;          // sum |q| T w_s margin: the error band of the samples
-    int ac_bits = 0;
-#pragma unroll
-    for (int k = 0; k < 8 * PIECES; ++k) {
-        const int nat = zz[k], u = nat >> 3, x = nat & 7;
-        if (u >= M || x >= M) continue;
-        const int q = (k & 1) ? words[k >> 1] >> 16 : (int)(short)(words[k >> 1] & 0xFFFF);
-        v[M * u + x] = (float)(q * c_tab.qi[kind][nat]) * (1.f / 256.f);
-        energy = fmaf(fabsf((float)q), c_tab.sqw[M == 4 ? 0 : 1][kind][M * u + x], energy);
-        if (k) ac_bits |= q;
-    }
-    scaled_transform<M>(v);
-    float margin = 1e30f;
     uint32_t packed[M * M / 4];
-#pragma unroll
-    for (int i = 0; i < M * M; ++i) {
-        const float p = v[i] + 128.f;
-        const float r = (p + MAGIC) - MAGIC;
-        margin = fminf(margin, fabsf(p - r));
-        const uint32_t b = (uint32_t)__float2int_rz(p) & 0xFFu;               // truncate, wrap
-        if (i % 4 == 0) packed[i / 4] = b; else packed[i / 4] |= b << (8 * (i % 4));
-    }
-    if constexpr (M == 4)
-        reinterpret_cast<uint4*>(tiles)[gid] = make_uint4(packed[0], packed[1], packed[2], packed[3]);
-    else
-        reinterpret_cast<uint32_t*>(tiles)[gid] = packed[0];
-    // as K7: 2^-15 covers the rounding of the final + 128 below 1024 and of this comparison
-    const float band = (float)(4.0 / 16777216.0 / 256.0) * energy + 3.0517578125e-5f;
-    if (ac_bits != 0 && margin <= band) {
-        const uint32_t slot = atomicAdd(&stats[0], 1u);
-        if (slot < tie_capacity) {
-            hic_tie_record rec;
-            rec.block = (uint32_t)gid;
-            rec.reserved = 0;
-            rec.mask = ~0ull;
-            ties[slot] = rec;
-        } else {
-            atomicAdd(&stats[3], 1u);
-        }
-    }
+    const bool flagged = scaled_block<M>(s.blk, threadIdx.x, kind, packed);
+    store_tile<M>(tiles + gid * M * M, packed);
+    if (flagged) record_tie((uint32_t)gid, ties, tie_capacity, stats);
 }
 
 // The fix-up of K7S's flagged blocks: one thread per record, scaled_decoded_block<M> (the float64 definition) into
-// the block's tile.  stats[1] counts the samples re-evaluated, stats[2] those that changed.
-template <int M>
-__global__ void __launch_bounds__(128)
-scaled_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_t* __restrict__ tiles,
-                    const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+// the block's tile, which locate(global block index) gives.  stats[1] counts the samples re-evaluated, stats[2] those
+// that changed.
+template <int M, class Locate>
+__device__ __forceinline__ void scaled_fixup_body(const int16_t* __restrict__ coef, const hic_dct_geometry& g,
+                                                  const hic_tie_record* __restrict__ ties, uint32_t tie_capacity,
+                                                  uint32_t* __restrict__ stats, Locate locate) {
     const uint32_t n_rec = min(stats[0], tie_capacity);
     uint32_t changed = 0, done = 0;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_rec; i += gridDim.x * blockDim.x) {
@@ -1464,7 +1541,7 @@ scaled_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_
             for (int x = 0; x < M; ++x) cq[M * u + x] = (int32_t)blk[c_tab.izz[8 * u + x]] * c_tab.qi[kind][8 * u + x];
         double y[M * M];
         scaled_decoded_block<M>(cq, y);
-        uint8_t* dst = tiles + (size_t)b * M * M;
+        uint8_t* dst = locate(b);
 #pragma unroll
         for (int k = 0; k < M * M; ++k) {
             const uint8_t val = wrap_u8(y[k]);
@@ -1486,6 +1563,30 @@ scaled_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_
     }
 }
 
+template <int M>
+__global__ void __launch_bounds__(128)
+scaled_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_t* __restrict__ tiles,
+                    const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    scaled_fixup_body<M>(coef, g, ties, tie_capacity, stats, [&](uint32_t b) { return tiles + (size_t)b * M * M; });
+}
+
+// K8S's pyrUp of reduced chroma sample (cy, cx) of planes of ny x nx samples: the 2x2 quads up[c] of Cr (c = 0) and Cb
+// (c = 1), from the 3x3 neighbourhood chosen with K8's borders in those planes and read through sample(c, row, col).
+template <class Sample>
+__device__ __forceinline__ void scaled_up_quads(int cy, int cx, int ny, int nx, Sample sample, int (&up)[2][4]) {
+    const int ym = cy > 0 ? cy - 1 : (ny > 1 ? 1 : 0), yn = cy + 1 < ny ? cy + 1 : ny - 1;
+    const int xm = cx > 0 ? cx - 1 : (nx > 1 ? 1 : 0), xn = cx + 1 < nx ? cx + 1 : nx - 1;
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+        auto row = [&](int r, int* v) {
+            v[0] = sample(c, r, xm); v[1] = sample(c, r, cx); v[2] = sample(c, r, xn);
+        };
+        int s0[3], s1[3], s2[3];
+        row(ym, s0); row(cy, s1); row(yn, s2);
+        pyr_up_quad(s0, s1, s2, up[c]);
+    }
+}
+
 // K8S: one sample of the reduced chroma planes (M nby_c x M nbx_c, their whole block grids: the thumbnail's
 // convention) per thread, as K8: its 3x3 neighbourhood through pyr_up_quad, Y from the reduced luminance plane
 // (M nby_l x M nbx_l), K8's ycrcb_to_rgb, and the pixels of its 2x2 output quad inside sh x sw = ceil(out_h / s) x
@@ -1500,21 +1601,11 @@ scaled_colour_kernel(const uint8_t* __restrict__ tiles, hic_dct_geometry g, int 
     const int64_t img = gid / per;
     const int64_t rem = gid - img * per;
     const int cy = (int)(rem / qw), cx = (int)(rem % qw);
-    const int ny = M * g.nby_c, nx = M * g.nbx_c;
-    const int ym = cy > 0 ? cy - 1 : (ny > 1 ? 1 : 0), yn = cy + 1 < ny ? cy + 1 : ny - 1;
-    const int xm = cx > 0 ? cx - 1 : (nx > 1 ? 1 : 0), xn = cx + 1 < nx ? cx + 1 : nx - 1;
     const uint8_t* base = tiles + (size_t)img * g.blocks_per_image * M * M;
     int up[2][4];
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-        const uint8_t* p = base + (size_t)(g.nb_l + c * g.nb_c) * M * M;
-        auto row = [&](int r, int* v) {
-            v[0] = tile_sample(p, g.nbx_c, M, r, xm); v[1] = tile_sample(p, g.nbx_c, M, r, cx); v[2] = tile_sample(p, g.nbx_c, M, r, xn);
-        };
-        int s0[3], s1[3], s2[3];
-        row(ym, s0); row(cy, s1); row(yn, s2);
-        pyr_up_quad(s0, s1, s2, up[c]);
-    }
+    scaled_up_quads(cy, cx, M * g.nby_c, M * g.nbx_c, [&](int c, int r, int col) {
+        return tile_sample(base + (size_t)(g.nb_l + c * g.nb_c) * M * M, g.nbx_c, M, r, col);
+    }, up);
     uint8_t* dst = rgb + (size_t)img * sh * sw * 3;
 #pragma unroll
     for (int dy = 0; dy < 2; ++dy)
@@ -1525,6 +1616,112 @@ scaled_colour_kernel(const uint8_t* __restrict__ tiles, hic_dct_geometry g, int 
             int r, gg, b;
             ycrcb_to_rgb(tile_sample(base, g.nbx_l, M, oy, ox), up[0][2 * dy + dx], up[1][2 * dy + dx], r, gg, b);
             uint8_t* o = dst + ((size_t)oy * sw + ox) * 3;
+            o[0] = (uint8_t)r;
+            o[1] = (uint8_t)gg;
+            o[2] = (uint8_t)b;
+        }
+}
+
+// ---- scaled region decode: K7SR, its fix-up, K8SR (one rh x rw window of the 1/s image per image) ---------------
+// The rectangles come from the region rules at M samples per block (region_first<M>, region_span<M>); image i's
+// window-local tiles: Y at y + i * ly, the M x M tiles of the luminance rectangle's blocks, row by row (nx_l per row);
+// Cr and Cb at cr / cb + i * lc likewise (nx_c per row).
+template <int M>
+__device__ __forceinline__ uint8_t* region_tile(const RegionArgs& a, int64_t img, int p, int ly, int lx) {
+    if (p == 0) return a.y + img * a.ly + ((size_t)ly * a.s.nx_l + lx) * M * M;
+    return (p == 1 ? a.cr : a.cb) + img * a.lc + ((size_t)ly * a.s.nx_c + lx) * M * M;
+}
+
+// K7SR: one selected block per thread through K7S's arithmetic (scaled_block) into its window-local tile; ties are
+// recorded with the global block index, so exactly the blocks K7S flags are flagged.  The selected blocks are one run
+// per block row of each rectangle, so there is no box of consecutive blocks for one TMA load: the CTA's blocks come in
+// by plain 16-byte loads of their first PIECES pieces only (64 bytes at M = 4, 16 at M = 2), consecutive threads on
+// consecutive pieces, into K7S's staging layout.
+template <int M>
+__global__ void __launch_bounds__(K7S_THREADS)
+scaled_region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, int n, RegionArgs a,
+                             hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    constexpr int PIECES = K7SSmem<M>::PIECES;
+    __shared__ int4 s_blk[K7S_THREADS * PIECES];
+    __shared__ uint32_t s_src[K7S_THREADS];
+    // 32-bit indices: the selected blocks are at most the batch's blocks, fewer than 2^32 (hic_dct_scaled_region)
+    const uint32_t nl = (uint32_t)a.s.ny_l * a.s.nx_l, nc = (uint32_t)a.s.ny_c * a.s.nx_c, per = nl + 2 * nc;
+    const uint32_t first = blockIdx.x * K7S_THREADS, gid = first + threadIdx.x, total = per * (uint32_t)n;
+    const bool live = gid < total;
+    uint32_t img = 0;
+    int p = 0, ly = 0, lx = 0;
+    if (live) {
+        img = gid / per;
+        s_src[threadIdx.x] = (uint32_t)region_block<M>(g, a, img, gid - img * per, nl, nc, p, ly, lx);
+    }
+    __syncthreads();
+    const int count = (int)min((uint32_t)K7S_THREADS, total - first);
+    const int4* c4 = reinterpret_cast<const int4*>(coef);
+    for (int q = threadIdx.x; q < PIECES * count; q += K7S_THREADS) {
+        const int t = q / PIECES, j = q % PIECES;
+        s_blk[scaled_piece<M>(t, j)] = __ldg(c4 + (size_t)s_src[t] * 8 + j);
+    }
+    __syncthreads();
+    if (!live) return;
+    uint32_t packed[M * M / 4];
+    const bool flagged = scaled_block<M>(s_blk, threadIdx.x, p == 0 ? 0 : 1, packed);
+    store_tile<M>(region_tile<M>(a, img, p, ly, lx), packed);
+    if (flagged) record_tie(s_src[threadIdx.x], ties, tie_capacity, stats);
+}
+
+// The fix-up of K7SR's flagged blocks: scaled_fixup_kernel's arithmetic, each block landing in its window's tile.
+template <int M>
+__global__ void __launch_bounds__(128)
+scaled_region_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, RegionArgs a,
+                           const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    scaled_fixup_body<M>(coef, g, ties, tie_capacity, stats, [&](uint32_t b) {
+        const int64_t img = b / g.blocks_per_image;
+        int64_t local = b - img * g.blocks_per_image;
+        const RegionFirst f = region_first<M>(g, a, img);
+        if (local < g.nb_l) return region_tile<M>(a, img, 0, (int)(local / g.nbx_l) - f.by_l, (int)(local % g.nbx_l) - f.bx_l);
+        local -= g.nb_l;
+        const int p = (int)(local / g.nb_c);
+        local -= (int64_t)p * g.nb_c;
+        return region_tile<M>(a, img, 1 + p, (int)(local / g.nbx_c) - f.by_c, (int)(local % g.nbx_c) - f.bx_c);
+    });
+}
+
+// K8SR: K8S's taps over one window per image: a thread per reduced chroma sample the window covers (rh / 2 + 1 rows of
+// rw / 2 + 1, as K8R), producing the pixels of its 2x2 quad inside the window.  The neighbours are chosen in the whole
+// reduced chroma planes (M nby_c x M nbx_c, K8S's borders) and read from the window-local tiles; Y likewise; the
+// n x rh x rw x 3 result is written directly.
+template <int M>
+__global__ void __launch_bounds__(256)
+scaled_region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restrict__ rgb) {
+    const int ch = a.rh / 2 + 1, cw = a.rw / 2 + 1;
+    const int64_t per = (int64_t)ch * cw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * n) return;
+    const int64_t img = gid / per;
+    const int64_t rem = gid - img * per;
+    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
+    const int cy = (top >> 1) + (int)(rem / cw), cx = (left >> 1) + (int)(rem % cw);
+    if (2 * cy > top + a.rh - 1 || 2 * cx > left + a.rw - 1) return;
+    const RegionFirst f = region_first<M>(g, a, img);
+    const int r0 = M * f.by_c, c0 = M * f.bx_c;
+    const uint8_t* crp = a.cr + img * a.lc;
+    const uint8_t* cbp = a.cb + img * a.lc;
+    int up[2][4];
+    scaled_up_quads(cy, cx, M * g.nby_c, M * g.nbx_c, [&](int c, int r, int col) {
+        return tile_sample(c == 0 ? crp : cbp, a.s.nx_c, M, r - r0, col - c0);
+    }, up);
+    const uint8_t* ysrc = a.y + img * a.ly;
+    uint8_t* dst = rgb + (size_t)img * a.rh * a.rw * 3;
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < 2; ++dx) {
+            const int oy = 2 * cy + dy, ox = 2 * cx + dx;
+            if (oy < top || oy >= top + a.rh || ox < left || ox >= left + a.rw) continue;
+            int r, gg, b;
+            ycrcb_to_rgb(tile_sample(ysrc, a.s.nx_l, M, oy - M * f.by_l, ox - M * f.bx_l), up[0][2 * dy + dx],
+                         up[1][2 * dy + dx], r, gg, b);
+            uint8_t* o = dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3;
             o[0] = (uint8_t)r;
             o[1] = (uint8_t)gg;
             o[2] = (uint8_t)b;
@@ -1645,6 +1842,42 @@ static int scaled_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n
     HIC_LAUNCH("scaled_inverse_kernel", st, k7::scaled_inverse_kernel<M><<<grid_inv, k7::K7S_THREADS, 0, st>>>(tmap_blocks, g, n, d_work, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("scaled_fixup_kernel", st, k7::scaled_fixup_kernel<M><<<148 * 4, 128, 0, st>>>(d_coef, g, d_work, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("scaled_colour_kernel", st, k7::scaled_colour_kernel<M><<<grid_rgb, 256, 0, st>>>(d_work, g, n, sh, sw, d_rgb_out));
+    return HIC_OK;
+}
+
+// The kernels' view of a region work buffer of layout L (origins at its head, already copied there)
+static k7::RegionArgs region_args(uint8_t* d_work, int n, const RegionLayout& L, int rh, int rw) {
+    k7::RegionArgs a;
+    a.origin = reinterpret_cast<const int32_t*>(d_work);
+    a.y = d_work + L.head;
+    a.cr = a.y + (size_t)n * L.ly;
+    a.cb = a.cr + (size_t)n * L.lc;
+    a.ly = L.ly;
+    a.lc = L.lc;
+    a.s = L.s;
+    a.rh = rh;
+    a.rw = rw;
+    return a;
+}
+
+// The rest of hic_dct_scaled_region for M x M samples per block (scale 8 / M): the work buffer's checks, the origins'
+// copy, K7SR, its fix-up and K8SR
+template <int M>
+static int scaled_region_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
+                                uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity,
+                                uint32_t* d_stats, uint8_t* d_rgb_out, cudaStream_t st) {
+    const RegionLayout L = region_layout<M>(n, g, rh, rw);
+    HIC_REQUIRE(work_bytes >= L.total, "work buffer of %zu bytes is too small: %zu needed (hic_dct_scaled_region_sizes)", work_bytes, L.total);
+    HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
+                "d_coef and d_work must be 16-byte aligned");
+    const int rc = ensure_tables();
+    if (rc) return rc;
+    HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
+    HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    const k7::RegionArgs a = region_args(d_work, n, L, rh, rw);
+    HIC_LAUNCH("scaled_region_inverse_kernel", st, k7::scaled_region_inverse_kernel<M><<<grid_for((int64_t)L.blocks, k7::K7S_THREADS), k7::K7S_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH("scaled_region_fixup_kernel", st, k7::scaled_region_fixup_kernel<M><<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH("scaled_region_colour_kernel", st, k7::scaled_region_colour_kernel<M><<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
     return HIC_OK;
 }
 
@@ -1847,10 +2080,7 @@ int hic_dct_region_blocks(int32_t h, int32_t w, int32_t top, int32_t left, int32
     if (rc) return rc;
     rc = region_check(g, top, left, rh, rw);
     if (rc) return rc;
-    const RegionSpan s = region_span(g, rh, rw);
-    const int32_t out[8] = {region_first_l(top, s.ny_l, g.nby_l), region_first_l(left, s.nx_l, g.nbx_l), s.ny_l, s.nx_l,
-                            region_first_c(top, s.ny_c, g.nby_c), region_first_c(left, s.nx_c, g.nbx_c), s.ny_c, s.nx_c};
-    memcpy(rect, out, sizeof(out));
+    region_rect<8>(g, top, left, rh, rw, rect);
     return HIC_OK;
 }
 
@@ -1890,16 +2120,7 @@ int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const
     cudaStream_t st = as_stream(stream);
     HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
     HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    k7::RegionArgs a;
-    a.origin = reinterpret_cast<const int32_t*>(d_work);
-    a.y = d_work + L.head;
-    a.cr = a.y + (size_t)n * L.ly;
-    a.cb = a.cr + (size_t)n * L.lc;
-    a.ly = L.ly;
-    a.lc = L.lc;
-    a.s = L.s;
-    a.rh = rh;
-    a.rw = rw;
+    const k7::RegionArgs a = region_args(d_work, n, L, rh, rw);
     HIC_LAUNCH("region_inverse_kernel", st, k7::region_inverse_kernel<<<grid_for((int64_t)L.blocks, k7::K7R_THREADS), k7::K7R_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("region_fixup_kernel", st, k7::region_fixup_kernel<<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("region_colour_kernel", st, k7::region_colour_kernel<<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
@@ -1957,6 +2178,86 @@ int hic_dct_scaled(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32
     HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
     return scale == 2 ? scaled_launch<4>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st)
                       : scaled_launch<2>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st);
+}
+
+int hic_dct_scaled_region_blocks(int32_t h, int32_t w, int32_t scale, int32_t top, int32_t left, int32_t rh, int32_t rw,
+                                 int32_t* rect) {
+    using namespace hic;
+    HIC_REQUIRE(rect != nullptr, "NULL argument");
+    HIC_REQUIRE(scale == 2 || scale == 4, "scale must be 2 or 4 (got %d)", scale);
+    hic_dct_geometry g;
+    int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    rc = region_check(g, top, left, rh, rw, scale);
+    if (rc) return rc;
+    if (scale == 2)
+        region_rect<4>(g, top, left, rh, rw, rect);
+    else
+        region_rect<2>(g, top, left, rh, rw, rect);
+    return HIC_OK;
+}
+
+int hic_dct_scaled_region_sizes(int32_t n, int32_t h, int32_t w, int32_t scale, int32_t rh, int32_t rw, size_t* work_bytes,
+                                uint32_t* tie_capacity) {
+    using namespace hic;
+    HIC_REQUIRE(work_bytes && tie_capacity, "NULL argument");
+    HIC_REQUIRE(scale == 2 || scale == 4 || scale == 8, "scale must be 2, 4 or 8 (got %d)", scale);
+    hic_dct_geometry g;
+    int rc = batch_geometry(n, h, w, false, &g);
+    if (rc) return rc;
+    rc = region_check(g, 0, 0, rh, rw, scale);
+    if (rc) return rc;
+    if (scale == 8) {              // hic_dct_thumbnail_region: the origins alone, no tie stage
+        *work_bytes = (size_t)n * 2 * sizeof(int32_t);
+        *tie_capacity = 0;
+        return HIC_OK;
+    }
+    const RegionLayout L = scale == 2 ? region_layout<4>(n, g, rh, rw) : region_layout<2>(n, g, rh, rw);
+    HIC_REQUIRE(L.blocks < (1ull << 32), "batch too large: %llu selected blocks", (unsigned long long)L.blocks);
+    *work_bytes = L.total;
+    *tie_capacity = (uint32_t)L.blocks;
+    return HIC_OK;
+}
+
+int hic_dct_scaled_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32_t scale, const int32_t* h_origin,
+                          int32_t rh, int32_t rw, uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties,
+                          uint32_t tie_capacity, uint32_t* d_stats, uint8_t* d_rgb_out, void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_coef && h_origin && d_work && d_ties && d_stats && d_rgb_out, "NULL pointer");
+    HIC_REQUIRE(scale == 2 || scale == 4, "scale must be 2 or 4 (got %d; the 1/8-scale window is hic_dct_thumbnail_region)", scale);
+    hic_dct_geometry g;
+    int rc = batch_geometry(n, h, w, true, &g);
+    if (rc) return rc;
+    for (int i = 0; i < n; ++i) {
+        rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw, scale);
+        if (rc) return rc;
+    }
+    cudaStream_t st = as_stream(stream);
+    return scale == 2 ? scaled_region_launch<4>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity, d_stats, d_rgb_out, st)
+                      : scaled_region_launch<2>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity, d_stats, d_rgb_out, st);
+}
+
+int hic_dct_thumbnail_region(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, const int32_t* h_origin, int32_t rh,
+                             int32_t rw, uint8_t* d_work, size_t work_bytes, uint8_t* d_rgb_out, void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_dc && h_origin && d_work && d_rgb_out, "NULL pointer");
+    hic_dct_geometry g;
+    int rc = batch_geometry(n, h, w, false, &g);
+    if (rc) return rc;
+    for (int i = 0; i < n; ++i) {
+        rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw, 8);
+        if (rc) return rc;
+    }
+    const size_t need = (size_t)n * 2 * sizeof(int32_t);
+    HIC_REQUIRE(work_bytes >= need, "work buffer of %zu bytes is too small: %zu needed (hic_dct_scaled_region_sizes)", work_bytes, need);
+    HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_dc) & 1) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 3) == 0,
+                "d_dc must be 2-byte aligned and d_work 4-byte aligned");
+    rc = ensure_tables();
+    if (rc) return rc;
+    cudaStream_t st = as_stream(stream);
+    HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, need, cudaMemcpyHostToDevice, st));
+    HIC_LAUNCH("thumbnail_region_kernel", st, k7::thumbnail_region_kernel<<<grid_for((int64_t)n * rh * rw, 256), 256, 0, st>>>(d_dc, g, n, reinterpret_cast<const int32_t*>(d_work), rh, rw, d_rgb_out));
+    return HIC_OK;
 }
 
 }  // extern "C"

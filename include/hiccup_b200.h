@@ -199,6 +199,36 @@ int hic_dct_scaled(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32
                    size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity, uint32_t* d_stats,
                    uint8_t* d_rgb_out, void* stream);
 
+/* Scaled region -- one rh x rw window of the 1/s-scale image per image of the batch: window i equals
+ * hic_dct_scaled's image (s = 2, 4) or hic_dct_thumbnail's (s = 8) cropped to [top, top+rh) x [left, left+rw)
+ * bit for bit, (top, left) = h_origin[2i], h_origin[2i+1] in the coordinates of that sh x sw = ceil(out_h / s) x
+ * ceil(out_w / s) image; valid when top, left >= 0, rh, rw >= 1, top + rh <= sh and left + rw <= sw.
+ * hic_dct_scaled_region (s = 2, 4) selects blocks with the region rules at m = 8 / s samples per block side: the
+ * window reads rows [top, top+rh) of the reduced luminance plane and the pyrUp taps of the reduced chroma planes
+ * (m nby_c x m nbx_c, hic_dct_scaled's borders).  Only those blocks go through hic_dct_scaled's float32 transform,
+ * its error band and float64 fix-up (tie records carry the global block index) into window-local tiles in d_work,
+ * and only the window's pixels are upsampled and converted, straight into d_rgb_out (n * rh * rw * 3).  d_coef as
+ * hic_dct_scaled reads it (16-byte aligned; only the first 64 (s = 2) or 16 (s = 4) bytes of a selected block);
+ * d_work 16-byte aligned; d_stats as for hic_dct_scaled, zeroed by this call.
+ * hic_dct_thumbnail_region computes the 1/8-scale window's pixels straight from the DC values d_dc (as
+ * hic_dct_thumbnail reads them, 2-byte aligned); d_work (4-byte aligned) needs 8 n bytes, for the origins.
+ * Both check every origin on the host (HIC_ERR_INVALID for a window outside sh x sw or an empty size) before
+ * anything is launched and copy the origins to d_work with cudaMemcpyAsync on `stream`.
+ * hic_dct_scaled_region_blocks (host only, s = 2, 4) gives the block rectangles a window selects, as
+ * hic_dct_region_blocks does; every window of one size selects rectangles of one size.
+ * hic_dct_scaled_region_sizes (host only, s = 2, 4, 8) gives the d_work bytes and the tie capacity (one record per
+ * selected block; 0 at s = 8) for n windows of rh x rw.  hic_dct_scaled_region returns HIC_ERR_INVALID for a scale
+ * other than 2 or 4 before anything is launched. */
+int hic_dct_scaled_region_blocks(int32_t h, int32_t w, int32_t scale, int32_t top, int32_t left, int32_t rh, int32_t rw,
+                                 int32_t* rect);
+int hic_dct_scaled_region_sizes(int32_t n, int32_t h, int32_t w, int32_t scale, int32_t rh, int32_t rw,
+                                size_t* work_bytes, uint32_t* tie_capacity);
+int hic_dct_scaled_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32_t scale, const int32_t* h_origin,
+                          int32_t rh, int32_t rw, uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties,
+                          uint32_t tie_capacity, uint32_t* d_stats, uint8_t* d_rgb_out, void* stream);
+int hic_dct_thumbnail_region(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, const int32_t* h_origin,
+                             int32_t rh, int32_t rw, uint8_t* d_work, size_t work_bytes, uint8_t* d_rgb_out, void* stream);
+
 /* ---- wavelet ("HIC") mode --------------------------------------------------------------------- */
 /* Sub-band geometry of pywt.wavedec2(channel, "db1", level=3) (transform.py:196-209): level sizes
  * ceil(n / 2) per level; ten sub-bands per channel in the order [cA3, cH3, cV3, cD3, cH2, cV2, cD2,

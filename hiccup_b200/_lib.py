@@ -106,6 +106,8 @@ SIGNATURES = {
     "hic_wavelet_general_work_bytes": (c_int, [c_int32, c_int32, c_int32, ctypes.POINTER(c_size_t)]),
     "hic_wavelet_forward_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, ctypes.POINTER(WaveletParams), c_void_p, c_void_p, c_void_p]),
     "hic_wavelet_inverse_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, ctypes.POINTER(WaveletParams), c_void_p, c_void_p, c_void_p]),
+    "hic_wavelet_scaled_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, ctypes.POINTER(WaveletParams), c_int32, c_void_p,
+                                           c_void_p, c_void_p]),
     "hic_wavelet_flat_to_bands_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "hic_wavelet_bands_to_flat_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "hic_layout_dct": (c_int, [c_int32, c_int32, c_int32, ctypes.POINTER(StreamLayout)]),
@@ -469,6 +471,15 @@ def wavelet_pyramid(h, w, levels):
     g = WaveletPyramid()
     check(load().hic_wavelet_pyramid_of(int(h), int(w), int(levels), ctypes.byref(g)))
     return g
+
+
+def wavelet_scale_arg(scale, levels):
+    """k for a wavelet scaled decode's scale = 2^k of a file of `levels` levels (1 <= k <= levels), else ValueError."""
+    levels = int(levels)
+    if isinstance(scale, bool) or not isinstance(scale, (int, np.integer)) or int(scale) < 2 or int(scale) & (int(scale) - 1) \
+            or int(scale) > 1 << levels:
+        raise ValueError("scale must be 2^k with 1 <= k <= %d, the file's levels (got %r)" % (levels, scale))
+    return int(scale).bit_length() - 1
 
 
 def wavelet_work_bytes(n, h, w):

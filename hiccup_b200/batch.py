@@ -35,6 +35,7 @@ class _BatchCodec:
         self.encoder = entropy.EntropyEncoder(self.layout, value_bins)
         self.decoder = entropy.EntropyDecoder(self.layout)
         self._buffers = [self.d_rgb, self.d_coef, self.d_coef_dec, self.d_out]
+        self._reduced = {}
         # page-locked staging for the host-to-host entry points (grown on demand, reused every call)
         self._h_data = None
         self._h_out = None
@@ -248,7 +249,23 @@ class _BatchCodec:
     def _after_decode(self):
         pass
 
+    # ---- reduced outputs (thumbnails, regions, scaled images) ---------------------------------------------------------
+    def _reduced_buffers(self, kind, key, sizes):
+        """The buffers of reduced output `kind` for its parameters `key`.  Each kind keeps its own, made on first use (a
+        codec that never asks for one pays nothing) and remade only when its key changes; sizes() gives (output shape,
+        work bytes, tie capacity) for a new key."""
+        r = self._reduced.get(kind)
+        if r is not None and r.key == key:
+            return r
+        if r is not None:
+            self._reduced.pop(kind).free()
+        r = self._reduced[kind] = _ReducedOutput(key, *sizes())
+        return r
+
     def close(self):
+        for r in self._reduced.values():
+            r.free()
+        self._reduced = {}
         self.encoder.close()
         self.decoder.close()
         for b in self._buffers + [self._h_data, self._h_out] + self._h_tab_mem:
@@ -258,7 +275,7 @@ class _BatchCodec:
 
 
 class _ReducedOutput:
-    """The device buffers of one reduced output of DctBatchCodec (thumbnails, regions or scaled images) for one key,
+    """The device buffers of one reduced output of a batch codec (thumbnails, regions or scaled images) for one key,
     its parameters: the kernels' work area and the output, plus the page-locked staging a fetch without `out` makes."""
 
     def __init__(self, key, shape, work_bytes, tie_capacity):
@@ -293,7 +310,6 @@ class DctBatchCodec(_BatchCodec):
         self._buffers += [self.d_ties, self.d_stats, self.d_y, self.d_cr, self.d_cb]
         self.forward_stats = np.zeros(4, np.uint32)
         self.inverse_stats = np.zeros(4, np.uint32)
-        self._reduced = {}
 
     def _forward(self):
         _lib.check(self.lib.hic_dct_forward(self.d_rgb.ptr, self.n, self.h, self.w, self.d_coef.ptr, self.d_ties.ptr,
@@ -309,19 +325,6 @@ class DctBatchCodec(_BatchCodec):
 
     def _after_decode(self):
         self.inverse_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
-
-    # ---- reduced outputs: thumbnails, regions and scaled images -----------------------------------------------------
-    def _reduced_buffers(self, kind, key, sizes):
-        """The buffers of reduced output `kind` for its parameters `key`.  Each kind keeps its own, made on first use (a
-        codec that never asks for one pays nothing) and remade only when its key changes; sizes() gives (output shape,
-        work bytes, tie capacity) for a new key."""
-        r = self._reduced.get(kind)
-        if r is not None and r.key == key:
-            return r
-        if r is not None:
-            self._reduced.pop(kind).free()
-        r = self._reduced[kind] = _ReducedOutput(key, *sizes())
-        return r
 
     # ---- 1/8-scale thumbnails from the DC streams alone (codec.jpeg_thumbnail for the whole batch) ---------------
     @property
@@ -462,12 +465,6 @@ class DctBatchCodec(_BatchCodec):
         self.scaled_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
         return pixels
 
-    def close(self):
-        for r in self._reduced.values():
-            r.free()
-        self._reduced = {}
-        super().close()
-
     def coefficients(self):
         """Download the quantised zigzag blocks of the last encode: (n, blocks_per_image, 64) int16."""
         c = self.d_coef.download(np.int16, self.blocks * 64, self.stream)
@@ -516,16 +513,20 @@ class WaveletBatchCodec(_BatchCodec):
         self.general = not settings.wavelet_defaults()
         if self.general:
             g = self.g = _lib.wavelet_pyramid(h, w, settings.WAVELET_NUM_LEVELS)
-            self.params = wavelet._params(g)
-            self._params_ref = ctypes.byref(self.params)
         else:
             g = self.g = _lib.wavelet_geometry(h, w)
+        self.params = wavelet._params(g)           # the scaled decode runs the general kernels at every setting
+        self._params_ref = ctypes.byref(self.params)
         self.chan_elems = 64 * ((int(g.len) + 63) // 64)
         super().__init__(n, h, w, _lib.layout_flat(int(n), int(g.len)), 2 * self.chan_elems * 3 * int(n), (h, w),
                          value_bins, device, stream, device_codes)
+        self.d_work = None             # the general kernels' work area; a default-settings codec makes it for a scaled decode
         if self.general:
-            self.d_work = _lib.DeviceBuffer(_lib.wavelet_work_bytes(n, h, w))
-            self._buffers.append(self.d_work)
+            self._make_work()
+
+    def _make_work(self):
+        self.d_work = _lib.DeviceBuffer(_lib.wavelet_work_bytes(self.n, self.h, self.w))
+        self._buffers.append(self.d_work)
 
     def _forward(self):
         if self.general:
@@ -540,6 +541,50 @@ class WaveletBatchCodec(_BatchCodec):
                                                             self.d_work.ptr, self.d_out.ptr, self.stream))
         else:
             _lib.check(self.lib.hic_wavelet_inverse(self.d_coef_dec.ptr, self.n, self.h, self.w, self.d_out.ptr, self.stream))
+
+    # ---- 1/2- to 1/2^levels-scale images (codec.wavelet_scaled for the whole batch) --------------------------------
+    def scaled_shape(self, scale):
+        """(n, h / scale, w / scale, 3); ValueError for a scale other than 2^k, 1 <= k <= levels, or sides that are not
+        multiples of 2^levels."""
+        levels = int(getattr(self.g, "levels", 3))
+        s = 1 << _lib.wavelet_scale_arg(scale, levels)
+        if self.h % (1 << levels) or self.w % (1 << levels):
+            raise ValueError("a scaled decode of %d levels needs sides that are multiples of %d (got %dx%d)"
+                             % (levels, 1 << levels, self.h, self.w))
+        return (self.n, self.h // s, self.w // s, 3)
+
+    def _scaled_buffers(self, scale):
+        """Check the scale (ValueError before any device work); returns the output buffers for it.  The work area is the
+        codec's, kept across scales; a default-settings codec makes it with its first scaled decode."""
+        shape = self.scaled_shape(scale)
+        if self.d_work is None:
+            self._make_work()
+        return self._reduced_buffers("scaled", int(scale), lambda: (shape, 0, 0))
+
+    def _scaled(self, r):
+        _lib.check(self.lib.hic_wavelet_scaled_general(self.d_coef_dec.ptr, self.n, self.h, self.w, self._params_ref, r.key,
+                                                       self.d_work.ptr, r.d_out.ptr, self.stream))
+
+    def decode_scaled_device(self, scale):
+        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the 1/scale images;
+        they stay on the device (fetch_scaled)."""
+        r = self._scaled_buffers(scale)
+        self._decode_from_encoder(self.d_coef_dec)
+        self._scaled(r)
+
+    def decode_scaled(self, enc, scale, out=None):
+        """The 1/scale images of an EncodedStreams, host to host: image i equals codec.wavelet_scaled of its file.
+        out: optional preallocated uint8 array of scaled_shape(scale)."""
+        r = self._scaled_buffers(scale)
+        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
+        self._scaled(r)
+        return self.fetch_scaled(out)
+
+    def fetch_scaled(self, out=None):
+        """Download the images of the last decode_scaled() / decode_scaled_device()."""
+        r = self._reduced["scaled"]
+        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
+        return pixels
 
     def hic_images(self, enc, images=None):
         from hiccup_b200 import wavelet

@@ -388,3 +388,8 @@ def wavelet_encode(compressed: model.CompressedImage, restarts: bool = False) ->
 def wavelet_decode(hic: hicimage.HicImage) -> model.CompressedImage:
     from hiccup_b200 import wavelet
     return wavelet.wavelet_decode(hic)
+
+
+def wavelet_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
+    from hiccup_b200 import wavelet
+    return wavelet.wavelet_scaled(hic, scale)

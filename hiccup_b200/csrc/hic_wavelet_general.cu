@@ -240,6 +240,23 @@ finish_kernel(const double* __restrict__ plane, int64_t pixels, int64_t total, u
     o[2] = (uint8_t)b;
 }
 
+// finish_kernel for the 1/s-scale image: the running approximation A_k (s = 2^k) times 2^-k (exact) is the mean of
+// each s x s tile of the unrounded image
+__global__ void __launch_bounds__(256)
+scaled_finish_kernel(const double* __restrict__ plane, int64_t pixels, int64_t total, double inv_scale, uint8_t* __restrict__ rgb) {
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= total) return;
+    const int64_t img = gid / pixels, p = gid - img * pixels;
+    const double* s = plane + img * 3 * pixels + p;
+    int r, gg, b;
+    ycrcb_to_rgb(wrap_u8(dadd(dmul(s[0], inv_scale), 256.0)), wrap_u8(dadd(dmul(s[pixels], inv_scale), 256.0)),
+                 wrap_u8(dadd(dmul(s[2 * pixels], inv_scale), 256.0)), r, gg, b);
+    uint8_t* o = rgb + gid * 3;
+    o[0] = (uint8_t)r;
+    o[1] = (uint8_t)gg;
+    o[2] = (uint8_t)b;
+}
+
 // ---- layout converters: flat zigzag stream <-> 3 L + 1 raster int32 sub-bands ----
 __global__ void __launch_bounds__(256)
 flat_to_bands_kernel(const int16_t* __restrict__ flat, Pyr g, int64_t n3, int32_t* __restrict__ bands) {
@@ -372,6 +389,42 @@ int hic_wavelet_inverse_general(const int16_t* d_flat, int32_t n, int32_t h, int
     }
     // plane[cur] holds channel-planar float64 samples; its (image, channel) stride is h * w
     HIC_LAUNCH("wavelet_finish_kernel", st, wvg::finish_kernel<<<wvg::blocks_for(pixels * n), 256, 0, st>>>(plane[cur], pixels, pixels * n, d_rgb_out));
+    return HIC_OK;
+}
+
+int hic_wavelet_scaled_general(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, const hic_wavelet_params* params,
+                               int32_t scale, void* d_work, uint8_t* d_rgb_out, void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_rgb_out && d_flat && d_work, "NULL device pointer");
+    HIC_REQUIRE(n >= 1 && n <= 65535, "batch size must be in 1..65535 (got %d)", n);
+    int rc = wvg::check_params(params);
+    if (rc) return rc;
+    const int L = params->levels;
+    int k = 1;
+    while (k < L && (1 << k) < scale) ++k;
+    HIC_REQUIRE(scale == (1 << k), "scale must be 2^k with 1 <= k <= %d levels (got %d)", L, scale);
+    HIC_REQUIRE(h % (1 << L) == 0 && w % (1 << L) == 0, "a scaled decode of %d levels needs multiples of %d (got %dx%d)", L,
+                1 << L, h, w);
+    wvg::Pyr g;
+    rc = wvg::make(h, w, L, &g);
+    if (rc) return rc;
+    cudaStream_t st = as_stream(stream);
+    const int64_t n3 = 3 * (int64_t)n, pixels = (int64_t)g.p.lh[k] * g.p.lw[k];
+    double* plane[2] = {static_cast<double*>(d_work), static_cast<double*>(d_work) + wvg::plane_doubles(n, h, w)};
+    int cur = (L - k) & 1;                                          // so that the last level lands in plane[0]
+    HIC_LAUNCH("wavelet_approximation_load_kernel", st, wvg::approximation_load_kernel<<<wvg::blocks_for((int64_t)g.p.lh[L] * g.p.lw[L] * n3), 256, 0, st>>>(
+        d_flat, g, g.p.lh[L], g.p.lw[L], (int64_t)g.p.lh[L] * g.p.lw[L], n3, plane[cur]));
+    for (int l = L; l > k; --l) {                                   // the first L - k levels of the full inverse
+        const int ho = g.p.lh[l], wo = g.p.lw[l];
+        const int i = L - l;
+        const double mul = params->multiplier * (double)(i * i + 1);
+        HIC_LAUNCH("wavelet_inverse_level_kernel", st, wvg::inverse_level_kernel<<<wvg::blocks_for((int64_t)ho * wo * n3), 256, 0, st>>>(
+            plane[cur], ho, wo, (int64_t)ho * wo, plane[cur ^ 1], g.p.lh[l - 1], g.p.lw[l - 1], n3, g, 1 + 3 * i, mul, d_flat));
+        cur ^= 1;
+    }
+    // plane[cur] holds A_k, channel-planar; its (image, channel) stride is lh[k] * lw[k] = (h / scale) (w / scale)
+    HIC_LAUNCH("wavelet_scaled_finish_kernel", st, wvg::scaled_finish_kernel<<<wvg::blocks_for(pixels * n), 256, 0, st>>>(
+        plane[cur], pixels, pixels * n, 1.0 / scale, d_rgb_out));
     return HIC_OK;
 }
 

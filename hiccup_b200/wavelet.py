@@ -2,6 +2,7 @@
 
     wavelet_compression(rgb)      compression.py:59-85      wavelet_encode(c)    codec.py:116-163
     wavelet_decompression(c)      compression.py:88-100     wavelet_decode(hic)  codec.py:199-239
+    wavelet_scaled(hic, scale)    no reference counterpart: the 1/2- to 1/2^L-scale image (include/hiccup_b200.h)
 
 The numeric work runs in csrc/hic_wavelet.cu (K9 / K10, the fused kernels for the default settings),
 csrc/hic_wavelet_general.cu (any WAVELET_NUM_LEVELS in 1..5, multiplier, threshold and quality factor:
@@ -294,17 +295,52 @@ def wavelet_decompression(channels: model.CompressedImage) -> np.ndarray:
         if levels == 3 and settings.WAVELET_SUBBAND_QUANTIZATION_MULTIPLIER == 1 and h % 8 == 0 and w % 8 == 0:
             _lib.check(lib.hic_wavelet_inverse(flat.ptr, 1, h, w, rgb.ptr, None))
         else:
-            params = _lib.WaveletParams()
-            params.levels, params.multiplier = levels, float(settings.WAVELET_SUBBAND_QUANTIZATION_MULTIPLIER)
-            params.threshold, params.threshold_index = 0.0, -1
-            work = _lib.scratch(_lib.wavelet_work_bytes(1, h, w))
-            try:
-                _lib.check(lib.hic_wavelet_inverse_general(flat.ptr, 1, h, w, ctypes.byref(params), work.ptr, rgb.ptr, None))
-                _lib.sync()
-            finally:
-                work.free()
+            _run_general(lib.hic_wavelet_inverse_general, flat, h, w, levels, (), rgb)
         out = rgb.download(np.uint8, h * w * 3).reshape(h, w, 3)
     finally:
         flat.free()
         rgb.free()
     return out
+
+
+def _run_general(entry, flat, h, w, levels, extra, rgb):
+    """hic_wavelet_inverse_general or hic_wavelet_scaled_general (extra = (scale,)) on one image, with a work area of its
+    own, at `levels` and the multiplier of the settings now."""
+    params = _lib.WaveletParams()
+    params.levels, params.multiplier = levels, float(settings.WAVELET_SUBBAND_QUANTIZATION_MULTIPLIER)
+    params.threshold, params.threshold_index = 0.0, -1
+    work = _lib.scratch(_lib.wavelet_work_bytes(1, h, w))
+    try:
+        _lib.check(entry(flat.ptr, 1, h, w, ctypes.byref(params), *extra, work.ptr, rgb.ptr, None))
+        _lib.sync()
+    finally:
+        work.free()
+
+
+def wavelet_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
+    """The 1/scale image of a wavelet-mode file of L levels: (h / scale, w / scale, 3) uint8, scale = 2^k with
+    1 <= k <= L.  Each sample is astype(uint8)(A_k * 2^-k + 256) of the running approximation A_k the full inverse holds
+    after its first L - k levels -- the mean of each scale x scale tile of the unrounded full reconstruction -- and the
+    three planes are converted to RGB as wavelet_decompression does (include/hiccup_b200.h, hic_wavelet_scaled_general,
+    at the file's levels and the multiplier of the settings now).  The entropy decode is wavelet_decode's (restart
+    records used when the file has them); the inverse transform stops k levels early and reads only the coarse
+    sub-bands.  NotImplementedError for a DCT-mode file, ValueError for a bad scale or a pyramid pyramid_of_file
+    refuses, all before any device work."""
+    from hiccup_b200 import codec
+    if codec._is_dct(hic):
+        raise NotImplementedError("wavelet scaled decode works on wavelet-mode (HIC) files; this is a DCT-mode (JPEG) file")
+    settings.check_wavelet_supported()
+    g = pyramid_of_file(hic)
+    h, w, levels = int(g.h), int(g.w), _levels_of(g)
+    _lib.wavelet_scale_arg(scale, levels)
+    scale = int(scale)
+    _lib.require_device()
+    sh, sw = h // scale, w // scale
+    flat, _ = decode_to_device_flat(hic)
+    rgb = _lib.scratch(sh * sw * 3)
+    try:
+        _run_general(_lib.load().hic_wavelet_scaled_general, flat, h, w, levels, (scale,), rgb)
+        return rgb.download(np.uint8, sh * sw * 3).reshape(sh, sw, 3)
+    finally:
+        flat.free()
+        rgb.free()

@@ -288,6 +288,20 @@ int hic_wavelet_forward_general(const uint8_t* d_rgb, int32_t n, int32_t h, int3
  * image pywt.waverec2 returns (it trims the extra row / column between levels of odd size) */
 int hic_wavelet_inverse_general(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, const hic_wavelet_params* params,
                                 void* d_work, uint8_t* d_rgb_out, void* stream);
+/* Scaled decode -- the 1/s-scale image of a wavelet file of L = params->levels levels, s = 2^k with
+ * 1 <= k <= L, h and w multiples of 2^L: (h / s) x (w / s) x 3 per image into d_rgb_out.  Per channel:
+ * dequantise as compression.wavelet_decompression does (A_L = cA_L; detail group i, 0 = coarsest, times
+ * params->multiplier * (i*i + 1); the thresholds are not used); A_k is the running approximation after the
+ * first L - k reconstruction levels of waverec2 -- the same operations in the same order as
+ * hic_wavelet_inverse_general, so bit for bit the intermediate it holds (at k = L, cA_L itself);
+ * sample = astype(uint8)(A_k * 2^-k + 256) (the product is exact; truncation toward zero, wrap).  The three
+ * reduced planes go through ycrcb_to_rgb (no chroma subsampling, no crop).  For db1, A_k * 2^-k is the mean
+ * of each s x s tile of the unrounded full reconstruction.  Only cA_L and the detail bands of levels
+ * L .. k + 1 are read.  d_work: hic_wavelet_general_work_bytes(n, h, w).  Returns HIC_ERR_INVALID for a bad
+ * scale or shape before anything is launched.  This is also the path at the default settings: a fused
+ * K10-style kernel measured slower on a B200 (DESIGN.md section 6). */
+int hic_wavelet_scaled_general(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, const hic_wavelet_params* params,
+                               int32_t scale, void* d_work, uint8_t* d_rgb_out, void* stream);
 int hic_wavelet_flat_to_bands_general(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, int32_t levels, int32_t* d_bands,
                                       void* stream);
 int hic_wavelet_bands_to_flat_general(const int32_t* d_bands, int32_t n, int32_t h, int32_t w, int32_t levels, int16_t* d_flat,

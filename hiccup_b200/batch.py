@@ -11,6 +11,7 @@ kernels as the single-image drop-in functions (compression.py / codec.py / wavel
 images.  Host-side results are views of page-locked staging owned by the codec (valid until the next
 call of the same method).
 """
+import functools
 import os
 
 import numpy as np
@@ -175,6 +176,14 @@ class _BatchCodec:
         run = self.decoder.run_dc if dc_only else self.decoder.run
         run(enc._out.ptr, enc.byte_off, enc.nbits, d_dst.ptr, st)
 
+    def _decode_from_streams(self, enc, d_dst, dc_only=False):
+        """D1-D3 of an EncodedStreams (its tables and bytes go up) into d_dst: the coefficient blocks, or with dc_only the
+        DC streams alone, one value per block (only their tables and bytes go up; EntropyDecoder.decode_dc)."""
+        if dc_only:
+            self.decoder.decode_dc(*entropy.dc_streams_only(enc), d_dst.ptr, self.stream)
+        else:
+            self.decoder.decode_streams(enc, d_dst.ptr, self.stream)
+
     # ---- host-to-host entry points -----------------------------------------------------------
     def encode(self, rgb):
         self.upload(rgb)
@@ -220,7 +229,7 @@ class _BatchCodec:
 
     def decode_resident(self, enc):
         """Entropy-decode and inverse-transform an EncodedStreams; the pixels stay on the device."""
-        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
+        self._decode_from_streams(enc, self.d_coef_dec)
         self._inverse()
 
     def fetch(self, out=None):
@@ -249,6 +258,9 @@ class _BatchCodec:
     def _after_decode(self):
         pass
 
+    def _after_scaled(self):
+        pass
+
     # ---- reduced outputs (thumbnails, regions, scaled images) ---------------------------------------------------------
     def _reduced_buffers(self, kind, key, sizes):
         """The buffers of reduced output `kind` for its parameters `key`.  Each kind keeps its own, made on first use (a
@@ -261,6 +273,43 @@ class _BatchCodec:
             self._reduced.pop(kind).free()
         r = self._reduced[kind] = _ReducedOutput(key, *sizes())
         return r
+
+    def _run_reduced(self, r, launch, enc=None, dc_only=False, d_src=None):
+        """D1-D3 into d_src (default the coefficient buffer of decode_device) -- from the encoder's own device-resident
+        output (decode_device's hand-over) or, given `enc`, from that EncodedStreams; all streams, or with dc_only the DC
+        streams alone -- then launch(r), the kernels of reduced output r."""
+        d_src = self.d_coef_dec if d_src is None else d_src
+        if enc is None:
+            self._decode_from_encoder(d_src, dc_only)
+        else:
+            self._decode_from_streams(enc, d_src, dc_only)
+        launch(r)
+
+    def _fetch_reduced(self, r, out):
+        """Download reduced output r into `out` or, without one, into its page-locked staging."""
+        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
+        return pixels
+
+    # ---- 1/scale images (codec.jpeg_scaled or codec.wavelet_scaled for the whole batch); the subclasses provide
+    # scaled_shape(scale), _scaled_buffers(scale) and _scaled(r) ------------------------------------------------------
+    def decode_scaled_device(self, scale):
+        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the 1/scale images;
+        they stay on the device (fetch_scaled)."""
+        self._run_reduced(self._scaled_buffers(scale), self._scaled)
+
+    def decode_scaled(self, enc, scale, out=None):
+        """The 1/scale images of an EncodedStreams, host to host: image i equals codec.jpeg_scaled (scale 2 or 4) or
+        codec.wavelet_scaled of its file, as the codec's mode.  out: optional preallocated uint8 array of
+        scaled_shape(scale)."""
+        self._run_reduced(self._scaled_buffers(scale), self._scaled, enc)
+        return self.fetch_scaled(out)
+
+    def fetch_scaled(self, out=None):
+        """Download the images of the last decode_scaled() / decode_scaled_device() (and, in DCT mode, their tie
+        statistics into scaled_stats)."""
+        pixels = self._fetch_reduced(self._reduced["scaled"], out)
+        self._after_scaled()
+        return pixels
 
     def close(self):
         for r in self._reduced.values():
@@ -343,24 +392,19 @@ class DctBatchCodec(_BatchCodec):
         """DC-only D1 + D3 and the thumbnail kernel from the encoder's own device-resident output (decode_device's
         hand-over); the thumbnails stay on the device (fetch_thumbnails)."""
         r = self._thumbnail_buffers()
-        self._decode_from_encoder(r.d_work, dc_only=True)
-        self._thumbnail(r)
+        self._run_reduced(r, self._thumbnail, dc_only=True, d_src=r.d_work)
 
     def thumbnails(self, enc, out=None):
         """Thumbnails of an EncodedStreams (encode() or read_files() / streams_from_files()), host to host: only the
         DC streams' tables and bytes go up, n x th x tw x 3 comes down.  out: optional preallocated uint8 array of
         thumbnail_shape."""
         r = self._thumbnail_buffers()
-        index, symbols, packed, data, byte_off, nbits = entropy.dc_streams_only(enc)
-        self.decoder.decode_dc(index, symbols, packed, data, byte_off, nbits, r.d_work.ptr, self.stream)
-        self._thumbnail(r)
+        self._run_reduced(r, self._thumbnail, enc, dc_only=True, d_src=r.d_work)
         return self.fetch_thumbnails(out)
 
     def fetch_thumbnails(self, out=None):
         """Download the thumbnails of the last thumbnails() / thumbnails_device()."""
-        r = self._thumbnail_buffers()
-        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
-        return pixels
+        return self._fetch_reduced(self._thumbnail_buffers(), out)
 
     # ---- regions: one height x width window per image, of the full-resolution image (codec.jpeg_region for the whole
     # batch) or of the 1/2-, 1/4- or 1/8-scale image (jpeg_region(..., scale)) ----------------------------------------
@@ -399,8 +443,7 @@ class DctBatchCodec(_BatchCodec):
         thumbnails_device), then the windows of size = (height, width) at origins ((n, 2) of (top, left), in the
         coordinates of the 1/scale image); they stay on the device (fetch_regions)."""
         origins, r = self._region_buffers(origins, size, scale)
-        self._decode_from_encoder(self.d_coef_dec, dc_only=r.key[2] == 8)
-        self._region(origins, r)
+        self._run_reduced(r, functools.partial(self._region, origins), dc_only=r.key[2] == 8)
 
     def decode_regions(self, enc, origins, size, out=None, scale=1):
         """Windows of an EncodedStreams, host to host: image i's window is decode(enc)[i, top:top+height,
@@ -408,19 +451,14 @@ class DctBatchCodec(_BatchCodec):
         same window of decode_scaled(enc, scale)[i], at scale 8 of thumbnails(enc)[i] (only the DC streams go up).
         out: optional preallocated uint8 array of (n, height, width, 3)."""
         origins, r = self._region_buffers(origins, size, scale)
-        if r.key[2] == 8:
-            index, symbols, packed, data, byte_off, nbits = entropy.dc_streams_only(enc)
-            self.decoder.decode_dc(index, symbols, packed, data, byte_off, nbits, self.d_coef_dec.ptr, self.stream)
-        else:
-            self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
-        self._region(origins, r)
+        self._run_reduced(r, functools.partial(self._region, origins), enc, dc_only=r.key[2] == 8)
         return self.fetch_regions(out)
 
     def fetch_regions(self, out=None):
         """Download the windows of the last decode_regions() / decode_regions_device() (and their tie statistics
         into region_stats; all zero at scale 8, which has no tie stage)."""
         r = self._reduced["region"]
-        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
+        pixels = self._fetch_reduced(r, out)
         if r.key[2] == 8:
             self.region_stats = np.zeros(_lib.TIE_STATS, np.uint32)
         else:
@@ -442,28 +480,8 @@ class DctBatchCodec(_BatchCodec):
         _lib.check(self.lib.hic_dct_scaled(self.d_coef_dec.ptr, self.n, self.h, self.w, r.key, r.d_work.ptr, r.work_bytes,
                                            self.d_ties.ptr, r.tie_capacity, self.d_stats.ptr, r.d_out.ptr, self.stream))
 
-    def decode_scaled_device(self, scale):
-        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the 1/scale images;
-        they stay on the device (fetch_scaled)."""
-        r = self._scaled_buffers(scale)
-        self._decode_from_encoder(self.d_coef_dec)
-        self._scaled(r)
-
-    def decode_scaled(self, enc, scale, out=None):
-        """The 1/scale images (scale 2 or 4) of an EncodedStreams, host to host: image i equals
-        codec.jpeg_scaled of its file.  out: optional preallocated uint8 array of scaled_shape(scale)."""
-        r = self._scaled_buffers(scale)
-        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
-        self._scaled(r)
-        return self.fetch_scaled(out)
-
-    def fetch_scaled(self, out=None):
-        """Download the images of the last decode_scaled() / decode_scaled_device() (and their tie statistics into
-        scaled_stats)."""
-        r = self._reduced["scaled"]
-        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
+    def _after_scaled(self):
         self.scaled_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
-        return pixels
 
     def coefficients(self):
         """Download the quantised zigzag blocks of the last encode: (n, blocks_per_image, 64) int16."""
@@ -564,27 +582,6 @@ class WaveletBatchCodec(_BatchCodec):
     def _scaled(self, r):
         _lib.check(self.lib.hic_wavelet_scaled_general(self.d_coef_dec.ptr, self.n, self.h, self.w, self._params_ref, r.key,
                                                        self.d_work.ptr, r.d_out.ptr, self.stream))
-
-    def decode_scaled_device(self, scale):
-        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over), then the 1/scale images;
-        they stay on the device (fetch_scaled)."""
-        r = self._scaled_buffers(scale)
-        self._decode_from_encoder(self.d_coef_dec)
-        self._scaled(r)
-
-    def decode_scaled(self, enc, scale, out=None):
-        """The 1/scale images of an EncodedStreams, host to host: image i equals codec.wavelet_scaled of its file.
-        out: optional preallocated uint8 array of scaled_shape(scale)."""
-        r = self._scaled_buffers(scale)
-        self.decoder.decode_streams(enc, self.d_coef_dec.ptr, self.stream)
-        self._scaled(r)
-        return self.fetch_scaled(out)
-
-    def fetch_scaled(self, out=None):
-        """Download the images of the last decode_scaled() / decode_scaled_device()."""
-        r = self._reduced["scaled"]
-        pixels, r.h_out = self._download(r.d_out, r.shape, out, r.h_out)
-        return pixels
 
     def hic_images(self, enc, images=None):
         from hiccup_b200 import wavelet

@@ -279,16 +279,9 @@ def jpeg_thumbnail(hic: hicimage.HicImage) -> np.ndarray:
     settings.check_supported()
     _lib.require_device()
     _, h, w, g = _dct_header(hic)
-    th, tw = _lib.thumbnail_shape(h, w)
-    d_dc = _lib.scratch(2 * g.blocks_per_image)
-    out = _lib.scratch(3 * th * tw)
-    try:
-        _decode_dc(hic, h, w, d_dc.ptr)
-        _lib.check(_lib.load().hic_dct_thumbnail(d_dc.ptr, 1, h, w, out.ptr, None))
-        return out.download(np.uint8, 3 * th * tw).reshape(th, tw, 3)
-    finally:
-        d_dc.free()
-        out.free()
+    lib = _lib.load()
+    return _reduced_decode(hic, h, w, g, _lib.thumbnail_shape(h, w) + (3,),
+                           lambda dc, out: lib.hic_dct_thumbnail(dc, 1, h, w, out, None), dc_only=True)
 
 
 def _decode_dc(hic, h, w, d_dc):
@@ -309,21 +302,31 @@ def _decode_dc(hic, h, w, d_dc):
     dec.decode_dc(index, syms, packed, data, offs, nbits, d_dc, restarts=records)
 
 
-def _reduced_decode(hic, h, w, g, launch, params, sizes, shape):
-    """jpeg_decode's entropy stage into a coefficient buffer, then `launch` -- hic_dct_region or hic_dct_scaled, called as
-    (coef, 1, h, w, *params, work, work bytes, ties, tie capacity, stats, out, stream) with the (work bytes, tie capacity)
-    of `sizes` -- into a uint8 image of `shape`, which is returned."""
-    work_bytes, tie_cap = sizes
-    bufs = [_lib.scratch(g.blocks_per_image * 128), _lib.scratch(work_bytes), _lib.scratch(tie_cap * _lib.TIE_RECORD_BYTES),
-            _lib.scratch(4 * _lib.TIE_STATS), _lib.scratch(int(np.prod(shape)))]
-    coef, work, ties, stats, out = bufs
+def _reduced_decode(hic, h, w, g, shape, launch, scratch=(), dc_only=False):
+    """jpeg_decode's entropy stage into a device buffer -- all nine streams into coefficient blocks, or (dc_only) the DC
+    streams alone into one int16 per block (_decode_dc) -- then launch(src, out, *scratch pointers) with that buffer, a
+    uint8 image of `shape` and one scratch buffer per byte count in `scratch`.  The image is returned."""
+    size = int(np.prod(shape))
+    bufs = [_lib.scratch(g.blocks_per_image * (2 if dc_only else 128)), _lib.scratch(size)]
+    bufs += [_lib.scratch(b) for b in scratch]
     try:
-        _decode_coefficients(hic, h, w, coef.ptr)
-        _lib.check(launch(coef.ptr, 1, h, w, *params, work.ptr, work_bytes, ties.ptr, tie_cap, stats.ptr, out.ptr, None))
-        return out.download(np.uint8, int(np.prod(shape))).reshape(shape)
+        (_decode_dc if dc_only else _decode_coefficients)(hic, h, w, bufs[0].ptr)
+        _lib.check(launch(*(b.ptr for b in bufs)))
+        return bufs[1].download(np.uint8, size).reshape(shape)
     finally:
         for b in bufs:
             b.free()
+
+
+def _tie_stage(entry, h, w, params, sizes):
+    """(launch, scratch) of _reduced_decode for hic_dct_region, hic_dct_scaled or hic_dct_scaled_region, called as
+    (coef, 1, h, w, *params, work, work bytes, ties, tie capacity, stats, out, stream) with the (work bytes, tie
+    capacity) of `sizes`."""
+    work_bytes, tie_cap = sizes
+
+    def launch(coef, out, work, ties, stats):
+        return entry(coef, 1, h, w, *params, work, work_bytes, ties, tie_cap, stats, out, None)
+    return launch, (work_bytes, tie_cap * _lib.TIE_RECORD_BYTES, 4 * _lib.TIE_STATS)
 
 
 def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int, scale: int = 1) -> np.ndarray:
@@ -343,24 +346,19 @@ def jpeg_region(hic: hicimage.HicImage, top: int, left: int, height: int, width:
     settings.check_supported()
     _lib.require_device()
     height, width = int(height), int(width)
-    lib = _lib.load()
+    lib, o = _lib.load(), origin.ctypes.data
     if scale == 1:
-        return _reduced_decode(hic, h, w, g, lib.hic_dct_region, (origin.ctypes.data, height, width),
-                               _lib.region_sizes(1, h, w, height, width), (height, width, 3))
-    sizes = _lib.scaled_region_sizes(1, h, w, scale, height, width)
-    if scale != 8:
-        return _reduced_decode(hic, h, w, g, lib.hic_dct_scaled_region, (scale, origin.ctypes.data, height, width), sizes,
-                               (height, width, 3))
-    bufs = [_lib.scratch(2 * g.blocks_per_image), _lib.scratch(sizes[0]), _lib.scratch(3 * height * width)]
-    d_dc, work, out = bufs
-    try:
-        _decode_dc(hic, h, w, d_dc.ptr)
-        _lib.check(lib.hic_dct_thumbnail_region(d_dc.ptr, 1, h, w, origin.ctypes.data, height, width, work.ptr, sizes[0],
-                                                out.ptr, None))
-        return out.download(np.uint8, 3 * height * width).reshape(height, width, 3)
-    finally:
-        for b in bufs:
-            b.free()
+        launch, scratch = _tie_stage(lib.hic_dct_region, h, w, (o, height, width), _lib.region_sizes(1, h, w, height, width))
+    elif scale != 8:
+        launch, scratch = _tie_stage(lib.hic_dct_scaled_region, h, w, (scale, o, height, width),
+                                     _lib.scaled_region_sizes(1, h, w, scale, height, width))
+    else:
+        work_bytes = _lib.scaled_region_sizes(1, h, w, 8, height, width)[0]
+        scratch = (work_bytes,)
+
+        def launch(dc, out, work):
+            return lib.hic_dct_thumbnail_region(dc, 1, h, w, o, height, width, work, work_bytes, out, None)
+    return _reduced_decode(hic, h, w, g, (height, width, 3), launch, scratch, dc_only=scale == 8)
 
 
 def jpeg_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
@@ -375,8 +373,8 @@ def jpeg_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
     _, h, w, g = _dct_header(hic)
     settings.check_supported()
     _lib.require_device()
-    return _reduced_decode(hic, h, w, g, _lib.load().hic_dct_scaled, (scale,), _lib.scaled_sizes(1, h, w, scale),
-                           _lib.scaled_shape(h, w, scale) + (3,))
+    return _reduced_decode(hic, h, w, g, _lib.scaled_shape(h, w, scale) + (3,),
+                           *_tie_stage(_lib.load().hic_dct_scaled, h, w, (scale,), _lib.scaled_sizes(1, h, w, scale)))
 
 
 def wavelet_encode(compressed: model.CompressedImage, restarts: bool = False) -> hicimage.HicImage:

@@ -9,6 +9,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <mutex>
+#include <type_traits>
 #include "hic_core.cuh"
 #include "hic_dct_bound.h"
 #include "hic_f32x2.cuh"
@@ -1829,6 +1830,15 @@ static int coef_block_map(CUtensorMap* map, const int16_t* d_coef, int64_t block
     return HIC_OK;
 }
 
+// f(std::integral_constant<int, M>()) for M = 8 / scale samples per block side: scale 2 or 4, or 1 too where FULL (the
+// scaled launches leave it out, so that no scaled kernel is instantiated for M = 8)
+template <bool FULL, class F>
+static auto by_samples(int scale, F f) {
+    if constexpr (FULL)
+        if (scale == 1) return f(std::integral_constant<int, 8>());
+    return scale == 2 ? f(std::integral_constant<int, 4>()) : f(std::integral_constant<int, 2>());
+}
+
 // K7S, its fix-up and K8S of hic_dct_scaled for M x M samples per block (scale 8 / M)
 template <int M>
 static int scaled_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, int sh, int sw, uint8_t* d_work,
@@ -1845,37 +1855,66 @@ static int scaled_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n
     return HIC_OK;
 }
 
-// The kernels' view of a region work buffer of layout L (origins at its head, already copied there)
-static k7::RegionArgs region_args(uint8_t* d_work, int n, const RegionLayout& L, int rh, int rw) {
-    k7::RegionArgs a;
-    a.origin = reinterpret_cast<const int32_t*>(d_work);
-    a.y = d_work + L.head;
-    a.cr = a.y + (size_t)n * L.ly;
-    a.cb = a.cr + (size_t)n * L.lc;
-    a.ly = L.ly;
-    a.lc = L.lc;
-    a.s = L.s;
-    a.rh = rh;
-    a.rw = rw;
-    return a;
+// Every origin of the windowed entries names an rh x rw window inside the 1/scale image
+static int check_origins(const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw, int scale) {
+    for (int i = 0; i < n; ++i) {
+        const int rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw, scale);
+        if (rc) return rc;
+    }
+    return HIC_OK;
 }
 
-// The rest of hic_dct_scaled_region for M x M samples per block (scale 8 / M): the work buffer's checks, the origins'
-// copy, K7SR, its fix-up and K8SR
+// The body of hic_dct_region_blocks (scale 1) and hic_dct_scaled_region_blocks (scale 2 or 4)
+static int region_blocks(int h, int w, int scale, int top, int left, int rh, int rw, int32_t* rect) {
+    hic_dct_geometry g;
+    int rc = geometry_of(h, w, &g);
+    if (rc) return rc;
+    rc = region_check(g, top, left, rh, rw, scale);
+    if (rc) return rc;
+    by_samples<true>(scale, [&](auto m) { region_rect<decltype(m)::value>(g, top, left, rh, rw, rect); });
+    return HIC_OK;
+}
+
+// The work buffer and tie capacity of n rh x rw windows at scale 1, 2 or 4, once the sizes entries' checks hold
+static int region_sizes(int n, const hic_dct_geometry& g, int scale, int rh, int rw, size_t* work_bytes, uint32_t* tie_capacity) {
+    const RegionLayout L = by_samples<true>(scale, [&](auto m) { return region_layout<decltype(m)::value>(n, g, rh, rw); });
+    HIC_REQUIRE(L.blocks < (1ull << 32), "batch too large: %llu selected blocks", (unsigned long long)L.blocks);
+    *work_bytes = L.total;
+    *tie_capacity = (uint32_t)L.blocks;
+    return HIC_OK;
+}
+
+// hic_dct_region's (M = 8) and hic_dct_scaled_region's (M = 4, 2) set-up once the origins are checked: *a is the
+// kernels' view of the work buffer, with the origins copied to its head, and *blocks the number of selected blocks
 template <int M>
-static int scaled_region_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
-                                uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity,
-                                uint32_t* d_stats, uint8_t* d_rgb_out, cudaStream_t st) {
+static int region_prepare(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
+                          uint8_t* d_work, size_t work_bytes, uint32_t* d_stats, cudaStream_t st, k7::RegionArgs* a,
+                          int64_t* blocks) {
     const RegionLayout L = region_layout<M>(n, g, rh, rw);
-    HIC_REQUIRE(work_bytes >= L.total, "work buffer of %zu bytes is too small: %zu needed (hic_dct_scaled_region_sizes)", work_bytes, L.total);
+    HIC_REQUIRE(work_bytes >= L.total, "work buffer of %zu bytes is too small: %zu needed (%s)", work_bytes, L.total,
+                M == 8 ? "hic_dct_region_sizes" : "hic_dct_scaled_region_sizes");
     HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
                 "d_coef and d_work must be 16-byte aligned");
     const int rc = ensure_tables();
     if (rc) return rc;
     HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
     HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    const k7::RegionArgs a = region_args(d_work, n, L, rh, rw);
-    HIC_LAUNCH("scaled_region_inverse_kernel", st, k7::scaled_region_inverse_kernel<M><<<grid_for((int64_t)L.blocks, k7::K7S_THREADS), k7::K7S_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
+    uint8_t* y = d_work + L.head;     // the n Y planes, then the n Cr and the n Cb planes
+    *a = {reinterpret_cast<const int32_t*>(d_work), y, y + (size_t)n * L.ly, y + (size_t)n * (L.ly + L.lc), L.ly, L.lc, L.s, rh, rw};
+    *blocks = (int64_t)L.blocks;
+    return HIC_OK;
+}
+
+// K7SR, its fix-up and K8SR of hic_dct_scaled_region for M x M samples per block (scale 8 / M)
+template <int M>
+static int scaled_region_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
+                                uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity,
+                                uint32_t* d_stats, uint8_t* d_rgb_out, cudaStream_t st) {
+    k7::RegionArgs a;
+    int64_t blocks = 0;
+    const int rc = region_prepare<M>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_stats, st, &a, &blocks);
+    if (rc) return rc;
+    HIC_LAUNCH("scaled_region_inverse_kernel", st, k7::scaled_region_inverse_kernel<M><<<grid_for(blocks, k7::K7S_THREADS), k7::K7S_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("scaled_region_fixup_kernel", st, k7::scaled_region_fixup_kernel<M><<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("scaled_region_colour_kernel", st, k7::scaled_region_colour_kernel<M><<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
     return HIC_OK;
@@ -2075,13 +2114,7 @@ int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint
 int hic_dct_region_blocks(int32_t h, int32_t w, int32_t top, int32_t left, int32_t rh, int32_t rw, int32_t* rect) {
     using namespace hic;
     HIC_REQUIRE(rect != nullptr, "NULL argument");
-    hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
-    if (rc) return rc;
-    rc = region_check(g, top, left, rh, rw);
-    if (rc) return rc;
-    region_rect<8>(g, top, left, rh, rw, rect);
-    return HIC_OK;
+    return region_blocks(h, w, 1, top, left, rh, rw, rect);
 }
 
 int hic_dct_region_sizes(int32_t n, int32_t h, int32_t w, int32_t rh, int32_t rw, size_t* work_bytes, uint32_t* tie_capacity) {
@@ -2092,11 +2125,7 @@ int hic_dct_region_sizes(int32_t n, int32_t h, int32_t w, int32_t rh, int32_t rw
     if (rc) return rc;
     rc = region_check(g, 0, 0, rh, rw);
     if (rc) return rc;
-    const RegionLayout L = region_layout(n, g, rh, rw);
-    HIC_REQUIRE(L.blocks < (1ull << 32), "batch too large: %llu selected blocks", (unsigned long long)L.blocks);
-    *work_bytes = L.total;
-    *tie_capacity = (uint32_t)L.blocks;
-    return HIC_OK;
+    return region_sizes(n, g, 1, rh, rw, work_bytes, tie_capacity);
 }
 
 int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const int32_t* h_origin, int32_t rh,
@@ -2107,21 +2136,14 @@ int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const
     hic_dct_geometry g;
     int rc = batch_geometry(n, h, w, true, &g);
     if (rc) return rc;
-    for (int i = 0; i < n; ++i) {
-        rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw);
-        if (rc) return rc;
-    }
-    const RegionLayout L = region_layout(n, g, rh, rw);
-    HIC_REQUIRE(work_bytes >= L.total, "work buffer of %zu bytes is too small: %zu needed (hic_dct_region_sizes)", work_bytes, L.total);
-    HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
-                "d_coef and d_work must be 16-byte aligned");
-    rc = ensure_tables();
+    rc = check_origins(g, n, h_origin, rh, rw, 1);
     if (rc) return rc;
     cudaStream_t st = as_stream(stream);
-    HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
-    HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    const k7::RegionArgs a = region_args(d_work, n, L, rh, rw);
-    HIC_LAUNCH("region_inverse_kernel", st, k7::region_inverse_kernel<<<grid_for((int64_t)L.blocks, k7::K7R_THREADS), k7::K7R_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
+    k7::RegionArgs a;
+    int64_t blocks = 0;
+    rc = region_prepare<8>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_stats, st, &a, &blocks);
+    if (rc) return rc;
+    HIC_LAUNCH("region_inverse_kernel", st, k7::region_inverse_kernel<<<grid_for(blocks, k7::K7R_THREADS), k7::K7R_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("region_fixup_kernel", st, k7::region_fixup_kernel<<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
     HIC_LAUNCH("region_colour_kernel", st, k7::region_colour_kernel<<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
     return HIC_OK;
@@ -2166,18 +2188,17 @@ int hic_dct_scaled(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32
     HIC_REQUIRE(work_bytes >= need, "work buffer of %zu bytes is too small: %zu needed (hic_dct_scaled_sizes)", work_bytes, need);
     HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
                 "d_coef and d_work must be 16-byte aligned");
-    hic_dct_geometry g;
-    rc = batch_geometry(n, h, w, false, &g);
+    hic_dct_geometry g;           // what hic_dct_scaled_sizes checked
+    rc = geometry_of(h, w, &g);
     if (rc) return rc;
-    int32_t sh = 0, sw = 0;
-    rc = hic_dct_scaled_shape(h, w, scale, &sh, &sw);
-    if (rc) return rc;
+    const int sh = ceil_div(g.out_h, scale), sw = ceil_div(g.out_w, scale);
     rc = ensure_tables();
     if (rc) return rc;
     cudaStream_t st = as_stream(stream);
     HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
-    return scale == 2 ? scaled_launch<4>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st)
-                      : scaled_launch<2>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st);
+    return by_samples<false>(scale, [&](auto m) {
+        return scaled_launch<decltype(m)::value>(d_coef, g, n, sh, sw, d_work, d_ties, tie_capacity, d_stats, d_rgb_out, st);
+    });
 }
 
 int hic_dct_scaled_region_blocks(int32_t h, int32_t w, int32_t scale, int32_t top, int32_t left, int32_t rh, int32_t rw,
@@ -2185,16 +2206,7 @@ int hic_dct_scaled_region_blocks(int32_t h, int32_t w, int32_t scale, int32_t to
     using namespace hic;
     HIC_REQUIRE(rect != nullptr, "NULL argument");
     HIC_REQUIRE(scale == 2 || scale == 4, "scale must be 2 or 4 (got %d)", scale);
-    hic_dct_geometry g;
-    int rc = geometry_of(h, w, &g);
-    if (rc) return rc;
-    rc = region_check(g, top, left, rh, rw, scale);
-    if (rc) return rc;
-    if (scale == 2)
-        region_rect<4>(g, top, left, rh, rw, rect);
-    else
-        region_rect<2>(g, top, left, rh, rw, rect);
-    return HIC_OK;
+    return region_blocks(h, w, scale, top, left, rh, rw, rect);
 }
 
 int hic_dct_scaled_region_sizes(int32_t n, int32_t h, int32_t w, int32_t scale, int32_t rh, int32_t rw, size_t* work_bytes,
@@ -2212,11 +2224,7 @@ int hic_dct_scaled_region_sizes(int32_t n, int32_t h, int32_t w, int32_t scale, 
         *tie_capacity = 0;
         return HIC_OK;
     }
-    const RegionLayout L = scale == 2 ? region_layout<4>(n, g, rh, rw) : region_layout<2>(n, g, rh, rw);
-    HIC_REQUIRE(L.blocks < (1ull << 32), "batch too large: %llu selected blocks", (unsigned long long)L.blocks);
-    *work_bytes = L.total;
-    *tie_capacity = (uint32_t)L.blocks;
-    return HIC_OK;
+    return region_sizes(n, g, scale, rh, rw, work_bytes, tie_capacity);
 }
 
 int hic_dct_scaled_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, int32_t scale, const int32_t* h_origin,
@@ -2228,13 +2236,13 @@ int hic_dct_scaled_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w
     hic_dct_geometry g;
     int rc = batch_geometry(n, h, w, true, &g);
     if (rc) return rc;
-    for (int i = 0; i < n; ++i) {
-        rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw, scale);
-        if (rc) return rc;
-    }
+    rc = check_origins(g, n, h_origin, rh, rw, scale);
+    if (rc) return rc;
     cudaStream_t st = as_stream(stream);
-    return scale == 2 ? scaled_region_launch<4>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity, d_stats, d_rgb_out, st)
-                      : scaled_region_launch<2>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity, d_stats, d_rgb_out, st);
+    return by_samples<false>(scale, [&](auto m) {
+        return scaled_region_launch<decltype(m)::value>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity,
+                                                        d_stats, d_rgb_out, st);
+    });
 }
 
 int hic_dct_thumbnail_region(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, const int32_t* h_origin, int32_t rh,
@@ -2244,10 +2252,8 @@ int hic_dct_thumbnail_region(const int16_t* d_dc, int32_t n, int32_t h, int32_t 
     hic_dct_geometry g;
     int rc = batch_geometry(n, h, w, false, &g);
     if (rc) return rc;
-    for (int i = 0; i < n; ++i) {
-        rc = region_check(g, h_origin[2 * i], h_origin[2 * i + 1], rh, rw, 8);
-        if (rc) return rc;
-    }
+    rc = check_origins(g, n, h_origin, rh, rw, 8);
+    if (rc) return rc;
     const size_t need = (size_t)n * 2 * sizeof(int32_t);
     HIC_REQUIRE(work_bytes >= need, "work buffer of %zu bytes is too small: %zu needed (hic_dct_scaled_region_sizes)", work_bytes, need);
     HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_dc) & 1) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 3) == 0,

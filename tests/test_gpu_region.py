@@ -10,41 +10,16 @@ import pytest
 
 from oracle import hiccup_oracle as orc
 from tests.conftest import load_golden
+from tests.reduced_helpers import GOLDENS_WITH_PIXELS, fixed_windows, kernels_of
 
 pytestmark = pytest.mark.gpu
 
-GOLDENS_WITH_PIXELS = ["flat32", "flat32b", "gh256", "lenna512", "noise32x64", "syn128x160", "syn48x80", "syn64", "tiny16"]
 NEW_KERNELS = {"region_inverse_kernel", "region_fixup_kernel", "region_colour_kernel"}
-
-
-def _kernels_of(fn):
-    from hiccup_b200 import _lib
-    _lib.profile_enable(True)
-    _lib.profile_report()
-    try:
-        out = fn()
-        _lib.sync()
-        return out, set(_lib.profile_report())
-    finally:
-        _lib.profile_enable(False)
-
-
-def _windows(out_h, out_w):
-    """Corners, edges, 1x1, single rows and columns, odd sizes at odd origins and the whole image."""
-    wins = {(0, 0, out_h, out_w), (0, 0, 1, 1), (out_h - 1, out_w - 1, 1, 1), (0, out_w - 1, 1, 1), (out_h - 1, 0, 1, 1),
-            (0, 0, 1, out_w), (out_h - 1, 0, 1, out_w), (0, 0, out_h, 1), (0, out_w - 1, out_h, 1)}
-    for rh, rw in ((7, 9), (16, 16), (17, 33), (out_h // 2 + 1, out_w // 2 + 3), (out_h - 1, out_w - 1)):
-        rh, rw = max(1, min(rh, out_h)), max(1, min(rw, out_w))
-        for top in sorted({0, 1, (out_h - rh) // 2 | 1, out_h - rh}):
-            for left in sorted({0, 3, (out_w - rw) // 2, out_w - rw}):
-                if top + rh <= out_h and left + rw <= out_w:
-                    wins.add((top, left, rh, rw))
-    return sorted(wins)
 
 
 def _check_windows(hi, full):
     from hiccup_b200 import codec
-    for top, left, rh, rw in _windows(*full.shape[:2]):
+    for top, left, rh, rw in fixed_windows(*full.shape[:2]):
         got = codec.jpeg_region(hi, top, left, rh, rw)
         assert got.shape == (rh, rw, 3) and got.dtype == np.uint8
         assert np.array_equal(got, full[top:top + rh, left:left + rw]), (top, left, rh, rw)
@@ -127,7 +102,7 @@ def test_ties(h, w, seed, tmp_path):
         assert int(bc.region_stats[0]) == flagged and int(bc.region_stats[1]) == int(bc.inverse_stats[1])
         assert int(bc.region_stats[3]) == 0
         seen = 0
-        for top, left, rh, rw in _windows(out_h, out_w):
+        for top, left, rh, rw in fixed_windows(out_h, out_w):
             got = bc.decode_regions(enc, [(top, left)], (rh, rw))
             assert np.array_equal(got[0], full[top:top + rh, left:left + rw]), (top, left, rh, rw)
             assert int(bc.region_stats[0]) <= flagged
@@ -146,9 +121,9 @@ def test_restart_records():
     ext = hicimage.HicImage.from_bytes(codec.jpeg_encode(comp, restarts=True).byte_stream())
     for top, left, rh, rw in [(37, 101, 224, 224), (0, 0, 426, 640), (425, 639, 1, 1)]:
         want = full[top:top + rh, left:left + rw]
-        got, k_plain = _kernels_of(lambda: codec.jpeg_region(plain, top, left, rh, rw))
+        got, k_plain = kernels_of(lambda: codec.jpeg_region(plain, top, left, rh, rw))
         assert np.array_equal(got, want) and "huffman_sync_kernel" in k_plain
-        got, k_ext = _kernels_of(lambda: codec.jpeg_region(ext, top, left, rh, rw))
+        got, k_ext = kernels_of(lambda: codec.jpeg_region(ext, top, left, rh, rw))
         assert np.array_equal(got, want)
         assert "restart_load_kernel" in k_ext and "huffman_sync_kernel" not in k_ext
 
@@ -158,7 +133,7 @@ def test_kernels():
     from hiccup_b200 import codec, hicimage
     g = load_golden("lenna512")
     hi = hicimage.HicImage.from_bytes(pickle.loads(g["hic"].tobytes()))
-    got, kernels = _kernels_of(lambda: codec.jpeg_region(hi, 100, 203, 64, 77))
+    got, kernels = kernels_of(lambda: codec.jpeg_region(hi, 100, 203, 64, 77))
     assert np.array_equal(got, g["rgb_out"][100:164, 203:280])
     assert NEW_KERNELS <= kernels and "expand_scatter_kernel" in kernels
     assert not kernels & {"inverse_kernel", "inverse_fixup_kernel", "upsample_colour_kernel"}

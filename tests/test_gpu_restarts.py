@@ -5,20 +5,9 @@ import numpy as np
 import pytest
 
 from oracle import hiccup_oracle as orc
+from tests.reduced_helpers import kernels_of
 
 pytestmark = pytest.mark.gpu
-
-
-def _kernels_of(fn):
-    from hiccup_b200 import _lib
-    _lib.profile_enable(True)
-    _lib.profile_report()
-    try:
-        out = fn()
-        _lib.sync()
-        return out, set(_lib.profile_report())
-    finally:
-        _lib.profile_enable(False)
 
 
 def _same_planes(a, b):
@@ -40,8 +29,8 @@ def test_dct_file_with_restart_records(shape, seed):
         assert off.size == cnt.size == n_sub
         assert int(cnt.astype(np.int64).sum()) > 0 and off.max(initial=0) < 58 and cnt.max(initial=0) <= 128
     back = hicimage.HicImage.from_bytes(ext.byte_stream())           # through the wire
-    want, k_plain = _kernels_of(lambda: codec.jpeg_decode(plain))
-    got, k_ext = _kernels_of(lambda: codec.jpeg_decode(back))
+    want, k_plain = kernels_of(lambda: codec.jpeg_decode(plain))
+    got, k_ext = kernels_of(lambda: codec.jpeg_decode(back))
     assert _same_planes(got, want)
     assert "huffman_sync_kernel" in k_plain and "huffman_sync_kernel" not in k_ext and "huffman_resync_kernel" not in k_ext
     assert "restart_load_kernel" in k_ext
@@ -60,12 +49,12 @@ def test_records_that_do_not_fit_are_ignored():
     # (a) wrong contents: the write pass finds out, the decoder synchronises by itself
     bad = [(np.zeros_like(o), np.ones_like(c)) for o, c in ext.restarts.records]
     hx = hicimage.HicImage(ext.hic_type, ext.settings, ext.payloads, [hicimage.RestartP(bad)])
-    got, kernels = _kernels_of(lambda: codec.jpeg_decode(hx))
+    got, kernels = kernels_of(lambda: codec.jpeg_decode(hx))
     assert _same_planes(got, want) and "huffman_sync_kernel" in kernels
     # (b) wrong sizes: not even tried
     short = [(o[:-1], c[:-1]) for o, c in ext.restarts.records]
     hy = hicimage.HicImage(ext.hic_type, ext.settings, ext.payloads, [hicimage.RestartP(short)])
-    got, kernels = _kernels_of(lambda: codec.jpeg_decode(hy))
+    got, kernels = kernels_of(lambda: codec.jpeg_decode(hy))
     assert _same_planes(got, want) and "restart_load_kernel" not in kernels
 
 
@@ -77,7 +66,7 @@ def test_wavelet_file_with_restart_records():
     ext = codec.wavelet_encode(comp, restarts=True)
     assert ext.byte_stream()[:15] == plain.byte_stream() and len(ext.restarts.records) == 6
     want = codec.wavelet_decode(plain)
-    got, kernels = _kernels_of(lambda: codec.wavelet_decode(hicimage.HicImage.from_bytes(ext.byte_stream())))
+    got, kernels = kernels_of(lambda: codec.wavelet_decode(hicimage.HicImage.from_bytes(ext.byte_stream())))
     assert "huffman_sync_kernel" not in kernels and "restart_load_kernel" in kernels
     assert all(np.array_equal(x, y) for ch in ("lum", "cr", "cb") for x, y in zip(got.as_dict[ch], want.as_dict[ch]))
     assert np.array_equal(compression.wavelet_decompression(got), orc.wavelet_decompression(orc.wavelet_compression(rgb)))

@@ -11,27 +11,11 @@ import pytest
 from oracle import hiccup_oracle as orc
 from tests import scaled_oracle as so
 from tests.conftest import load_golden
+from tests.reduced_helpers import GOLDENS_WITH_PIXELS, ODD, kernels_of, planes, tie_planes
 
 pytestmark = pytest.mark.gpu
 
-GOLDENS_WITH_PIXELS = ["flat32", "flat32b", "gh256", "lenna512", "noise32x64", "syn128x160", "syn48x80", "syn64", "tiny16"]
 NEW_KERNELS = {"scaled_inverse_kernel", "scaled_fixup_kernel", "scaled_colour_kernel"}
-
-
-def _kernels_of(fn):
-    from hiccup_b200 import _lib
-    _lib.profile_enable(True)
-    _lib.profile_report()
-    try:
-        out = fn()
-        _lib.sync()
-        return out, set(_lib.profile_report())
-    finally:
-        _lib.profile_enable(False)
-
-
-def _planes(comp):
-    return {ch: np.asarray(v) for ch, v in comp.as_dict.items()}
 
 
 @pytest.mark.parametrize("scale", [2, 4])
@@ -47,9 +31,6 @@ def test_reference_files(name, scale):
     assert np.array_equal(got, want)
 
 
-ODD = [(26, 40), (33, 47), (2, 2), (3, 5), (5, 3), (9, 17), (17, 2), (2, 31), (15, 15), (64, 106)]
-
-
 @pytest.mark.parametrize("shape", ODD + [(int(h), int(w)) for h, w in np.random.default_rng(77).integers(2, 300, (6, 2))])
 def test_odd_shapes_against_the_oracle(shape):
     """syn26x40, syn33x47, random sizes, and sizes whose chroma planes are one sample (or one block) wide or high."""
@@ -58,28 +39,7 @@ def test_odd_shapes_against_the_oracle(shape):
     comp = compression.jpeg_compression(rgb)
     hi = codec.jpeg_encode(comp)
     for scale in (2, 4):
-        assert np.array_equal(codec.jpeg_scaled(hi, scale), so.jpeg_scaled(_planes(comp), scale)), (shape, scale)
-
-
-def _tie_planes(h, w, scale, seed):
-    """Large DC terms (samples that wrap) and large AC terms; the first blocks of every plane are ones whose float32
-    samples truncate differently from the float64 definition -- found by K7S's arithmetic on the host (the CPU harness
-    runs the same float32 code) -- so the fix-up must change samples."""
-    from tests.test_scaled_host import _harness, _harness_blocks
-    lib = _harness()
-    rng = np.random.default_rng(seed)
-    planes = {}
-    for ch, shape in (("lum", (h, w)), ("cr", (h // 2, w // 2)), ("cb", (h // 2, w // 2))):
-        nb = (shape[0] // 8) * (shape[1] // 8)
-        pool = rng.integers(-1500, 1501, (200000, 64)) * (rng.random((200000, 64)) < 0.7)
-        pool[:, 0] = rng.integers(-6000, 6000, len(pool))
-        out, _, _, exact = _harness_blocks(lib, pool, 0 if ch == "lum" else 1, 8 // scale)
-        miss = (out != exact).any(axis=1)
-        zz = np.concatenate([pool[miss], pool[~miss]])[:nb]
-        nat = np.zeros((nb, 64), np.int64)
-        nat[:, orc.ZIGZAG8] = zz
-        planes[ch] = orc.merge_blocks(nat.reshape(nb, 8, 8), shape).astype(np.int32)
-    return planes
+        assert np.array_equal(codec.jpeg_scaled(hi, scale), so.jpeg_scaled(planes(comp), scale)), (shape, scale)
 
 
 @pytest.mark.parametrize("scale", [2, 4])
@@ -88,7 +48,7 @@ def test_ties(scale, tmp_path):
     from hiccup_b200 import codec, model
     from hiccup_b200.batch import DctBatchCodec
     h, w = 256, 384
-    planes = _tie_planes(h, w, scale, 40 + scale)
+    planes = tie_planes(h, w, scale, 40 + scale)
     hi = codec.jpeg_encode(model.CompressedImage(planes["lum"], planes["cr"], planes["cb"]))
     want = so.jpeg_scaled(planes, scale)
     assert np.array_equal(codec.jpeg_scaled(hi, scale), want)
@@ -112,10 +72,10 @@ def test_restart_records():
     plain = codec.jpeg_encode(comp)
     ext = hicimage.HicImage.from_bytes(codec.jpeg_encode(comp, restarts=True).byte_stream())
     for scale in (2, 4):
-        want = so.jpeg_scaled(_planes(comp), scale)
-        got, k_plain = _kernels_of(lambda: codec.jpeg_scaled(plain, scale))
+        want = so.jpeg_scaled(planes(comp), scale)
+        got, k_plain = kernels_of(lambda: codec.jpeg_scaled(plain, scale))
         assert np.array_equal(got, want) and "huffman_sync_kernel" in k_plain
-        got, k_ext = _kernels_of(lambda: codec.jpeg_scaled(ext, scale))
+        got, k_ext = kernels_of(lambda: codec.jpeg_scaled(ext, scale))
         assert np.array_equal(got, want)
         assert "restart_load_kernel" in k_ext and "huffman_sync_kernel" not in k_ext
 
@@ -127,7 +87,7 @@ def test_kernels():
     hi = hicimage.HicImage.from_bytes(pickle.loads(g["hic"].tobytes()))
     planes = {ch: g["coef_" + ch] for ch in orc.CHANNELS}
     for scale in (2, 4):
-        got, kernels = _kernels_of(lambda: codec.jpeg_scaled(hi, scale))
+        got, kernels = kernels_of(lambda: codec.jpeg_scaled(hi, scale))
         assert np.array_equal(got, so.jpeg_scaled(planes, scale))
         assert NEW_KERNELS <= kernels and "expand_scatter_kernel" in kernels
         assert not kernels & {"inverse_kernel", "inverse_fixup_kernel", "upsample_colour_kernel"}

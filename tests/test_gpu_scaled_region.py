@@ -13,8 +13,7 @@ from oracle import hiccup_oracle as orc
 from tests import scaled_oracle as so
 from tests import thumbnail_oracle as tho
 from tests.conftest import load_golden
-from tests.test_gpu_region import GOLDENS_WITH_PIXELS, _kernels_of, _windows
-from tests.test_gpu_scaled import ODD, _planes, _tie_planes
+from tests.reduced_helpers import GOLDENS_WITH_PIXELS, ODD, fixed_windows, kernels_of, planes, tie_planes
 
 pytestmark = pytest.mark.gpu
 
@@ -30,7 +29,7 @@ def _whole(hi, scale):
 
 def _check_windows(hi, full, scale):
     from hiccup_b200 import codec
-    for top, left, rh, rw in _windows(*full.shape[:2]):
+    for top, left, rh, rw in fixed_windows(*full.shape[:2]):
         got = codec.jpeg_region(hi, top, left, rh, rw, scale=scale)
         assert got.shape == (rh, rw, 3) and got.dtype == np.uint8
         assert np.array_equal(got, full[top:top + rh, left:left + rw]), (scale, top, left, rh, rw)
@@ -54,7 +53,7 @@ def test_odd_shapes(shape):
     comp = compression.jpeg_compression(rgb)
     hi = codec.jpeg_encode(comp)
     for scale in (2, 4, 8):
-        want = tho.jpeg_thumbnail(_planes(comp)) if scale == 8 else so.jpeg_scaled(_planes(comp), scale)
+        want = tho.jpeg_thumbnail(planes(comp)) if scale == 8 else so.jpeg_scaled(planes(comp), scale)
         assert np.array_equal(_whole(hi, scale), want), (shape, scale)
         _check_windows(hi, want, scale)
 
@@ -66,7 +65,7 @@ def test_ties(scale, tmp_path):
     from hiccup_b200 import codec, model
     from hiccup_b200.batch import DctBatchCodec
     h, w = 256, 384
-    planes = _tie_planes(h, w, scale, 60 + scale)
+    planes = tie_planes(h, w, scale, 60 + scale)
     hi = codec.jpeg_encode(model.CompressedImage(planes["lum"], planes["cr"], planes["cb"]))
     want = so.jpeg_scaled(planes, scale)
     sh, sw = want.shape[:2]
@@ -93,9 +92,9 @@ def test_restart_records():
     for scale, (top, left, rh, rw) in ((2, (17, 31, 112, 112)), (4, (50, 103, 56, 56)), (8, (25, 51, 28, 28))):
         full = _whole(plain, scale)
         want = full[top:top + rh, left:left + rw]
-        got, k_plain = _kernels_of(lambda: codec.jpeg_region(plain, top, left, rh, rw, scale=scale))
+        got, k_plain = kernels_of(lambda: codec.jpeg_region(plain, top, left, rh, rw, scale=scale))
         assert np.array_equal(got, want) and "huffman_sync_kernel" in k_plain
-        got, k_ext = _kernels_of(lambda: codec.jpeg_region(ext, top, left, rh, rw, scale=scale))
+        got, k_ext = kernels_of(lambda: codec.jpeg_region(ext, top, left, rh, rw, scale=scale))
         assert np.array_equal(got, want)
         assert "restart_load_kernel" in k_ext and "huffman_sync_kernel" not in k_ext
 
@@ -108,7 +107,7 @@ def test_kernels():
     hi = hicimage.HicImage.from_bytes(pickle.loads(g["hic"].tobytes()))
     for scale, win in ((2, (31, 45, 112, 80)), (4, (10, 7, 56, 56)), (8, (3, 5, 28, 40))):
         full = _whole(hi, scale)
-        got, kernels = _kernels_of(lambda: codec.jpeg_region(hi, *win, scale=scale))
+        got, kernels = kernels_of(lambda: codec.jpeg_region(hi, *win, scale=scale))
         top, left, rh, rw = win
         assert np.array_equal(got, full[top:top + rh, left:left + rw])
         if scale == 8:

@@ -11,25 +11,9 @@ import pytest
 from oracle import hiccup_oracle as orc
 from tests import thumbnail_oracle as tho
 from tests.conftest import load_golden
-from tests.test_thumbnail_host import DCT_GOLDENS
+from tests.reduced_helpers import DCT_GOLDENS, kernels_of, planes
 
 pytestmark = pytest.mark.gpu
-
-
-def _planes(comp):
-    return {ch: np.asarray(v) for ch, v in comp.as_dict.items()}
-
-
-def _kernels_of(fn):
-    from hiccup_b200 import _lib
-    _lib.profile_enable(True)
-    _lib.profile_report()
-    try:
-        out = fn()
-        _lib.sync()
-        return out, set(_lib.profile_report())
-    finally:
-        _lib.profile_enable(False)
 
 
 @pytest.mark.parametrize("name", DCT_GOLDENS)
@@ -37,7 +21,7 @@ def test_reference_files(name):
     from hiccup_b200 import codec, hicimage
     g = load_golden(name)
     hi = hicimage.HicImage.from_bytes(pickle.loads(g["hic"].tobytes()))
-    got, kernels = _kernels_of(lambda: codec.jpeg_thumbnail(hi))
+    got, kernels = kernels_of(lambda: codec.jpeg_thumbnail(hi))
     want = tho.jpeg_thumbnail({ch: g["coef_" + ch] for ch in orc.CHANNELS})
     assert got.shape == want.shape and np.array_equal(got, want)
     assert "thumbnail_kernel" in kernels and "validate_dc_kernel" in kernels
@@ -50,7 +34,7 @@ def test_odd_sizes(shape):
     rgb = orc.synthetic_image(shape[0], shape[1], 300 + shape[0] * 7 + shape[1])
     comp = compression.jpeg_compression(rgb)
     got = codec.jpeg_thumbnail(codec.jpeg_encode(comp))
-    assert np.array_equal(got, tho.jpeg_thumbnail(_planes(comp)))
+    assert np.array_equal(got, tho.jpeg_thumbnail(planes(comp)))
 
 
 def test_dc_values_that_wrap():
@@ -75,23 +59,23 @@ def test_restart_records():
     from hiccup_b200 import codec, compression, hicimage
     rgb = orc.synthetic_image(426, 640, 2000)
     comp = compression.jpeg_compression(rgb)
-    want = tho.jpeg_thumbnail(_planes(comp))
+    want = tho.jpeg_thumbnail(planes(comp))
     plain = codec.jpeg_encode(comp)
     ext = hicimage.HicImage.from_bytes(codec.jpeg_encode(comp, restarts=True).byte_stream())
-    got, k_plain = _kernels_of(lambda: codec.jpeg_thumbnail(plain))
+    got, k_plain = kernels_of(lambda: codec.jpeg_thumbnail(plain))
     assert np.array_equal(got, want) and "huffman_sync_kernel" in k_plain
-    got, k_ext = _kernels_of(lambda: codec.jpeg_thumbnail(ext))
+    got, k_ext = kernels_of(lambda: codec.jpeg_thumbnail(ext))
     assert np.array_equal(got, want)
     assert "restart_load_kernel" in k_ext and "huffman_sync_kernel" not in k_ext
     # records that do not belong: the write pass finds out and the decode synchronises by itself
     bad = [(np.zeros_like(o), np.ones_like(c)) for o, c in ext.restarts.records]
     hx = hicimage.HicImage(ext.hic_type, ext.settings, ext.payloads, [hicimage.RestartP(bad)])
-    got, kernels = _kernels_of(lambda: codec.jpeg_thumbnail(hx))
+    got, kernels = kernels_of(lambda: codec.jpeg_thumbnail(hx))
     assert np.array_equal(got, want) and "huffman_sync_kernel" in kernels
     # records of the wrong size are not even tried
     short = [(o[:-1], c[:-1]) for o, c in ext.restarts.records]
     hy = hicimage.HicImage(ext.hic_type, ext.settings, ext.payloads, [hicimage.RestartP(short)])
-    got, kernels = _kernels_of(lambda: codec.jpeg_thumbnail(hy))
+    got, kernels = kernels_of(lambda: codec.jpeg_thumbnail(hy))
     assert np.array_equal(got, want) and "restart_load_kernel" not in kernels
 
 
@@ -125,7 +109,7 @@ def test_ac_streams_are_never_read():
     rgb = orc.synthetic_image(96, 136, 44)
     comp = compression.jpeg_compression(rgb)
     hi = codec.jpeg_encode(comp)
-    want = tho.jpeg_thumbnail(_planes(comp))
+    want = tho.jpeg_thumbnail(planes(comp))
     p = hi.payloads
     order = [kind * 3 + c for c in range(3) for kind in range(3)]          # stream s = channel * 3 + kind
     rows, syms, lens, codes = codec._tables_to_arrays([p[i] for i in order])
@@ -161,7 +145,7 @@ def test_short_dc_stream_is_corrupt():
     rgb = orc.synthetic_image(64, 96, 45)
     comp = compression.jpeg_compression(rgb)
     hi = codec.jpeg_encode(comp)
-    streams = orc.jpeg_streams(_planes(comp))
+    streams = orc.jpeg_streams(planes(comp))
     for c, ch in enumerate(orc.CHANNELS):
         table = [(int(sym), code) for sym, code in hi.payloads[c].rows]
         bits = orc.huffman_encode_bits(streams["dc"][ch][:-1], table)
@@ -170,7 +154,7 @@ def test_short_dc_stream_is_corrupt():
         cut = hicimage.HicImage(hi.hic_type, hi.settings, payloads, [])
         with pytest.raises(_lib.HicError, match="error -4"):
             codec.jpeg_thumbnail(cut)
-    assert np.array_equal(codec.jpeg_thumbnail(hi), tho.jpeg_thumbnail(_planes(comp)))
+    assert np.array_equal(codec.jpeg_thumbnail(hi), tho.jpeg_thumbnail(planes(comp)))
 
 
 @pytest.mark.parametrize("n,h,w", [(5, 40, 41), (3, 33, 47), (4, 64, 96)])

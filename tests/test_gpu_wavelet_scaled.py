@@ -13,24 +13,13 @@ import pytest
 from oracle import hiccup_oracle as orc
 from tests import wavelet_scaled_oracle as wso
 from tests.conftest import load_golden
+from tests.reduced_helpers import kernels_of
 from tests.test_gpu_wavelet_settings import wavelet_settings
 from tests.test_wavelet_scaled_host import random_planes
 
 pytestmark = pytest.mark.gpu
 
 DEFAULT = dict(levels=3, multiplier=1, threshold=5, quality_factor=1)
-
-
-def _kernels_of(fn):
-    from hiccup_b200 import _lib
-    _lib.profile_enable(True)
-    _lib.profile_report()
-    try:
-        out = fn()
-        _lib.sync()
-        return out, set(_lib.profile_report())
-    finally:
-        _lib.profile_enable(False)
 
 
 def _planes(comp):
@@ -134,7 +123,7 @@ def test_settings(cfg):
             hi = codec.wavelet_encode(compression.wavelet_compression(rgb[0]))
             planes = _planes(codec.wavelet_decode(hi))
             for k in range(1, L + 1):
-                got, kernels = _kernels_of(lambda: codec.wavelet_scaled(hi, 1 << k))
+                got, kernels = kernels_of(lambda: codec.wavelet_scaled(hi, 1 << k))
                 assert np.array_equal(got, wso.wavelet_scaled(planes, 1 << k, cfg["multiplier"])), k
                 assert "wavelet_scaled_finish_kernel" in kernels and "wavelet_finish_kernel" not in kernels
 
@@ -146,7 +135,7 @@ def test_kernels_at_the_defaults():
     hi = codec.wavelet_encode(compression.wavelet_compression(rgb))
     planes = _planes(codec.wavelet_decode(hi))
     for s in (2, 4, 8):
-        got, kernels = _kernels_of(lambda: codec.wavelet_scaled(hi, s))
+        got, kernels = kernels_of(lambda: codec.wavelet_scaled(hi, s))
         assert np.array_equal(got, wso.wavelet_scaled(planes, s))
         assert "wavelet_scaled_finish_kernel" in kernels and "expand_scatter_kernel" in kernels
         assert ("wavelet_inverse_level_kernel" in kernels) == (s != 8)
@@ -201,9 +190,9 @@ def test_restart_records():
     planes = _planes(codec.wavelet_decode(plain))
     for s in (2, 4, 8):
         want = wso.wavelet_scaled(planes, s)
-        got, k_plain = _kernels_of(lambda: codec.wavelet_scaled(plain, s))
+        got, k_plain = kernels_of(lambda: codec.wavelet_scaled(plain, s))
         assert np.array_equal(got, want) and "huffman_sync_kernel" in k_plain
-        got, k_ext = _kernels_of(lambda: codec.wavelet_scaled(ext, s))
+        got, k_ext = kernels_of(lambda: codec.wavelet_scaled(ext, s))
         assert np.array_equal(got, want)
         assert "restart_load_kernel" in k_ext and "huffman_sync_kernel" not in k_ext
 

@@ -2,12 +2,11 @@
 work and tie sizes, the argument checks of every entry point (they all refuse before any device work, so they run
 here) and the command line."""
 import os
-import pickle
 
 import numpy as np
 import pytest
 
-from tests.conftest import load_golden
+from tests.reduced_helpers import random_windows, write_goldens
 
 SIZES = [(2, 2), (3, 5), (5, 3), (2, 17), (17, 2), (3, 3), (7, 9), (8, 8), (9, 17), (15, 17), (16, 16), (17, 33),
          (26, 40), (33, 47), (40, 41), (64, 106), (96, 136), (426, 640)]
@@ -23,19 +22,6 @@ def _rows_read(top, rh, n_out, n_c):
         yn = min(cy + 1, n_c - 1)
         chroma |= {ym, cy, yn}
     return lum, chroma
-
-
-def _windows(out_h, out_w, rng):
-    """Corners, edges, 1x1, single rows and columns, the whole image and a few random windows."""
-    yield 0, 0, out_h, out_w
-    for rh, rw in {(1, 1), (1, out_w), (out_h, 1), (min(7, out_h), min(9, out_w)), (min(16, out_h), min(16, out_w)),
-                   (min(17, out_h), min(33, out_w)), ((out_h + 1) // 2, (out_w + 1) // 2)}:
-        for top in {0, (out_h - rh) // 2, out_h - rh}:
-            for left in {0, (out_w - rw) // 2, out_w - rw}:
-                yield top, left, rh, rw
-    for _ in range(12):
-        rh, rw = int(rng.integers(1, out_h + 1)), int(rng.integers(1, out_w + 1))
-        yield int(rng.integers(0, out_h - rh + 1)), int(rng.integers(0, out_w - rw + 1)), rh, rw
 
 
 def _check_cover(g, top, left, rh, rw, lum_rect, c_rect):
@@ -56,7 +42,7 @@ def test_selection_covers_every_sample_k8_reads(h, w):
     from hiccup_b200 import _lib
     g = _lib.geometry(h, w)
     rng = np.random.default_rng(h * 1000 + w)
-    for top, left, rh, rw in _windows(g.out_h, g.out_w, rng):
+    for top, left, rh, rw in random_windows(g.out_h, g.out_w, rng):
         lum_rect, c_rect = _lib.region_blocks(h, w, top, left, rh, rw)
         _check_cover(g, top, left, rh, rw, lum_rect, c_rect)
 
@@ -139,19 +125,11 @@ def test_python_checks_windows():
             _lib.region_origins(64, 81, origins, size)
 
 
-def _write_goldens(tmp_path):
-    wp, dp = os.path.join(tmp_path, "w.hic"), os.path.join(tmp_path, "d.hic")
-    for path, name in ((wp, "w_syn64"), (dp, "syn64")):
-        with open(path, "wb") as f:
-            f.write(pickle.dumps(pickle.loads(load_golden(name)["hic"].tobytes())))
-    return wp, dp
-
-
 def test_bad_windows_are_refused_before_any_work(tmp_path):
     """An empty window or one the 64 x 64 image does not hold: ValueError from every entry point, before a device is
     needed (this runs without one) and before any file is written."""
     from hiccup_b200 import codec, hicimage, run
-    _, dp = _write_goldens(tmp_path)
+    _, dp = write_goldens(tmp_path)
     hi = hicimage.HicImage.from_file(dp)
     for top, left, rh, rw in [(0, 0, 0, 4), (0, 0, 4, 0), (-1, 0, 4, 4), (0, -2, 4, 4), (61, 0, 4, 4), (0, 0, 65, 64),
                               (0, 60, 1, 5)]:
@@ -173,7 +151,7 @@ def test_bad_windows_are_refused_before_any_work(tmp_path):
 
 def test_wavelet_files_are_refused_before_any_work(tmp_path):
     from hiccup_b200 import codec, hicimage, run
-    wp, dp = _write_goldens(tmp_path)
+    wp, dp = write_goldens(tmp_path)
     with pytest.raises(NotImplementedError, match="wavelet"):
         codec.jpeg_region(hicimage.HicImage.from_file(wp), 0, 0, 4, 4)
     with pytest.raises(NotImplementedError, match="wavelet"):

@@ -4,7 +4,6 @@ oracle, the float32 path's flagging and error bound, the shapes, the argument ch
 command line."""
 import ctypes
 import os
-import pickle
 
 import numpy as np
 import pytest
@@ -13,6 +12,7 @@ from oracle import hiccup_oracle as orc
 from tests import scaled_oracle as so
 from tests import thumbnail_oracle as tho
 from tests.conftest import load_golden
+from tests.reduced_helpers import DCT_GOLDENS, write_goldens
 from tests.test_oracle_dct import _ptr
 
 HARNESS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "cpu_harness", "libhic_scaled_harness.so")
@@ -24,8 +24,6 @@ def _harness():
         __graft_entry__.build()
     return ctypes.CDLL(HARNESS)
 
-DCT_GOLDENS = ["lenna512", "gh256", "syn64", "syn48x80", "syn64x106", "syn128x160", "syn26x40", "syn33x47",
-               "tiny16", "flat32", "flat32b", "noise32x64"]
 TABLES = {0: orc.LUM_TABLE, 1: orc.CHROMA_TABLE}
 
 
@@ -202,19 +200,11 @@ def test_python_checks_the_scale():
             _lib.scale_arg(bad)
 
 
-def _write_goldens(tmp_path):
-    wp, dp = os.path.join(tmp_path, "w.hic"), os.path.join(tmp_path, "d.hic")
-    for path, name in ((wp, "w_syn64"), (dp, "syn64")):
-        with open(path, "wb") as f:
-            f.write(pickle.dumps(pickle.loads(load_golden(name)["hic"].tobytes())))
-    return wp, dp
-
-
 def test_bad_scales_and_wavelet_files_are_refused_before_any_work(tmp_path):
     """A scale other than 2 or 4 raises ValueError and a wavelet file NotImplementedError from every entry point, before
     a device is needed (this runs without one) and before any file is written."""
     from hiccup_b200 import codec, hicimage, run
-    wp, dp = _write_goldens(tmp_path)
+    wp, dp = write_goldens(tmp_path)
     hi = hicimage.HicImage.from_file(dp)
     for bad in (1, 3, 8, 2.5):
         with pytest.raises(ValueError):

@@ -4,7 +4,7 @@ the argument checks of every new entry point (they all refuse before any device 
 import numpy as np
 import pytest
 
-from tests.test_region_host import _windows, _write_goldens
+from tests.reduced_helpers import random_windows, write_goldens
 
 SHAPES = [(2, 2), (3, 5), (5, 3), (17, 2), (2, 17), (9, 17), (26, 40), (33, 47), (64, 81), (426, 640)] + \
     [(int(h), int(w)) for h, w in np.random.default_rng(5).integers(2, 400, (8, 2))]
@@ -54,7 +54,7 @@ def test_selection_covers_every_tap(h, w, scale):
     g = _lib.geometry(h, w)
     (sh, sw), _, _ = _reduced(g, scale)
     assert (sh, sw) == _lib.scaled_shape(h, w, scale)
-    windows = list(_windows(sh, sw, np.random.default_rng(h * 1000 + w + scale)))
+    windows = list(random_windows(sh, sw, np.random.default_rng(h * 1000 + w + scale)))
     if sh * sw <= 400:
         windows += [(t, l, 1, 1) for t in range(sh) for l in range(sw)]
     shapes = {}
@@ -192,7 +192,7 @@ def test_bad_scales_and_windows_are_refused_before_any_work(tmp_path):
     """jpeg_region with a bad scale or a window outside the 1/scale image raises ValueError, and with a wavelet file
     NotImplementedError, before a device is needed (this runs without one)."""
     from hiccup_b200 import codec, hicimage
-    wp, dp = _write_goldens(tmp_path)
+    wp, dp = write_goldens(tmp_path)
     hi = hicimage.HicImage.from_file(dp)            # 64 x 64: 1/2 32 x 32, 1/4 16 x 16, 1/8 8 x 8
     for bad in (0, 3, 16, 2.0, "4", True):
         with pytest.raises(ValueError):

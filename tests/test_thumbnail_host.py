@@ -10,9 +10,7 @@ import pytest
 from oracle import hiccup_oracle as orc
 from tests import thumbnail_oracle as tho
 from tests.conftest import load_golden
-
-DCT_GOLDENS = ["lenna512", "gh256", "syn64", "syn48x80", "syn64x106", "syn128x160", "syn26x40", "syn33x47",
-               "tiny16", "flat32", "flat32b", "noise32x64"]
+from tests.reduced_helpers import DCT_GOLDENS
 
 
 @pytest.mark.parametrize("table", ["lum", "chroma"])

@@ -116,8 +116,7 @@ static int geometry_of(int h, int w, hic_dct_geometry* g) {
 // row the window reads, moved back where it would run past the plane's last block.
 // The scaled region decode uses the same rules at M = 8 / scale samples per block side: a window of the 1/scale image
 // reads rows of the reduced planes (M nby_l x M nbx_l luminance, M nby_c x M nbx_c chroma) exactly as a window of the
-// full decode reads rows of the full-size planes, so only the block size changes.  M is a template argument so that
-// the full-resolution callers (M = 8) compile to what they always did.
+// full decode reads rows of the full-size planes, so only the block size changes.
 struct RegionSpan {
     int ny_l, nx_l;   // luminance rectangle, blocks
     int ny_c, nx_c;   // chroma rectangle (Cr and Cb alike)
@@ -125,18 +124,18 @@ struct RegionSpan {
 
 template <int M>
 constexpr int log2_side() { return M == 8 ? 3 : (M == 4 ? 2 : 1); }
-template <int M = 8>
+template <int M>
 __host__ __device__ inline int region_span_l(int r, int nb) { return min(nb, (r + M - 2) / M + 1); }   // r samples
-template <int M = 8>
+template <int M>
 __host__ __device__ inline int region_span_c(int r, int nb) { return min(nb, (r / 2 + 3 + M - 2) / M + 1); }
-template <int M = 8>
+template <int M>
 __host__ __device__ inline RegionSpan region_span(const hic_dct_geometry& g, int rh, int rw) {
     return {region_span_l<M>(rh, g.nby_l), region_span_l<M>(rw, g.nbx_l), region_span_c<M>(rh, g.nby_c), region_span_c<M>(rw, g.nbx_c)};
 }
 // first block row (column) of the luminance / chroma rectangle of a window whose first output row (column) is t
-template <int M = 8>
+template <int M>
 __host__ __device__ inline int region_first_l(int t, int span, int nb) { return min(t >> log2_side<M>(), nb - span); }
-template <int M = 8>
+template <int M>
 __host__ __device__ inline int region_first_c(int t, int span, int nb) {
     return min(max(0, (t >> 1) - 1) >> log2_side<M>(), nb - span);
 }
@@ -163,14 +162,14 @@ static void region_rect(const hic_dct_geometry& g, int top, int left, int rh, in
     memcpy(rect, out, sizeof(out));
 }
 
-// window-local planes of one image (bytes, M x M samples per block) and the work buffer: n origins, then the n Y
-// planes, Cr planes, Cb planes
+// window-local tiles of one image (bytes, M x M samples per block) and the work buffer: n origins, then the n images'
+// Y tiles, Cr tiles, Cb tiles
 struct RegionLayout {
     RegionSpan s;
     size_t head, ly, lc, total;
     uint64_t blocks;      // selected blocks of the batch
 };
-template <int M = 8>
+template <int M>
 static RegionLayout region_layout(int n, const hic_dct_geometry& g, int rh, int rw) {
     RegionLayout L;
     L.s = region_span<M>(g, rh, rw);
@@ -848,6 +847,20 @@ fixup_kernel(const uint8_t* __restrict__ rgb, int h, int w, hic_dct_geometry g, 
 namespace k7 {
 constexpr float MAGIC = 12582912.0f;
 
+__device__ __forceinline__ void record_tie(uint32_t block, hic_tie_record* __restrict__ ties, uint32_t tie_capacity,
+                                           uint32_t* __restrict__ stats) {
+    const uint32_t slot = atomicAdd(&stats[0], 1u);
+    if (slot < tie_capacity) {
+        hic_tie_record rec;
+        rec.block = block;
+        rec.reserved = 0;
+        rec.mask = ~0ull;
+        ties[slot] = rec;
+    } else {
+        atomicAdd(&stats[3], 1u);
+    }
+}
+
 // in: the block's 128-byte row of the staging area (TMA 128-byte swizzle: piece j sits at position j ^ sw)
 template <int KIND>
 __device__ __forceinline__ void inverse_block(const int4* __restrict__ in, int sw, uint8_t* __restrict__ plane, int ph,
@@ -910,18 +923,61 @@ __device__ __forceinline__ void inverse_block(const int4* __restrict__ in, int s
     // energy = sum |coef| q w(u, v) margin: the rigorous per-input error weights of hic_dct_bound.h; 2^-15 covers the
     // rounding of the final + 128 (half an ulp of a value below 512) and of this comparison
     const float band = (float)(4.0 / 16777216.0 / 256.0) * energy + 3.0517578125e-5f;
-    if (ac_bits != 0 && margin <= band) {
-        const uint32_t slot = atomicAdd(&stats[0], 1u);
-        if (slot < tie_capacity) {
-            hic_tie_record rec;
-            rec.block = block_index;
-            rec.reserved = 0;
-            rec.mask = ~0ull;
-            ties[slot] = rec;
-        } else {
-            atomicAdd(&stats[3], 1u);
-        }
+    if (ac_bits != 0 && margin <= band) record_tie(block_index, ties, tie_capacity, stats);
+}
+
+// One TMA tensor load of the CTA's box of K7's [block][64 int16] map (box_rows blocks from block blockIdx.x * box_rows)
+// into dst (bytes long): thread 0 issues it on the mbarrier bar, and every thread returns once it has landed.
+__device__ __forceinline__ void load_block_box(const CUtensorMap& tmap, int box_rows, void* dst, uint32_t bytes,
+                                               unsigned long long* bar_p) {
+    const uint32_t bar = (uint32_t)__cvta_generic_to_shared(bar_p);
+    if (threadIdx.x == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+        asm volatile(
+            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+            ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(reinterpret_cast<uint64_t>(&tmap)), "r"(0),
+            "r"((int)(blockIdx.x * box_rows)), "r"(bar)
+            : "memory");
     }
+    __syncthreads();
+    asm volatile(
+        "{\n"
+        ".reg .pred P1;\n"
+        "LAB_WAIT:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], 0;\n"
+        "@P1 bra DONE;\n"
+        "bra LAB_WAIT;\n"
+        "DONE:\n"
+        "}\n" ::"r"(bar)
+        : "memory");
+}
+
+// Global block index b of the batch (per image its Y blocks, then Cr, then Cb, each row by row): its image, plane p
+// (0 = Y, 1 = Cr, 2 = Cb) and block row and column in that plane.
+struct BlockPos {
+    int64_t img;
+    int p, by, bx;
+};
+__device__ __forceinline__ BlockPos block_pos(const hic_dct_geometry& g, int64_t b) {
+    BlockPos q;
+    q.img = b / g.blocks_per_image;
+    int64_t local = b - q.img * g.blocks_per_image;
+    int nbx = g.nbx_l;
+    q.p = 0;
+    if (local >= g.nb_l) {
+        local -= g.nb_l;
+        q.p = 1;
+        if (local >= g.nb_c) {
+            local -= g.nb_c;
+            q.p = 2;
+        }
+        nbx = g.nbx_c;
+    }
+    q.by = (int)(local / nbx);
+    q.bx = (int)(local % nbx);
+    return q;
 }
 
 // A CTA takes K7_THREADS consecutive blocks of the coefficient buffer: ONE TMA tensor load (the buffer as
@@ -940,28 +996,7 @@ inverse_kernel(const __grid_constant__ CUtensorMap tmap_blocks, hic_dct_geometry
                uint8_t* __restrict__ crp, uint8_t* __restrict__ cbp, hic_tie_record* __restrict__ ties,
                uint32_t tie_capacity, uint32_t* __restrict__ stats) {
     __shared__ K7Smem s;
-    const uint32_t bar = (uint32_t)__cvta_generic_to_shared(&s.bar);
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)sizeof(s.blk)) : "memory");
-        asm volatile(
-            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-            ::"r"((uint32_t)__cvta_generic_to_shared(s.blk)), "l"(reinterpret_cast<uint64_t>(&tmap_blocks)), "r"(0),
-            "r"((int)(blockIdx.x * K7_THREADS)), "r"(bar)
-            : "memory");
-    }
-    __syncthreads();
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], 0;\n"
-        "@P1 bra DONE;\n"
-        "bra LAB_WAIT;\n"
-        "DONE:\n"
-        "}\n" ::"r"(bar)
-        : "memory");
+    load_block_box(tmap_blocks, K7_THREADS, s.blk, sizeof(s.blk), &s.bar);
     const int64_t total = (int64_t)n * g.blocks_per_image;
     const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (gid >= total) return;
@@ -1076,9 +1111,36 @@ inverse_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8
     });
 }
 
-// K8: cv2.pyrUp of both chroma planes + crop + YCrCb -> RGB.  One thread per chroma sample,
-// producing the 2x2 output quad.  pyrUp per axis: even = s[i-1] + 6 s[i] + s[i+1],
-// odd = 4 (s[i] + s[i+1]); s[-1] = s[1], s[n] = s[n-1]; (v + 32) >> 6 after both axes.
+// K8's pyrUp neighbours of sample i on an axis of n samples: i - 1 and i + 1, with s[-1] = s[1] and s[n] = s[n-1]
+__device__ __forceinline__ void pyr_neighbours(int i, int n, int& prev, int& next) {
+    prev = i > 0 ? i - 1 : (n > 1 ? 1 : 0);
+    next = i + 1 < n ? i + 1 : n - 1;
+}
+
+// K8's pyrUp of one chroma sample's 2x2 output quad [2 dy + dx] from its 3x3 neighbourhood: r0, r1, r2 the rows
+// ym, cy, yn, each at columns xm, cx, xn (pyr_neighbours).  Per axis even = s[i-1] + 6 s[i] + s[i+1], odd =
+// 4 (s[i] + s[i+1]); (v + 32) >> 6 after both axes.
+__device__ __forceinline__ void pyr_up_quad(const int* r0, const int* r1, const int* r2, int* up) {
+    const int e0 = r0[0] + 6 * r0[1] + r0[2], o0 = 4 * (r0[1] + r0[2]);
+    const int e1 = r1[0] + 6 * r1[1] + r1[2], o1 = 4 * (r1[1] + r1[2]);
+    const int e2 = r2[0] + 6 * r2[1] + r2[2], o2 = 4 * (r2[1] + r2[2]);
+    up[0] = (e0 + 6 * e1 + e2 + 32) >> 6;
+    up[1] = (o0 + 6 * o1 + o2 + 32) >> 6;
+    up[2] = (4 * (e1 + e2) + 32) >> 6;
+    up[3] = (4 * (o1 + o2) + 32) >> 6;
+}
+
+// K8's ycrcb_to_rgb of one pixel, written to o[0..2]
+__device__ __forceinline__ void store_rgb(uint8_t* o, int y, int cr, int cb) {
+    int r, gg, b;
+    ycrcb_to_rgb(y, cr, cb, r, gg, b);
+    o[0] = (uint8_t)r;
+    o[1] = (uint8_t)gg;
+    o[2] = (uint8_t)b;
+}
+
+// K8: cv2.pyrUp of both chroma planes + crop + YCrCb -> RGB.  One thread per chroma sample, producing the 2x2 output
+// quad through pyr_up_quad.
 __global__ void __launch_bounds__(256)
 upsample_colour_kernel(const uint8_t* __restrict__ yp, const uint8_t* __restrict__ crp,
                        const uint8_t* __restrict__ cbp, hic_dct_geometry g, int n, uint8_t* __restrict__ rgb) {
@@ -1088,8 +1150,9 @@ upsample_colour_kernel(const uint8_t* __restrict__ yp, const uint8_t* __restrict
     const int64_t img = gid / per;
     const int64_t rem = gid - img * per;
     const int cy = (int)(rem / g.wc), cx = (int)(rem % g.wc);
-    const int ym = cy > 0 ? cy - 1 : (g.hc > 1 ? 1 : 0), yn = cy + 1 < g.hc ? cy + 1 : g.hc - 1;
-    const int xm = cx > 0 ? cx - 1 : (g.wc > 1 ? 1 : 0), xn = cx + 1 < g.wc ? cx + 1 : g.wc - 1;
+    int ym, yn, xm, xn;
+    pyr_neighbours(cy, g.hc, ym, yn);
+    pyr_neighbours(cx, g.wc, xm, xn);
     int up[2][4];      // [channel][2*dy + dx]
 #pragma unroll
     for (int ch = 0; ch < 2; ++ch) {
@@ -1097,14 +1160,7 @@ upsample_colour_kernel(const uint8_t* __restrict__ yp, const uint8_t* __restrict
         const int r0[3] = {p[(size_t)ym * g.wc + xm], p[(size_t)ym * g.wc + cx], p[(size_t)ym * g.wc + xn]};
         const int r1[3] = {p[(size_t)cy * g.wc + xm], p[(size_t)cy * g.wc + cx], p[(size_t)cy * g.wc + xn]};
         const int r2[3] = {p[(size_t)yn * g.wc + xm], p[(size_t)yn * g.wc + cx], p[(size_t)yn * g.wc + xn]};
-        // horizontal pass on the three rows: even column, odd column
-        const int e0 = r0[0] + 6 * r0[1] + r0[2], o0 = 4 * (r0[1] + r0[2]);
-        const int e1 = r1[0] + 6 * r1[1] + r1[2], o1 = 4 * (r1[1] + r1[2]);
-        const int e2 = r2[0] + 6 * r2[1] + r2[2], o2 = 4 * (r2[1] + r2[2]);
-        up[ch][0] = (e0 + 6 * e1 + e2 + 32) >> 6;
-        up[ch][1] = (o0 + 6 * o1 + o2 + 32) >> 6;
-        up[ch][2] = (4 * (e1 + e2) + 32) >> 6;
-        up[ch][3] = (4 * (o1 + o2) + 32) >> 6;
+        pyr_up_quad(r0, r1, r2, up[ch]);
     }
     const uint8_t* ysrc = yp + (size_t)img * g.h * g.w;
     uint8_t* dst = rgb + (size_t)img * g.out_h * g.out_w * 3;
@@ -1134,7 +1190,8 @@ upsample_colour_vec_kernel(const uint8_t* __restrict__ yp, const uint8_t* __rest
     const int64_t img = gid / per;
     const int64_t rem = gid - img * per;
     const int cy = (int)(rem / groups), cx = 4 * (int)(rem % groups);
-    const int ym = cy > 0 ? cy - 1 : (g.hc > 1 ? 1 : 0), yn = cy + 1 < g.hc ? cy + 1 : g.hc - 1;
+    int ym, yn;
+    pyr_neighbours(cy, g.hc, ym, yn);
     int up[2][2][8];          // [channel][output row parity][output column]
 #pragma unroll
     for (int ch = 0; ch < 2; ++ch) {
@@ -1187,19 +1244,6 @@ upsample_colour_vec_kernel(const uint8_t* __restrict__ yp, const uint8_t* __rest
 // constant sample: trunc(q T00 / 256 + 128) mod 256 = ((q T00 + 32768) / 256, truncated toward zero) & 255.
 __device__ __forceinline__ int dc_block_sample(int q, int t00) { return ((q * t00 + 32768) / 256) & 255; }
 
-// K8's pyrUp of one chroma sample's 2x2 output quad [2 dy + dx] from its 3x3 neighbourhood: r0, r1, r2 the rows
-// ym, cy, yn, each at columns xm, cx, xn (s[-1] = s[1], s[n] = s[n-1] already applied by the caller).  Per axis even =
-// s[i-1] + 6 s[i] + s[i+1], odd = 4 (s[i] + s[i+1]); (v + 32) >> 6 after both axes.
-__device__ __forceinline__ void pyr_up_quad(const int* r0, const int* r1, const int* r2, int* up) {
-    const int e0 = r0[0] + 6 * r0[1] + r0[2], o0 = 4 * (r0[1] + r0[2]);
-    const int e1 = r1[0] + 6 * r1[1] + r1[2], o1 = 4 * (r1[1] + r1[2]);
-    const int e2 = r2[0] + 6 * r2[1] + r2[2], o2 = 4 * (r2[1] + r2[2]);
-    up[0] = (e0 + 6 * e1 + e2 + 32) >> 6;
-    up[1] = (o0 + 6 * o1 + o2 + 32) >> 6;
-    up[2] = (4 * (e1 + e2) + 32) >> 6;
-    up[3] = (4 * (o1 + o2) + 32) >> 6;
-}
-
 // Thumbnail: one pixel per 8x8 tile of the full decode's output (th = ceil(out_h / 8), tw = ceil(out_w / 8)),
 // from the DC values alone (one int16 per block, global block order).  The luminance block (ty, tx) gives Y; the
 // chroma planes of block samples (nby_c x nbx_c) go through K8's pyrUp taps on the fly, s[-1] = s[1] and s[n] =
@@ -1211,8 +1255,9 @@ __device__ __forceinline__ void thumbnail_pixel(const int16_t* __restrict__ bloc
     const int y = dc_block_sample(__ldg(blocks + (int64_t)ty * g.nbx_l + tx), t_l);
     const int cy = ty >> 1, cx = tx >> 1;
     const bool odd_y = ty & 1, odd_x = tx & 1;
-    const int ym = cy > 0 ? cy - 1 : (g.nby_c > 1 ? 1 : 0), yn = cy + 1 < g.nby_c ? cy + 1 : g.nby_c - 1;
-    const int xm = cx > 0 ? cx - 1 : (g.nbx_c > 1 ? 1 : 0), xn = cx + 1 < g.nbx_c ? cx + 1 : g.nbx_c - 1;
+    int ym, yn, xm, xn;
+    pyr_neighbours(cy, g.nby_c, ym, yn);
+    pyr_neighbours(cx, g.nbx_c, xm, xn);
     int up[2];
 #pragma unroll
     for (int ch = 0; ch < 2; ++ch) {
@@ -1223,11 +1268,7 @@ __device__ __forceinline__ void thumbnail_pixel(const int16_t* __restrict__ bloc
         const int v = odd_y ? 4 * (hor(cy) + hor(yn)) : hor(ym) + 6 * hor(cy) + hor(yn);
         up[ch] = (v + 32) >> 6;
     }
-    int r, gg, b;
-    ycrcb_to_rgb(y, up[0], up[1], r, gg, b);
-    o[0] = (uint8_t)r;
-    o[1] = (uint8_t)gg;
-    o[2] = (uint8_t)b;
+    store_rgb(o, y, up[0], up[1]);
 }
 
 __global__ void __launch_bounds__(256)
@@ -1254,200 +1295,49 @@ thumbnail_region_kernel(const int16_t* __restrict__ dc, hic_dct_geometry g, int 
     thumbnail_pixel(dc + img * g.blocks_per_image, g, top + (int)(rem / rw), left + (int)(rem % rw), rgb + gid * 3);
 }
 
-// ---- region decode: K7R, its fix-up, K8R (one rh x rw window per image, its origin per image) -----------------
-// Image i's window-local planes: Y at y + i * ly, 8 ny_l rows of 8 nx_l samples holding the luminance block
-// rectangle (region_first_l, region_span); Cr and Cb at cr / cb + i * lc, the chroma rectangle likewise.  (The scaled
-// region decode keeps M x M tiles of the rectangles' blocks there instead, block row by block row.)
-struct RegionArgs {
-    const int32_t* origin;      // n x (top, left), output coordinates (of the 1/scale image for the scaled decode)
-    uint8_t *y, *cr, *cb;
-    size_t ly, lc;
-    RegionSpan s;
-    int rh, rw;
-};
-struct RegionFirst {
-    int by_l, bx_l, by_c, bx_c;
-};
-template <int M = 8>
-__device__ __forceinline__ RegionFirst region_first(const hic_dct_geometry& g, const RegionArgs& a, int64_t img) {
-    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
-    return {region_first_l<M>(top, a.s.ny_l, g.nby_l), region_first_l<M>(left, a.s.nx_l, g.nbx_l),
-            region_first_c<M>(top, a.s.ny_c, g.nby_c), region_first_c<M>(left, a.s.nx_c, g.nbx_c)};
-}
-
-// Selected block `local` of image img (the nl luminance blocks of its rectangle row by row, then the nc of Cr, then
-// Cb): its plane p (0 = Y, 1 = Cr, 2 = Cb), its place (ly, lx) in the rectangle, and its global block index.
-template <int M = 8>
-__device__ __forceinline__ int64_t region_block(const hic_dct_geometry& g, const RegionArgs& a, int64_t img, int64_t local,
-                                                int64_t nl, int64_t nc, int& p, int& ly, int& lx) {
-    const RegionFirst f = region_first<M>(g, a, img);
-    int64_t block = img * g.blocks_per_image;
-    if (local < nl) {
-        ly = (int)(local / a.s.nx_l);
-        lx = (int)(local % a.s.nx_l);
-        block += (int64_t)(f.by_l + ly) * g.nbx_l + f.bx_l + lx;
-    } else {
-        local -= nl;
-        p = 1 + (int)(local / nc);
-        local -= (int64_t)(p - 1) * nc;
-        ly = (int)(local / a.s.nx_c);
-        lx = (int)(local % a.s.nx_c);
-        block += g.nb_l + (int64_t)(p - 1) * g.nb_c + (int64_t)(f.by_c + ly) * g.nbx_c + f.bx_c + lx;
-    }
-    return block;
-}
-
-// K7R: one selected block per thread through K7's inverse_block, into the window-local planes; ties are recorded
-// with the global block index, so exactly the blocks K7 flags are flagged.  The selected blocks are one run per
-// block row of each rectangle, so there is no box of consecutive blocks for one TMA load: the CTA's 128 blocks
-// come in by plain 16-byte loads, a warp reading four whole 128-byte blocks per instruction, into shared memory
-// with K7's 128-byte swizzle (piece j of block t at j ^ (t & 7)).
-constexpr int K7R_THREADS = 128;
-__global__ void __launch_bounds__(K7R_THREADS)
-region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, int n, RegionArgs a,
-                      hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
-    __shared__ int4 s_blk[K7R_THREADS * 8];
-    __shared__ uint32_t s_src[K7R_THREADS];
-    const int64_t nl = (int64_t)a.s.ny_l * a.s.nx_l, nc = (int64_t)a.s.ny_c * a.s.nx_c, per = nl + 2 * nc;
-    const int64_t first = (int64_t)blockIdx.x * K7R_THREADS, gid = first + threadIdx.x;
-    const bool live = gid < per * n;
-    int64_t img = 0;
-    int p = 0, ly = 0, lx = 0;
-    if (live) {
-        img = gid / per;
-        s_src[threadIdx.x] = (uint32_t)region_block(g, a, img, gid - img * per, nl, nc, p, ly, lx);
-    }
-    __syncthreads();
-    const int count = (int)min((int64_t)K7R_THREADS, per * n - first);
-    const int4* c4 = reinterpret_cast<const int4*>(coef);
-    for (int q = threadIdx.x; q < 8 * count; q += K7R_THREADS) {
-        const int t = q >> 3, j = q & 7;
-        s_blk[8 * t + (j ^ (t & 7))] = __ldg(c4 + (size_t)s_src[t] * 8 + j);
-    }
-    __syncthreads();
-    if (!live) return;
-    const int4* src = &s_blk[threadIdx.x * 8];
-    const int sw = threadIdx.x & 7;
-    if (p == 0)
-        inverse_block<0>(src, sw, a.y + img * a.ly, 8 * a.s.ny_l, 8 * a.s.nx_l, ly, lx, s_src[threadIdx.x], ties,
-                         tie_capacity, stats);
-    else
-        inverse_block<1>(src, sw, (p == 1 ? a.cr : a.cb) + img * a.lc, 8 * a.s.ny_c, 8 * a.s.nx_c, ly, lx,
-                         s_src[threadIdx.x], ties, tie_capacity, stats);
-}
-
-// The fix-up of K7R's flagged blocks: inverse_fixup_kernel's arithmetic, each block landing in its window.
-__global__ void __launch_bounds__(128)
-region_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, RegionArgs a,
-                    const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
-    inverse_fixup_body(coef, g, ties, tie_capacity, stats, [&](int64_t img, int p, int BY, int BX) {
-        const RegionFirst f = region_first(g, a, img);
-        if (p == 0) return BlockDst{a.y + img * a.ly, 8 * a.s.ny_l, 8 * a.s.nx_l, BY - f.by_l, BX - f.bx_l};
-        return BlockDst{(p == 1 ? a.cr : a.cb) + img * a.lc, 8 * a.s.ny_c, 8 * a.s.nx_c, BY - f.by_c, BX - f.bx_c};
-    });
-}
-
-// K8R: K8's pyrUp taps and ycrcb_to_rgb over one window per image: a thread per chroma sample the window covers,
-// producing the pixels of its 2x2 output quad that lie inside the window (cw = rw / 2 + 1 samples per row cover any
-// origin's columns, ch = rh / 2 + 1 its rows).  The neighbours are chosen in image coordinates (hc, wc of the whole
-// image: reflect at row / column 0, replicate at the last) and then read from the window-local planes; the
-// n x rh x rw x 3 result is written directly.
-__global__ void __launch_bounds__(256)
-region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restrict__ rgb) {
-    const int ch = a.rh / 2 + 1, cw = a.rw / 2 + 1;
-    const int64_t per = (int64_t)ch * cw;
-    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= per * n) return;
-    const int64_t img = gid / per;
-    const int64_t rem = gid - img * per;
-    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
-    const int cy = (top >> 1) + (int)(rem / cw), cx = (left >> 1) + (int)(rem % cw);
-    if (2 * cy > top + a.rh - 1 || 2 * cx > left + a.rw - 1) return;
-    const RegionFirst f = region_first(g, a, img);
-    const int ym = cy > 0 ? cy - 1 : (g.hc > 1 ? 1 : 0), yn = cy + 1 < g.hc ? cy + 1 : g.hc - 1;
-    const int xm = cx > 0 ? cx - 1 : (g.wc > 1 ? 1 : 0), xn = cx + 1 < g.wc ? cx + 1 : g.wc - 1;
-    const int r0 = 8 * f.by_c, c0 = 8 * f.bx_c, pw = 8 * a.s.nx_c;
-    int up[2][4];      // [channel][2*dy + dx], as K8
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-        const uint8_t* p = (c == 0 ? a.cr : a.cb) + img * a.lc;
-        auto row = [&](int r, int* v) {
-            const uint8_t* q = p + (size_t)(r - r0) * pw - c0;
-            v[0] = q[xm]; v[1] = q[cx]; v[2] = q[xn];
-        };
-        int s0[3], s1[3], s2[3];
-        row(ym, s0); row(cy, s1); row(yn, s2);
-        pyr_up_quad(s0, s1, s2, up[c]);
-    }
-    const uint8_t* ysrc = a.y + img * a.ly;
-    uint8_t* dst = rgb + (size_t)img * a.rh * a.rw * 3;
-#pragma unroll
-    for (int dy = 0; dy < 2; ++dy)
-#pragma unroll
-        for (int dx = 0; dx < 2; ++dx) {
-            const int oy = 2 * cy + dy, ox = 2 * cx + dx;
-            if (oy < top || oy >= top + a.rh || ox < left || ox >= left + a.rw) continue;
-            int r, gg, b;
-            ycrcb_to_rgb(ysrc[(size_t)(oy - 8 * f.by_l) * (8 * a.s.nx_l) + (ox - 8 * f.bx_l)], up[0][2 * dy + dx],
-                         up[1][2 * dy + dx], r, gg, b);
-            uint8_t* o = dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3;
-            o[0] = (uint8_t)r;
-            o[1] = (uint8_t)gg;
-            o[2] = (uint8_t)b;
-        }
-}
-
 // ---- scaled decode: K7S, its fix-up, K8S (1/s scale, M = 8 / s samples per block side) ----------------------
 // The work buffer holds one M x M tile of samples per block of the batch, in global block order: block b's samples
-// at work + b M^2, row major.  K8S reads the reduced planes through that layout.
-__device__ __forceinline__ int tile_sample(const uint8_t* plane, int nbx, int M, int r, int c) {
-    return plane[(((r / M) * nbx + c / M) * M + r % M) * M + c % M];
+// at work + b M^2, row major.  K8S reads the reduced planes through that layout (r, c >= 0).
+template <int M>
+__device__ __forceinline__ int tile_sample(const uint8_t* plane, int nbx, unsigned r, unsigned c) {
+    return plane[((r / M * nbx + c / M) * M + r % M) * M + c % M];
+}
+
+// The 16-byte pieces (8 scan entries each) of a block that the decode at M x M samples per block reads: all eight at
+// M = 8; entries 0..31 at M = 4 (its 4 x 4 corner ends at entry 24); entries 0..7 at M = 2 (the 2 x 2 corner ends at 4).
+template <int M>
+constexpr int block_pieces() { return M == 8 ? 8 : (M == 4 ? 4 : 1); }
+
+// Piece j of staged block t (16-byte units of a CTA's staging area): K7's 128-byte swizzle at M = 8 (j ^ (t & 7)),
+// the 64-byte swizzle at M = 4 (j ^ ((t >> 1) & 3): the eight blocks of a quarter warp hit eight different 16-byte
+// bank groups), none at M = 2.
+template <int M>
+__device__ __forceinline__ int staged_piece(int t, int j) {
+    return block_pieces<M>() * t + (M == 8 ? j ^ (t & 7) : (M == 4 ? j ^ ((t >> 1) & 3) : j));
 }
 
 // K7S: one block per thread.  The CTA's 128 blocks arrive by one TMA tensor load over K7's [block][64 int16] map of
-// the coefficient buffer, only the scan entries the block needs: M = 4 reads entries 0..31 (its 4 x 4 corner ends at
-// entry 24) as a box of {32, 128} in the 64-byte swizzle (piece j of block t at j ^ ((t >> 1) & 3): the eight blocks
-// of a quarter warp hit eight different 16-byte bank groups); M = 2 reads entries 0..7 (the 2 x 2 corner ends at 4)
-// as a box of {8, 128}.  The float32 path is scaled_transform<M> on q T / 256 (exact); a block with AC terms and a
-// sample within its band of an integer (where the uint8 truncation steps) is recorded for the float64 fix-up.
+// the coefficient buffer, only the pieces the block needs (block_pieces): a box of {32, 128} in the 64-byte swizzle
+// at M = 4, of {8, 128} at M = 2.  The float32 path is scaled_transform<M> on q T / 256 (exact); a block with AC
+// terms and a sample within its band of an integer (where the uint8 truncation steps) is recorded for the float64
+// fix-up.
 constexpr int K7S_THREADS = 128;
 template <int M>
 struct K7SSmem {
-    static constexpr int PIECES = M == 4 ? 4 : 1;      // 16-byte pieces (8 scan entries each) read per block
-    alignas(1024) int4 blk[K7S_THREADS * PIECES];
+    alignas(1024) int4 blk[K7S_THREADS * block_pieces<M>()];
     alignas(8) unsigned long long bar;
 };
-
-// piece j of staged block t (16-byte units of the CTA's staging area)
-template <int M>
-__device__ __forceinline__ int scaled_piece(int t, int j) {
-    return K7SSmem<M>::PIECES * t + (M == 4 ? j ^ ((t >> 1) & 3) : j);
-}
-
-__device__ __forceinline__ void record_tie(uint32_t block, hic_tie_record* __restrict__ ties, uint32_t tie_capacity,
-                                           uint32_t* __restrict__ stats) {
-    const uint32_t slot = atomicAdd(&stats[0], 1u);
-    if (slot < tie_capacity) {
-        hic_tie_record rec;
-        rec.block = block;
-        rec.reserved = 0;
-        rec.mask = ~0ull;
-        ties[slot] = rec;
-    } else {
-        atomicAdd(&stats[3], 1u);
-    }
-}
 
 // K7S's arithmetic on staged block t of kind 0 (luminance) / 1 (chroma): its M x M tile, four samples per word, into
 // packed; true when the block has AC terms and a sample within its error band of an integer.
 template <int M>
 __device__ __forceinline__ bool scaled_block(const int4* __restrict__ blk, int t, int kind, uint32_t (&packed)[M * M / 4]) {
-    constexpr int PIECES = K7SSmem<M>::PIECES;
+    constexpr int PIECES = block_pieces<M>();
     constexpr uint8_t zz[64] = HIC_ZIGZAG8;
     int words[4 * PIECES];                              // the block's first 8 PIECES scan entries, two per word
 #pragma unroll
     for (int j = 0; j < PIECES; ++j) {
-        const int4 wv = blk[scaled_piece<M>(t, j)];
+        const int4 wv = blk[staged_piece<M>(t, j)];
         words[4 * j] = wv.x; words[4 * j + 1] = wv.y; words[4 * j + 2] = wv.z; words[4 * j + 3] = wv.w;
     }
     float v[M * M];
@@ -1490,34 +1380,12 @@ __global__ void __launch_bounds__(K7S_THREADS)
 scaled_inverse_kernel(const __grid_constant__ CUtensorMap tmap_blocks, hic_dct_geometry g, int n, uint8_t* __restrict__ tiles,
                       hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
     __shared__ K7SSmem<M> s;
-    const uint32_t bar = (uint32_t)__cvta_generic_to_shared(&s.bar);
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)sizeof(s.blk)) : "memory");
-        asm volatile(
-            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-            ::"r"((uint32_t)__cvta_generic_to_shared(s.blk)), "l"(reinterpret_cast<uint64_t>(&tmap_blocks)), "r"(0),
-            "r"((int)(blockIdx.x * K7S_THREADS)), "r"(bar)
-            : "memory");
-    }
-    __syncthreads();
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], 0;\n"
-        "@P1 bra DONE;\n"
-        "bra LAB_WAIT;\n"
-        "DONE:\n"
-        "}\n" ::"r"(bar)
-        : "memory");
+    load_block_box(tmap_blocks, K7S_THREADS, s.blk, sizeof(s.blk), &s.bar);
     const int64_t total = (int64_t)n * g.blocks_per_image;
     const int64_t gid = (int64_t)blockIdx.x * K7S_THREADS + threadIdx.x;
     if (gid >= total) return;
-    const int kind = gid % g.blocks_per_image < g.nb_l ? 0 : 1;
     uint32_t packed[M * M / 4];
-    const bool flagged = scaled_block<M>(s.blk, threadIdx.x, kind, packed);
+    const bool flagged = scaled_block<M>(s.blk, threadIdx.x, block_pos(g, gid).p == 0 ? 0 : 1, packed);
     store_tile<M>(tiles + gid * M * M, packed);
     if (flagged) record_tie((uint32_t)gid, ties, tie_capacity, stats);
 }
@@ -1533,7 +1401,7 @@ __device__ __forceinline__ void scaled_fixup_body(const int16_t* __restrict__ co
     uint32_t changed = 0, done = 0;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_rec; i += gridDim.x * blockDim.x) {
         const uint32_t b = ties[i].block;
-        const int kind = b % g.blocks_per_image < g.nb_l ? 0 : 1;
+        const int kind = block_pos(g, b).p == 0 ? 0 : 1;
         const int16_t* blk = coef + (size_t)b * 64;
         int32_t cq[M * M];
 #pragma unroll
@@ -1571,12 +1439,21 @@ scaled_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, uint8_
     scaled_fixup_body<M>(coef, g, ties, tie_capacity, stats, [&](uint32_t b) { return tiles + (size_t)b * M * M; });
 }
 
-// K8S's pyrUp of reduced chroma sample (cy, cx) of planes of ny x nx samples: the 2x2 quads up[c] of Cr (c = 0) and Cb
-// (c = 1), from the 3x3 neighbourhood chosen with K8's borders in those planes and read through sample(c, row, col).
+// The chroma planes (rows, columns) whose borders K8's taps reflect and replicate at, M samples per block side: the
+// full decode's hc x wc at M = 8; the reduced planes' whole block grids, M nby_c x M nbx_c, below (the thumbnail's
+// convention).  The two differ wherever hc or wc is not a multiple of 8.
+template <int M>
+__device__ __forceinline__ int2 chroma_extent(const hic_dct_geometry& g) {
+    return M == 8 ? make_int2(g.hc, g.wc) : make_int2(M * g.nby_c, M * g.nbx_c);
+}
+
+// The pyrUp of chroma sample (cy, cx) of planes of ny x nx samples: the 2x2 quads up[c] of Cr (c = 0) and Cb (c = 1),
+// from the 3x3 neighbourhood chosen with K8's borders in those planes and read through sample(c, row, col).
 template <class Sample>
-__device__ __forceinline__ void scaled_up_quads(int cy, int cx, int ny, int nx, Sample sample, int (&up)[2][4]) {
-    const int ym = cy > 0 ? cy - 1 : (ny > 1 ? 1 : 0), yn = cy + 1 < ny ? cy + 1 : ny - 1;
-    const int xm = cx > 0 ? cx - 1 : (nx > 1 ? 1 : 0), xn = cx + 1 < nx ? cx + 1 : nx - 1;
+__device__ __forceinline__ void chroma_up_quads(int cy, int cx, int2 extent, Sample sample, int (&up)[2][4]) {
+    int ym, yn, xm, xn;
+    pyr_neighbours(cy, extent.x, ym, yn);
+    pyr_neighbours(cx, extent.y, xm, xn);
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
         auto row = [&](int r, int* v) {
@@ -1588,10 +1465,9 @@ __device__ __forceinline__ void scaled_up_quads(int cy, int cx, int ny, int nx, 
     }
 }
 
-// K8S: one sample of the reduced chroma planes (M nby_c x M nbx_c, their whole block grids: the thumbnail's
-// convention) per thread, as K8: its 3x3 neighbourhood through pyr_up_quad, Y from the reduced luminance plane
-// (M nby_l x M nbx_l), K8's ycrcb_to_rgb, and the pixels of its 2x2 output quad inside sh x sw = ceil(out_h / s) x
-// ceil(out_w / s) written to n x sh x sw x 3 directly.
+// K8S: one sample of the reduced chroma planes (chroma_extent) per thread, as K8: its 3x3 neighbourhood through
+// pyr_up_quad, Y from the reduced luminance plane (M nby_l x M nbx_l), K8's ycrcb_to_rgb, and the pixels of its 2x2
+// output quad inside sh x sw = ceil(out_h / s) x ceil(out_w / s) written to n x sh x sw x 3 directly.
 template <int M>
 __global__ void __launch_bounds__(256)
 scaled_colour_kernel(const uint8_t* __restrict__ tiles, hic_dct_geometry g, int n, int sh, int sw, uint8_t* __restrict__ rgb) {
@@ -1604,8 +1480,8 @@ scaled_colour_kernel(const uint8_t* __restrict__ tiles, hic_dct_geometry g, int 
     const int cy = (int)(rem / qw), cx = (int)(rem % qw);
     const uint8_t* base = tiles + (size_t)img * g.blocks_per_image * M * M;
     int up[2][4];
-    scaled_up_quads(cy, cx, M * g.nby_c, M * g.nbx_c, [&](int c, int r, int col) {
-        return tile_sample(base + (size_t)(g.nb_l + c * g.nb_c) * M * M, g.nbx_c, M, r, col);
+    chroma_up_quads(cy, cx, chroma_extent<M>(g), [&](int c, int r, int col) {
+        return tile_sample<M>(base + (size_t)(g.nb_l + c * g.nb_c) * M * M, g.nbx_c, r, col);
     }, up);
     uint8_t* dst = rgb + (size_t)img * sh * sw * 3;
 #pragma unroll
@@ -1614,38 +1490,94 @@ scaled_colour_kernel(const uint8_t* __restrict__ tiles, hic_dct_geometry g, int 
         for (int dx = 0; dx < 2; ++dx) {
             const int oy = 2 * cy + dy, ox = 2 * cx + dx;
             if (oy >= sh || ox >= sw) continue;
-            int r, gg, b;
-            ycrcb_to_rgb(tile_sample(base, g.nbx_l, M, oy, ox), up[0][2 * dy + dx], up[1][2 * dy + dx], r, gg, b);
-            uint8_t* o = dst + ((size_t)oy * sw + ox) * 3;
-            o[0] = (uint8_t)r;
-            o[1] = (uint8_t)gg;
-            o[2] = (uint8_t)b;
+            store_rgb(dst + ((size_t)oy * sw + ox) * 3, tile_sample<M>(base, g.nbx_l, oy, ox), up[0][2 * dy + dx],
+                      up[1][2 * dy + dx]);
         }
 }
 
-// ---- scaled region decode: K7SR, its fix-up, K8SR (one rh x rw window of the 1/s image per image) ---------------
-// The rectangles come from the region rules at M samples per block (region_first<M>, region_span<M>); image i's
-// window-local tiles: Y at y + i * ly, the M x M tiles of the luminance rectangle's blocks, row by row (nx_l per row);
-// Cr and Cb at cr / cb + i * lc likewise (nx_c per row).
+// ---- region decode: K7R, its fix-up, K8R (one rh x rw window per image, its origin per image) ------------------
+// One template per stage for M = 8 / s samples per block side: M = 8 is the window of the decoded image, M = 4 and 2
+// the window of its 1/2- and 1/4-scale image.  The rectangles come from the region rules at M (region_first<M>,
+// region_span<M>).  Image i's window-local tiles: Y at y + i * ly, the M x M tiles of the luminance rectangle's blocks,
+// block row by block row (nx_l per row); Cr and Cb at cr / cb + i * lc likewise (nx_c per row).
+struct RegionArgs {
+    const int32_t* origin;      // n x (top, left), output coordinates (of the 1/scale image for the scaled decode)
+    uint8_t *y, *cr, *cb;
+    size_t ly, lc;
+    RegionSpan s;
+    int rh, rw;
+};
+struct RegionFirst {
+    int by_l, bx_l, by_c, bx_c;
+};
+template <int M>
+__device__ __forceinline__ RegionFirst region_first(const hic_dct_geometry& g, const RegionArgs& a, int64_t img) {
+    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
+    return {region_first_l<M>(top, a.s.ny_l, g.nby_l), region_first_l<M>(left, a.s.nx_l, g.nbx_l),
+            region_first_c<M>(top, a.s.ny_c, g.nby_c), region_first_c<M>(left, a.s.nx_c, g.nbx_c)};
+}
+
+// Selected block `local` of image img (the nl luminance blocks of its rectangle row by row, then the nc of Cr, then
+// Cb): its plane p (0 = Y, 1 = Cr, 2 = Cb), its place (ly, lx) in the rectangle, and its global block index.
+template <int M>
+__device__ __forceinline__ int64_t region_block(const hic_dct_geometry& g, const RegionArgs& a, int64_t img, int64_t local,
+                                                int64_t nl, int64_t nc, int& p, int& ly, int& lx) {
+    const RegionFirst f = region_first<M>(g, a, img);
+    int64_t block = img * g.blocks_per_image;
+    if (local < nl) {
+        ly = (int)(local / a.s.nx_l);
+        lx = (int)(local % a.s.nx_l);
+        block += (int64_t)(f.by_l + ly) * g.nbx_l + f.bx_l + lx;
+    } else {
+        local -= nl;
+        p = 1 + (int)(local / nc);
+        local -= (int64_t)(p - 1) * nc;
+        ly = (int)(local / a.s.nx_c);
+        lx = (int)(local % a.s.nx_c);
+        block += g.nb_l + (int64_t)(p - 1) * g.nb_c + (int64_t)(f.by_c + ly) * g.nbx_c + f.bx_c + lx;
+    }
+    return block;
+}
+
 template <int M>
 __device__ __forceinline__ uint8_t* region_tile(const RegionArgs& a, int64_t img, int p, int ly, int lx) {
     if (p == 0) return a.y + img * a.ly + ((size_t)ly * a.s.nx_l + lx) * M * M;
     return (p == 1 ? a.cr : a.cb) + img * a.lc + ((size_t)ly * a.s.nx_c + lx) * M * M;
 }
 
-// K7SR: one selected block per thread through K7S's arithmetic (scaled_block) into its window-local tile; ties are
-// recorded with the global block index, so exactly the blocks K7S flags are flagged.  The selected blocks are one run
-// per block row of each rectangle, so there is no box of consecutive blocks for one TMA load: the CTA's blocks come in
-// by plain 16-byte loads of their first PIECES pieces only (64 bytes at M = 4, 16 at M = 2), consecutive threads on
-// consecutive pieces, into K7S's staging layout.
+// Staged block t of plane p through K7's arithmetic (M = 8) or K7S's into its tile; a flagged block is recorded with
+// its global block index `block`.
+template <int M>
+__device__ __forceinline__ void region_tile_block(const int4* __restrict__ blk, int t, int p, uint8_t* __restrict__ tile,
+                                                  uint32_t block, hic_tie_record* __restrict__ ties, uint32_t tie_capacity,
+                                                  uint32_t* __restrict__ stats) {
+    if constexpr (M == 8) {
+        if (p == 0)
+            inverse_block<0>(blk + 8 * t, t & 7, tile, 8, 8, 0, 0, block, ties, tie_capacity, stats);
+        else
+            inverse_block<1>(blk + 8 * t, t & 7, tile, 8, 8, 0, 0, block, ties, tie_capacity, stats);
+    } else {
+        uint32_t packed[M * M / 4];
+        const bool flagged = scaled_block<M>(blk, t, p == 0 ? 0 : 1, packed);
+        store_tile<M>(tile, packed);
+        if (flagged) record_tie(block, ties, tie_capacity, stats);
+    }
+}
+
+// K7R: one selected block per thread into its window-local tile (region_tile_block); ties are recorded with the global
+// block index, so exactly the blocks K7 (K7S) flags are flagged.  The selected blocks are one run per block row of
+// each rectangle, so there is no box of consecutive blocks for one TMA load: the CTA's blocks come in by plain 16-byte
+// loads of the pieces the arithmetic reads (block_pieces: 128 bytes at M = 8, 64 at M = 4, 16 at M = 2), consecutive
+// threads on consecutive pieces, into K7's (K7S's) staging layout.
 template <int M>
 __global__ void __launch_bounds__(K7S_THREADS)
-scaled_region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, int n, RegionArgs a,
-                             hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
-    constexpr int PIECES = K7SSmem<M>::PIECES;
+region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, int n, RegionArgs a,
+                      hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    constexpr int PIECES = block_pieces<M>();
     __shared__ int4 s_blk[K7S_THREADS * PIECES];
     __shared__ uint32_t s_src[K7S_THREADS];
-    // 32-bit indices: the selected blocks are at most the batch's blocks, fewer than 2^32 (hic_dct_scaled_region)
+    // 32-bit indices: the selected blocks are at most the batch's blocks, fewer than 2^32 (hic_dct_region and
+    // hic_dct_scaled_region check it)
     const uint32_t nl = (uint32_t)a.s.ny_l * a.s.nx_l, nc = (uint32_t)a.s.ny_c * a.s.nx_c, per = nl + 2 * nc;
     const uint32_t first = blockIdx.x * K7S_THREADS, gid = first + threadIdx.x, total = per * (uint32_t)n;
     const bool live = gid < total;
@@ -1660,40 +1592,38 @@ scaled_region_inverse_kernel(const int16_t* __restrict__ coef, hic_dct_geometry 
     const int4* c4 = reinterpret_cast<const int4*>(coef);
     for (int q = threadIdx.x; q < PIECES * count; q += K7S_THREADS) {
         const int t = q / PIECES, j = q % PIECES;
-        s_blk[scaled_piece<M>(t, j)] = __ldg(c4 + (size_t)s_src[t] * 8 + j);
+        s_blk[staged_piece<M>(t, j)] = __ldg(c4 + (size_t)s_src[t] * 8 + j);
     }
     __syncthreads();
     if (!live) return;
-    uint32_t packed[M * M / 4];
-    const bool flagged = scaled_block<M>(s_blk, threadIdx.x, p == 0 ? 0 : 1, packed);
-    store_tile<M>(region_tile<M>(a, img, p, ly, lx), packed);
-    if (flagged) record_tie(s_src[threadIdx.x], ties, tie_capacity, stats);
+    region_tile_block<M>(s_blk, threadIdx.x, p, region_tile<M>(a, img, p, ly, lx), s_src[threadIdx.x], ties, tie_capacity, stats);
 }
 
-// The fix-up of K7SR's flagged blocks: scaled_fixup_kernel's arithmetic, each block landing in its window's tile.
+// The fix-up of K7R's flagged blocks: inverse_fixup_kernel's arithmetic at M = 8, scaled_fixup_kernel's below, each
+// block landing in its window-local tile.
 template <int M>
 __global__ void __launch_bounds__(128)
-scaled_region_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, RegionArgs a,
-                           const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
-    scaled_fixup_body<M>(coef, g, ties, tie_capacity, stats, [&](uint32_t b) {
-        const int64_t img = b / g.blocks_per_image;
-        int64_t local = b - img * g.blocks_per_image;
-        const RegionFirst f = region_first<M>(g, a, img);
-        if (local < g.nb_l) return region_tile<M>(a, img, 0, (int)(local / g.nbx_l) - f.by_l, (int)(local % g.nbx_l) - f.bx_l);
-        local -= g.nb_l;
-        const int p = (int)(local / g.nb_c);
-        local -= (int64_t)p * g.nb_c;
-        return region_tile<M>(a, img, 1 + p, (int)(local / g.nbx_c) - f.by_c, (int)(local % g.nbx_c) - f.bx_c);
-    });
+region_fixup_kernel(const int16_t* __restrict__ coef, hic_dct_geometry g, RegionArgs a,
+                    const hic_tie_record* __restrict__ ties, uint32_t tie_capacity, uint32_t* __restrict__ stats) {
+    auto tile = [&](const BlockPos& q) {
+        const RegionFirst f = region_first<M>(g, a, q.img);
+        if (q.p == 0) return region_tile<M>(a, q.img, 0, q.by - f.by_l, q.bx - f.bx_l);
+        return region_tile<M>(a, q.img, q.p, q.by - f.by_c, q.bx - f.bx_c);
+    };
+    if constexpr (M == 8)
+        inverse_fixup_body(coef, g, ties, tie_capacity, stats,
+                           [&](int64_t img, int p, int by, int bx) { return BlockDst{tile({img, p, by, bx}), 8, 8, 0, 0}; });
+    else
+        scaled_fixup_body<M>(coef, g, ties, tie_capacity, stats, [&](uint32_t b) { return tile(block_pos(g, b)); });
 }
 
-// K8SR: K8S's taps over one window per image: a thread per reduced chroma sample the window covers (rh / 2 + 1 rows of
-// rw / 2 + 1, as K8R), producing the pixels of its 2x2 quad inside the window.  The neighbours are chosen in the whole
-// reduced chroma planes (M nby_c x M nbx_c, K8S's borders) and read from the window-local tiles; Y likewise; the
-// n x rh x rw x 3 result is written directly.
+// K8R: the colour stage over one window per image: a thread per chroma sample the window covers, producing the pixels
+// of its 2x2 output quad that lie inside the window (cw = rw / 2 + 1 samples per row cover any origin's columns,
+// ch = rh / 2 + 1 its rows).  The neighbours are chosen in the whole chroma planes with K8's borders (chroma_extent)
+// and read from the window-local tiles; Y likewise; the n x rh x rw x 3 result is written directly.
 template <int M>
 __global__ void __launch_bounds__(256)
-scaled_region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restrict__ rgb) {
+region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __restrict__ rgb) {
     const int ch = a.rh / 2 + 1, cw = a.rw / 2 + 1;
     const int64_t per = (int64_t)ch * cw;
     const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1708,8 +1638,8 @@ scaled_region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __
     const uint8_t* crp = a.cr + img * a.lc;
     const uint8_t* cbp = a.cb + img * a.lc;
     int up[2][4];
-    scaled_up_quads(cy, cx, M * g.nby_c, M * g.nbx_c, [&](int c, int r, int col) {
-        return tile_sample(c == 0 ? crp : cbp, a.s.nx_c, M, r - r0, col - c0);
+    chroma_up_quads(cy, cx, chroma_extent<M>(g), [&](int c, int r, int col) {
+        return tile_sample<M>(c == 0 ? crp : cbp, a.s.nx_c, r - r0, col - c0);
     }, up);
     const uint8_t* ysrc = a.y + img * a.ly;
     uint8_t* dst = rgb + (size_t)img * a.rh * a.rw * 3;
@@ -1719,13 +1649,8 @@ scaled_region_colour_kernel(hic_dct_geometry g, int n, RegionArgs a, uint8_t* __
         for (int dx = 0; dx < 2; ++dx) {
             const int oy = 2 * cy + dy, ox = 2 * cx + dx;
             if (oy < top || oy >= top + a.rh || ox < left || ox >= left + a.rw) continue;
-            int r, gg, b;
-            ycrcb_to_rgb(tile_sample(ysrc, a.s.nx_l, M, oy - M * f.by_l, ox - M * f.bx_l), up[0][2 * dy + dx],
-                         up[1][2 * dy + dx], r, gg, b);
-            uint8_t* o = dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3;
-            o[0] = (uint8_t)r;
-            o[1] = (uint8_t)gg;
-            o[2] = (uint8_t)b;
+            store_rgb(dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3,
+                      tile_sample<M>(ysrc, a.s.nx_l, oy - M * f.by_l, ox - M * f.bx_l), up[0][2 * dy + dx], up[1][2 * dy + dx]);
         }
 }
 }  // namespace k7
@@ -1884,39 +1809,29 @@ static int region_sizes(int n, const hic_dct_geometry& g, int scale, int rh, int
     return HIC_OK;
 }
 
-// hic_dct_region's (M = 8) and hic_dct_scaled_region's (M = 4, 2) set-up once the origins are checked: *a is the
-// kernels' view of the work buffer, with the origins copied to its head, and *blocks the number of selected blocks
+// K7R, its fix-up and K8R of hic_dct_region (M = 8) and hic_dct_scaled_region (M = 4, 2) once the origins are
+// checked; the origins are copied to the work buffer's head, the window-local tiles follow.  The launches keep the
+// labels of the entry they serve: region_* at M = 8, scaled_region_* below.
 template <int M>
-static int region_prepare(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
-                          uint8_t* d_work, size_t work_bytes, uint32_t* d_stats, cudaStream_t st, k7::RegionArgs* a,
-                          int64_t* blocks) {
+static int region_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
+                         uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity,
+                         uint32_t* d_stats, uint8_t* d_rgb_out, cudaStream_t st) {
+    constexpr bool full = M == 8;
     const RegionLayout L = region_layout<M>(n, g, rh, rw);
     HIC_REQUIRE(work_bytes >= L.total, "work buffer of %zu bytes is too small: %zu needed (%s)", work_bytes, L.total,
-                M == 8 ? "hic_dct_region_sizes" : "hic_dct_scaled_region_sizes");
+                full ? "hic_dct_region_sizes" : "hic_dct_scaled_region_sizes");
     HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
                 "d_coef and d_work must be 16-byte aligned");
     const int rc = ensure_tables();
     if (rc) return rc;
     HIC_CUDA(cudaMemsetAsync(d_stats, 0, HIC_TIE_STATS * sizeof(uint32_t), st));
     HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    uint8_t* y = d_work + L.head;     // the n Y planes, then the n Cr and the n Cb planes
-    *a = {reinterpret_cast<const int32_t*>(d_work), y, y + (size_t)n * L.ly, y + (size_t)n * (L.ly + L.lc), L.ly, L.lc, L.s, rh, rw};
-    *blocks = (int64_t)L.blocks;
-    return HIC_OK;
-}
-
-// K7SR, its fix-up and K8SR of hic_dct_scaled_region for M x M samples per block (scale 8 / M)
-template <int M>
-static int scaled_region_launch(const int16_t* d_coef, const hic_dct_geometry& g, int n, const int32_t* h_origin, int rh, int rw,
-                                uint8_t* d_work, size_t work_bytes, hic_tie_record* d_ties, uint32_t tie_capacity,
-                                uint32_t* d_stats, uint8_t* d_rgb_out, cudaStream_t st) {
-    k7::RegionArgs a;
-    int64_t blocks = 0;
-    const int rc = region_prepare<M>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_stats, st, &a, &blocks);
-    if (rc) return rc;
-    HIC_LAUNCH("scaled_region_inverse_kernel", st, k7::scaled_region_inverse_kernel<M><<<grid_for(blocks, k7::K7S_THREADS), k7::K7S_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
-    HIC_LAUNCH("scaled_region_fixup_kernel", st, k7::scaled_region_fixup_kernel<M><<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
-    HIC_LAUNCH("scaled_region_colour_kernel", st, k7::scaled_region_colour_kernel<M><<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
+    uint8_t* y = d_work + L.head;     // the n images' Y tiles, then their Cr and their Cb tiles
+    const k7::RegionArgs a = {reinterpret_cast<const int32_t*>(d_work), y, y + (size_t)n * L.ly, y + (size_t)n * (L.ly + L.lc),
+                              L.ly, L.lc, L.s, rh, rw};
+    HIC_LAUNCH(full ? "region_inverse_kernel" : "scaled_region_inverse_kernel", st, k7::region_inverse_kernel<M><<<grid_for((int64_t)L.blocks, k7::K7S_THREADS), k7::K7S_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH(full ? "region_fixup_kernel" : "scaled_region_fixup_kernel", st, k7::region_fixup_kernel<M><<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
+    HIC_LAUNCH(full ? "region_colour_kernel" : "scaled_region_colour_kernel", st, k7::region_colour_kernel<M><<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
     return HIC_OK;
 }
 
@@ -2138,15 +2053,8 @@ int hic_dct_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w, const
     if (rc) return rc;
     rc = check_origins(g, n, h_origin, rh, rw, 1);
     if (rc) return rc;
-    cudaStream_t st = as_stream(stream);
-    k7::RegionArgs a;
-    int64_t blocks = 0;
-    rc = region_prepare<8>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_stats, st, &a, &blocks);
-    if (rc) return rc;
-    HIC_LAUNCH("region_inverse_kernel", st, k7::region_inverse_kernel<<<grid_for(blocks, k7::K7R_THREADS), k7::K7R_THREADS, 0, st>>>(d_coef, g, n, a, d_ties, tie_capacity, d_stats));
-    HIC_LAUNCH("region_fixup_kernel", st, k7::region_fixup_kernel<<<148 * 4, 128, 0, st>>>(d_coef, g, a, d_ties, tie_capacity, d_stats));
-    HIC_LAUNCH("region_colour_kernel", st, k7::region_colour_kernel<<<grid_for((int64_t)n * (rh / 2 + 1) * (rw / 2 + 1), 256), 256, 0, st>>>(g, n, a, d_rgb_out));
-    return HIC_OK;
+    return region_launch<8>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity, d_stats, d_rgb_out,
+                            as_stream(stream));
 }
 
 int hic_dct_scaled_shape(int32_t h, int32_t w, int32_t scale, int32_t* sh, int32_t* sw) {
@@ -2240,8 +2148,8 @@ int hic_dct_scaled_region(const int16_t* d_coef, int32_t n, int32_t h, int32_t w
     if (rc) return rc;
     cudaStream_t st = as_stream(stream);
     return by_samples<false>(scale, [&](auto m) {
-        return scaled_region_launch<decltype(m)::value>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity,
-                                                        d_stats, d_rgb_out, st);
+        return region_launch<decltype(m)::value>(d_coef, g, n, h_origin, rh, rw, d_work, work_bytes, d_ties, tie_capacity,
+                                                 d_stats, d_rgb_out, st);
     });
 }
 

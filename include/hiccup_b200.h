@@ -160,7 +160,7 @@ int hic_dct_thumbnail(const int16_t* d_dc, int32_t n, int32_t h, int32_t w, uint
  * borders at the image's edges (reflect at the top and left, replicate at the bottom and right), the real
  * neighbouring samples everywhere else.  Only the blocks covering those samples are inverse-transformed
  * (K7's float32 path, its error band and float64 fix-up; tie records carry the global block index) into
- * window-local planes in d_work, and only the window's pixels are upsampled and converted (K8's integer
+ * window-local 8x8 tiles in d_work, and only the window's pixels are upsampled and converted (K8's integer
  * arithmetic) straight into d_rgb_out (n * rh * rw * 3).
  * hic_dct_region_blocks (host only) gives the block rectangles a window at (top, left) selects:
  * rect = {by, bx, nby, nbx} of the luminance plane, then the same of each chroma plane; every window of one

@@ -108,6 +108,8 @@ SIGNATURES = {
     "hic_wavelet_inverse_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, ctypes.POINTER(WaveletParams), c_void_p, c_void_p, c_void_p]),
     "hic_wavelet_scaled_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, ctypes.POINTER(WaveletParams), c_int32, c_void_p,
                                            c_void_p, c_void_p]),
+    "hic_wavelet_region": (c_int, [c_void_p, c_int32, c_int32, c_int32, ctypes.POINTER(WaveletParams), c_int32, c_void_p, c_int32,
+                                   c_int32, c_void_p, c_size_t, c_void_p, c_void_p]),
     "hic_wavelet_flat_to_bands_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "hic_wavelet_bands_to_flat_general": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "hic_layout_dct": (c_int, [c_int32, c_int32, c_int32, ctypes.POINTER(StreamLayout)]),
@@ -255,7 +257,22 @@ def region_origins(h, w, origins, size, scale=1):
     g = geometry(h, w)
     scale = region_scale_arg(scale)
     ih, iw = (g.out_h, g.out_w) if scale == 1 else (-(-g.out_h // scale), -(-g.out_w // scale))
-    what = "decoded image" if scale == 1 else "1/%d-scale image" % scale
+    return _window_origins(ih, iw, "decoded image" if scale == 1 else "1/%d-scale image" % scale, origins, size)
+
+
+def wavelet_region_origins(h, w, levels, origins, size, scale=1):
+    """region_origins() for a wavelet file of `levels` levels and h x w (multiples of 2^levels): windows of the
+    full-resolution image (scale 1) or of the (h / scale) x (w / scale) image, scale = 2^k with 1 <= k <= levels."""
+    levels = int(levels)
+    k = wavelet_scale_arg(scale, levels, lowest=0)
+    if h % (1 << levels) or w % (1 << levels):
+        raise ValueError("a region decode of %d levels needs sides that are multiples of %d (got %dx%d)" % (levels, 1 << levels, h, w))
+    return _window_origins(h >> k, w >> k, "image" if k == 0 else "1/%d-scale image" % (1 << k), origins, size)
+
+
+def _window_origins(ih, iw, what, origins, size):
+    """The origins ((n, 2) of (top, left)) of windows of size = (rh, rw) inside an ih x iw image (`what`, for the
+    message) as a contiguous (n, 2) int32 array, or ValueError."""
     rh, rw = (int(v) for v in size)
     o = np.asarray(origins)
     if o.ndim != 2 or o.shape[1] != 2 or o.shape[0] < 1 or not np.issubdtype(o.dtype, np.integer):
@@ -473,12 +490,13 @@ def wavelet_pyramid(h, w, levels):
     return g
 
 
-def wavelet_scale_arg(scale, levels):
-    """k for a wavelet scaled decode's scale = 2^k of a file of `levels` levels (1 <= k <= levels), else ValueError."""
+def wavelet_scale_arg(scale, levels, lowest=1):
+    """k for a wavelet scaled decode's scale = 2^k of a file of `levels` levels (lowest <= k <= levels; a region decode
+    takes lowest = 0, the full-resolution image), else ValueError."""
     levels = int(levels)
-    if isinstance(scale, bool) or not isinstance(scale, (int, np.integer)) or int(scale) < 2 or int(scale) & (int(scale) - 1) \
-            or int(scale) > 1 << levels:
-        raise ValueError("scale must be 2^k with 1 <= k <= %d, the file's levels (got %r)" % (levels, scale))
+    if isinstance(scale, bool) or not isinstance(scale, (int, np.integer)) or int(scale) < 1 << lowest \
+            or int(scale) & (int(scale) - 1) or int(scale) > 1 << levels:
+        raise ValueError("scale must be 2^k with %d <= k <= %d, the file's levels (got %r)" % (lowest, levels, scale))
     return int(scale).bit_length() - 1
 
 

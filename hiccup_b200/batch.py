@@ -311,6 +311,41 @@ class _BatchCodec:
         self._after_scaled()
         return pixels
 
+    # ---- windows: one height x width window per image of the full-resolution or 1/scale image (codec.jpeg_region or
+    # codec.wavelet_region for the whole batch); the subclasses provide _region_buffers(origins, size, scale),
+    # _region(origins, r) and _after_regions(r) --------------------------------------------------------------------------
+    def decode_regions_device(self, origins, size, scale=1):
+        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over; in DCT mode DC-only at scale 8,
+        as thumbnails_device), then the windows of size = (height, width) at origins ((n, 2) of (top, left), in the
+        coordinates of the 1/scale image); they stay on the device (fetch_regions)."""
+        origins, r, dc_only = self._region_buffers(origins, size, scale)
+        self._run_reduced(r, functools.partial(self._region, origins), dc_only=dc_only)
+
+    def decode_regions(self, enc, origins, size, out=None, scale=1):
+        """Windows of an EncodedStreams, host to host: image i's window is decode(enc)[i, top:top+height,
+        left:left+width] with (top, left) = origins[i] and (height, width) = size, bit for bit -- or the same window of
+        decode_scaled(enc, scale)[i] (DCT mode: scale 2 or 4; wavelet mode: 2^k, 1 <= k <= levels), in DCT mode at
+        scale 8 of thumbnails(enc)[i] (only the DC streams go up).  out: optional preallocated uint8 array of
+        (n, height, width, 3)."""
+        origins, r, dc_only = self._region_buffers(origins, size, scale)
+        self._run_reduced(r, functools.partial(self._region, origins), enc, dc_only=dc_only)
+        return self.fetch_regions(out)
+
+    def fetch_regions(self, out=None):
+        """Download the windows of the last decode_regions() / decode_regions_device() (and, in DCT mode, their tie
+        statistics into region_stats; all zero at scale 8, which has no tie stage)."""
+        r = self._reduced["region"]
+        pixels = self._fetch_reduced(r, out)
+        self._after_regions(r)
+        return pixels
+
+    def _after_regions(self, r):
+        pass
+
+    def _check_origin_count(self, origins):
+        if origins.shape[0] != self.n:
+            raise ValueError("%d origins for a batch of %d images" % (origins.shape[0], self.n))
+
     def close(self):
         for r in self._reduced.values():
             r.free()
@@ -409,18 +444,17 @@ class DctBatchCodec(_BatchCodec):
     # ---- regions: one height x width window per image, of the full-resolution image (codec.jpeg_region for the whole
     # batch) or of the 1/2-, 1/4- or 1/8-scale image (jpeg_region(..., scale)) ----------------------------------------
     def _region_buffers(self, origins, size, scale):
-        """Check the scale and the windows (ValueError before any device work); returns the origins as (n, 2) int32 and
-        the buffers for their size and scale."""
+        """Check the scale and the windows (ValueError before any device work); returns the origins as (n, 2) int32, the
+        buffers for their size and scale, and whether the decode is DC-only (scale 8, as thumbnails)."""
         scale = _lib.region_scale_arg(scale)
         origins = _lib.region_origins(self.h, self.w, origins, size, scale)
-        if origins.shape[0] != self.n:
-            raise ValueError("%d origins for a batch of %d images" % (origins.shape[0], self.n))
+        self._check_origin_count(origins)
         rh, rw = int(size[0]), int(size[1])
         if scale == 1:
             sizes = lambda: _lib.region_sizes(self.n, self.h, self.w, rh, rw)
         else:
             sizes = lambda: _lib.scaled_region_sizes(self.n, self.h, self.w, scale, rh, rw)
-        return origins, self._reduced_buffers("region", (rh, rw, scale), lambda: ((self.n, rh, rw, 3),) + sizes())
+        return origins, self._reduced_buffers("region", (rh, rw, scale), lambda: ((self.n, rh, rw, 3),) + sizes()), scale == 8
 
     def _region(self, origins, r):
         """The region kernels of r's scale on the decoded coefficients -- at scale 8 on the DC values, which the DC-only
@@ -438,32 +472,12 @@ class DctBatchCodec(_BatchCodec):
                                                       rh, rw, r.d_work.ptr, r.work_bytes, self.d_ties.ptr, r.tie_capacity,
                                                       self.d_stats.ptr, r.d_out.ptr, self.stream))
 
-    def decode_regions_device(self, origins, size, scale=1):
-        """D1-D3 from the encoder's own device-resident output (decode_device's hand-over; DC-only at scale 8, as
-        thumbnails_device), then the windows of size = (height, width) at origins ((n, 2) of (top, left), in the
-        coordinates of the 1/scale image); they stay on the device (fetch_regions)."""
-        origins, r = self._region_buffers(origins, size, scale)
-        self._run_reduced(r, functools.partial(self._region, origins), dc_only=r.key[2] == 8)
-
-    def decode_regions(self, enc, origins, size, out=None, scale=1):
-        """Windows of an EncodedStreams, host to host: image i's window is decode(enc)[i, top:top+height,
-        left:left+width] with (top, left) = origins[i] and (height, width) = size, bit for bit -- or at scale 2 or 4 the
-        same window of decode_scaled(enc, scale)[i], at scale 8 of thumbnails(enc)[i] (only the DC streams go up).
-        out: optional preallocated uint8 array of (n, height, width, 3)."""
-        origins, r = self._region_buffers(origins, size, scale)
-        self._run_reduced(r, functools.partial(self._region, origins), enc, dc_only=r.key[2] == 8)
-        return self.fetch_regions(out)
-
-    def fetch_regions(self, out=None):
-        """Download the windows of the last decode_regions() / decode_regions_device() (and their tie statistics
-        into region_stats; all zero at scale 8, which has no tie stage)."""
-        r = self._reduced["region"]
-        pixels = self._fetch_reduced(r, out)
+    def _after_regions(self, r):
+        """The tie statistics of the windows into region_stats: all zero at scale 8, which has no tie stage."""
         if r.key[2] == 8:
             self.region_stats = np.zeros(_lib.TIE_STATS, np.uint32)
         else:
             self.region_stats = self.d_stats.download(np.uint32, _lib.TIE_STATS, self.stream)
-        return pixels
 
     # ---- 1/2- and 1/4-scale images (codec.jpeg_scaled for the whole batch) ----------------------------------------
     def scaled_shape(self, scale):
@@ -582,6 +596,20 @@ class WaveletBatchCodec(_BatchCodec):
     def _scaled(self, r):
         _lib.check(self.lib.hic_wavelet_scaled_general(self.d_coef_dec.ptr, self.n, self.h, self.w, self._params_ref, r.key,
                                                        self.d_work.ptr, r.d_out.ptr, self.stream))
+
+    # ---- windows of the full-resolution or 1/2- to 1/2^levels-scale image (codec.wavelet_region for the whole batch) ---
+    def _region_buffers(self, origins, size, scale):
+        """Check the scale and the windows (ValueError before any device work); returns the origins as (n, 2) int32, the
+        buffers for their size and scale (the work area holds the origins alone) and False: the decode is never DC-only."""
+        origins = _lib.wavelet_region_origins(self.h, self.w, self.params.levels, origins, size, scale)
+        self._check_origin_count(origins)
+        rh, rw = int(size[0]), int(size[1])
+        return origins, self._reduced_buffers("region", (rh, rw, int(scale)), lambda: ((self.n, rh, rw, 3), origins.nbytes, 0)), False
+
+    def _region(self, origins, r):
+        rh, rw, scale = r.key
+        _lib.check(self.lib.hic_wavelet_region(self.d_coef_dec.ptr, self.n, self.h, self.w, self._params_ref, scale,
+                                               origins.ctypes.data, rh, rw, r.d_work.ptr, r.work_bytes, r.d_out.ptr, self.stream))
 
     def hic_images(self, enc, images=None):
         from hiccup_b200 import wavelet

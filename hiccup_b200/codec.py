@@ -391,3 +391,8 @@ def wavelet_decode(hic: hicimage.HicImage) -> model.CompressedImage:
 def wavelet_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
     from hiccup_b200 import wavelet
     return wavelet.wavelet_scaled(hic, scale)
+
+
+def wavelet_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int, scale: int = 1) -> np.ndarray:
+    from hiccup_b200 import wavelet
+    return wavelet.wavelet_region(hic, top, left, height, width, scale)

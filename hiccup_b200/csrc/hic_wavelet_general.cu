@@ -195,6 +195,21 @@ __device__ __forceinline__ void ihaar_pair(double a, double d, double& even, dou
     odd = dadd(ca, -cd);
 }
 
+// one reconstruction step at the position whose zigzag index in the level's bands is `pos`: the approximation
+// sample v_aa and the three detail coefficients there, times `mul` (quantization.py:72-77) -> the 2 x 2 children
+// q[row][col] of the next finer level
+__device__ __forceinline__ void inverse_quad(double v_aa, const int16_t* __restrict__ src, const Pyr& g, int band0, int64_t pos,
+                                             double mul, double (&q)[2][2]) {
+    const double v_da = dmul((double)src[g.p.band_off[band0] + pos], mul);
+    const double v_ad = dmul((double)src[g.p.band_off[band0 + 1] + pos], mul);
+    const double v_dd = dmul((double)src[g.p.band_off[band0 + 2] + pos], mul);
+    double a_e, a_o, d_e, d_o;                                                    // idwtn undoes the LAST axis first
+    ihaar_pair(v_aa, v_ad, a_e, a_o);
+    ihaar_pair(v_da, v_dd, d_e, d_o);
+    ihaar_pair(a_e, d_e, q[0][0], q[1][0]);
+    ihaar_pair(a_o, d_o, q[0][1], q[1][1]);
+}
+
 // one reconstruction level: aa (ho x wo) + the level's detail bands times `mul` -> out (H x W), H = 2 ho or
 // 2 ho - 1: pywt.waverec2 trims the extra row / column when the next detail band is one smaller
 __global__ void __launch_bounds__(256)
@@ -209,21 +224,25 @@ inverse_level_kernel(const double* __restrict__ aa, int ho, int wo, int64_t in_s
     const int16_t* src = flat + cs * g.chan_elems;
     const int64_t pos = zigzag_pos(k, j, ho, wo);
     const double v_aa = aa[cs * in_stride + e];
-    const double v_da = dmul((double)src[g.p.band_off[band0] + pos], mul);          // quantization.py:72-77
-    const double v_ad = dmul((double)src[g.p.band_off[band0 + 1] + pos], mul);
-    const double v_dd = dmul((double)src[g.p.band_off[band0 + 2] + pos], mul);
-    double a_e, a_o, d_e, d_o;                                                    // idwtn undoes the LAST axis first
-    ihaar_pair(v_aa, v_ad, a_e, a_o);
-    ihaar_pair(v_da, v_dd, d_e, d_o);
+    double q[2][2];
+    inverse_quad(v_aa, src, g, band0, pos, mul, q);
     double* o = out + cs * ((int64_t)H * W);
     const bool row1 = 2 * k + 1 < H, col1 = 2 * j + 1 < W;
-    double t0, t1;
-    ihaar_pair(a_e, d_e, t0, t1);
-    o[(int64_t)(2 * k) * W + 2 * j] = t0;
-    if (row1) o[(int64_t)(2 * k + 1) * W + 2 * j] = t1;
-    ihaar_pair(a_o, d_o, t0, t1);
-    if (col1) o[(int64_t)(2 * k) * W + 2 * j + 1] = t0;
-    if (row1 && col1) o[(int64_t)(2 * k + 1) * W + 2 * j + 1] = t1;
+    o[(int64_t)(2 * k) * W + 2 * j] = q[0][0];
+    if (row1) o[(int64_t)(2 * k + 1) * W + 2 * j] = q[1][0];
+    if (col1) o[(int64_t)(2 * k) * W + 2 * j + 1] = q[0][1];
+    if (row1 && col1) o[(int64_t)(2 * k + 1) * W + 2 * j + 1] = q[1][1];
+}
+
+// one channel sample: + 2^8, astype(uint8): truncate, wrap (compression.py:95)
+__device__ __forceinline__ int finish_sample(double v) { return wrap_u8(dadd(v, 256.0)); }
+
+__device__ __forceinline__ void store_pixel(int y, int cr, int cb, uint8_t* __restrict__ o) {
+    int r, gg, b;
+    ycrcb_to_rgb(y, cr, cb, r, gg, b);
+    o[0] = (uint8_t)r;
+    o[1] = (uint8_t)gg;
+    o[2] = (uint8_t)b;
 }
 
 __global__ void __launch_bounds__(256)
@@ -232,12 +251,7 @@ finish_kernel(const double* __restrict__ plane, int64_t pixels, int64_t total, u
     if (gid >= total) return;
     const int64_t img = gid / pixels, p = gid - img * pixels;
     const double* s = plane + img * 3 * pixels + p;
-    int r, gg, b;                                                 // + 2^8, astype(uint8): truncate, wrap (compression.py:95)
-    ycrcb_to_rgb(wrap_u8(dadd(s[0], 256.0)), wrap_u8(dadd(s[pixels], 256.0)), wrap_u8(dadd(s[2 * pixels], 256.0)), r, gg, b);
-    uint8_t* o = rgb + gid * 3;
-    o[0] = (uint8_t)r;
-    o[1] = (uint8_t)gg;
-    o[2] = (uint8_t)b;
+    store_pixel(finish_sample(s[0]), finish_sample(s[pixels]), finish_sample(s[2 * pixels]), rgb + gid * 3);
 }
 
 // finish_kernel for the 1/s-scale image: the running approximation A_k (s = 2^k) times 2^-k (exact) is the mean of
@@ -248,13 +262,73 @@ scaled_finish_kernel(const double* __restrict__ plane, int64_t pixels, int64_t t
     if (gid >= total) return;
     const int64_t img = gid / pixels, p = gid - img * pixels;
     const double* s = plane + img * 3 * pixels + p;
-    int r, gg, b;
-    ycrcb_to_rgb(wrap_u8(dadd(dmul(s[0], inv_scale), 256.0)), wrap_u8(dadd(dmul(s[pixels], inv_scale), 256.0)),
-                 wrap_u8(dadd(dmul(s[2 * pixels], inv_scale), 256.0)), r, gg, b);
-    uint8_t* o = rgb + gid * 3;
-    o[0] = (uint8_t)r;
-    o[1] = (uint8_t)gg;
-    o[2] = (uint8_t)b;
+    store_pixel(finish_sample(dmul(s[0], inv_scale)), finish_sample(dmul(s[pixels], inv_scale)),
+                finish_sample(dmul(s[2 * pixels], inv_scale)), rgb + gid * 3);
+}
+
+// ---- region: one rh x rw window of the 1/s-scale image (s = 2^k, 0 <= k <= L) per image ----
+// db1 has no halo: a level-(l-1) sample at (y, x) reads only the level-l approximation at (y >> 1, x >> 1) and the
+// three detail coefficients there.  So a window needs, at each level l > k, only the dyadic parent rectangle of its
+// rows [top >> (l-k), (top+rh-1) >> (l-k)] (columns alike), and every sample on that path is the very float64 value
+// the full inverse computes at that position.
+struct RegionArgs {
+    const int32_t* origin;         // (top, left) per image, in the coordinates of the 1/s image
+    int n, rh, rw;
+    double mul[HIC_WAVELET_MAX_LEVELS];   // detail group i's dequantisation factor (0 = coarsest)
+    double inv_scale;              // 2^-k
+};
+
+// D = L - k levels to reconstruct.  D = 0: one thread per window pixel, straight from cA_L.  D >= 1: one thread per
+// level-(k+1) sample of the window's parent rectangle (a 2 x 2 output quad), all three channels (ycrcb_to_rgb needs
+// them together); per channel it starts from cA_L, keeps only the child on its own path through levels L .. k+2, and
+// finishes with inverse_level_kernel's quad.  No float64 planes, no intermediate traffic.
+template <int D>
+__global__ void __launch_bounds__(256)
+region_kernel(const int16_t* __restrict__ flat, Pyr g, RegionArgs a, uint8_t* __restrict__ rgb) {
+    constexpr int Q = D == 0 ? 1 : 2;                  // output pixels per thread along each axis
+    const int L = g.p.levels, k = L - D;
+    const int ph = D == 0 ? a.rh : a.rh / 2 + 1, pw = D == 0 ? a.rw : a.rw / 2 + 1;
+    const int64_t per = (int64_t)ph * pw;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= per * a.n) return;
+    const int64_t img = gid / per;
+    const int rem = (int)(gid - img * per);
+    const int top = __ldg(a.origin + 2 * img), left = __ldg(a.origin + 2 * img + 1);
+    // this thread's position at level k + (D > 0): the window pixel itself, or the parent of a quad
+    const int py = (D == 0 ? top : top >> 1) + rem / pw, px = (D == 0 ? left : left >> 1) + rem % pw;
+    if (Q * py > top + a.rh - 1 || Q * px > left + a.rw - 1) return;
+    int u[3][Q][Q];                                   // finished samples, by channel
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const int16_t* src = flat + (3 * img + c) * g.chan_elems;
+        double s = (double)src[g.p.band_off[0] + zigzag_pos(py >> (D > 0 ? D - 1 : 0), px >> (D > 0 ? D - 1 : 0), g.p.lh[L], g.p.lw[L])];
+        if constexpr (D == 0) {
+            u[c][0][0] = finish_sample(dmul(s, a.inv_scale));
+        } else {
+            double q[2][2];
+#pragma unroll
+            for (int i = 0; i < D - 1; ++i) {          // level L - i -> L - i - 1, keeping the child on this path
+                const int sh = D - 1 - i, l = L - i;
+                inverse_quad(s, src, g, 1 + 3 * i, zigzag_pos(py >> sh, px >> sh, g.p.lh[l], g.p.lw[l]), a.mul[i], q);
+                const bool ry = (py >> (sh - 1)) & 1, rx = (px >> (sh - 1)) & 1;     // selects, not a local-memory index
+                s = ry ? (rx ? q[1][1] : q[1][0]) : (rx ? q[0][1] : q[0][0]);
+            }
+            inverse_quad(s, src, g, 1 + 3 * (D - 1), zigzag_pos(py, px, g.p.lh[k + 1], g.p.lw[k + 1]), a.mul[D - 1], q);
+#pragma unroll
+            for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+                for (int dx = 0; dx < 2; ++dx) u[c][dy][dx] = finish_sample(dmul(q[dy][dx], a.inv_scale));
+        }
+    }
+    uint8_t* dst = rgb + (size_t)img * a.rh * a.rw * 3;
+#pragma unroll
+    for (int dy = 0; dy < Q; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < Q; ++dx) {
+            const int oy = Q * py + dy, ox = Q * px + dx;
+            if (oy < top || oy >= top + a.rh || ox < left || ox >= left + a.rw) continue;
+            store_pixel(u[0][dy][dx], u[1][dy][dx], u[2][dy][dx], dst + ((size_t)(oy - top) * a.rw + (ox - left)) * 3);
+        }
 }
 
 // ---- layout converters: flat zigzag stream <-> 3 L + 1 raster int32 sub-bands ----
@@ -425,6 +499,52 @@ int hic_wavelet_scaled_general(const int16_t* d_flat, int32_t n, int32_t h, int3
     // plane[cur] holds A_k, channel-planar; its (image, channel) stride is lh[k] * lw[k] = (h / scale) (w / scale)
     HIC_LAUNCH("wavelet_scaled_finish_kernel", st, wvg::scaled_finish_kernel<<<wvg::blocks_for(pixels * n), 256, 0, st>>>(
         plane[cur], pixels, pixels * n, 1.0 / scale, d_rgb_out));
+    return HIC_OK;
+}
+
+int hic_wavelet_region(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, const hic_wavelet_params* params, int32_t scale,
+                       const int32_t* h_origin, int32_t rh, int32_t rw, void* d_work, size_t work_bytes, uint8_t* d_rgb_out,
+                       void* stream) {
+    using namespace hic;
+    HIC_REQUIRE(d_flat && h_origin && d_work && d_rgb_out, "NULL pointer");
+    HIC_REQUIRE(n >= 1 && n <= 65535, "batch size must be in 1..65535 (got %d)", n);
+    int rc = wvg::check_params(params);
+    if (rc) return rc;
+    const int L = params->levels;
+    int k = 0;
+    while (k < L && (1 << k) < scale) ++k;
+    HIC_REQUIRE(scale == (1 << k), "scale must be 2^k with 0 <= k <= %d levels (got %d)", L, scale);
+    HIC_REQUIRE(h % (1 << L) == 0 && w % (1 << L) == 0, "a region decode of %d levels needs multiples of %d (got %dx%d)", L,
+                1 << L, h, w);
+    wvg::Pyr g;
+    rc = wvg::make(h, w, L, &g);
+    if (rc) return rc;
+    HIC_REQUIRE(rh >= 1 && rw >= 1, "empty region %dx%d", rh, rw);
+    const int ih = h >> k, iw = w >> k;
+    for (int i = 0; i < n; ++i) {
+        const int64_t top = h_origin[2 * i], left = h_origin[2 * i + 1];
+        HIC_REQUIRE(top >= 0 && left >= 0 && top + rh <= ih && left + rw <= iw,
+                    "region %dx%d at (%lld, %lld) is not inside the %dx%d 1/%d-scale image", rh, rw, (long long)top,
+                    (long long)left, ih, iw, scale);
+    }
+    const size_t need = (size_t)n * 2 * sizeof(int32_t);
+    HIC_REQUIRE(work_bytes >= need, "work buffer of %zu bytes is too small: %zu needed for the origins", work_bytes, need);
+    HIC_REQUIRE((reinterpret_cast<uintptr_t>(d_work) & 3) == 0, "d_work must be 4-byte aligned");
+    cudaStream_t st = as_stream(stream);
+    HIC_CUDA(cudaMemcpyAsync(d_work, h_origin, need, cudaMemcpyHostToDevice, st));
+    wvg::RegionArgs a = {reinterpret_cast<const int32_t*>(d_work), n, rh, rw, {}, 1.0 / scale};
+    for (int i = 0; i < L; ++i) a.mul[i] = params->multiplier * (double)(i * i + 1);
+    const int D = L - k;
+    const int64_t threads = (int64_t)n * (D == 0 ? (int64_t)rh * rw : (int64_t)(rh / 2 + 1) * (rw / 2 + 1));
+    HIC_REQUIRE(threads <= 256ll * INT32_MAX, "batch too large: %lld threads", (long long)threads);
+    const unsigned blocks = wvg::blocks_for(threads);
+    switch (D) {                     // one instantiation per number of levels to reconstruct, so the walk unrolls
+#define HIC_WAVELET_REGION(d) \
+        case d: HIC_LAUNCH("wavelet_region_kernel", st, wvg::region_kernel<d><<<blocks, 256, 0, st>>>(d_flat, g, a, d_rgb_out)); break;
+        HIC_WAVELET_REGION(0) HIC_WAVELET_REGION(1) HIC_WAVELET_REGION(2) HIC_WAVELET_REGION(3) HIC_WAVELET_REGION(4)
+        HIC_WAVELET_REGION(5)
+#undef HIC_WAVELET_REGION
+    }
     return HIC_OK;
 }
 

@@ -3,6 +3,7 @@
     wavelet_compression(rgb)      compression.py:59-85      wavelet_encode(c)    codec.py:116-163
     wavelet_decompression(c)      compression.py:88-100     wavelet_decode(hic)  codec.py:199-239
     wavelet_scaled(hic, scale)    no reference counterpart: the 1/2- to 1/2^L-scale image (include/hiccup_b200.h)
+    wavelet_region(hic, top, left, height, width, scale)    no reference counterpart: one window of the full or 1/scale image
 
 The numeric work runs in csrc/hic_wavelet.cu (K9 / K10, the fused kernels for the default settings),
 csrc/hic_wavelet_general.cu (any WAVELET_NUM_LEVELS in 1..5, multiplier, threshold and quality factor:
@@ -295,7 +296,8 @@ def wavelet_decompression(channels: model.CompressedImage) -> np.ndarray:
         if levels == 3 and settings.WAVELET_SUBBAND_QUANTIZATION_MULTIPLIER == 1 and h % 8 == 0 and w % 8 == 0:
             _lib.check(lib.hic_wavelet_inverse(flat.ptr, 1, h, w, rgb.ptr, None))
         else:
-            _run_general(lib.hic_wavelet_inverse_general, flat, h, w, levels, (), rgb)
+            _run_general(levels, _lib.wavelet_work_bytes(1, h, w),
+                         lambda params, work: lib.hic_wavelet_inverse_general(flat.ptr, 1, h, w, params, work, rgb.ptr, None))
         out = rgb.download(np.uint8, h * w * 3).reshape(h, w, 3)
     finally:
         flat.free()
@@ -303,15 +305,15 @@ def wavelet_decompression(channels: model.CompressedImage) -> np.ndarray:
     return out
 
 
-def _run_general(entry, flat, h, w, levels, extra, rgb):
-    """hic_wavelet_inverse_general or hic_wavelet_scaled_general (extra = (scale,)) on one image, with a work area of its
-    own, at `levels` and the multiplier of the settings now."""
+def _run_general(levels, work_bytes, launch):
+    """launch(params, work) -- a general entry on one image -- with a work area of work_bytes of its own, at `levels`
+    and the multiplier of the settings now."""
     params = _lib.WaveletParams()
     params.levels, params.multiplier = levels, float(settings.WAVELET_SUBBAND_QUANTIZATION_MULTIPLIER)
     params.threshold, params.threshold_index = 0.0, -1
-    work = _lib.scratch(_lib.wavelet_work_bytes(1, h, w))
+    work = _lib.scratch(work_bytes)
     try:
-        _lib.check(entry(flat.ptr, 1, h, w, ctypes.byref(params), *extra, work.ptr, rgb.ptr, None))
+        _lib.check(launch(ctypes.byref(params), work.ptr))
         _lib.sync()
     finally:
         work.free()
@@ -334,13 +336,44 @@ def wavelet_scaled(hic: hicimage.HicImage, scale: int) -> np.ndarray:
     h, w, levels = int(g.h), int(g.w), _levels_of(g)
     _lib.wavelet_scale_arg(scale, levels)
     scale = int(scale)
+    lib = _lib.load()
+    return _reduced_decode(hic, levels, (h // scale, w // scale, 3), _lib.wavelet_work_bytes(1, h, w),
+                           lambda flat, params, work, rgb: lib.hic_wavelet_scaled_general(flat, 1, h, w, params, scale, work, rgb, None))
+
+
+def wavelet_region(hic: hicimage.HicImage, top: int, left: int, height: int, width: int, scale: int = 1) -> np.ndarray:
+    """One window of a wavelet-mode file of L levels: (height, width, 3) uint8.  At scale 1 it equals
+    wavelet_decompression(wavelet_decode(hic))[top:top+height, left:left+width] bit for bit; at scale = 2^k,
+    1 <= k <= L, the same window of wavelet_scaled(hic, scale), (top, left) in the coordinates of that image.  The
+    entropy decode is wavelet_decode's (restart records used when the file has them); then only the window's dyadic
+    parent rectangles of the sub-bands are read and inverse-transformed, with the full inverse's operations, straight
+    into the window's pixels (include/hiccup_b200.h, hic_wavelet_region, at the file's levels and the multiplier of the
+    settings now).  NotImplementedError for a DCT-mode file, ValueError for a bad scale, a window outside the 1/scale
+    image or a pyramid pyramid_of_file refuses, all before any device work."""
+    from hiccup_b200 import codec
+    if codec._is_dct(hic):
+        raise NotImplementedError("wavelet region decode works on wavelet-mode (HIC) files; this is a DCT-mode (JPEG) file")
+    settings.check_wavelet_supported()
+    g = pyramid_of_file(hic)
+    h, w, levels = int(g.h), int(g.w), _levels_of(g)
+    origin = _lib.wavelet_region_origins(h, w, levels, [(top, left)], (height, width), scale)
+    scale, height, width = int(scale), int(height), int(width)
+    lib = _lib.load()
+    return _reduced_decode(hic, levels, (height, width, 3), origin.nbytes,
+                           lambda flat, params, work, rgb: lib.hic_wavelet_region(flat, 1, h, w, params, scale, origin.ctypes.data,
+                                                                                  height, width, work, origin.nbytes, rgb, None))
+
+
+def _reduced_decode(hic, levels, shape, work_bytes, launch):
+    """wavelet_decode's entropy stage into the flat stream on the device, then launch(flat, params, work, out) of a
+    general entry into a uint8 image of `shape`, which is returned."""
     _lib.require_device()
-    sh, sw = h // scale, w // scale
+    size = int(np.prod(shape))
     flat, _ = decode_to_device_flat(hic)
-    rgb = _lib.scratch(sh * sw * 3)
+    rgb = _lib.scratch(size)
     try:
-        _run_general(_lib.load().hic_wavelet_scaled_general, flat, h, w, levels, (scale,), rgb)
-        return rgb.download(np.uint8, sh * sw * 3).reshape(sh, sw, 3)
+        _run_general(levels, work_bytes, lambda params, work: launch(flat.ptr, params, work, rgb.ptr))
+        return rgb.download(np.uint8, size).reshape(shape)
     finally:
         flat.free()
         rgb.free()

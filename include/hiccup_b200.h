@@ -302,6 +302,22 @@ int hic_wavelet_inverse_general(const int16_t* d_flat, int32_t n, int32_t h, int
  * K10-style kernel measured slower on a B200 (DESIGN.md section 6). */
 int hic_wavelet_scaled_general(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, const hic_wavelet_params* params,
                                int32_t scale, void* d_work, uint8_t* d_rgb_out, void* stream);
+/* Region -- one rh x rw window of the full-resolution (s = 1) or 1/s-scale image per image of the batch,
+ * s = 2^k with 0 <= k <= L = params->levels, h and w multiples of 2^L: window i equals
+ * hic_wavelet_inverse_general's image (s = 1; K10's at the defaults) or hic_wavelet_scaled_general's (s >= 2)
+ * cropped to [top, top+rh) x [left, left+rw) bit for bit, (top, left) = h_origin[2i], h_origin[2i+1] in the
+ * coordinates of that (h / s) x (w / s) image; valid when top, left >= 0, rh, rw >= 1, top + rh <= h / s and
+ * left + rw <= w / s.  The arithmetic is at params->levels and params->multiplier; the thresholds are not used.
+ * db1 has no halo, so at each level l > k only the window's dyadic parent rectangle, rows
+ * [top >> (l - k), (top + rh - 1) >> (l - k)] and the same for columns, of cA_L and of the detail bands is read,
+ * and each sample on that path is computed with the full inverse's operations in its order, straight into
+ * d_rgb_out (n * rh * rw * 3): no float64 planes.  d_work (4-byte aligned) needs 8 n bytes, for the origins,
+ * which are copied there with cudaMemcpyAsync on `stream`.  Returns HIC_ERR_INVALID for a scale other than 2^k,
+ * 0 <= k <= L, sides that are not multiples of 2^L, an empty size, a window outside (h / s) x (w / s) or
+ * work_bytes < 8 n, all checked on the host before anything is launched. */
+int hic_wavelet_region(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, const hic_wavelet_params* params,
+                       int32_t scale, const int32_t* h_origin, int32_t rh, int32_t rw, void* d_work, size_t work_bytes,
+                       uint8_t* d_rgb_out, void* stream);
 int hic_wavelet_flat_to_bands_general(const int16_t* d_flat, int32_t n, int32_t h, int32_t w, int32_t levels, int32_t* d_bands,
                                       void* stream);
 int hic_wavelet_bands_to_flat_general(const int32_t* d_bands, int32_t n, int32_t h, int32_t w, int32_t levels, int16_t* d_flat,
